@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- `inquiSTR call` hot path on B200: STR loci genotyped / s and CIGAR ops / s.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 3] [--scale S]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 3] [--scale S] [--dump-outputs DIR]
 
 A step = one pass of the hot path (join -> CIGAR scan -> pair sums -> medians) over the whole
 workload. `value` is measured with the reads already resident in HBM (CUDA events on the library's
@@ -46,7 +46,35 @@ def parse_args():
     ap.add_argument("--no-cohort", action="store_true", help="skip the extra.cohort_outlier block (SURVEY 8f rank 3 kernels)")
     ap.add_argument("--parity-seconds", type=float, default=6.0, help="budget of the per-rank oracle check at N > 1")
     ap.add_argument("--no-e2e", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the medians of the last timed step as DIR/phase1.npy and DIR/phase2.npy (float64, 0 where no "
+                         "call) and their valid_mask (include/inqcall.h) as DIR/valid_mask.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours (the reference arm times a sample of the loci sized by the clock)")
+    return args
+
+
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: str, phase1: np.ndarray, phase2: np.ndarray) -> None:
+    """phase1 / phase2 as the caller of Context.genotype receives them, one value per catalog locus, written as finite
+    arrays: the medians with 0 where there is no call (NaN in phase1 / phase2) and valid_mask, bit 0 = H1 called,
+    bit 1 = H2 called. A catalog too large for DUMP_MAX_BYTES is cut to a fixed seeded sample of loci, whose catalog
+    indices go to locus_index.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    n = len(phase1)
+    ok1, ok2 = ~np.isnan(phase1), ~np.isnan(phase2)
+    arrays = {"phase1": np.where(ok1, phase1, 0.0), "phase2": np.where(ok2, phase2, 0.0), "valid_mask": ok1 + 2.0 * ok2}
+    if len(arrays) * 8 * n > DUMP_MAX_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(n, DUMP_MAX_BYTES // ((len(arrays) + 1) * 8), replace=False))
+        arrays = {name: a[keep] for name, a in arrays.items()}
+        arrays["locus_index"] = keep.astype(np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
 
 
 def dist_env():
@@ -353,6 +381,8 @@ def main():
     dev_per_rank = gather_ranks(dev_ms / args.steps)
     st = cst.as_dict()
     res = q.GenotypeResult(out[0], out[1], out[2], st)
+    # phase1 / phase2 are fresh arrays: the e2e and diagnostic passes below overwrite `out`
+    last_step = (res.phase1, res.phase2) if args.dump_outputs else None
 
     # ---- timed: end to end from pinned host buffers through the C ABI
     e2e = None
@@ -483,6 +513,13 @@ def main():
             cohort_block = cohort_outlier_block(peak)
         except Exception as ex:
             cohort_block = {"error": repr(ex)}
+    if args.dump_outputs:
+        if world > 1:
+            parts = [None] * world
+            dist.all_gather_object(parts, last_step)          # the ranks' catalog shards are contiguous, in rank order
+            last_step = tuple(np.concatenate([p[k] for p in parts]) for k in (0, 1))
+        if rank == 0:
+            dump_outputs(args.dump_outputs, *last_step)
     if world > 1:
         dist.barrier()
 

@@ -103,9 +103,11 @@ def reads_to_bam(path, ref_names, ref_lens, reads, rng=None, sa_for_flags=True, 
     write_bam(path, ref_names, ref_lens, recs)
 
 
-def index_bam(path: str) -> str:
+def index_bam(path: str, meta: bool = False) -> str:
     """Pure-Python BAI builder (SAM spec 5.2) for coordinate-sorted BAMs written by this module or by
-    synth.write_bam: bins with merged chunks, 16 kb linear index. Returns the .bai path."""
+    synth.write_bam: bins with merged chunks, 16 kb linear index. meta=True adds what htslib writes on
+    top: the metadata pseudo-bin 37450 of every populated reference (its first and last virtual offset,
+    mapped / unmapped counts) and the n_no_coor trailer. Returns the .bai path."""
     data = open(path, "rb").read()
     # pass 1: BGZF blocks -> (compressed offset, inflated bytes)
     blocks, off = [], 0
@@ -142,6 +144,8 @@ def index_bam(path: str) -> str:
         l_name = struct.unpack_from("<I", stream, p)[0]; p += 4 + l_name + 4
     bins = [dict() for _ in range(n_ref)]
     linear = [dict() for _ in range(n_ref)]
+    span = [None] * n_ref            # [first v0, last v1, mapped, unmapped] per reference
+    n_no_coor = 0
     while p + 4 <= len(stream):
         bs = struct.unpack_from("<I", stream, p)[0]
         tid, pos, l_name, mapq, _bin, n_cig, flag, l_seq = struct.unpack_from("<iiBBHHHI", stream, p + 4)
@@ -162,19 +166,29 @@ def index_bam(path: str) -> str:
             for w in range(pos >> 14, ((end - 1) >> 14) + 1):
                 if w not in linear[tid]:
                     linear[tid][w] = v0
+            s = span[tid] = span[tid] or [v0, v1, 0, 0]
+            s[1] = v1
+            s[3 if flag & 4 else 2] += 1
+        else:
+            n_no_coor += 1
         p += 4 + bs
     out = bytearray(b"BAI\1" + struct.pack("<i", n_ref))
     for t in range(n_ref):
-        out += struct.pack("<i", len(bins[t]))
+        has_meta = meta and span[t] is not None
+        out += struct.pack("<i", len(bins[t]) + has_meta)
         for b, chunks in bins[t].items():
             out += struct.pack("<Ii", b, len(chunks))
             for v0, v1 in chunks:
                 out += struct.pack("<QQ", v0, v1)
+        if has_meta:
+            out += struct.pack("<IiQQQQ", 37450, 2, *span[t])
         n_intv = (max(linear[t]) + 1) if linear[t] else 0
         out += struct.pack("<i", n_intv)
         last = 0
         for w in range(n_intv):
             last = linear[t].get(w, last)
             out += struct.pack("<Q", last)
+    if meta:
+        out += struct.pack("<Q", n_no_coor)
     open(path + ".bai", "wb").write(bytes(out))
     return path + ".bai"

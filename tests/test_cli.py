@@ -219,8 +219,9 @@ def test_host_bam_reader_matches_workload(cli, tmp_path):
 def test_own_deflate_decoder_equals_zlib_on_every_block(cli, tmp_path):
     """`bgzf-check`: the host ingest's own DEFLATE decoder against zlib, block by block, bytes compared -- stored blocks
     (level 0), the match-heavy streams of level 1, the literal-heavy ones of level 6 (with SEQ/QUAL: long dynamic
-    codes, two-level tables), and the reference's own BGZF fixture where it exists. A declined block would fall back
-    to zlib in the product; here it fails the test."""
+    codes, two-level tables), and a plain gzip file like the reference's `file1.inq.gz`. A declined block would fall
+    back to zlib in the product; here it fails the test."""
+    import gzip
     import json
     from synth import synth as S
     w = S.make_workload(3, scale=0.0006, threads=2)
@@ -231,10 +232,11 @@ def test_own_deflate_decoder_equals_zlib_on_every_block(cli, tmp_path):
         assert r.returncode == 0, r.stderr
         st = json.loads(r.stdout)
         assert st["blocks"] > 1 and st["mismatch"] == 0 and st["fast_declined"] == 0, (level, st)
-    ref_gz = "/root/reference/test-data/file1.inq.gz"
-    if os.path.exists(ref_gz):                      # plain gzip is not BGZF: the walker says so
-        r = run(cli, "bgzf-check", ref_gz)
-        assert r.returncode == 1 and b"not a BGZF member" in r.stdout
+    plain_gz = str(tmp_path / "file1.inq.gz")       # plain gzip is not BGZF: the walker says so
+    with gzip.open(plain_gz, "wt") as f:
+        f.write("".join(f"chr7\t{154778571 + i}\t{154779363 + i}\t{i}.0\t{2 * i}.5\n" for i in range(50)))
+    r = run(cli, "bgzf-check", plain_gz)
+    assert r.returncode == 1 and b"not a BGZF member" in r.stdout
 
 
 def test_clmul_crc32_equals_zlib(tmp_path):

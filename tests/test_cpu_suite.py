@@ -1,5 +1,5 @@
 """CPU-only checks (-m "not gpu"): golden fixtures vs the oracle, C-ABI exports, the synthetic
-generator, range-sharding (world_size 2 over gloo) and the reference arm of bench.py."""
+generator, range-sharding (world_size 2 over gloo), the reference arm of bench.py and its output dump."""
 import ctypes
 import json
 import os
@@ -205,3 +205,45 @@ def test_bench_reference_arm_prints_contract_line():
     line = json.loads(out.stdout.strip().splitlines()[-1])
     assert line["impl"] == "reference" and line["unit"] == "loci/s" and line["value"] > 0
     assert line["cpu_baseline"]["kind"] == "port" and line["e2e"]["h2d_bytes_per_step"] == 0
+
+
+def test_bench_rejects_zero_steps_and_a_reference_dump(tmp_path):
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path)]):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *extra], capture_output=True, text=True, timeout=60)
+        assert out.returncode == 2 and out.stdout == "", extra
+    assert os.listdir(tmp_path) == []
+
+
+def test_bench_dump_outputs_float64_and_size_cap(tmp_path, monkeypatch):
+    import bench
+    rng = np.random.default_rng(3)
+    p1 = rng.integers(0, 400, 1000) / 2.0
+    p2 = p1 + 1.5
+    p1[::7] = np.nan
+    p1[0] = 0.0                                     # a called median of 0 stays apart from "no call" through the mask
+    p2[::11] = np.nan
+    bench.dump_outputs(str(tmp_path / "all"), p1, p2)
+    files = ["phase1.npy", "phase2.npy", "valid_mask.npy"]
+    assert sorted(os.listdir(tmp_path / "all")) == files
+    a1, a2, vm = (np.load(tmp_path / "all" / f) for f in files)
+    assert a1.dtype == a2.dtype == vm.dtype == np.float64
+    assert all(np.isfinite(a).all() for a in (a1, a2, vm))
+    assert np.array_equal(vm, np.where(np.isnan(p1), 0, 1) + np.where(np.isnan(p2), 0, 2))
+    assert np.array_equal(np.where(vm % 2 == 1, a1, np.nan), p1, equal_nan=True)
+    assert np.array_equal(np.where(vm >= 2, a2, np.nan), p2, equal_nan=True)
+    assert np.all(a1[np.isnan(p1)] == 0) and np.all(a2[np.isnan(p2)] == 0)
+    # over the cap: a fixed seeded sample of the loci, the same on every run, with its catalog indices
+    monkeypatch.setattr(bench, "DUMP_MAX_BYTES", 4 * 8 * 100)
+    for d in ("s1", "s2"):
+        bench.dump_outputs(str(tmp_path / d), p1, p2)
+    files = ["locus_index.npy", "phase1.npy", "phase2.npy", "valid_mask.npy"]
+    assert sorted(os.listdir(tmp_path / "s1")) == files
+    assert sum(os.path.getsize(tmp_path / "s1" / f) for f in files) <= 4 * 8 * 100 + 4 * 128
+    for f in files:
+        a = np.load(tmp_path / "s1" / f)
+        assert np.isfinite(a).all() and np.array_equal(a, np.load(tmp_path / "s2" / f))
+    idx = np.load(tmp_path / "s1" / "locus_index.npy")
+    assert idx.dtype == np.float64 and len(idx) == 100 and np.all(np.diff(idx) > 0)
+    k = idx.astype(np.int64)
+    for f in ("phase1.npy", "phase2.npy", "valid_mask.npy"):
+        assert np.array_equal(np.load(tmp_path / "s1" / f), np.load(tmp_path / "all" / f)[k])

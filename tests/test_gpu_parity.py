@@ -423,3 +423,30 @@ def test_routed_push_over_catalog_shards(sort_reads):
         assert same(np.concatenate(g1), p1) and same(np.concatenate(g2), p2)
         assert tot_visits == visits
         assert tot_taken < 3 * rd.n                      # nobody takes everything
+
+
+def test_bench_dump_outputs_are_the_timed_results(tmp_path):
+    """bench.py --dump-outputs: the medians of the last timed step, as the caller of Context.genotype gets them,
+    equal the oracle's on the same seeded workload; --steps is the number of timed steps"""
+    import json
+    import os
+    import subprocess
+    import sys
+    from synth.synth import make_workload
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--scale", "0.002", "--steps", "2", "--warmup", "0",
+                        "--no-cpu-baseline", "--no-e2e", "--no-cohort", "--bam-scale", "0", "--dump-outputs", str(tmp_path)],
+                       capture_output=True, text=True, timeout=600)
+    assert r.returncode == 0, r.stderr[-2000:]
+    line = json.loads(r.stdout.strip().splitlines()[-1])
+    assert line["steps"] == 2
+    w = make_workload(3, scale=0.002, threads=2, pack_filter=True)
+    rc, p1, p2, _ = O.genotype_loci(w.reads, w.n_contigs, w.locus_contig, w.locus_start.astype(np.uint32),
+                                    w.locus_end.astype(np.uint32), w.minlen, w.support, w.unphased, threads=4)
+    assert rc == 0
+    assert sorted(os.listdir(tmp_path)) == ["phase1.npy", "phase2.npy", "valid_mask.npy"]
+    d1, d2, vm = (np.load(tmp_path / f) for f in ("phase1.npy", "phase2.npy", "valid_mask.npy"))
+    assert d1.dtype == d2.dtype == vm.dtype == np.float64
+    assert all(np.isfinite(a).all() for a in (d1, d2, vm))
+    assert np.isnan(p1).any() and np.isnan(p2).any()              # the workload has loci without a call
+    assert same(np.where(vm % 2 == 1, d1, np.nan), p1) and same(np.where(vm >= 2, d2, np.nan), p2)
