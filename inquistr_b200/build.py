@@ -44,7 +44,7 @@ def build_cli(force: bool = False) -> str:
     target = os.path.join(bindir, "inquistr-b200")
     host = os.path.join(CSRC, "host")
     sources = [os.path.join(host, "main.cpp"), os.path.join(host, "bam_reader.cpp"), os.path.join(host, "cohort_cli.cpp"),
-               os.path.join(host, "shard_driver.cpp")]
+               os.path.join(host, "shard_driver.cpp"), os.path.join(host, "call_common.cpp"), os.path.join(host, "cohort_call.cpp")]
     deps = sources + [os.path.join(host, f) for f in sorted(os.listdir(host)) if f.endswith(".hpp")] + [os.path.join(os.path.dirname(HERE), "include", "inqcall.h"),
                       os.path.join(os.path.dirname(HERE), "include", "inqcohort.h"),
                       os.path.join(LIBDIR, "libinqcall.so")]

@@ -149,7 +149,29 @@ void ShardWorker::add(int32_t tid, int32_t pos, int32_t end, uint8_t mapq, uint8
 
 void ShardWorker::finish()
 {
+    end_sample();
+    stop();
+}
+
+void ShardWorker::end_sample()
+{
     submit();
+    { std::lock_guard<std::mutex> g(mu_); full_.push_back(nullptr); }
+    cv_.notify_all();
+}
+
+bool ShardWorker::take_result(ShardResult &out)
+{
+    std::unique_lock<std::mutex> lk(mu_);
+    cv_.wait(lk, [this] { return !done_.empty() || failed_; });
+    if (done_.empty()) { out = res_; return false; }
+    out = std::move(done_.front());
+    done_.pop_front();
+    return true;
+}
+
+void ShardWorker::stop()
+{
     { std::lock_guard<std::mutex> g(mu_); done_input_ = true; }
     cv_.notify_all();
     if (th_.joinable()) th_.join();
@@ -176,8 +198,9 @@ void ShardWorker::run()
         inq_host_register(b.cigar, ReadBatch::kWords * 4);
         inq_host_register(b.meta_block, meta_bytes());
     }
-    res_.s_ctx = now_s() - t0;
+    res_.s_ctx = s_ctx_ = now_s() - t0;
 
+    bool need_clear = false;             // a sample has been genotyped: its reads go before the next sample's first push
     for (;;) {
         ReadBatch *b = nullptr;
         {
@@ -189,6 +212,29 @@ void ShardWorker::run()
             b = full_.front();
             full_.pop_front();
         }
+        if (need_clear) {
+            need_clear = false;
+            rc = inq_clear_reads(ctx);
+            if (rc != INQ_OK) { fail(rc, inq_last_error(ctx)); break; }
+        }
+        if (!b) {                        // end of a sample: genotype the whole catalog against its reads
+            const size_t L = hi_ - lo_;
+            res_.t1.resize(L); res_.t2.resize(L); res_.valid.resize(L);
+            const double tg = now_s();
+            rc = inq_genotype(ctx, minlen_, support_, unphased_ ? 1 : 0, res_.t1.data(), res_.t2.data(), res_.valid.data(), &res_.stats);
+            res_.s_genotype = now_s() - tg;
+            if (rc != INQ_OK) { fail(rc, inq_last_error(ctx)); break; }
+            {
+                std::lock_guard<std::mutex> g(mu_);
+                done_.push_back(std::move(res_));
+                res_ = ShardResult();
+                memset(&res_.stats, 0, sizeof(res_.stats));
+                res_.s_ctx = s_ctx_;
+            }
+            cv_.notify_all();
+            need_clear = true;
+            continue;
+        }
         const double tp = now_s();
         if (b->n) {
             rc = inq_push_reads(ctx, b->n, b->contig, b->start, b->end, b->mapq, b->hp, b->flags, b->off, b->cigar);
@@ -199,14 +245,6 @@ void ShardWorker::run()
         if (rc != INQ_OK) { fail(rc, inq_last_error(ctx)); break; }
         { std::lock_guard<std::mutex> g(mu_); free_.push_back(b); }
         cv_.notify_all();
-    }
-    if (res_.rc == INQ_OK) {
-        const size_t L = hi_ - lo_;
-        res_.t1.resize(L); res_.t2.resize(L); res_.valid.resize(L);
-        const double tg = now_s();
-        rc = inq_genotype(ctx, minlen_, support_, unphased_ ? 1 : 0, res_.t1.data(), res_.t2.data(), res_.valid.data(), &res_.stats);
-        res_.s_genotype = now_s() - tg;
-        if (rc != INQ_OK) fail(rc, inq_last_error(ctx));
     }
     for (ReadBatch &b : batches_) { inq_host_unregister(b.cigar); inq_host_unregister(b.meta_block); }
     inq_ctx_destroy(ctx);

@@ -9,6 +9,9 @@
 //     genotypes its range once the input ends;
 //   * results are concatenated in shard order, which is catalog order. No collective, no device-to-device traffic.
 // A device may be listed several times (one context each), which exercises the sharding on a single GPU.
+// A worker may also genotype several samples in turn (`call-cohort`): end_sample() closes one sample's input, the
+// worker genotypes it and clears the reads, and the reader may already fill batches of the next sample meanwhile;
+// take_result() hands the samples' results back in the order they were ended. Context and catalog are set up once.
 #pragma once
 
 #include <condition_variable>
@@ -55,6 +58,7 @@ public:
     ShardWorker(const ShardWorker &) = delete;
     ShardWorker &operator=(const ShardWorker &) = delete;
 
+    int device() const { return device_; }
     size_t lo() const { return lo_; }
     size_t hi() const { return hi_; }
     // would htslib's fetch return a record [pos, end) on tid for some locus of this shard?
@@ -62,8 +66,15 @@ public:
     // append one record to the shard's current batch (reader thread); blocks while both batches are in flight
     void add(int32_t tid, int32_t pos, int32_t end, uint8_t mapq, uint8_t hp, uint8_t flags, const uint32_t *cigar, uint32_t n_cigar);
     void finish();                       // no more input: flush, genotype, join
-    ShardResult &result() { return res_; }
+    ShardResult &result() { return done_.empty() ? res_ : done_.front(); }     // after finish()
     bool failed();                       // the worker hit an error (the reader may stop early)
+    // per-sample cycle (reader thread): close the current sample's input; the worker genotypes it after the batches
+    // added before, then clears the reads for the next sample
+    void end_sample();
+    // results of the ended samples, oldest first; blocks until the next one is genotyped. false if the worker failed
+    // (out then carries the error)
+    bool take_result(ShardResult &out);
+    void stop();                         // no more samples: join the worker (no genotype of its own)
 
 private:
     void run();
@@ -82,11 +93,13 @@ private:
     std::thread th_;
     std::mutex mu_;
     std::condition_variable cv_;
-    std::deque<ReadBatch *> free_, full_;
+    std::deque<ReadBatch *> free_, full_; // full_: a null entry marks the end of a sample
     std::vector<ReadBatch> batches_;
     ReadBatch *cur_ = nullptr;
     bool ready_ = false, done_input_ = false, failed_ = false;
-    ShardResult res_;
+    ShardResult res_;                    // the sample being pushed (or the error)
+    std::deque<ShardResult> done_;       // genotyped samples not yet taken
+    double s_ctx_ = 0;
 };
 
 // cut [0, L) into n contiguous ranges of (nearly) equal total weight; weight may be null (all ones)

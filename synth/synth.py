@@ -155,11 +155,12 @@ def pack_keep_mask(mapq, hp, unphased: bool) -> np.ndarray:
 
 def make_workload(config: int, scale: float = 1.0, seed: int | None = None, threads: int = 0,
                   pinned: bool = False, shard: tuple = (0, 1), depth: float | None = None,
-                  n_loci: int | None = None, pack_filter: bool = False) -> Workload:
+                  n_loci: int | None = None, pack_filter: bool = False, read_seed: int | None = None) -> Workload:
     """Build one of the BASELINE.json configurations. `shard=(rank, world)` keeps only the loci of
     the rank's contiguous slice of the sorted catalog and the reads that can overlap them.
     `pack_filter` applies the host packer's per-read predicate (pack_keep_mask) while packing: the same
-    reads are drawn, the ones that can never pair are not emitted."""
+    reads are drawn, the ones that can never pair are not emitted.
+    `read_seed` draws the reads from their own seed over the catalog of `seed`: samples of one cohort."""
     L = lib()
     seed = config if seed is None else seed
     p_tagged, p_big_trunc, mode, unphased = 0.85, 0.0, 0, False
@@ -220,7 +221,7 @@ def make_workload(config: int, scale: float = 1.0, seed: int | None = None, thre
         reg_s = np.zeros(nc, np.int64)
         reg_e = contig_len - 1
     cfg = _Cfg()
-    cfg.seed, cfg.n_contigs, cfg.threads = seed, nc, threads
+    cfg.seed, cfg.n_contigs, cfg.threads = (seed if read_seed is None else read_seed), nc, threads
     cfg.contig_len = contig_len.ctypes.data
     cfg.contig_locus_off, cfg.lstart, cfg.lend = off.ctypes.data, ls.ctypes.data, le.ctypes.data
     cfg.delta_h1, cfg.delta_h2 = d1.ctypes.data, d2.ctypes.data
