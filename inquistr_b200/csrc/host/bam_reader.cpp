@@ -535,25 +535,13 @@ bool BamReader::next_parsed(const RecFilter &filter, int parse_threads, std::vec
             for (size_t i = a; i < b; ++i) {
                 if (!parse_bam_record(base + recs[i].first, recs[i].second, rv, cg, pc.err)) break;
                 if (filter.reach && !filter.reach(filter.ctx, rv.tid, rv.pos, rv.end)) continue;
-                const bool hp_odd = filter.need_hp && (rv.hp_type == HpType::OtherInt || rv.hp_type == HpType::NotInt);
-                if (!hp_odd && (rv.mapq <= 10 || (filter.need_hp && rv.hp_type == HpType::Absent))) {
-                    // fails the filter at every locus: counted by the caller through n_records - recs.size(), never shipped.
-                    // (kept as a stub without CIGAR so that the caller's counters can tell "unpairable" from "unreachable")
-                    BamRecLite l{rv.tid, rv.pos, rv.end, 0, nullptr, rv.hp_value, rv.flag, rv.mapq, rv.hp_type, false, false};
-                    pc.recs.push_back(l);
-                    cig_off.push_back((size_t)-1);
-                    continue;
-                }
-                bool sa_panic = false, has_clip = false;
-                for (uint32_t k = 0; k < rv.n_cigar && !has_clip; ++k) has_clip = (cg[k] & 0xF) == 4;
-                const bool two_d = has_clip ? is_accidental_2d(rv, &sa_panic) : false;
-                BamRecLite l{rv.tid, rv.pos, rv.end, rv.n_cigar, nullptr, rv.hp_value, rv.flag, rv.mapq, rv.hp_type, two_d, sa_panic};
+                const BamRecLite l = lite_record(rv, filter.need_hp);
                 cig_off.push_back(pc.cigar.size());
-                pc.cigar.insert(pc.cigar.end(), cg.begin(), cg.begin() + rv.n_cigar);
+                pc.cigar.insert(pc.cigar.end(), l.cigar, l.cigar + l.n_cigar);
                 pc.recs.push_back(l);
             }
             for (size_t k = 0; k < pc.recs.size(); ++k)
-                if (cig_off[k] != (size_t)-1) pc.recs[k].cigar = pc.cigar.data() + cig_off[k];
+                pc.recs[k].cigar = pc.recs[k].n_cigar ? pc.cigar.data() + cig_off[k] : nullptr;
         }
     };
     const int nt = (int)std::min<size_t>((size_t)std::max(1, parse_threads), n_chunks);
@@ -565,6 +553,23 @@ bool BamReader::next_parsed(const RecFilter &filter, int parse_threads, std::vec
     for (auto &pc : chunks)
         if (!pc.err.empty()) { err_ = pc.err; return false; }
     return true;
+}
+
+BamRecLite lite_record(const BamRecordView &rv, bool need_hp)
+{
+    BamRecLite l{rv.tid, rv.pos, rv.end, 0, nullptr, rv.hp_value, rv.flag, rv.mapq, rv.hp_type, false, false};
+    // fails the filter at every locus: never shipped, but kept as a stub without CIGAR so that the caller's counters
+    // can tell "unpairable" from "unreachable"
+    const bool hp_odd = need_hp && (rv.hp_type == HpType::OtherInt || rv.hp_type == HpType::NotInt);
+    if (!hp_odd && (rv.mapq <= 10 || (need_hp && rv.hp_type == HpType::Absent))) return l;
+    // is_accidental_2d is only consulted on S ops of reads that passed the filter (call.rs:394): what it would panic on
+    // travels as a flag and is raised by the GPU only if the read really pairs with a locus
+    bool has_clip = false;
+    for (uint32_t k = 0; k < rv.n_cigar && !has_clip; ++k) has_clip = (rv.cigar[k] & 0xF) == 4;
+    if (has_clip) l.two_d = is_accidental_2d(rv, &l.sa_panic);
+    l.n_cigar = rv.n_cigar;
+    l.cigar = rv.cigar;
+    return l;
 }
 
 bool parse_bam_record(const uint8_t *p, uint32_t block_size, BamRecordView &rec, std::vector<uint32_t> &cg_, std::string &err_)

@@ -48,7 +48,7 @@ struct BamRecordView {
 struct BamRecLite {
     int32_t tid, pos, end;
     uint32_t n_cigar;
-    const uint32_t *cigar;        // into the chunk's own storage; null when the record was not kept
+    const uint32_t *cigar;        // into the chunk's own storage; null for a stub (n_cigar 0)
     int64_t hp_value;
     uint16_t flag;
     uint8_t mapq;
@@ -266,5 +266,10 @@ bool bgzf_selfcheck(const std::string &path, std::string *report);
 int64_t cigar_text_to_rlen(const std::string &cigar);
 // call.rs:415-459 ; *panic set when the reference would panic (SA not a string)
 bool is_accidental_2d(const BamRecordView &rec, bool *panic);
+// What the `call` driver keeps of a record that some locus window reaches. A record with mapq <= 10 or, when need_hp,
+// without an HP tag fails the filter at every locus (call.rs:297-300,350-352) and becomes a stub without CIGAR, unless
+// its HP tag has a type the reference panics on (call.rs:487). Otherwise the CIGAR points into rv and, for a record
+// with a soft clip, two_d / sa_panic are what is_accidental_2d says.
+BamRecLite lite_record(const BamRecordView &rv, bool need_hp);
 
 }  // namespace inqhost

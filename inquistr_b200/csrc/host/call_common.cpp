@@ -18,6 +18,12 @@ void panic(const std::string &msg)
     exit(101);
 }
 
+void usage_error(const std::string &usage, const std::string &msg)
+{
+    fprintf(stderr, "error: %s\n\nUsage: %s\n\nFor more information, try '--help'.\n", msg.c_str(), usage.c_str());
+    exit(2);
+}
+
 bool parse_u64(const std::string &s, uint64_t *out)
 {
     if (s.empty()) return false;

@@ -1,4 +1,4 @@
-// call_common.hpp -- pieces of the `call` driver (main.cpp) that `call-cohort` (cohort_call.cpp) uses as they are:
+// call_common.hpp -- helpers of the `call` / `call-cohort` driver (call_driver.cpp): errors, option values, paths,
 // sample names, catalog parsing and validation, output order and number format.
 #pragma once
 
@@ -11,6 +11,7 @@
 namespace inqhost {
 
 [[noreturn]] void panic(const std::string &msg);     // a panic in the reference: message on stderr, exit code 101
+[[noreturn]] void usage_error(const std::string &usage, const std::string &msg);   // clap's usage error: exit code 2
 bool parse_u64(const std::string &s, uint64_t *out);
 bool parse_device_list(const std::string &v, std::vector<int> *out);   // "A,B,...": 1..64 devices, each <= 1023
 bool is_file(const std::string &p);

@@ -48,7 +48,6 @@ ShardWorker::ShardWorker(int device, size_t lo, size_t hi, int n_contigs, const 
         int32_t m = INT32_MIN;
         for (int64_t i = off_[c]; i < off_[c + 1]; ++i) { m = std::max(m, lend_[i]); pmax_[i] = m; }
     }
-    memset(&res_.stats, 0, sizeof(res_.stats));
     // staging batches: the reader fills one while others are on their way to the device (or wait for the context)
     batches_.resize((size_t)std::max(2, n_batches));
     for (ReadBatch &b : batches_) {
@@ -104,10 +103,7 @@ bool ShardWorker::failed()
 ReadBatch *ShardWorker::take_free()
 {
     std::unique_lock<std::mutex> lk(mu_);
-    const double t0 = now_s();
     cv_.wait(lk, [this] { return !free_.empty() || failed_; });
-    res_.s_wait_input += 0;               // (reader-side wait; the worker-side wait is accounted in run())
-    (void)t0;
     if (failed_) return nullptr;
     ReadBatch *b = free_.front();
     free_.pop_front();
@@ -130,7 +126,7 @@ void ShardWorker::add(int32_t tid, int32_t pos, int32_t end, uint8_t mapq, uint8
     if (cur_ && !cur_->room_for(n_cigar)) submit();
     if (!cur_) {
         cur_ = take_free();
-        if (!cur_) return;                                       // worker failed: the error surfaces in finish()
+        if (!cur_) return;                                       // worker failed: the error surfaces in take_result()
     }
     if (n_cigar > ReadBatch::kWords) {                            // cannot happen with BAM (CG tag max 2^32/4 > kWords is theoretical): fail loudly
         std::lock_guard<std::mutex> g(mu_);
@@ -145,12 +141,6 @@ void ShardWorker::add(int32_t tid, int32_t pos, int32_t end, uint8_t mapq, uint8
     memcpy(b.cigar + b.words, cigar, (size_t)n_cigar * 4);
     b.words += n_cigar;
     b.off[++b.n] = b.words;
-}
-
-void ShardWorker::finish()
-{
-    end_sample();
-    stop();
 }
 
 void ShardWorker::end_sample()
@@ -205,9 +195,7 @@ void ShardWorker::run()
         ReadBatch *b = nullptr;
         {
             std::unique_lock<std::mutex> lk(mu_);
-            const double tw = now_s();
             cv_.wait(lk, [this] { return !full_.empty() || done_input_; });
-            res_.s_wait_input += now_s() - tw;
             if (full_.empty()) break;
             b = full_.front();
             full_.pop_front();
@@ -228,7 +216,6 @@ void ShardWorker::run()
                 std::lock_guard<std::mutex> g(mu_);
                 done_.push_back(std::move(res_));
                 res_ = ShardResult();
-                memset(&res_.stats, 0, sizeof(res_.stats));
                 res_.s_ctx = s_ctx_;
             }
             cv_.notify_all();
@@ -236,11 +223,7 @@ void ShardWorker::run()
             continue;
         }
         const double tp = now_s();
-        if (b->n) {
-            rc = inq_push_reads(ctx, b->n, b->contig, b->start, b->end, b->mapq, b->hp, b->flags, b->off, b->cigar);
-            res_.reads += b->n;
-            res_.words += b->words;
-        }
+        if (b->n) rc = inq_push_reads(ctx, b->n, b->contig, b->start, b->end, b->mapq, b->hp, b->flags, b->off, b->cigar);
         res_.s_push += now_s() - tp;
         if (rc != INQ_OK) { fail(rc, inq_last_error(ctx)); break; }
         { std::lock_guard<std::mutex> g(mu_); free_.push_back(b); }

@@ -44,9 +44,8 @@ struct ShardResult {
     std::string error;
     std::vector<int64_t> t1, t2;
     std::vector<uint8_t> valid;
-    inq_stats stats;
-    double s_ctx = 0, s_push = 0, s_genotype = 0, s_wait_input = 0;
-    uint64_t reads = 0, words = 0;
+    inq_stats stats{};
+    double s_ctx = 0, s_push = 0, s_genotype = 0;
 };
 
 class ShardWorker {
@@ -65,8 +64,6 @@ public:
     bool reaches(int32_t tid, int32_t pos, int32_t end) const;
     // append one record to the shard's current batch (reader thread); blocks while both batches are in flight
     void add(int32_t tid, int32_t pos, int32_t end, uint8_t mapq, uint8_t hp, uint8_t flags, const uint32_t *cigar, uint32_t n_cigar);
-    void finish();                       // no more input: flush, genotype, join
-    ShardResult &result() { return done_.empty() ? res_ : done_.front(); }     // after finish()
     bool failed();                       // the worker hit an error (the reader may stop early)
     // per-sample cycle (reader thread): close the current sample's input; the worker genotypes it after the batches
     // added before, then clears the reads for the next sample

@@ -143,7 +143,7 @@ def _alloc(n, dtype, pinned):
 
 
 def pack_keep_mask(mapq, hp, unphased: bool) -> np.ndarray:
-    """The host packer's per-read predicate (`consider()` in csrc/host/main.cpp): a read with mapq <= 10
+    """The host packer's per-read predicate (`lite_record()` in csrc/host/bam_reader.cpp): a read with mapq <= 10
     fails both filters (call.rs:297-300,350-352), and without an HP tag it fails the phased one, for
     every locus -- such a read can never pair, so the host does not ship it. HP 0 and HP > 2 reads are
     kept: they pass the filter (the reference walks them / panics on them)."""

@@ -327,6 +327,11 @@ def test_panel_with_and_without_index(cli, panel_bam, tmp_path):
         assert r.returncode == 0, r.stderr
         assert r.stdout == exp
         outs[mode] = json.load(open(stats))
+    keys = {"used_index", "records", "records_pushed", "records_unpairable", "bytes_inflated", "bytes_inflated_on_gpu", "n_loci",
+            "n_reads", "n_cigar_words", "n_pairs", "n_events", "ms_total", "ms_cigar", "ms_h2d", "launches", "n_shards",
+            "records_routed", "s_ctx_create_set_loci", "s_bam_scan", "s_push_under_scan", "s_flush_genotype", "s_total",
+            "s_scan_wait_inflate", "s_scan_index", "s_scan_parse"}
+    assert set(outs["1"]) == set(outs["0"]) == keys
     assert outs["1"]["used_index"] == 1 and outs["0"]["used_index"] == 0
     assert outs["1"]["records"] <= outs["0"]["records"]          # only records near the loci are decoded
     assert outs["1"]["records_pushed"] == outs["0"]["records_pushed"]

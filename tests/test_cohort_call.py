@@ -161,6 +161,9 @@ def test_equals_combine_of_calls(cli, tmp_path, cfg, scale, n, modes):
         assert r.stdout == exp, (threads, unphased, idx)
         assert r.stdout == oracle_table(bams, ws, rows, unphased, threads)
         st = json.load(open(stats))
+        assert set(st) == {"n_samples", "n_contexts", "n_loci", "s_ctx_create_set_loci", "s_total", "samples"}
+        assert all(set(s) == {"bam", "context", "used_index", "records", "records_pushed", "records_unpairable", "bytes_inflated",
+                              "n_pairs", "ms_total", "s_bam_scan", "s_genotype"} for s in st["samples"])
         assert st["n_samples"] == n and st["n_contexts"] == 1 and len(st["samples"]) == n
         assert all(s["used_index"] == int(idx) for s in st["samples"])
         assert all(s["records_pushed"] > 0 and s["ms_total"] > 0 for s in st["samples"])
