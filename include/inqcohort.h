@@ -11,6 +11,10 @@
  *                        outliers = Noise
  * What the caller keeps: the sample names (suffix stripping outlier.rs:112,130), --subset filtering
  * (outlier.rs:59-67) and the TSV text.
+ *
+ * inq_assoc: per-locus association of STR length with a trait (`inquistr-b200 assoc`, DESIGN.md 5e); the model is
+ * this project's own (the reference has it only as an external R script): OLS with a Student t test, or logistic
+ * IRLS as R's glm.fit without step-halving with a Wald z test; design [1, covariates..., x], x last.
  */
 #ifndef INQCOHORT_H
 #define INQCOHORT_H
@@ -36,6 +40,29 @@ extern "C" {
 int inq_outlier(int device, int method, uint64_t n_rows, uint32_t n_cols, const float *values,
                 uint32_t minsize, float zscore_cutoff, uint8_t *row_kept,
                 uint64_t *n_hits, uint64_t *hits, uint64_t cap, float *ms_kernel /* nullable */);
+
+#define INQ_ASSOC_LINEAR 0         /* OLS, t test with n - rank degrees of freedom */
+#define INQ_ASSOC_LOGISTIC 1       /* binomial / logit IRLS, Wald z test, dispersion 1 */
+#define INQ_ASSOC_SUM 0            /* predictor H1 + H2, missing if either is NaN */
+#define INQ_ASSOC_MAX 1            /* predictor max of the non-NaN alleles, missing if both are NaN */
+
+#define INQ_ASSOC_OK 0
+#define INQ_ASSOC_FEW_SAMPLES 1    /* n <= rank, or (logistic) only one class among the samples used */
+#define INQ_ASSOC_SINGULAR 2       /* x aliased by the intercept and covariates */
+#define INQ_ASSOC_NO_CONVERGENCE 3 /* logistic: 25 iterations without meeting the deviance criterion */
+#define INQ_ASSOC_SEPARATION 4     /* logistic: a fitted probability below 10 eps or above 1 - 10 eps */
+
+#define INQ_ASSOC_MAX_COV 30       /* design columns: intercept + covariates + x <= 32 */
+
+/* Tests every row of `haps` (host memory, row-major n_rows x 2 * n_samples f64: H1, H2 of each sample, NaN = no
+ * call) for association with the trait `y[n_samples]` (logistic: every value 0 or 1), adjusted for the covariates
+ * `cov` (row-major n_samples x n_cov, no missing values). Per row: beta, se, stat (t or z), two-sided p (NaN when
+ * the status is FEW_SAMPLES or SINGULAR), n_used (samples with a predictor) and status (INQ_ASSOC_*);
+ * n_iter (nullable) is the number of weighted solves of a logistic fit (0 for linear).
+ * Returns 0 or a negative INQ_ERR_* code (inqcall.h); inq_cohort_last_error() describes the failure. */
+int inq_assoc(int device, int model, int predictor, uint64_t n_rows, uint32_t n_samples, const double *haps,
+              const double *y, uint32_t n_cov, const double *cov, double *beta, double *se, double *stat, double *p,
+              uint32_t *n_used, uint8_t *status, uint8_t *n_iter /* nullable */, float *ms_kernel /* nullable */);
 
 const char *inq_cohort_last_error(void);
 

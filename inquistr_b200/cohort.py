@@ -1,4 +1,4 @@
-"""ctypes binding of include/inqcohort.h (cohort `outlier` rows, part of libinqcall.so). No CPU fallback."""
+"""ctypes binding of include/inqcohort.h (cohort `outlier` rows and `assoc`, part of libinqcall.so). No CPU fallback."""
 from __future__ import annotations
 
 import ctypes as C
@@ -9,7 +9,11 @@ from .api import INQ_OK, InqError, load_library
 
 ZSCORE, DBSCAN = 0, 1
 INQ_ERR_NO_MODE, INQ_ERR_HITS_CAP = -15, -16
-EXPORTS = ["inq_outlier", "inq_cohort_last_error"]
+LINEAR, LOGISTIC = 0, 1
+PRED_SUM, PRED_MAX = 0, 1
+ASSOC_OK, ASSOC_FEW_SAMPLES, ASSOC_SINGULAR, ASSOC_NO_CONVERGENCE, ASSOC_SEPARATION = 0, 1, 2, 3, 4
+ASSOC_STATUS_NAMES = ["ok", "few_samples", "singular", "no_convergence", "separation"]
+EXPORTS = ["inq_outlier", "inq_assoc", "inq_cohort_last_error"]
 
 _BOUND = False
 
@@ -21,6 +25,10 @@ def _lib():
         L.inq_outlier.restype = C.c_int
         L.inq_outlier.argtypes = [C.c_int, C.c_int, C.c_uint64, C.c_uint32, C.c_void_p, C.c_uint32, C.c_float,
                                   C.c_void_p, C.POINTER(C.c_uint64), C.c_void_p, C.c_uint64, C.POINTER(C.c_float)]
+        L.inq_assoc.restype = C.c_int
+        L.inq_assoc.argtypes = [C.c_int, C.c_int, C.c_int, C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint32,
+                                C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                C.c_void_p, C.POINTER(C.c_float)]
         L.inq_cohort_last_error.restype = C.c_char_p
         L.inq_cohort_last_error.argtypes = []
         _BOUND = True
@@ -49,3 +57,32 @@ def outlier(matrix, minsize: int = 10, cutoff: float = 3.0, method: str = "zscor
             raise InqError(rc, L.inq_cohort_last_error().decode())
         h = hits[:int(n.value)]
         return kept, (h >> np.uint64(32)).astype(np.int64), (h & np.uint64(0xFFFFFFFF)).astype(np.int64), float(ms.value)
+
+
+def assoc(haps, y, cov=None, model: str = "linear", predictor: str = "sum", device: int = 0):
+    """Per-row association of STR length with the trait y (include/inqcohort.h inq_assoc).
+    haps: rows x 2*samples f64 (H1, H2 of each sample, NaN = no call); y: samples; cov: samples x n_cov or None.
+    -> dict of per-row arrays beta, se, stat, p (f64), n (u32), status (u8, ASSOC_*), n_iter (u8), and ms_kernel."""
+    h = np.ascontiguousarray(haps, dtype=np.float64)
+    rows, cols = h.shape
+    if cols % 2:
+        raise ValueError("haps needs two columns per sample")
+    ns = cols // 2
+    yy = np.ascontiguousarray(y, dtype=np.float64)
+    if yy.shape != (ns,):
+        raise ValueError("y needs one value per sample")
+    c = np.zeros((ns, 0)) if cov is None else np.ascontiguousarray(np.asarray(cov, np.float64).reshape(ns, -1))
+    out = {k: np.zeros(rows, np.float64) for k in ("beta", "se", "stat", "p")}
+    out["n"] = np.zeros(rows, np.uint32)
+    out["status"] = np.zeros(rows, np.uint8)
+    out["n_iter"] = np.zeros(rows, np.uint8)
+    ms = C.c_float(0)
+    L = _lib()
+    rc = L.inq_assoc(device, {"linear": LINEAR, "logistic": LOGISTIC}[model], {"sum": PRED_SUM, "max": PRED_MAX}[predictor],
+                     rows, ns, h.ctypes.data, yy.ctypes.data, c.shape[1], c.ctypes.data if c.size else None,
+                     out["beta"].ctypes.data, out["se"].ctypes.data, out["stat"].ctypes.data, out["p"].ctypes.data,
+                     out["n"].ctypes.data, out["status"].ctypes.data, out["n_iter"].ctypes.data, C.byref(ms))
+    if rc != INQ_OK:
+        raise InqError(rc, L.inq_cohort_last_error().decode())
+    out["ms_kernel"] = float(ms.value)
+    return out

@@ -1,16 +1,20 @@
-// cohort_cli.cpp -- `inquistr-b200 combine` and `inquistr-b200 outlier` (SURVEY 8f rank 3).
+// cohort_cli.cpp -- `inquistr-b200 combine`, `inquistr-b200 outlier` (SURVEY 8f rank 3) and `inquistr-b200 assoc`.
 // Host side of the reference's src/combine.rs:27-59 and src/outlier.rs:33-72 / src/main.rs:75-99,202-229
 // above the C ABI of include/inqcohort.h: text in, text out; the per-row arithmetic runs on the GPU.
-// A Rust panic in the reference maps to exit code 101, clap usage errors to 2.
+// A Rust panic in the reference maps to exit code 101, clap usage errors to 2. `assoc` has no counterpart in the
+// reference's binary (DESIGN.md 5e): its input errors exit 1 with `inquistr-b200: <file>:<line>: ...`.
 #include <sys/stat.h>
 #include <zlib.h>
 
 #include <algorithm>
+#include <charconv>
+#include <chrono>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
 #include <string>
+#include <unordered_map>
 #include <unordered_set>
 #include <vector>
 
@@ -269,6 +273,268 @@ int outlier_main(const std::vector<std::string> &v, int device)
         if (keys.size() == batch_rows) flush();
     }
     flush();
+    return 0;
+}
+
+namespace {
+
+[[noreturn]] void afail(const std::string &msg)
+{
+    fflush(stdout);
+    fprintf(stderr, "inquistr-b200: %s\n", msg.c_str());
+    exit(1);
+}
+
+// a finite decimal number, the whole field
+bool parse_f64(const std::string &s, double *out)
+{
+    if (s.empty() || isspace((unsigned char)s[0])) return false;
+    char *end = nullptr;
+    *out = strtod(s.c_str(), &end);
+    return end && *end == '\0' && std::isfinite(*out);
+}
+
+// a value of the combined table: a finite number or NaN (no call)
+bool parse_call(const std::string &s, double *out)
+{
+    if (s.size() == 3 && tolower((unsigned char)s[0]) == 'n' && tolower((unsigned char)s[1]) == 'a' && tolower((unsigned char)s[2]) == 'n') {
+        *out = NAN;
+        return true;
+    }
+    return parse_f64(s, out);
+}
+
+void append_f64(std::string &out, double v)
+{
+    if (std::isnan(v)) { out += "NaN"; return; }
+    char buf[64];
+    const auto r = std::to_chars(buf, buf + sizeof(buf), v);          // shortest form that round-trips
+    out.append(buf, r.ptr);
+}
+
+}  // namespace
+
+// `assoc`: one regression per row of a combined table (DESIGN.md 5e)
+int assoc_main(const std::vector<std::string> &v, int device)
+{
+    const char *usage = "assoc --phenotype <TSV> --trait <COL> --model <linear|logistic> [--covariates A,B,...] [--predictor sum|max] [--device N] <COMBINED>";
+    std::string combined, pheno, trait, model, predictor = "sum", covs, stats_json;
+    bool has_cov = false;
+    for (size_t i = 0; i < v.size(); ++i) {
+        const std::string &a = v[i];
+        auto value = [&](const char *name) -> std::string {
+            if (i + 1 >= v.size()) cusage(std::string("a value is required for '") + name + "' but none was supplied", usage);
+            return v[++i];
+        };
+        if (a == "--phenotype") pheno = value("--phenotype <TSV>");
+        else if (a == "--trait") trait = value("--trait <COL>");
+        else if (a == "--model") {
+            model = value("--model <MODEL>");
+            if (model != "linear" && model != "logistic") cusage("invalid value '" + model + "' for '--model <MODEL>'\n  [possible values: linear, logistic]", usage);
+        } else if (a == "--covariates") { covs = value("--covariates <A,B,...>"); has_cov = true; }
+        else if (a == "--predictor") {
+            predictor = value("--predictor <PREDICTOR>");
+            if (predictor != "sum" && predictor != "max") cusage("invalid value '" + predictor + "' for '--predictor <PREDICTOR>'\n  [possible values: sum, max]", usage);
+        } else if (a == "--device") {
+            const std::string s = value("--device <N>");
+            char *e = nullptr;
+            const long d = strtol(s.c_str(), &e, 10);
+            if (s.empty() || *e || d < 0 || d > 1024) cusage("invalid value '" + s + "' for '--device <N>'", usage);
+            device = (int)d;
+        } else if (a == "--stats-json") stats_json = value("--stats-json <FILE>");
+        else if (a == "-h" || a == "--help") {
+            printf("Test every locus of a combined table for association with a phenotype\n\nUsage: inquistr-b200 %s\n\n"
+                   "Arguments:\n  <COMBINED>  combined table of calls (`call-cohort` or `combine` output, plain or gzip)\n\nOptions:\n"
+                   "      --phenotype <TSV>        tab-separated phenotype table with a header; first column: sample names\n"
+                   "      --trait <COL>            response column\n"
+                   "      --model <MODEL>          linear (OLS, t test) or logistic (0/1 trait, IRLS, Wald z test) [possible values: linear, logistic]\n"
+                   "      --covariates <A,B,...>   0 to %d covariate columns; samples with a missing value (NA, NaN, empty) are left out\n"
+                   "      --predictor <PREDICTOR>  per sample and locus: H1 + H2, or the larger allele [default: sum] [possible values: sum, max]\n"
+                   "      --device <N>             CUDA device [default: 0]\n"
+                   "      --stats-json <FILE>      write parse, device and output times to FILE\n"
+                   "  -h, --help                   Print help\n\n"
+                   "Output: chromosome begin end n beta se stat p status, one row per input row; status is one of ok,\n"
+                   "few_samples, singular, no_convergence, separation\n", usage, INQ_ASSOC_MAX_COV);
+            return 0;
+        } else if (!a.empty() && a[0] == '-' && a.size() > 1) cusage("unexpected argument '" + a + "' found", usage);
+        else if (combined.empty()) combined = a;
+        else cusage("unexpected argument '" + a + "' found", usage);
+    }
+    std::string missing;
+    if (pheno.empty()) missing += "\n  --phenotype <TSV>";
+    if (trait.empty()) missing += "\n  --trait <COL>";
+    if (model.empty()) missing += "\n  --model <MODEL>";
+    if (combined.empty()) missing += "\n  <COMBINED>";
+    if (!missing.empty()) cusage("the following required arguments were not provided:" + missing, usage);
+    std::vector<std::string> cov_names;
+    if (has_cov && !covs.empty()) {
+        size_t a = 0;
+        for (;;) {
+            const size_t b = covs.find(',', a);
+            cov_names.emplace_back(covs, a, b == std::string::npos ? std::string::npos : b - a);
+            if (b == std::string::npos) break;
+            a = b + 1;
+        }
+    }
+    if (cov_names.size() > INQ_ASSOC_MAX_COV)
+        cusage("invalid value '" + covs + "' for '--covariates <A,B,...>': " + std::to_string(cov_names.size()) + " covariates, at most " +
+               std::to_string(INQ_ASSOC_MAX_COV), usage);
+    for (size_t c = 0; c < cov_names.size(); ++c) {
+        if (cov_names[c].empty()) cusage("invalid value '" + covs + "' for '--covariates <A,B,...>': an empty column name", usage);
+        if (cov_names[c] == trait) cusage("the trait '" + trait + "' is also listed as a covariate", usage);
+        for (size_t d = 0; d < c; ++d)
+            if (cov_names[d] == cov_names[c]) cusage("covariate '" + cov_names[c] + "' is listed twice", usage);
+    }
+    const bool logistic = model == "logistic";
+    const auto t_start = std::chrono::steady_clock::now();
+
+    // phenotype table: sample -> trait, covariates; rows with a missing value are left out
+    const size_t n_cov = cov_names.size();
+    std::unordered_map<std::string, std::vector<double>> ph;          // complete rows: [trait, covariates...]
+    std::unordered_set<std::string> ph_seen;
+    size_t ph_missing = 0;
+    {
+        LineReader pr;
+        if (!exists(pheno) || !pr.open(pheno)) afail(pheno + ": cannot open the phenotype table");
+        std::string line;
+        std::vector<std::string> cols;
+        if (!pr.next(line)) afail(pheno + ":1: empty file (a header row is needed)");
+        split_tabs(line, cols);
+        const std::vector<std::string> head = cols;
+        std::vector<std::string> want_names{trait};                   // [trait, covariates...]
+        want_names.insert(want_names.end(), cov_names.begin(), cov_names.end());
+        std::vector<size_t> want;
+        for (const std::string &name : want_names) {
+            size_t k = 1;
+            while (k < head.size() && head[k] != name) ++k;
+            if (k >= head.size()) afail(pheno + ":1: column '" + name + "' is not in the header");
+            want.push_back(k);
+        }
+        for (uint64_t ln = 2; pr.next(line); ++ln) {
+            if (line.empty()) continue;
+            split_tabs(line, cols);
+            const std::string where = pheno + ":" + std::to_string(ln) + ": ";
+            if (cols.size() != head.size())
+                afail(where + std::to_string(cols.size()) + " fields, the header has " + std::to_string(head.size()));
+            if (!ph_seen.insert(cols[0]).second) afail(where + "column '" + head[0] + "': sample '" + cols[0] + "' appears twice");
+            std::vector<double> vals(want.size());
+            bool complete = true;
+            for (size_t w = 0; w < want.size(); ++w) {
+                const std::string &f = cols[want[w]];
+                if (f.empty() || f == "NA" || f == "NaN") { complete = false; continue; }
+                if (!parse_f64(f, &vals[w])) afail(where + "column '" + head[want[w]] + "': '" + f + "' is not a number");
+                if (w == 0 && logistic && vals[w] != 0.0 && vals[w] != 1.0)
+                    afail(where + "column '" + head[want[w]] + "': '" + f + "' is not 0 or 1 (--model logistic)");
+            }
+            if (complete) ph.emplace(cols[0], std::move(vals));
+            else ++ph_missing;
+        }
+    }
+
+    // combined table header: chromosome begin end <S>_H1 <S>_H2 ...
+    if (!exists(combined)) afail(combined + ": no such file");
+    LineReader rd;
+    if (!rd.open(combined)) afail(combined + ": cannot open");
+    std::string line;
+    std::vector<std::string> cols;
+    if (!rd.next(line)) afail(combined + ":1: empty file (a header row is needed)");
+    split_tabs(line, cols);
+    if (cols.size() < 3 || cols[0] != "chromosome" || cols[1] != "begin" || cols[2] != "end")
+        afail(combined + ":1: the header does not start with 'chromosome begin end'");
+    const size_t n_val = cols.size() - 3;
+    if (n_val % 2) afail(combined + ":1: " + std::to_string(n_val) + " value columns: not in <S>_H1 <S>_H2 pairs");
+    const size_t n_tab = n_val / 2;
+    std::vector<uint32_t> use_idx;                       // table sample index of every used sample, in table order
+    std::vector<double> y, cov;
+    {
+        std::unordered_set<std::string> names;
+        for (size_t k = 0; k < n_tab; ++k) {
+            const std::string &h1 = cols[3 + 2 * k], &h2 = cols[4 + 2 * k];
+            const bool pair = h1.size() > 3 && h2.size() == h1.size() && h1.compare(h1.size() - 3, 3, "_H1") == 0 &&
+                              h2.compare(h2.size() - 3, 3, "_H2") == 0 && h1.compare(0, h1.size() - 3, h2, 0, h2.size() - 3) == 0;
+            if (!pair) afail(combined + ":1: columns " + std::to_string(4 + 2 * k) + "-" + std::to_string(5 + 2 * k) + " ('" + h1 + "', '" + h2 +
+                             "') are not a <S>_H1 <S>_H2 pair");
+            const std::string s = h1.substr(0, h1.size() - 3);
+            if (!names.insert(s).second) afail(combined + ":1: sample '" + s + "' appears twice");
+            const auto it = ph.find(s);
+            if (it == ph.end()) continue;
+            use_idx.push_back((uint32_t)k);
+            y.push_back(it->second[0]);
+            cov.insert(cov.end(), it->second.begin() + 1, it->second.end());
+        }
+        size_t ph_only = 0;
+        for (const std::string &s : ph_seen) ph_only += !names.count(s);
+        fprintf(stderr, "assoc: %zu samples used, %zu in the table only, %zu in the phenotype table only (%zu phenotype rows with a missing value left out)\n",
+                use_idx.size(), n_tab - use_idx.size(), ph_only, ph_missing);
+        if (use_idx.empty()) afail("no sample is in both " + combined + " and " + pheno);
+    }
+    const uint32_t ns = (uint32_t)use_idx.size();
+    fputs("chromosome\tbegin\tend\tn\tbeta\tse\tstat\tp\tstatus\n", stdout);
+    const char *status_names[] = {"ok", "few_samples", "singular", "no_convergence", "separation"};
+    const int mdl = logistic ? INQ_ASSOC_LOGISTIC : INQ_ASSOC_LINEAR, prd = predictor == "max" ? INQ_ASSOC_MAX : INQ_ASSOC_SUM;
+
+    // rows in batches of at most 256 MB of values
+    const size_t batch_rows = std::max<size_t>(1, (256u << 20) / ((size_t)ns * 2 * sizeof(double)));
+    std::vector<double> haps, beta, se, stat, pv, rowvals(n_val);
+    std::vector<uint32_t> n_used;
+    std::vector<uint8_t> status;
+    std::vector<std::string> keys;
+    double s_device = 0.0, s_write = 0.0;
+    uint64_t n_rows = 0;
+    std::string out;
+    auto flush = [&]() {
+        const size_t rows = keys.size();
+        if (!rows) return;
+        beta.resize(rows); se.resize(rows); stat.resize(rows); pv.resize(rows); n_used.resize(rows); status.resize(rows);
+        const auto t0 = std::chrono::steady_clock::now();
+        const int rc = inq_assoc(device, mdl, prd, rows, ns, haps.data(), y.data(), (uint32_t)n_cov, n_cov ? cov.data() : nullptr,
+                                 beta.data(), se.data(), stat.data(), pv.data(), n_used.data(), status.data(), nullptr, nullptr);
+        const auto t1 = std::chrono::steady_clock::now();
+        s_device += std::chrono::duration<double>(t1 - t0).count();
+        if (rc != INQ_OK) afail(inq_cohort_last_error());
+        out.clear();
+        for (size_t r = 0; r < rows; ++r) {
+            out += keys[r];
+            out.push_back('\t');
+            out += std::to_string(n_used[r]);
+            for (double x : {beta[r], se[r], stat[r], pv[r]}) { out.push_back('\t'); append_f64(out, x); }
+            out.push_back('\t');
+            out += status[r] < 5 ? status_names[status[r]] : "?";
+            out.push_back('\n');
+            if (out.size() >= (4u << 20)) { fwrite(out.data(), 1, out.size(), stdout); out.clear(); }
+        }
+        fwrite(out.data(), 1, out.size(), stdout);
+        s_write += std::chrono::duration<double>(std::chrono::steady_clock::now() - t1).count();
+        n_rows += rows;
+        haps.clear();
+        keys.clear();
+    };
+    for (uint64_t ln = 2; rd.next(line); ++ln) {
+        split_tabs(line, cols);
+        const std::string where = combined + ":" + std::to_string(ln) + ": ";
+        if (cols.size() != 3 + n_val) {
+            flush();
+            afail(where + std::to_string(cols.size() < 3 ? 0 : cols.size() - 3) + " values, the header has " + std::to_string(n_val));
+        }
+        for (size_t c = 0; c < n_val; ++c)
+            if (!parse_call(cols[3 + c], &rowvals[c])) {
+                flush();
+                afail(where + "column " + std::to_string(4 + c) + ": '" + cols[3 + c] + "' is not a number");
+            }
+        for (uint32_t k : use_idx) { haps.push_back(rowvals[2 * k]); haps.push_back(rowvals[2 * k + 1]); }
+        keys.push_back(cols[0] + "\t" + cols[1] + "\t" + cols[2]);
+        if (keys.size() == batch_rows) flush();
+    }
+    flush();
+    fflush(stdout);
+    if (!stats_json.empty()) {
+        const double total = std::chrono::duration<double>(std::chrono::steady_clock::now() - t_start).count();
+        FILE *f = fopen(stats_json.c_str(), "w");
+        if (!f) afail(stats_json + ": cannot write");
+        fprintf(f, "{\"rows\": %llu, \"samples_used\": %u, \"s_total\": %.6f, \"s_device\": %.6f, \"s_write\": %.6f, \"s_parse\": %.6f}\n",
+                (unsigned long long)n_rows, ns, total, s_device, s_write, total - s_device - s_write);
+        fclose(f);
+    }
     return 0;
 }
 

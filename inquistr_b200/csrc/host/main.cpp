@@ -1,6 +1,6 @@
 // inquistr-b200 -- C++ host CLI of the `inquiSTR` drop-in: the subcommand dispatch and the extension subcommands
-// `bgzf-check`, `baistat` and `bamstat`. `call` and `call-cohort` run in call_driver.cpp, `combine` and `outlier` in
-// cohort_cli.cpp. stdout carries only the output; diagnostics go to stderr, clap usage errors exit with code 2.
+// `bgzf-check`, `baistat` and `bamstat`. `call` and `call-cohort` run in call_driver.cpp, `combine`, `outlier` and
+// `assoc` in cohort_cli.cpp. stdout carries only the output; diagnostics go to stderr, clap usage errors exit with code 2.
 #include <algorithm>
 #include <chrono>
 #include <cstdio>
@@ -17,6 +17,7 @@ namespace inqhost {
 int call_main(const std::vector<std::string> &args, bool cohort, std::vector<int> devices);   // call_driver.cpp
 int combine_main(const std::vector<std::string> &files);                                    // cohort_cli.cpp
 int outlier_main(const std::vector<std::string> &args, int device);
+int assoc_main(const std::vector<std::string> &args, int device);
 }
 using namespace inqhost;
 
@@ -32,7 +33,9 @@ int main(int argc, char **argv)
                "Usage: inquistr-b200 <COMMAND>\n\nCommands:\n  call         Call lengths\n"
                "  call-cohort  Call lengths in several bams against one catalog and print the combined TSV\n"
                "  combine      Combine lengths from multiple bams to a TSV\n"
-               "  outlier      Find outliers from TSV\n  help         Print this message\n");
+               "  outlier      Find outliers from TSV\n"
+               "  assoc        Test every locus of a combined TSV for association with a phenotype\n"
+               "  help         Print this message\n");
         exit(v.empty() ? 2 : 0);
     }
     if (v[0] == "-V" || v[0] == "--version") { printf("inquistr-b200 %s\n", inq_version()); exit(0); }
@@ -130,7 +133,8 @@ int main(int argc, char **argv)
     const std::vector<std::string> rest(v.begin() + 1, v.end());
     if (v[0] == "combine") return combine_main(rest);
     if (v[0] == "outlier") return outlier_main(rest, devices[0]);
+    if (v[0] == "assoc") return assoc_main(rest, devices[0]);
     if (v[0] == "call" || v[0] == "call-cohort") return call_main(rest, v[0] == "call-cohort", devices);
     usage_error("inquistr-b200 call [OPTIONS] <BAM>",
-                "unrecognized subcommand '" + v[0] + "' (`call`, `call-cohort`, `combine` and `outlier` are implemented in this build)");
+                "unrecognized subcommand '" + v[0] + "' (`call`, `call-cohort`, `combine`, `outlier` and `assoc` are implemented in this build)");
 }

@@ -1,0 +1,307 @@
+// inq_assoc.cuh -- sm_100a kernel of `assoc`: per-locus linear / logistic regression of a trait on STR length.
+//
+// One warp per locus, four loci per CTA. The design is [1, covariates..., x] with x last (p <= 32 columns); lane j
+// owns row j of the (weighted) Gram matrix G and entry j of X'Wz, in f64 registers (P = p rounded up to 4, 8, 16 or
+// 32 is a template parameter, so the rows stay in registers). The CTA stages tiles of 32 samples of the design rows
+// shared by all loci (intercept + covariates, centred by their mean over the samples used) and of the trait in
+// shared memory, so the sample count is not bounded by shared memory. Lane l of a warp reads sample s0 + l of its
+// locus (two haplotype values), forms the predictor, and computes that sample's eta, mu, weight and working response;
+// the warp then walks the valid samples of the tile and every lane adds its row's terms.
+//
+// The predictor is centred per locus (mean over the samples used there), so the normal equations see centred
+// columns. The rank rule compares each elimination pivot d_j (the weighted residual sum of squares of column j
+// after the kept earlier columns, which centring does not change) with 1e-10 * G_jj of the UNcentred design.
+// Elimination is symmetric Gaussian elimination (LDL') without pivoting, one row per lane; an aliased column is
+// skipped (coefficient 0, rank - 1). With x last, (G^-1)_xx = 1 / d_x.
+//
+// Linear: pass 0 accumulates G (W = 1, z = y - mean y), solve, pass 1 sums the squared residuals.
+// Logistic (R's glm.fit without step-halving): pass t evaluates eta = X beta_t (t = 0: the start mu = (y + 1/2) / 2),
+// mu, the deviance of beta_t, and the weights / working response of the next solve, and accumulates that solve's G.
+// The warps of a CTA run their passes in lock step (the tiles are shared); a warp whose locus is done idles.
+#pragma once
+
+#include <cuda_runtime.h>
+#include <float.h>
+#include <stdint.h>
+
+#include "../../include/inqcohort.h"
+
+namespace inqa {
+
+constexpr int kAWarps = 4;                 // loci per CTA
+constexpr int kATile = 32;                 // samples per shared-memory tile
+constexpr int kAMaxIter = 25;              // glm.control(maxit = 25)
+constexpr double kAEpsilon = 1e-8;         // glm.control(epsilon = 1e-8)
+constexpr double kAAlias = 1e-10;          // pivot d_j <= kAAlias * G_jj: column j aliased
+
+// R's logit link (src/library/stats/src/family.c): THRESH = 30, MTHRESH = -30, INVEPS = 1 / DBL_EPSILON.
+// linkinv gives mu = t / (1 + t) and also 1 - mu = 1 / (1 + t): R forms 1 - mu by subtraction, which keeps only
+// eps / (1 - mu) of relative precision; for a misclassified sample near mu = 1 the IRLS term W (y - mu) / mu.eta is
+// of order 1 and would inherit that error (1e-8 at |eta| = 18). Same model, no cancellation.
+__host__ __device__ inline void logit_linkinv(double eta, double *mu, double *omu)
+{
+    const double t = eta < -30.0 ? DBL_EPSILON : (eta > 30.0 ? 1.0 / DBL_EPSILON : exp(eta));
+    *mu = t / (1.0 + t);
+    *omu = 1.0 / (1.0 + t);
+}
+__host__ __device__ inline double logit_mu_eta(double eta)
+{
+    const double opexp = 1.0 + exp(eta);
+    return (eta > 30.0 || eta < -30.0) ? DBL_EPSILON : exp(eta) / (opexp * opexp);
+}
+
+// regularised incomplete beta I_x(a, b), continued fraction (modified Lentz), f64
+__device__ inline double betacf(double a, double b, double x)
+{
+    const double tiny = 1e-300;
+    double c = 1.0, d = 1.0 - (a + b) * x / (a + 1.0);
+    if (fabs(d) < tiny) d = tiny;
+    d = 1.0 / d;
+    double h = d;
+    for (int m = 1; m <= 1000; ++m) {
+        const double m2 = 2.0 * m;
+        double aa = m * (b - m) * x / ((a + m2 - 1.0) * (a + m2));
+        d = 1.0 + aa * d; if (fabs(d) < tiny) d = tiny;
+        c = 1.0 + aa / c; if (fabs(c) < tiny) c = tiny;
+        d = 1.0 / d; h *= d * c;
+        aa = -(a + m) * (a + b + m) * x / ((a + m2) * (a + m2 + 1.0));
+        d = 1.0 + aa * d; if (fabs(d) < tiny) d = tiny;
+        c = 1.0 + aa / c; if (fabs(c) < tiny) c = tiny;
+        d = 1.0 / d;
+        const double del = d * c;
+        h *= del;
+        if (fabs(del - 1.0) < 1e-16) break;
+    }
+    return h;
+}
+__device__ inline double betai(double a, double b, double x)
+{
+    if (x <= 0.0) return 0.0;
+    if (x >= 1.0) return 1.0;
+    const double lf = lgamma(a + b) - lgamma(a) - lgamma(b) + a * log(x) + b * log1p(-x);
+    if (x < (a + 1.0) / (a + b + 2.0)) return exp(lf) * betacf(a, b, x) / a;
+    return 1.0 - exp(lf) * betacf(b, a, 1.0 - x) / b;
+}
+// two-sided p of Student t with df degrees of freedom
+__device__ inline double t_two_sided(double t, double df)
+{
+    if (t != t) return t;
+    return betai(0.5 * df, 0.5, df / (df + t * t));
+}
+
+__device__ __forceinline__ double warp_sum(double v)
+{
+#pragma unroll
+    for (int o = 16; o; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+    return v;
+}
+
+struct AssocOut {
+    double *beta, *se, *stat, *p;
+    uint32_t *n_used;
+    uint8_t *status, *n_iter;
+};
+
+// design: n_samples x P (row stride P): [1, centred covariates..., 0 (the slot of x), 0 padding]
+// shift : P column shifts (covariate means; 0 for the intercept and x), to rebuild the uncentred G_jj
+// y     : n_samples trait values (linear: centred by their mean)
+template <int P>
+__global__ void __launch_bounds__(kAWarps * 32)
+k_assoc(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_samples, uint32_t p, int logistic, int use_max,
+        const double *__restrict__ design, const double *__restrict__ shift, const double *__restrict__ y, AssocOut out)
+{
+    constexpr int S = P + 1;                              // odd row stride in doubles: lane-per-row reads spread over banks
+    __shared__ double s_des[kATile][S];
+    __shared__ double s_y[kATile];
+    __shared__ double s_beta[kAWarps][P];
+    const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const uint64_t row = (uint64_t)blockIdx.x * kAWarps + warp;
+    const bool have = row < n_rows;
+    const double2 *h = reinterpret_cast<const double2 *>(haps + (have ? row : 0) * 2ull * n_samples);
+    const uint32_t xcol = p - 1;
+
+    // pass A: samples used, mean of x, cases
+    double sx = 0.0, sy = 0.0;
+    uint32_t cnt = 0;
+    if (have)
+        for (uint32_t s = lane; s < n_samples; s += 32) {
+            const double2 v = h[s];
+            const double x = use_max ? fmax(v.x, v.y) : v.x + v.y;
+            if (x == x) { sx += x; sy += y[s]; ++cnt; }
+        }
+    uint32_t n = cnt;
+#pragma unroll
+    for (int o = 16; o; o >>= 1) n += __shfl_xor_sync(0xffffffffu, n, o);
+    const double xbar = n ? warp_sum(sx) / n : 0.0;
+    const double cases = warp_sum(sy);
+
+    uint8_t status = INQ_ASSOC_OK;
+    bool done = !have;
+    if (have && (n == 0 || (logistic && (cases == 0.0 || cases == (double)n)))) { status = INQ_ASSOC_FEW_SAMPLES; done = true; }
+    if (lane < P) s_beta[warp][lane] = 0.0;
+
+    const double my_shift = lane == xcol ? xbar : (lane < P ? shift[lane] : 0.0);
+    double beta_lane = 0.0, dx = 0.0, dev_old = 0.0;
+    int iter = 0, pass = 0, rank = 0;
+    for (;;) {
+        if (__syncthreads_and(done)) break;
+        // per-pass accumulators: row `lane` of G, X'Wz, uncentred G_jj; deviance / RSS and the separation test
+        double G[P];
+#pragma unroll
+        for (int k = 0; k < P; ++k) G[k] = 0.0;
+        double gx = 0.0, rhs = 0.0, diag = 0.0, dsum = 0.0;
+        bool sep_l = false;
+        const bool need_gram = !done && (logistic || pass == 0);
+        for (uint32_t s0 = 0; s0 < n_samples; s0 += kATile) {
+            __syncthreads();
+            for (uint32_t t = threadIdx.x; t < (uint32_t)kATile * P; t += blockDim.x) {
+                const uint32_t r = t / P, c = t % P, s = s0 + r;
+                s_des[r][c] = s < n_samples ? design[(uint64_t)s * P + c] : 0.0;
+            }
+            if (threadIdx.x < kATile) s_y[threadIdx.x] = s0 + threadIdx.x < n_samples ? y[s0 + threadIdx.x] : 0.0;
+            __syncthreads();
+            if (done) continue;
+            const uint32_t s = s0 + lane;
+            double xt = __longlong_as_double(0x7ff8000000000000ll);
+            if (s < n_samples) {
+                const double2 v = h[s];
+                xt = (use_max ? fmax(v.x, v.y) : v.x + v.y) - xbar;
+            }
+            const bool valid = xt == xt;
+            const double yl = s_y[lane];
+            // eta of this lane's sample under the current coefficients
+            double eta = 0.0;
+#pragma unroll
+            for (int k = 0; k < P; ++k) eta = fma(s_beta[warp][k], s_des[lane][k], eta);
+            eta = fma(s_beta[warp][xcol], xt, eta);     // the x slot of s_des is 0
+            double W = 1.0, z = yl;
+            if (logistic) {
+                if (pass == 0) {
+                    const double mu0 = (yl + 0.5) * 0.5;
+                    eta = log(mu0 / (1.0 - mu0));
+                }
+                double mu, omu;
+                logit_linkinv(eta, &mu, &omu);
+                const double me = logit_mu_eta(eta);
+                if (valid) {
+                    dsum += yl != 0.0 ? -2.0 * log(mu) : -2.0 * log(omu);
+                    sep_l |= mu < 10.0 * DBL_EPSILON || omu < 10.0 * DBL_EPSILON;
+                }
+                W = me * me / (mu * omu);
+                z = eta + (yl != 0.0 ? omu : -mu) / me;
+            } else if (pass == 1 && valid) {
+                const double r = yl - eta;
+                dsum = fma(r, r, dsum);
+            }
+            if (!need_gram) continue;
+            unsigned m = __ballot_sync(0xffffffffu, valid);
+            while (m) {
+                const int i = __ffs(m) - 1;
+                m &= m - 1;
+                const double xi = __shfl_sync(0xffffffffu, xt, i);
+                const double wi = __shfl_sync(0xffffffffu, W, i);
+                const double zi = __shfl_sync(0xffffffffu, z, i);
+                const double uj = lane == xcol ? xi : (lane < P ? s_des[i][lane < P ? lane : 0] : 0.0);
+                const double a = wi * uj;
+#pragma unroll
+                for (int k = 0; k < P; ++k) G[k] = fma(a, s_des[i][k], G[k]);
+                gx = fma(a, xi, gx);
+                rhs = fma(a, zi, rhs);
+                const double raw = uj + my_shift;
+                diag = fma(wi * raw, raw, diag);
+            }
+        }
+        if (!done) {
+            const double dev = warp_sum(dsum);             // deviance of the current coefficients (linear: RSS)
+            const bool any_sep = __any_sync(0xffffffffu, sep_l);
+            bool solve = true;
+            if (!logistic && pass == 1) {
+                // RSS known: t statistic
+                const double df = (double)n - rank;
+                const double sigma2 = dev / df;
+                const double se = sqrt(sigma2 / dx);
+                const double beta = __shfl_sync(0xffffffffu, beta_lane, xcol);
+                if (lane == 0) {
+                    const double t = beta / se;
+                    out.beta[row] = beta; out.se[row] = se; out.stat[row] = t; out.p[row] = t_two_sided(t, df);
+                }
+                done = true;
+                solve = false;
+            } else if (logistic && pass > 0) {
+                const double crit = fabs(dev - dev_old) / (fabs(dev) + 0.1);
+                if (crit < kAEpsilon || iter == kAMaxIter) {
+                    if (crit >= kAEpsilon) status = INQ_ASSOC_NO_CONVERGENCE;
+                    else if (any_sep) status = INQ_ASSOC_SEPARATION;
+                    const double se = sqrt(1.0 / dx);
+                    const double beta = __shfl_sync(0xffffffffu, beta_lane, xcol);
+                    if (lane == 0) {
+                        const double zs = beta / se;
+                        out.beta[row] = beta; out.se[row] = se; out.stat[row] = zs; out.p[row] = erfc(fabs(zs) * M_SQRT1_2);
+                    }
+                    done = true;
+                    solve = false;
+                }
+            }
+            dev_old = dev;
+            if (solve) {
+                // G[k] for the x column: gx; symmetric elimination, one row per lane
+#pragma unroll
+                for (int k = 0; k < P; ++k) if (k == (int)xcol) G[k] = gx;
+                uint32_t kept = 0;
+                int rk = 0;
+                double d_x = 0.0;
+#pragma unroll
+                for (int c = 0; c < P; ++c) {
+                    if (c >= (int)p) break;
+                    const double d = __shfl_sync(0xffffffffu, G[c], c);
+                    const double sc = __shfl_sync(0xffffffffu, diag, c);
+                    if (!(d > kAAlias * sc)) continue;          // aliased (or empty) column: dropped
+                    kept |= 1u << c;
+                    ++rk;
+                    if (c == (int)xcol) d_x = d;
+                    const double l = G[c] / d;
+                    const double bc = __shfl_sync(0xffffffffu, rhs, c);
+#pragma unroll
+                    for (int k = c + 1; k < P; ++k) {
+                        if (k >= (int)p) break;
+                        const double gck = __shfl_sync(0xffffffffu, G[k], c);
+                        if ((int)lane > c) G[k] = fma(-l, gck, G[k]);
+                    }
+                    if ((int)lane > c) rhs = fma(-l, bc, rhs);
+                }
+                double acc = 0.0, b = 0.0;
+#pragma unroll
+                for (int c = P - 1; c >= 0; --c) {
+                    if (c >= (int)p || !((kept >> c) & 1u)) continue;
+                    const double bc = __shfl_sync(0xffffffffu, (rhs - acc) / G[c], c);
+                    if ((int)lane == c) b = bc;
+                    if ((int)lane < c) acc = fma(G[c], bc, acc);
+                }
+                if (pass == 0) rank = rk;
+                if (pass == 0 && n <= (uint32_t)rk) { status = INQ_ASSOC_FEW_SAMPLES; done = true; }
+                else if (!((kept >> xcol) & 1u)) { status = INQ_ASSOC_SINGULAR; done = true; }
+                else {
+                    rank = rk;
+                    dx = d_x;
+                    beta_lane = b;
+                    __syncwarp();
+                    if (lane < P) s_beta[warp][lane] = b;
+                    __syncwarp();
+                    if (logistic) ++iter;
+                }
+            }
+        }
+        ++pass;
+    }
+    if (have && lane == 0) {
+        if (status == INQ_ASSOC_FEW_SAMPLES || status == INQ_ASSOC_SINGULAR) {
+            const double nan = __longlong_as_double(0x7ff8000000000000ll);
+            out.beta[row] = nan; out.se[row] = nan; out.stat[row] = nan; out.p[row] = nan;
+        }
+        out.n_used[row] = n;
+        out.status[row] = status;
+        if (out.n_iter) out.n_iter[row] = (uint8_t)iter;
+    }
+}
+
+}  // namespace inqa

@@ -1,14 +1,17 @@
 // inq_cohort_capi.cu -- extern "C" entry points of include/inqcohort.h (part of libinqcall.so)
 #include "../../include/inqcall.h"
 #include "../../include/inqcohort.h"
+#include "inq_assoc.cuh"
 #include "inq_cohort.cuh"
 
 #include <algorithm>
 #include <cstdarg>
 #include <cstdio>
 #include <cstdlib>
+#include <cmath>
 #include <cstring>
 #include <string>
+#include <vector>
 
 namespace {
 
@@ -161,6 +164,106 @@ int inq_outlier(int device, int method, uint64_t n_rows, uint32_t n_cols, const 
         std::sort(hits, hits + n);                            // (row, column) = the reference's print order
     }
     if (h.n_hits > cap) return cfail(INQ_ERR_HITS_CAP, "inq_outlier: %llu outliers, capacity %llu", (unsigned long long)h.n_hits, (unsigned long long)cap);
+    return INQ_OK;
+}
+
+int inq_assoc(int device, int model, int predictor, uint64_t n_rows, uint32_t n_samples, const double *haps,
+              const double *y, uint32_t n_cov, const double *cov, double *beta, double *se, double *stat, double *p,
+              uint32_t *n_used, uint8_t *status, uint8_t *n_iter, float *ms_kernel)
+{
+    using namespace inqa;
+    if (ms_kernel) *ms_kernel = 0.f;
+    if (model != INQ_ASSOC_LINEAR && model != INQ_ASSOC_LOGISTIC) return cfail(INQ_ERR_ARG, "inq_assoc: unknown model %d", model);
+    if (predictor != INQ_ASSOC_SUM && predictor != INQ_ASSOC_MAX) return cfail(INQ_ERR_ARG, "inq_assoc: unknown predictor %d", predictor);
+    if (n_cov > INQ_ASSOC_MAX_COV) return cfail(INQ_ERR_ARG, "inq_assoc: %u covariates (at most %d)", n_cov, INQ_ASSOC_MAX_COV);
+    if (n_rows == 0) return INQ_OK;
+    if (n_samples == 0) return cfail(INQ_ERR_ARG, "inq_assoc: no samples");
+    if (!haps || !y || (n_cov && !cov) || !beta || !se || !stat || !p || !n_used || !status) return cfail(INQ_ERR_ARG, "inq_assoc: NULL array");
+    if ((n_rows + kAWarps - 1) / kAWarps > 0x7FFFFFFFull) return cfail(INQ_ERR_TOO_LARGE, "inq_assoc: too many rows");
+    for (uint32_t s = 0; s < n_samples; ++s) {
+        if (!std::isfinite(y[s])) return cfail(INQ_ERR_ARG, "inq_assoc: trait of sample %u is not a finite number", s);
+        if (model == INQ_ASSOC_LOGISTIC && y[s] != 0.0 && y[s] != 1.0) return cfail(INQ_ERR_ARG, "inq_assoc: logistic trait of sample %u is not 0 or 1", s);
+        for (uint32_t c = 0; c < n_cov; ++c)
+            if (!std::isfinite(cov[(size_t)s * n_cov + c])) return cfail(INQ_ERR_ARG, "inq_assoc: covariate %u of sample %u is not a finite number", c, s);
+    }
+    const uint32_t pdim = n_cov + 2;
+    const int P = pdim <= 4 ? 4 : pdim <= 8 ? 8 : pdim <= 16 ? 16 : 32;
+    // shared design rows [1, covariates centred by their mean, 0 (x), 0 ...]; the linear trait centred by its mean
+    std::vector<double> design((size_t)n_samples * P, 0.0), shift(P, 0.0), yc(y, y + n_samples);
+    for (uint32_t c = 0; c < n_cov; ++c) {
+        double m = 0.0;
+        for (uint32_t s = 0; s < n_samples; ++s) m += cov[(size_t)s * n_cov + c];
+        shift[1 + c] = m / n_samples;
+    }
+    for (uint32_t s = 0; s < n_samples; ++s) {
+        design[(size_t)s * P] = 1.0;
+        for (uint32_t c = 0; c < n_cov; ++c) design[(size_t)s * P + 1 + c] = cov[(size_t)s * n_cov + c] - shift[1 + c];
+    }
+    if (model == INQ_ASSOC_LINEAR) {
+        double m = 0.0;
+        for (uint32_t s = 0; s < n_samples; ++s) m += y[s];
+        m /= n_samples;
+        for (double &v : yc) v -= m;
+    }
+
+    CC_TRY(cudaSetDevice(device));
+    struct AGuard {
+        std::vector<void *> p;
+        cudaStream_t s = nullptr;
+        cudaEvent_t e0 = nullptr, e1 = nullptr;
+        ~AGuard()
+        {
+            for (void *q : p) cudaFree(q);
+            if (e0) cudaEventDestroy(e0);
+            if (e1) cudaEventDestroy(e1);
+            if (s) cudaStreamDestroy(s);
+        }
+    } g;
+    auto dalloc = [&](void **q, size_t bytes) -> cudaError_t {
+        const cudaError_t e = cudaMalloc(q, bytes);
+        if (e == cudaSuccess) g.p.push_back(*q);
+        return e;
+    };
+    CC_TRY(cudaStreamCreateWithFlags(&g.s, cudaStreamNonBlocking));
+    CC_TRY(cudaEventCreate(&g.e0));
+    CC_TRY(cudaEventCreate(&g.e1));
+    const size_t hap_bytes = (size_t)n_rows * 2 * n_samples * sizeof(double);
+    void *d_haps, *d_des, *d_shift, *d_y, *d_res, *d_n, *d_st, *d_it;
+    CC_TRY(dalloc(&d_haps, hap_bytes));
+    CC_TRY(dalloc(&d_des, design.size() * sizeof(double)));
+    CC_TRY(dalloc(&d_shift, shift.size() * sizeof(double)));
+    CC_TRY(dalloc(&d_y, n_samples * sizeof(double)));
+    CC_TRY(dalloc(&d_res, (size_t)n_rows * 4 * sizeof(double)));
+    CC_TRY(dalloc(&d_n, (size_t)n_rows * sizeof(uint32_t)));
+    CC_TRY(dalloc(&d_st, (size_t)n_rows));
+    CC_TRY(dalloc(&d_it, (size_t)n_rows));
+    CC_TRY(cudaMemcpyAsync(d_haps, haps, hap_bytes, cudaMemcpyHostToDevice, g.s));
+    CC_TRY(cudaMemcpyAsync(d_des, design.data(), design.size() * sizeof(double), cudaMemcpyHostToDevice, g.s));
+    CC_TRY(cudaMemcpyAsync(d_shift, shift.data(), shift.size() * sizeof(double), cudaMemcpyHostToDevice, g.s));
+    CC_TRY(cudaMemcpyAsync(d_y, yc.data(), n_samples * sizeof(double), cudaMemcpyHostToDevice, g.s));
+    double *r = (double *)d_res;
+    const AssocOut out{r, r + n_rows, r + 2 * n_rows, r + 3 * n_rows, (uint32_t *)d_n, (uint8_t *)d_st, (uint8_t *)d_it};
+    const unsigned grid = (unsigned)((n_rows + kAWarps - 1) / kAWarps);
+    const int lg = model == INQ_ASSOC_LOGISTIC, mx = predictor == INQ_ASSOC_MAX;
+    const double *dh = (const double *)d_haps, *dd = (const double *)d_des, *ds = (const double *)d_shift, *dy = (const double *)d_y;
+    CC_TRY(cudaEventRecord(g.e0, g.s));
+    switch (P) {
+    case 4: k_assoc<4><<<grid, kAWarps * 32, 0, g.s>>>(dh, n_rows, n_samples, pdim, lg, mx, dd, ds, dy, out); break;
+    case 8: k_assoc<8><<<grid, kAWarps * 32, 0, g.s>>>(dh, n_rows, n_samples, pdim, lg, mx, dd, ds, dy, out); break;
+    case 16: k_assoc<16><<<grid, kAWarps * 32, 0, g.s>>>(dh, n_rows, n_samples, pdim, lg, mx, dd, ds, dy, out); break;
+    default: k_assoc<32><<<grid, kAWarps * 32, 0, g.s>>>(dh, n_rows, n_samples, pdim, lg, mx, dd, ds, dy, out); break;
+    }
+    CC_TRY(cudaGetLastError());
+    CC_TRY(cudaEventRecord(g.e1, g.s));
+    CC_TRY(cudaMemcpyAsync(beta, r, n_rows * sizeof(double), cudaMemcpyDeviceToHost, g.s));
+    CC_TRY(cudaMemcpyAsync(se, r + n_rows, n_rows * sizeof(double), cudaMemcpyDeviceToHost, g.s));
+    CC_TRY(cudaMemcpyAsync(stat, r + 2 * n_rows, n_rows * sizeof(double), cudaMemcpyDeviceToHost, g.s));
+    CC_TRY(cudaMemcpyAsync(p, r + 3 * n_rows, n_rows * sizeof(double), cudaMemcpyDeviceToHost, g.s));
+    CC_TRY(cudaMemcpyAsync(n_used, d_n, n_rows * sizeof(uint32_t), cudaMemcpyDeviceToHost, g.s));
+    CC_TRY(cudaMemcpyAsync(status, d_st, n_rows, cudaMemcpyDeviceToHost, g.s));
+    if (n_iter) CC_TRY(cudaMemcpyAsync(n_iter, d_it, n_rows, cudaMemcpyDeviceToHost, g.s));
+    CC_TRY(cudaStreamSynchronize(g.s));
+    if (ms_kernel) cudaEventElapsedTime(ms_kernel, g.e0, g.e1);
     return INQ_OK;
 }
 

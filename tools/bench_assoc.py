@@ -1,0 +1,139 @@
+#!/usr/bin/env python
+"""Measures `assoc` (include/inqcohort.h inq_assoc) at the scale the reference's R script reports: 654,000 loci x 268
+samples, 12 covariates, 10 % missing calls, about 20 % constant loci, seeded. Prints one JSON line per model x
+predictor with the kernel time (CUDA events, H2D excluded; median of --reps runs after a warm-up), loci/s, the f64
+FMAs the fits need (from shapes and iteration counts) and GFLOP/s, and parity of --parity random loci against the
+numpy restatement (oracle/assoc.py, not R) with its host time. Then one line per model for the CLI on the same table
+written as TSV: wall time with text parse, device and output time separated (`--stats-json`). The card's name and
+power limit are read in the same run. Temporary files go to a temporary directory."""
+import argparse
+import json
+import os
+import subprocess
+import sys
+import tempfile
+import time
+
+import numpy as np
+
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
+
+
+def card():
+    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader"], capture_output=True, text=True)
+    return q.stdout.strip().splitlines()[0] if q.returncode == 0 and q.stdout.strip() else "unknown"
+
+
+def workload(rows, samples, n_cov, seed=2024):
+    rng = np.random.default_rng(seed)
+    haps = np.round(rng.gamma(2.0, 12.0, (rows, 2 * samples)) * 2) / 2
+    big = rng.random(haps.shape) < 0.02
+    haps[big] = np.round(rng.pareto(1.5, big.sum()) * 100 + 100)    # heavy tail: expansions
+    haps = np.minimum(haps, 3000.0)
+    haps[rng.random(rows) < 0.2] = 30.0                                # constant loci
+    haps[rng.random(haps.shape) < 0.1] = np.nan
+    cov = np.empty((samples, n_cov))
+    for c in range(n_cov):
+        cov[:, c] = rng.normal(50, 15, samples) if c == 0 else (rng.integers(0, 2, samples) if c == 1 else rng.normal(0, 1, samples))
+    y_lin = 3 + 0.01 * cov[:, 0] + rng.normal(size=samples)
+    y_bin = (rng.random(samples) < 0.4).astype(float)
+    return haps, cov, y_lin, y_bin
+
+
+def fmas(res, p, model):
+    """f64 FMAs of the passes over the samples, n samples used and p design columns per locus:
+    linear   one Gram pass, n * (p^2 + p) for G and X'y, and one residual pass, n * p for eta: n * (p^2 + 2p);
+    logistic n_iter + 1 passes, each n * p for eta and n * (p^2 + p) for G and X'Wz (the last pass's G is accumulated
+             and not solved): (n_iter + 1) * n * (p^2 + 2p).
+    few_samples loci (no solve) count nothing; the elimination (about p^3 / 3 per solve) is small next to these."""
+    n = res["n"].astype(np.float64)
+    fit = res["status"] != 1                                           # few_samples
+    if model == "linear":
+        return float(np.sum(n[fit] * (p * p + 2 * p)))
+    passes = res["n_iter"].astype(np.float64) + 1
+    return float(np.sum(n[fit] * passes[fit] * (p * p + 2 * p)))
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--rows", type=int, default=654_000)
+    ap.add_argument("--samples", type=int, default=268)
+    ap.add_argument("--cov", type=int, default=12)
+    ap.add_argument("--reps", type=int, default=5)
+    ap.add_argument("--parity", type=int, default=2000)
+    ap.add_argument("--no-cli", action="store_true")
+    args = ap.parse_args()
+    from inquistr_b200 import cohort
+    from oracle import assoc as A
+    name = card()
+    haps, cov, y_lin, y_bin = workload(args.rows, args.samples, args.cov)
+    p = args.cov + 2
+    sel = np.sort(np.random.default_rng(7).choice(args.rows, min(args.parity, args.rows), replace=False))
+    for model in ("linear", "logistic"):
+        y = y_lin if model == "linear" else y_bin
+        for pred in ("sum", "max"):
+            res = cohort.assoc(haps, y, cov, model, pred)                # warm-up
+            ms = []
+            for _ in range(args.reps):
+                res = cohort.assoc(haps, y, cov, model, pred)
+                ms.append(res["ms_kernel"])
+            med = float(np.median(ms))
+            f = fmas(res, p, model)
+            t0 = time.perf_counter()
+            ref = A.assoc_matrix(haps[sel], y, cov, model, pred)
+            oracle_s = time.perf_counter() - t0
+            st = res["status"][sel]
+            ok = (ref["status"] == A.OK) & (st == A.OK)
+            if model == "logistic":
+                ok &= res["n_iter"][sel] == ref["n_iter"]
+            rb = np.abs(res["beta"][sel][ok] - ref["beta"][ok]) / (np.abs(ref["beta"][ok]) + ref["se"][ok])
+            rs = np.abs(res["se"][sel][ok] / ref["se"][ok] - 1)
+            lp = np.abs(np.log10(np.maximum(res["p"][sel][ok], 1e-300)) - np.log10(np.maximum(ref["p"][ok], 1e-300)))
+            print(json.dumps({
+                "bench": "assoc_kernel", "card": name, "model": model, "predictor": pred, "loci": args.rows,
+                "samples": args.samples, "covariates": args.cov, "kernel_ms_median": med, "kernel_ms_all": ms,
+                "loci_per_s": args.rows / (med * 1e-3), "f64_fma": f, "gflops": 2 * f / (med * 1e-3) / 1e9,
+                "status_counts": {A.STATUS_NAMES[k]: int((res["status"] == k).sum()) for k in range(5)},
+                "mean_iterations": float(res["n_iter"][res["status"] != 1].mean()) if model == "logistic" else 0.0,
+                "parity": {"loci": int(len(sel)), "status_equal": bool(np.array_equal(st, ref["status"])),
+                           "iter_equal": bool(np.array_equal(res["n_iter"][sel], ref["n_iter"])),
+                           "compared": int(ok.sum()), "max_beta_err_rel_to_abs_beta_plus_se": float(rb.max()) if ok.any() else None,
+                           "max_se_rel_err": float(rs.max()) if ok.any() else None, "max_dlog10_p": float(lp.max()) if ok.any() else None},
+                "numpy_oracle_s": oracle_s, "numpy_oracle_loci_per_s": len(sel) / oracle_s}), flush=True)
+    if args.no_cli:
+        return
+    from inquistr_b200 import build
+    exe = os.path.join(os.path.dirname(build.__file__), "bin", "inquistr-b200")
+    with tempfile.TemporaryDirectory() as d:
+        samples = [f"S{i}" for i in range(args.samples)]
+        lut = np.array([f"{v / 2:g}" for v in range(0, 6001)] + ["NaN"], dtype=object)
+        idx = np.where(np.isnan(haps), 6001, np.nan_to_num(haps * 2).astype(np.int64))
+        t0 = time.perf_counter()
+        table = os.path.join(d, "cohort.tsv")
+        with open(table, "w") as f:
+            f.write("chromosome\tbegin\tend\t" + "\t".join(f"{s}_H1\t{s}_H2" for s in samples) + "\n")
+            for i in range(args.rows):
+                f.write(f"chr{1 + i // 30000}\t{1000 + 100 * i}\t{1040 + 100 * i}\t" + "\t".join(lut[idx[i]]) + "\n")
+        write_s = time.perf_counter() - t0
+        ph = os.path.join(d, "pheno.tsv")
+        with open(ph, "w") as f:
+            f.write("sample\tlin\tbin\t" + "\t".join(f"c{c}" for c in range(args.cov)) + "\n")
+            for i, s in enumerate(samples):
+                f.write(f"{s}\t{float(y_lin[i])!r}\t{int(y_bin[i])}\t" + "\t".join(repr(float(v)) for v in cov[i]) + "\n")
+        for model, trait in (("linear", "lin"), ("logistic", "bin")):
+            sj = os.path.join(d, "stats.json")
+            t0 = time.perf_counter()
+            r = subprocess.run([exe, "assoc", "--phenotype", ph, "--trait", trait, "--model", model, "--covariates",
+                                ",".join(f"c{c}" for c in range(args.cov)), "--stats-json", sj, table],
+                               stdout=subprocess.PIPE, stderr=subprocess.PIPE)
+            wall = time.perf_counter() - t0
+            st = json.load(open(sj)) if r.returncode == 0 else {}
+            out_rows = r.stdout.count(b"\n") - 1
+            print(json.dumps({"bench": "assoc_cli", "card": name, "model": model, "predictor": "sum", "rc": r.returncode,
+                              "table_bytes": os.path.getsize(table), "table_write_s": write_s, "wall_s": wall,
+                              "rows_out": out_rows, **st, "stderr_tail": r.stderr.decode()[-300:]}), flush=True)
+
+
+if __name__ == "__main__":
+    main()
