@@ -77,16 +77,16 @@ typedef struct inq_stats {
     float ms_total;              /* start of the pass -> everything done, results in host memory */
     float ms_index;              /* memsets */
     float ms_join;               /* K1 read x locus overlap join + segment offsets (second stream, under K2) */
-    float ms_cigar;              /* K2 CIGAR scan (dominant kernel), summed over the ranges of the pass */
-    float ms_fixup;              /* prefix scans over the warp-tile totals, summed over the ranges */
-    float ms_scan;               /* tail: last range scanned -> end of the pass (what the overlap does not hide) */
-    float ms_pairs;              /* K2b event staging, per-pair window sums, scatter into buckets (runs under K2 of the next range) */
+    float ms_cigar;              /* K2 CIGAR scan (dominant kernel) */
+    float ms_fixup;              /* CIGAR scan done -> K2b start: prefix scan over the warp-tile totals (and any wait for K1) */
+    float ms_scan;               /* tail: CIGAR stream scanned -> end of the pass (what the overlap does not hide) */
+    float ms_pairs;              /* K2b event staging, per-pair window sums, scatter into buckets */
     float ms_median;             /* K3 per-locus sort / support filter / median: first chunk start -> last chunk end */
     float ms_h2d;                /* host->device copies of the last inq_push_reads */
     float ms_d2h;                /* last median chunk done -> last result copy done */
-    uint32_t n_ranges;           /* ranges the CIGAR stream was scanned in (pair/median work of range k runs under scan k+1) */
+    uint32_t n_ranges;           /* always 1: the CIGAR stream is scanned in one launch (kept for the layout) */
     uint32_t used_graph;         /* 1: the pass was replayed from a captured CUDA graph */
-    uint32_t reads_sorted;       /* 1: reads were pushed in (contig, ref_start) order: finished loci are reduced and copied early */
+    uint32_t reads_sorted;       /* 1: reads were pushed in (contig, ref_start) order */
     uint32_t n_median_chunks;
 } inq_stats;
 
@@ -97,23 +97,12 @@ const char *inq_last_error(const inq_ctx *ctx);   /* ctx may be NULL: message of
 const char *inq_version(void);
 
 /*
- * Tuning knobs (all optional; the defaults are what bench.py measures). Returns INQ_ERR_ARG for an
- * unknown name or a value out of range.
- *   "ranges"          number of ranges the CIGAR stream is scanned in (0 = automatic, max 16)
- *   "max_ranges"      upper bound of the automatic choice (default 1: one scan launch; ranges > 1 let the
- *                     pair / median kernels of a range run next to the scan of the following one)
- *   "min_range_tiles" automatic choice: at least this many 4 KB warp tiles per range (default 65536)
+ * Options (both optional; the defaults are what bench.py measures). Returns INQ_ERR_ARG for any other
+ * name or a value out of range.
  *   "graph"           1 (default): replay the steady state from a CUDA graph; 0: always launch directly
  *   "timing"          1 (default): three CUDA event records per pass -> inq_stats.ms_total, ms_cigar, ms_scan;
  *                     2: one per stage as well -> every inq_stats.ms_* (each record is a node of the replayed graph
  *                     and costs ~5 us on the chain: ~50 us per pass); 0: none
- *   "push_kernel"     1 (default): a chunk's results are stored into the caller's pinned arrays by a kernel;
- *                     0: three copy-engine operations per chunk
- *   "push_ctas"       CTAs of that kernel (default 8: its stores are PCIe-bound)
- *   "join_coop"       1 (default): k_join_ranges finds a warp's lower bounds together; 0: two binary searches per read
- *   "evict_first"     1 (default): k_cigar_scan loads the stream with the L2 evict-first policy
- *   "median_pieces"   median chunks per pass (default 12; the transfer of one runs under the medians of the next)
- *   "min_piece"       ... but no chunk smaller than this many loci (default 65536)
  */
 int inq_set_option(inq_ctx *ctx, const char *name, int64_t value);
 

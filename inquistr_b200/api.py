@@ -178,8 +178,7 @@ class Context:
         self.n_loci = len(s)
 
     def set_option(self, name: str, value: int):
-        """inq_set_option: "ranges", "max_ranges", "min_range_tiles", "graph", "timing" (0/1/2), "push_kernel", "push_ctas",
-        "join_coop", "evict_first", "median_pieces", "min_piece" (include/inqcall.h)."""
+        """inq_set_option: "graph" (0/1) or "timing" (0/1/2) (include/inqcall.h)."""
         self._check(self._lib.inq_set_option(self._h, name.encode(), int(value)))
 
     def reserve_reads(self, n_reads, n_words):

@@ -3,12 +3,11 @@
 // No CPU implementation of the hot path lives here: without a CUDA device every entry fails.
 //
 // One genotyping pass is a small DAG over four streams (DESIGN.md section 3b):
-//   S0  counter memset, k_cigar_scan(k) per range k of the CIGAR stream; with one range (the default) also the prefix
-//       sum over its warp-tile totals (k_exclusive_scan2)
-//   S1  k_zero, k_join_ranges + two offset scans (next to scan(0)), then -- with several ranges k_exclusive_scan2(k)
-//       and -- k_pair_eval(k) as soon as range k is scanned
-//   S2  k_locus_median (+ the CTA-path kernel where the last pass had deep loci) over the catalog chunk that became
-//       complete with pair(k); the counters go home from here
+//   S0  counter memset, k_cigar_scan over the whole CIGAR stream, then the prefix sum over its warp-tile totals
+//       (k_exclusive_scan2)
+//   S1  k_zero, k_join_ranges + two offset scans (next to the CIGAR scan), then k_pair_eval once S0 is done
+//   S2  k_locus_median (+ the CTA-path kernel where the last pass had deep loci) per catalog chunk; the counters go
+//       home from here
 //   S3  k_push_results: finished chunks stored into the caller's pinned arrays (copy engines when they are not mapped)
 // The steady state (same reads, same parameters, same pinned outputs) is replayed from a CUDA graph; the first call
 // of a shape and every retry (speculative buffer regrown, CTA-path guess wrong) launch the same DAG directly.
@@ -25,17 +24,6 @@
 #include <vector>
 
 using namespace inq;
-
-// shape of the pass (compile-time; the defaults are what the sweeps in profiles/README.md picked)
-#ifndef INQ_STREAM_PRIORITIES
-#define INQ_STREAM_PRIORITIES 1       // bit i: stream Si is high priority
-#endif
-#ifndef INQ_SCAN_FIRST
-#define INQ_SCAN_FIRST 0              // 1: enqueue the scan kernels before the join chain
-#endif
-#ifndef INQ_BIG_ON_S3
-#define INQ_BIG_ON_S3 0               // 1: CTA-path medians run on the copy stream instead of between two chunks
-#endif
 
 namespace {
 
@@ -110,33 +98,26 @@ struct VmStream {
 };
 
 enum {
-    EV_START = 0, EV_END, EV_INDEX, EV_JOIN0, EV_JOIN, EV_MED0, EV_MED1, EV_D2H, EV_H2D0, EV_H2D1,
-    EV_SCAN0,                                   // + 2k, 2k+1: start / end of k_cigar_scan(k)
-    EV_XS0 = EV_SCAN0 + 2 * kMaxRanges,         // + 2k, 2k+1: start / end of k_exclusive_scan2(k)
-    EV_PAIR0 = EV_XS0 + 2 * kMaxRanges,         // + 2k, 2k+1: start / end of k_pair_eval(k)
-    EV_COUNT = EV_PAIR0 + 2 * kMaxRanges
+    EV_START = 0, EV_END, EV_INDEX, EV_JOIN, EV_MED0, EV_MED1, EV_D2H, EV_H2D0, EV_H2D1,
+    EV_SCAN0, EV_SCAN1,                         // start / end of k_cigar_scan
+    EV_PAIR0, EV_PAIR1,                         // start / end of k_pair_eval
+    EV_COUNT
 };
 // dependency-only events (no timing)
 enum {
-    DEP_FORK = 0, DEP_JOIN_DONE, DEP_S1_DONE, DEP_S2_DONE, DEP_S3_DONE, DEP_ZEROED, DEP_SCAN_ONLY,
-    DEP_SCANNED,                                // + k: range k scanned
-    DEP_PAIRED = DEP_SCANNED + kMaxRanges,      // + k: pair(k) done
-    DEP_CHUNK = DEP_PAIRED + kMaxRanges,        // + c: median chunk c done
+    DEP_FORK = 0, DEP_JOIN_DONE, DEP_S1_DONE, DEP_S2_DONE, DEP_S3_DONE, DEP_ZEROED, DEP_SCAN_ONLY, DEP_SCANNED, DEP_PAIRED,
+    DEP_CHUNK,                                  // + c: median chunk c done
     DEP_COUNT = DEP_CHUNK + kMaxMedianChunks
 };
 
 struct MedianChunk {
     uint32_t l0, l1;
-    int after_range;                            // runs once pair(after_range) is done
 };
 
-// How the pass is cut up; rebuilt whenever the reads or the catalog change.
+// How the medians are cut up; rebuilt whenever the reads or the catalog change.
 struct Plan {
     bool valid = false;
     uint64_t data_gen = 0;
-    int K = 1;
-    uint64_t tile_end[kMaxRanges + 1] = {};     // warp-tile boundaries, tile_end[0] = 0
-    uint64_t read_end[kMaxRanges + 1] = {};     // reads [read_end[k], read_end[k+1]) are evaluated after range k
     int n_chunks = 0;
     MedianChunk chunk[kMaxMedianChunks];
     bool reads_sorted = false;
@@ -159,13 +140,6 @@ struct GraphKey {
     }
 };
 
-struct ProbeOut {                               // k_plan_probe result per range boundary
-    uint32_t read_end;
-    uint32_t contig;                            // of read `read_end` (0xFFFFFFFF if none)
-    int32_t ref_start;
-    uint32_t pad;
-};
-
 }  // namespace
 
 struct inq_ctx {
@@ -176,30 +150,18 @@ struct inq_ctx {
     cudaStream_t stream_join = nullptr;   // S1: join, pair evaluation
     cudaStream_t stream_med = nullptr;    // S2: medians
     cudaStream_t stream_copy = nullptr;   // S3: result copies
-    uint32_t scan_debug = 0, pair_debug = 0;     // only honoured by builds with -DINQ_TIMING_EXPERIMENTS
     std::string err;
 
     // options (inq_set_option)
-    int opt_ranges = 0;                   // 0 = automatic
-    int64_t opt_min_range_tiles = 64 * 1024;
-    int opt_max_ranges = 1;               // measured (profiles/README.md, r2 sweeps): co-scheduling pair/median CTAs under the scan is zero-sum on B200
     int opt_graph = 1;
     int opt_timing = 1;
-    int opt_median_pieces = 12;       // median chunks per pass (the last one is a quarter piece)
-    int64_t opt_min_piece = 1 << 16;  // ... but no piece smaller than this many loci
-    unsigned long long *join_trace = nullptr;   // experiments (INQ_JOIN_TRACE=file): per-CTA start / end / SM of k_join_ranges
-    uint64_t join_trace_ctas = 0;
-    int opt_evict_first = 1;          // k_cigar_scan loads the stream with the L2 evict-first policy
-    int opt_join_coop = 1;            // k_join_ranges: warp-cooperative lower bounds (0: two scalar binary searches per read)
-    int opt_push_ctas = 8;            // CTAs of k_push_results (PCIe-bound stores: a few SMs' worth is plenty)
-    int opt_push_kernel = 1;          // results leave through k_push_results (0: three copy-engine operations per chunk)
 
     // locus catalog
     int32_t n_contigs = 0;
     int64_t L = 0;
     DevBuf<int64_t> contig_off;
     DevBuf<int32_t> lstart, lend, lpmax;
-    std::vector<int64_t> h_contig_off;    // host copies for the plan (which loci are complete after which read)
+    std::vector<int64_t> h_contig_off;    // host copies for inq_push_reads_routed (which reads can reach a locus)
     std::vector<int32_t> h_pmax, h_lstart;
     void *h_route_stage = nullptr;        // pinned staging of inq_push_reads_routed when the kept reads are scattered
 
@@ -228,8 +190,6 @@ struct inq_ctx {
     DevCounters *d_ctr = nullptr;
     DevCounters *h_ctr = nullptr;     // pinned
     uint32_t *h_total = nullptr;      // pinned
-    ProbeOut *d_probe = nullptr, *h_probe = nullptr;
-    uint64_t *d_probe_tiles = nullptr;
     void *h_stage = nullptr;          // pinned staging of the results when the caller's arrays are pageable
     size_t h_stage_bytes = 0;
 
@@ -448,6 +408,8 @@ __device__ __forceinline__ void push_bytes(unsigned char *__restrict__ dst, cons
     if (tid < n - tail0) dst[tail0 + tid] = src[tail0 + tid];
 }
 
+constexpr unsigned kPushCtas = 8;     // the stores are PCIe-bound: a few SMs' worth is plenty
+
 __global__ void __launch_bounds__(256)
 k_push_results(uint32_t l0, uint32_t l1, const int64_t *__restrict__ t1, const int64_t *__restrict__ t2, const uint8_t *__restrict__ valid,
                int64_t *__restrict__ o1, int64_t *__restrict__ o2, uint8_t *__restrict__ ov)
@@ -468,25 +430,6 @@ __global__ void k_zero(ZeroJobs jobs)
     }
 }
 
-// per range boundary k: the first read that is NOT entirely inside warp tiles [0, tile_end[k]) and where it starts
-__global__ void k_plan_probe(const uint32_t *__restrict__ tile_first, const uint64_t *__restrict__ tile_end, int K, uint64_t R,
-                             const int32_t *__restrict__ contig, const int32_t *__restrict__ rs, ProbeOut *__restrict__ out)
-{
-    const int k = threadIdx.x;
-    if (k >= K) return;
-    // tile_first[t] = first entry of cig_off[0, R] that is >= t * kWarpTileWords: every read before entry f - 1 has
-    // its end (= the next read's start) below the boundary
-    const uint32_t f = tile_first[tile_end[k]];
-    uint64_t b = f ? f - 1u : 0u;
-    if (b > R) b = R;
-    ProbeOut o;
-    o.read_end = (uint32_t)b;
-    o.contig = b < R ? (uint32_t)contig[b] : 0xFFFFFFFFu;
-    o.ref_start = b < R ? rs[b] : 0;
-    o.pad = 0;
-    out[k] = o;
-}
-
 struct RunParams {
     uint32_t minlen, support;
     int unphased;
@@ -497,76 +440,57 @@ struct RunParams {
     uint8_t *dv = nullptr;
 };
 
-// Cut the pass into ranges (see the file header). Needs one small device read-back, so it is cached until
-// the reads or the catalog change.
-int build_plan(inq_ctx *ctx, uint64_t n_wt)
+// The medians run in catalog chunks so that the transfer of one runs under the medians of the next; the very last
+// chunk is small (its transfer is the exposed one). profiles/r2_sweep_median_pieces.jsonl: flat within 1 % around these.
+constexpr int64_t kMedianPieces = 12;     // median chunks per pass
+constexpr int64_t kMinPiece = 1 << 16;    // ... but no chunk smaller than this many loci (the last one: a quarter of it)
+
+// Cut the catalog into median chunks and read whether the reads are sorted. Needs one small device read-back, so it is
+// cached until the reads or the catalog change.
+int build_plan(inq_ctx *ctx)
 {
     Plan &pl = ctx->plan;
     if (pl.valid && pl.data_gen == ctx->data_gen) return INQ_OK;
     pl = Plan();
-    const uint64_t R = ctx->R;
     const int64_t L = ctx->L;
-    int K = ctx->opt_ranges > 0 ? ctx->opt_ranges
-                                : (int)std::min<uint64_t>((uint64_t)ctx->opt_max_ranges, n_wt / (uint64_t)std::max<int64_t>(1, ctx->opt_min_range_tiles));
-    K = std::max(1, std::min(K, kMaxRanges));
-    if ((uint64_t)K > n_wt) K = (int)std::max<uint64_t>(1, n_wt);
-    pl.K = K;
-    for (int k = 0; k <= K; ++k) pl.tile_end[k] = n_wt * (uint64_t)k / (uint64_t)K;
-    pl.read_end[0] = 0;
-    pl.read_end[K] = R;
-    std::vector<int64_t> done(K + 1, 0);
-    done[K] = L;
-    if (R && L) {
+    if (ctx->R && L) {
         cudaStream_t s = ctx->stream;
-        if (K > 1) {
-            CU_TRY(ctx, cudaMemcpyAsync(ctx->d_probe_tiles, pl.tile_end + 1, (K - 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
-            k_plan_probe<<<1, 32, 0, s>>>(ctx->tile_first.p, ctx->d_probe_tiles, K - 1, R, ctx->contig.p, ctx->rs.p, ctx->d_probe);
-            CU_TRY(ctx, cudaGetLastError());
-            CU_TRY(ctx, cudaMemcpyAsync(ctx->h_probe, ctx->d_probe, (K - 1) * sizeof(ProbeOut), cudaMemcpyDeviceToHost, s));
-        }
         CU_TRY(ctx, cudaMemcpyAsync(ctx->h_total + 8, ctx->d_unsorted, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
         CU_TRY(ctx, cudaStreamSynchronize(s));
         pl.reads_sorted = ctx->h_total[8] == 0;
-        for (int k = 1; k < K; ++k) {
-            const ProbeOut &o = ctx->h_probe[k - 1];
-            pl.read_end[k] = std::max<uint64_t>(pl.read_end[k - 1], std::min<uint64_t>(o.read_end, R));
-            // Sorted reads: every read from read_end[k] on starts at (o.contig, o.ref_start) or later, so a locus whose
-            // running max of end (+10) lies at or before that start cannot be a candidate of any of them
-            // (k_join_ranges / candidate_range): its calls are complete once pair(k - 1) is done.
-            int64_t d = 0;
-            if (pl.reads_sorted) {
-                if (o.contig >= (uint32_t)ctx->n_contigs) d = L;
-                else {
-                    const int64_t a = ctx->h_contig_off[o.contig], b = ctx->h_contig_off[o.contig + 1];
-                    d = std::upper_bound(ctx->h_pmax.begin() + a, ctx->h_pmax.begin() + b, (int64_t)o.ref_start - 10,
-                                         [](int64_t v, int32_t p) { return v < (int64_t)p; }) - ctx->h_pmax.begin();
-                }
-            }
-            done[k] = std::max(done[k - 1], std::min<int64_t>(d, L));
-        }
     }
-    // median chunks: the loci that became complete with pair(k - 1), cut into pieces so that the copy of one piece
-    // runs under the medians of the next; the very last piece is small (its copy is the exposed one)
-    const int64_t piece = std::max<int64_t>(ctx->opt_min_piece, (L + ctx->opt_median_pieces - 1) / ctx->opt_median_pieces);
-    const int64_t last_piece = std::max<int64_t>(ctx->opt_min_piece / 4, L / (4 * ctx->opt_median_pieces));
-    for (int k = 1; k <= K; ++k) {
-        int64_t a = done[k - 1], b = done[k];
-        if (k == K && L == 0) break;
-        while (a < b) {
-            int64_t e = std::min(b, a + piece);
-            if (k == K) {
-                // the last group ends with a short piece
-                if (b - a > 2 * last_piece && e > b - last_piece) e = b - last_piece;
-            } else if (b - e < piece / 4) {
-                e = b;                                        // no tiny trailing piece
-            }
-            if (pl.n_chunks == kMaxMedianChunks - 1) e = b;
-            pl.chunk[pl.n_chunks++] = MedianChunk{(uint32_t)a, (uint32_t)e, k - 1};
-            a = e;
-        }
+    const int64_t piece = std::max<int64_t>(kMinPiece, (L + kMedianPieces - 1) / kMedianPieces);
+    const int64_t last_piece = std::max<int64_t>(kMinPiece / 4, L / (4 * kMedianPieces));
+    for (int64_t a = 0; a < L;) {
+        int64_t e = std::min(L, a + piece);
+        if (L - a > 2 * last_piece && e > L - last_piece) e = L - last_piece;
+        if (pl.n_chunks == kMaxMedianChunks - 1) e = L;
+        pl.chunk[pl.n_chunks++] = MedianChunk{(uint32_t)a, (uint32_t)e};
+        a = e;
     }
     pl.valid = true;
     pl.data_gen = ctx->data_gen;
+    return INQ_OK;
+}
+
+uint32_t loc_scan_tiles(int64_t L) { return (uint32_t)(((uint64_t)L + 1 + kXsTile - 1) / kXsTile); }
+
+// k_join_ranges, then the two offset scans over its difference array: lcnt[i+1] = number of candidate reads of locus
+// i, seg_off = exclusive scan of those counts. delta, desc_scan and the counters must be zero.
+int launch_join(inq_ctx *ctx, int unphased, cudaStream_t s)
+{
+    const int64_t L = ctx->L;
+    const uint64_t R = ctx->R;
+    const uint32_t tiles = loc_scan_tiles(L);
+    ReadView rv{ctx->contig.p, ctx->rs.p, ctx->re.p, ctx->mapq.p, ctx->hp.p, ctx->flags.p, ctx->cig_off.p, R};
+    LocusView lv{ctx->contig_off.p, ctx->lstart.p, ctx->lend.p, ctx->lpmax.p, ctx->n_contigs};
+    k_join_ranges<<<(unsigned)((R + 255) / 256), 256, 0, s>>>(rv, lv, unphased, ctx->cand_lo.p, ctx->cand_n.p, ctx->delta.p, ctx->d_ctr);
+    const unsigned g = std::min<unsigned>(tiles, (unsigned)ctx->sm_count * 4);
+    k_exclusive_scan<<<g, kXsThreads, 0, s>>>(ctx->delta.p, ctx->lcnt.p, (uint64_t)L + 1, tiles, ctx->desc_scan.p,
+                                              &ctx->d_ctr->scan_counter[2], nullptr);
+    k_exclusive_scan<<<g, kXsThreads, 0, s>>>(ctx->lcnt.p + 1, ctx->seg_off.p, (uint64_t)L, tiles,
+                                              ctx->desc_scan.p + tiles + 1, &ctx->d_ctr->scan_counter[3], &ctx->d_ctr->flags);
+    CU_TRY(ctx, cudaGetLastError());
     return INQ_OK;
 }
 
@@ -580,15 +504,13 @@ int enqueue_pass(inq_ctx *ctx, const RunParams &rp, bool capturing, uint32_t *n_
     cudaStream_t s0 = ctx->stream, s1 = ctx->stream_join, s2 = ctx->stream_med, s3 = ctx->stream_copy;
     const uint32_t ntiles = (uint32_t)((C + kTileWords - 1) / kTileWords);
     const uint64_t n_wt = (uint64_t)ntiles * (kTileWords / kWarpTileWords);
-    const uint32_t loc_scan_tiles = (uint32_t)(((uint64_t)L + 1 + kXsTile - 1) / kXsTile);
     const bool work = R && L;
+    const bool scan = n_wt && L;
     uint32_t launches = 0;
     auto stamp = [&](int e, cudaStream_t s, int level = 2) -> cudaError_t {
         if (rp.timing < level) return cudaSuccess;
         return cudaEventRecordWithFlags(ctx->ev[e], s, capturing ? cudaEventRecordExternal : cudaEventRecordDefault);
     };
-    ReadView rv{ctx->contig.p, ctx->rs.p, ctx->re.p, ctx->mapq.p, ctx->hp.p, ctx->flags.p, ctx->cig_off.p, R};
-    LocusView lv{ctx->contig_off.p, ctx->lstart.p, ctx->lend.p, ctx->lpmax.p, ctx->n_contigs};
 
     // S0 only needs the counters zeroed before the scan starts; everything the join / pair / median kernels need
     // zeroed is cleared on S1, off the scan's critical path
@@ -597,174 +519,123 @@ int enqueue_pass(inq_ctx *ctx, const RunParams &rp, bool capturing, uint32_t *n_
     // (EV_START / EV_END are plain event records on S0 around the pass -- or around the graph launch --, made by
     // inq_genotype: no nodes of the graph)
 
-    auto enqueue_join = [&]() -> int {
-        // ---- S1: K1 candidate ranges + difference array, then the per-locus segment offsets
-        CU_TRY(ctx, cudaStreamWaitEvent(s1, ctx->dep[DEP_FORK], 0));
-        {
-            // (buffers come from cudaMalloc: 256-byte aligned; the sizes are rounded up to 16 bytes inside their capacity)
-            ZeroJobs z;
-            z.n = 0;
-            auto add = [&](void *p, uint64_t bytes, uint64_t cap_bytes) { if (p && bytes) z.j[z.n++] = ZeroJob{p, std::min((bytes + 15) / 16 * 16, cap_bytes / 16 * 16)}; };
-            uint64_t biggest = 0;
-            if (L) {
-                add(ctx->delta.p, ((uint64_t)L + 2) * sizeof(uint32_t), ctx->delta.cap * sizeof(uint32_t));
-                add(ctx->seg_off.p, ((uint64_t)L + 2) * sizeof(uint32_t), ctx->seg_off.cap * sizeof(uint32_t));
-                add(ctx->cursor.p, ((uint64_t)L + 1) * sizeof(unsigned long long), ctx->cursor.cap * sizeof(unsigned long long));
-                add(ctx->desc_scan.p, 2 * ((uint64_t)loc_scan_tiles + 1) * sizeof(uint64_t), ctx->desc_scan.cap * sizeof(uint64_t));
-                biggest = ((uint64_t)L + 1) * sizeof(unsigned long long);
-            }
-            if (!ntiles) add(ctx->wt.p, 2 * sizeof(uint2), ctx->wt.cap * sizeof(uint2));      // no CIGAR words at all
-            if (n_wt) add(ctx->desc_wt.p, ctx->desc_wt.cap * sizeof(uint64_t), ctx->desc_wt.cap * sizeof(uint64_t));
-            if (z.n) {
-                const unsigned g = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((std::max<uint64_t>(biggest, 4096) / 16 + 255) / 256, (uint64_t)ctx->sm_count * 4));
-                k_zero<<<g, 256, 0, s1>>>(z);
-                CU_TRY(ctx, cudaGetLastError());
-            }
-            CU_TRY(ctx, cudaEventRecord(ctx->dep[DEP_ZEROED], s1));
-            CU_TRY(ctx, stamp(EV_INDEX, s1));
+    // ---- S1: K1 candidate ranges + difference array, then the per-locus segment offsets. Enqueued before the scan:
+    //      the order decides whose CTAs the SMs see first.
+    CU_TRY(ctx, cudaStreamWaitEvent(s1, ctx->dep[DEP_FORK], 0));
+    {
+        // (buffers come from cudaMalloc: 256-byte aligned; the sizes are rounded up to 16 bytes inside their capacity)
+        ZeroJobs z;
+        z.n = 0;
+        auto add = [&](void *p, uint64_t bytes, uint64_t cap_bytes) { if (p && bytes) z.j[z.n++] = ZeroJob{p, std::min((bytes + 15) / 16 * 16, cap_bytes / 16 * 16)}; };
+        uint64_t biggest = 0;
+        if (L) {
+            add(ctx->delta.p, ((uint64_t)L + 2) * sizeof(uint32_t), ctx->delta.cap * sizeof(uint32_t));
+            add(ctx->seg_off.p, ((uint64_t)L + 2) * sizeof(uint32_t), ctx->seg_off.cap * sizeof(uint32_t));
+            add(ctx->cursor.p, ((uint64_t)L + 1) * sizeof(unsigned long long), ctx->cursor.cap * sizeof(unsigned long long));
+            add(ctx->desc_scan.p, 2 * ((uint64_t)loc_scan_tiles(L) + 1) * sizeof(uint64_t), ctx->desc_scan.cap * sizeof(uint64_t));
+            biggest = ((uint64_t)L + 1) * sizeof(unsigned long long);
         }
-        if (work) {
-            k_join_ranges<<<(unsigned)((R + 255) / 256), 256, 0, s1>>>(rv, lv, rp.unphased, ctx->opt_join_coop, ctx->cand_lo.p, ctx->cand_n.p, ctx->delta.p, ctx->d_ctr, ctx->join_trace);
-            CU_TRY(ctx, stamp(EV_JOIN0, s1));
-            const unsigned g = std::min<unsigned>(loc_scan_tiles, (unsigned)ctx->sm_count * 4);
-            // lcnt[i+1] = number of candidate reads of locus i ; seg_off = exclusive scan of those counts
-            k_exclusive_scan<<<g, kXsThreads, 0, s1>>>(ctx->delta.p, ctx->lcnt.p, (uint64_t)L + 1, loc_scan_tiles, ctx->desc_scan.p,
-                                                       &ctx->d_ctr->scan_counter[2], nullptr);
-            k_exclusive_scan<<<g, kXsThreads, 0, s1>>>(ctx->lcnt.p + 1, ctx->seg_off.p, (uint64_t)L, loc_scan_tiles,
-                                                       ctx->desc_scan.p + loc_scan_tiles + 1, &ctx->d_ctr->scan_counter[3], &ctx->d_ctr->flags);
-            launches += 3;
-            CU_TRY(ctx, cudaGetLastError());
-            // the call buffer holds one slot per candidate; its size is only known on the device (checked after the pass)
-            // (read home on S2, idle until the first medians: a copy-engine operation in front of k_pair_eval costs the chain ~10 us)
-            CU_TRY(ctx, cudaEventRecord(ctx->dep[DEP_JOIN_DONE], s1));
-            CU_TRY(ctx, cudaStreamWaitEvent(s2, ctx->dep[DEP_JOIN_DONE], 0));
-            CU_TRY(ctx, cudaMemcpyAsync(ctx->h_total, ctx->seg_off.p + L, sizeof(uint32_t), cudaMemcpyDeviceToHost, s2));
-        }
-        CU_TRY(ctx, stamp(EV_JOIN, s1));
-
-        return INQ_OK;
-    };
-    uint64_t desc_base = 0;
-    auto enqueue_xscan2 = [&](int k, cudaStream_t st) -> int {
-        const uint64_t t0 = pl.tile_end[k], t1 = pl.tile_end[k + 1];
-        if (t1 > t0 && L) {
-            const uint64_t n = t1 - t0;
-            const uint32_t xt = (uint32_t)((n + kXsTile - 1) / kXsTile);
-            const unsigned g = std::min<unsigned>(xt, (unsigned)ctx->sm_count * 4);
-            uint64_t *dx = ctx->desc_wt.p + desc_base, *dy = dx + xt + 1;
-            desc_base += 2 * ((uint64_t)xt + 1);
-            k_exclusive_scan2<<<g, kXsThreads, 0, st>>>(ctx->wtot.p + t0, ctx->wt.p + t0, n, xt, dx, dy, &ctx->d_ctr->wt_scan_counter[k],
-                                                        ctx->d_ctr->wt_carry[k], ctx->d_ctr->wt_carry[k + 1], &ctx->d_ctr->flags);
-            ++launches;
+        if (!ntiles) add(ctx->wt.p, 2 * sizeof(uint2), ctx->wt.cap * sizeof(uint2));      // no CIGAR words at all
+        if (n_wt) add(ctx->desc_wt.p, ctx->desc_wt.cap * sizeof(uint64_t), ctx->desc_wt.cap * sizeof(uint64_t));
+        if (z.n) {
+            const unsigned g = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((std::max<uint64_t>(biggest, 4096) / 16 + 255) / 256, (uint64_t)ctx->sm_count * 4));
+            k_zero<<<g, 256, 0, s1>>>(z);
             CU_TRY(ctx, cudaGetLastError());
         }
-        return INQ_OK;
-    };
-    const bool xs_on_s0 = pl.K == 1 && !INQ_SCAN_FIRST;
-    auto enqueue_scans = [&]() -> int {
-        // ---- S0: K2, range after range, nothing in between (the scan of a range depends on nothing but the reads)
-        for (int k = 0; k < pl.K; ++k) {
-            const uint64_t t0 = pl.tile_end[k], t1 = pl.tile_end[k + 1];
-            CU_TRY(ctx, stamp(EV_SCAN0 + 2 * k, s0));
-            if (t1 > t0 && L) {
-                ScanParams sp;
-                sp.tile_first = ctx->tile_first.p; sp.cig_off = ctx->cig_off.p; sp.rd_pre = ctx->rd_pre.p; sp.wt = ctx->wtot.p;
-                sp.wt_sbase = ctx->wt_sbase.p; sp.evraw = ctx->evraw.p; sp.ctr = ctx->d_ctr; sp.raw_cap = ctx->evraw.cap;
-                sp.wt_begin = t0; sp.n_wt = t1; sp.neg1 = 0xFFFFFFFFu;
-                sp.thr = (std::min<uint32_t>(rp.minlen, (1u << 28) - 1u) << 4) | 15u;      // BAM op lengths have 28 bits
-                sp.evict_first = (uint32_t)ctx->opt_evict_first;
-                sp.debug = ctx->scan_debug;
-                const unsigned grid = (unsigned)std::min<uint64_t>((t1 - t0 + kScanWarps - 1) / kScanWarps, (uint64_t)ctx->sm_count * ctx->scan_ctas_per_sm);
-                if (sp.thr >> 31) k_cigar_scan<true><<<grid, kCtaThreads, kScanSmemBytes, s0>>>(ctx->tmap, sp);
-                else k_cigar_scan<false><<<grid, kCtaThreads, kScanSmemBytes, s0>>>(ctx->tmap, sp);
-                ++launches;
-                CU_TRY(ctx, cudaGetLastError());
-            }
-            if (xs_on_s0) {
-                // one range: the prefix sum over the warp-tile totals follows the scan on its own stream, so the join chain
-                // on S1 (slow under the scan) has until the end of it; the scan's end is time-stamped on the idle S3
-                CU_TRY(ctx, cudaEventRecord(ctx->dep[DEP_SCAN_ONLY], s0));
-                if (rp.timing >= 1) {
-                    CU_TRY(ctx, cudaStreamWaitEvent(s3, ctx->dep[DEP_SCAN_ONLY], 0));
-                    CU_TRY(ctx, stamp(EV_SCAN0 + 2 * k + 1, s3, 1));
-                }
-                CU_TRY(ctx, cudaStreamWaitEvent(s0, ctx->dep[DEP_ZEROED], 0));       // desc_wt is cleared by k_zero
-                TRY(enqueue_xscan2(k, s0));
-                CU_TRY(ctx, cudaEventRecord(ctx->dep[DEP_SCANNED + k], s0));
-            } else {
-                // the dependants hang off the kernel, not off the event-record node that follows it
-                CU_TRY(ctx, cudaEventRecord(ctx->dep[DEP_SCANNED + k], s0));
-                CU_TRY(ctx, stamp(EV_SCAN0 + 2 * k + 1, s0, k == pl.K - 1 ? 1 : 2));
-            }
-        }
+        CU_TRY(ctx, cudaEventRecord(ctx->dep[DEP_ZEROED], s1));
+        CU_TRY(ctx, stamp(EV_INDEX, s1));
+    }
+    if (work) {
+        TRY(launch_join(ctx, rp.unphased, s1));
+        launches += 3;
+        // the call buffer holds one slot per candidate; its size is only known on the device (checked after the pass)
+        // (read home on S2, idle until the first medians: a copy-engine operation in front of k_pair_eval costs the chain ~10 us)
+        CU_TRY(ctx, cudaEventRecord(ctx->dep[DEP_JOIN_DONE], s1));
+        CU_TRY(ctx, cudaStreamWaitEvent(s2, ctx->dep[DEP_JOIN_DONE], 0));
+        CU_TRY(ctx, cudaMemcpyAsync(ctx->h_total, ctx->seg_off.p + L, sizeof(uint32_t), cudaMemcpyDeviceToHost, s2));
+    }
+    CU_TRY(ctx, stamp(EV_JOIN, s1));
 
-        return INQ_OK;
-    };
-    // which of the two is enqueued first decides whose CTAs the SMs see first
-    if (INQ_SCAN_FIRST) { TRY(enqueue_scans()); TRY(enqueue_join()); }
-    else { TRY(enqueue_join()); TRY(enqueue_scans()); }
+    // ---- S0: K2, then the prefix sum over its warp-tile totals on the same stream, so that the join chain on S1
+    //      (slow under the scan) has until the end of the scan; the scan's end is time-stamped on the idle S3
+    CU_TRY(ctx, stamp(EV_SCAN0, s0));
+    if (scan) {
+        ScanParams sp;
+        sp.tile_first = ctx->tile_first.p; sp.cig_off = ctx->cig_off.p; sp.rd_pre = ctx->rd_pre.p; sp.wt = ctx->wtot.p;
+        sp.wt_sbase = ctx->wt_sbase.p; sp.evraw = ctx->evraw.p; sp.ctr = ctx->d_ctr; sp.raw_cap = ctx->evraw.cap;
+        sp.n_wt = n_wt; sp.neg1 = 0xFFFFFFFFu;
+        sp.thr = (std::min<uint32_t>(rp.minlen, (1u << 28) - 1u) << 4) | 15u;      // BAM op lengths have 28 bits
+        const unsigned grid = (unsigned)std::min<uint64_t>((n_wt + kScanWarps - 1) / kScanWarps, (uint64_t)ctx->sm_count * ctx->scan_ctas_per_sm);
+        if (sp.thr >> 31) k_cigar_scan<true><<<grid, kCtaThreads, kScanSmemBytes, s0>>>(ctx->tmap, sp);
+        else k_cigar_scan<false><<<grid, kCtaThreads, kScanSmemBytes, s0>>>(ctx->tmap, sp);
+        ++launches;
+        CU_TRY(ctx, cudaGetLastError());
+    }
+    CU_TRY(ctx, cudaEventRecord(ctx->dep[DEP_SCAN_ONLY], s0));
+    if (rp.timing >= 1) {
+        CU_TRY(ctx, cudaStreamWaitEvent(s3, ctx->dep[DEP_SCAN_ONLY], 0));
+        CU_TRY(ctx, stamp(EV_SCAN1, s3, 1));
+    }
+    CU_TRY(ctx, cudaStreamWaitEvent(s0, ctx->dep[DEP_ZEROED], 0));       // desc_wt is cleared by k_zero
+    if (scan) {
+        const uint32_t xt = (uint32_t)((n_wt + kXsTile - 1) / kXsTile);
+        const unsigned g = std::min<unsigned>(xt, (unsigned)ctx->sm_count * 4);
+        uint64_t *dx = ctx->desc_wt.p, *dy = dx + xt + 1;
+        k_exclusive_scan2<<<g, kXsThreads, 0, s0>>>(ctx->wtot.p, ctx->wt.p, n_wt, xt, dx, dy, &ctx->d_ctr->wt_scan_counter, &ctx->d_ctr->flags);
+        ++launches;
+        CU_TRY(ctx, cudaGetLastError());
+    }
+    CU_TRY(ctx, cudaEventRecord(ctx->dep[DEP_SCANNED], s0));
 
-    // ---- S1: prefix sum over the range's warp-tile totals, then K2b ; S2: K3 per finished catalog chunk ; S3: result copies
-    int c = 0;
+    // ---- S1: K2b once the stream is scanned ; S2: K3 per catalog chunk ; S3: result copies
+    CU_TRY(ctx, cudaStreamWaitEvent(s1, ctx->dep[DEP_SCANNED], 0));
+    CU_TRY(ctx, stamp(EV_PAIR0, s1));
+    if (work) {
+        const unsigned threads = kPairWarps * 32;
+        ReadView rv{ctx->contig.p, ctx->rs.p, ctx->re.p, ctx->mapq.p, ctx->hp.p, ctx->flags.p, ctx->cig_off.p, R};
+        LocusView lv{ctx->contig_off.p, ctx->lstart.p, ctx->lend.p, ctx->lpmax.p, ctx->n_contigs};
+        k_pair_eval<<<(unsigned)((R + threads - 1) / threads), threads, sizeof(PairSmem), s1>>>(
+            rv, 0, R, lv, rp.unphased, ctx->cand_lo.p, ctx->cand_n.p,
+            EventSource{ctx->wt.p, ctx->rd_pre.p, ctx->wt_sbase.p, ctx->evraw.p, ctx->evraw.cap}, ctx->seg_off.p, ctx->cursor.p,
+            ctx->vals.p, ctx->vals.cap, ctx->d_ctr);
+        ++launches;
+        CU_TRY(ctx, cudaGetLastError());
+    }
+    CU_TRY(ctx, stamp(EV_PAIR1, s1));
+    CU_TRY(ctx, cudaEventRecord(ctx->dep[DEP_PAIRED], s1));
     int64_t *o1 = rp.o1, *o2 = rp.o2;
     uint8_t *ov = rp.ov;
-    for (int k = 0; k < pl.K; ++k) {
-        const uint64_t r0 = pl.read_end[k], r1 = pl.read_end[k + 1];
-        CU_TRY(ctx, cudaStreamWaitEvent(s1, ctx->dep[DEP_SCANNED + k], 0));
-        if (!xs_on_s0) TRY(enqueue_xscan2(k, s1));
-        CU_TRY(ctx, stamp(EV_PAIR0 + 2 * k, s1));
-        if (work && r1 > r0) {
-            const unsigned threads = kPairWarps * 32;
-            k_pair_eval<<<(unsigned)((r1 - r0 + threads - 1) / threads), threads, sizeof(PairSmem), s1>>>(
-                rv, r0, r1, lv, rp.unphased, ctx->cand_lo.p, ctx->cand_n.p,
-                EventSource{ctx->wt.p, ctx->rd_pre.p, ctx->wt_sbase.p, ctx->evraw.p, ctx->evraw.cap}, ctx->seg_off.p, ctx->cursor.p,
-                ctx->vals.p, ctx->vals.cap, ctx->d_ctr, ctx->pair_debug);
-            ++launches;
-            CU_TRY(ctx, cudaGetLastError());
+    for (int c = 0; c < pl.n_chunks; ++c) {
+        const uint32_t l0 = pl.chunk[c].l0, l1 = pl.chunk[c].l1;
+        if (c == 0) {
+            // (S1 ran the join before the pair kernel: the first chunk also sees the empty segments of loci without reads)
+            CU_TRY(ctx, cudaStreamWaitEvent(s2, ctx->dep[DEP_PAIRED], 0));
+            CU_TRY(ctx, stamp(EV_MED0, s2));
         }
-        CU_TRY(ctx, stamp(EV_PAIR0 + 2 * k + 1, s1));
-        CU_TRY(ctx, cudaEventRecord(ctx->dep[DEP_PAIRED + k], s1));
-        bool waited = false;
-        for (; c < pl.n_chunks && pl.chunk[c].after_range == k; ++c) {
-            const uint32_t l0 = pl.chunk[c].l0, l1 = pl.chunk[c].l1;
-            if (!waited) {
-                CU_TRY(ctx, cudaStreamWaitEvent(s2, ctx->dep[DEP_PAIRED + k], 0));
-                // the first chunk also needs the (empty) segments of loci without reads: wait for the join if nothing was paired
-                waited = true;
-            }
-            if (c == 0) CU_TRY(ctx, stamp(EV_MED0, s2));
-            k_locus_median<<<(unsigned)((((uint64_t)(l1 - l0) + kMedianLociPerWarp - 1) / kMedianLociPerWarp * 32 + 255) / 256), 256, 0, s2>>>(l0, l1, c, rp.unphased, rp.support, ctx->seg_off.p, ctx->cursor.p,
-                                                                                              ctx->vals.p, ctx->vals.cap, ctx->t1.p, ctx->t2.p, ctx->valid.p,
-                                                                                              ctx->big_list.p, ctx->d_ctr);
-            CU_TRY(ctx, cudaGetLastError());
-            // the CTA path for the (rare) deep loci of the chunk: between two chunks on S2, or on the copy stream
-            cudaStream_t sb = INQ_BIG_ON_S3 ? s3 : s2;
-            if (INQ_BIG_ON_S3) {
-                CU_TRY(ctx, cudaEventRecord(ctx->dep[DEP_CHUNK + c], s2));
-                CU_TRY(ctx, cudaStreamWaitEvent(s3, ctx->dep[DEP_CHUNK + c], 0));
-            }
-            if (!pl.big_known || pl.need_big[c]) {
-                k_locus_median_big<<<(unsigned)ctx->sm_count * 2, kBigThreads, 0, sb>>>(l0, c, rp.unphased, rp.support, ctx->seg_off.p, ctx->cursor.p, ctx->vals.p,
-                                                                                      ctx->vals.cap, ctx->t1.p, ctx->t2.p, ctx->valid.p, ctx->big_list.p, ctx->d_ctr);
-                ++launches;
-            }
+        k_locus_median<<<(unsigned)((((uint64_t)(l1 - l0) + kMedianLociPerWarp - 1) / kMedianLociPerWarp * 32 + 255) / 256), 256, 0, s2>>>(l0, l1, c, rp.unphased, rp.support, ctx->seg_off.p, ctx->cursor.p,
+                                                                                          ctx->vals.p, ctx->vals.cap, ctx->t1.p, ctx->t2.p, ctx->valid.p,
+                                                                                          ctx->big_list.p, ctx->d_ctr);
+        CU_TRY(ctx, cudaGetLastError());
+        // the CTA path for the (rare) deep loci of the chunk, between two chunks on S2
+        if (!pl.big_known || pl.need_big[c]) {
+            k_locus_median_big<<<(unsigned)ctx->sm_count * 2, kBigThreads, 0, s2>>>(l0, c, rp.unphased, rp.support, ctx->seg_off.p, ctx->cursor.p, ctx->vals.p,
+                                                                                  ctx->vals.cap, ctx->t1.p, ctx->t2.p, ctx->valid.p, ctx->big_list.p, ctx->d_ctr);
+            ++launches;
+        }
+        ++launches;
+        CU_TRY(ctx, cudaGetLastError());
+        CU_TRY(ctx, cudaEventRecord(ctx->dep[DEP_CHUNK + c], s2));
+        CU_TRY(ctx, cudaStreamWaitEvent(s3, ctx->dep[DEP_CHUNK + c], 0));
+        const size_t n = l1 - l0;
+        if (rp.d1) {
+            const unsigned g = (unsigned)std::min<size_t>(kPushCtas, (n + 2047) / 2048);
+            k_push_results<<<std::max(g, 1u), 256, 0, s3>>>(l0, l1, ctx->t1.p, ctx->t2.p, ctx->valid.p, rp.d1, rp.d2, rp.dv);
             ++launches;
             CU_TRY(ctx, cudaGetLastError());
-            if (!INQ_BIG_ON_S3) {
-                CU_TRY(ctx, cudaEventRecord(ctx->dep[DEP_CHUNK + c], s2));
-                CU_TRY(ctx, cudaStreamWaitEvent(s3, ctx->dep[DEP_CHUNK + c], 0));
-            }
-            const size_t n = l1 - l0;
-            if (rp.d1) {
-                const unsigned g = (unsigned)std::min<size_t>((size_t)ctx->opt_push_ctas, (n + 2047) / 2048);
-                k_push_results<<<std::max(g, 1u), 256, 0, s3>>>(l0, l1, ctx->t1.p, ctx->t2.p, ctx->valid.p, rp.d1, rp.d2, rp.dv);
-                ++launches;
-                CU_TRY(ctx, cudaGetLastError());
-            } else {
-                CU_TRY(ctx, cudaMemcpyAsync(o1 + l0, ctx->t1.p + l0, n * sizeof(int64_t), cudaMemcpyDeviceToHost, s3));
-                CU_TRY(ctx, cudaMemcpyAsync(o2 + l0, ctx->t2.p + l0, n * sizeof(int64_t), cudaMemcpyDeviceToHost, s3));
-                CU_TRY(ctx, cudaMemcpyAsync(ov + l0, ctx->valid.p + l0, n, cudaMemcpyDeviceToHost, s3));
-            }
+        } else {
+            CU_TRY(ctx, cudaMemcpyAsync(o1 + l0, ctx->t1.p + l0, n * sizeof(int64_t), cudaMemcpyDeviceToHost, s3));
+            CU_TRY(ctx, cudaMemcpyAsync(o2 + l0, ctx->t2.p + l0, n * sizeof(int64_t), cudaMemcpyDeviceToHost, s3));
+            CU_TRY(ctx, cudaMemcpyAsync(ov + l0, ctx->valid.p + l0, n, cudaMemcpyDeviceToHost, s3));
         }
     }
     if (pl.n_chunks == 0) {                                   // nothing to do on S2/S3: keep them in the DAG for the join below
@@ -774,13 +645,12 @@ int enqueue_pass(inq_ctx *ctx, const RunParams &rp, bool capturing, uint32_t *n_
     }
     CU_TRY(ctx, stamp(EV_MED1, s2));
     // total number of events = the last prefix
-    if (n_wt && L) CU_TRY(ctx, cudaMemcpyAsync(ctx->h_total + 2, ctx->wt.p + n_wt, sizeof(uint2), cudaMemcpyDeviceToHost, s1));
+    if (scan) CU_TRY(ctx, cudaMemcpyAsync(ctx->h_total + 2, ctx->wt.p + n_wt, sizeof(uint2), cudaMemcpyDeviceToHost, s1));
     CU_TRY(ctx, cudaEventRecord(ctx->dep[DEP_S1_DONE], s1));
-    // the counters go home on S2 next to the last result copy (S3) instead of after it: S2 has seen every median kernel,
-    // S1 every join / prefix / pair kernel, and those waited for the scans
-    cudaStream_t sctr = INQ_BIG_ON_S3 ? s3 : s2;              // (the stream that runs the CTA-path medians, which also raise flags)
-    CU_TRY(ctx, cudaStreamWaitEvent(sctr, ctx->dep[DEP_S1_DONE], 0));
-    CU_TRY(ctx, cudaMemcpyAsync(ctx->h_ctr, ctx->d_ctr, sizeof(DevCounters), cudaMemcpyDeviceToHost, sctr));
+    // the counters go home on S2 next to the last result copy (S3) instead of after it: S2 has seen every median kernel
+    // (which raise flags), S1 every join / prefix / pair kernel, and those waited for the scans
+    CU_TRY(ctx, cudaStreamWaitEvent(s2, ctx->dep[DEP_S1_DONE], 0));
+    CU_TRY(ctx, cudaMemcpyAsync(ctx->h_ctr, ctx->d_ctr, sizeof(DevCounters), cudaMemcpyDeviceToHost, s2));
     CU_TRY(ctx, cudaEventRecord(ctx->dep[DEP_S2_DONE], s2));
     CU_TRY(ctx, stamp(EV_D2H, s3));
     CU_TRY(ctx, cudaEventRecord(ctx->dep[DEP_S3_DONE], s3));
@@ -838,13 +708,8 @@ int inq_ctx_create(int device, inq_ctx **out)
     int prio_lo = 0, prio_hi = 0;
     if ((e = cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi)) != cudaSuccess) return bail("cudaDeviceGetStreamPriorityRange", e);
     cudaStream_t *streams[4] = {&ctx->stream, &ctx->stream_join, &ctx->stream_med, &ctx->stream_copy};
-    for (int i = 0; i < 4; ++i) {
-        // INQ_STREAM_PRIORITIES bit i: stream Si gets the high priority (default: only the scan stream S0)
-        int prio_mask = INQ_STREAM_PRIORITIES;
-        if (const char *pm = getenv("INQ_STREAM_PRIORITY_MASK")) prio_mask = atoi(pm);       // experiments
-        const bool hi = (prio_mask >> i) & 1;
-        if ((e = cudaStreamCreateWithPriority(streams[i], cudaStreamNonBlocking, hi ? prio_hi : prio_lo)) != cudaSuccess) return bail("cudaStreamCreate", e);
-    }
+    for (int i = 0; i < 4; ++i)
+        if ((e = cudaStreamCreateWithPriority(streams[i], cudaStreamNonBlocking, i == 0 ? prio_hi : prio_lo)) != cudaSuccess) return bail("cudaStreamCreate", e);
     for (int i = 0; i < EV_COUNT; ++i)
         if ((e = cudaEventCreate(&ctx->ev[i])) != cudaSuccess) return bail("cudaEventCreate", e);
     for (int i = 0; i < DEP_COUNT; ++i)
@@ -852,11 +717,8 @@ int inq_ctx_create(int device, inq_ctx **out)
     if ((e = cudaMalloc(&ctx->d_ctr, sizeof(DevCounters))) != cudaSuccess) return bail("cudaMalloc", e);
     if ((e = cudaMalloc(&ctx->d_unsorted, sizeof(uint32_t))) != cudaSuccess) return bail("cudaMalloc", e);
     if ((e = cudaMemset(ctx->d_unsorted, 0, sizeof(uint32_t))) != cudaSuccess) return bail("cudaMemset", e);
-    if ((e = cudaMalloc(&ctx->d_probe, kMaxRanges * sizeof(ProbeOut))) != cudaSuccess) return bail("cudaMalloc", e);
-    if ((e = cudaMalloc(&ctx->d_probe_tiles, kMaxRanges * sizeof(uint64_t))) != cudaSuccess) return bail("cudaMalloc", e);
     if ((e = cudaMallocHost(&ctx->h_ctr, sizeof(DevCounters))) != cudaSuccess) return bail("cudaMallocHost", e);
     if ((e = cudaMallocHost(&ctx->h_total, 64)) != cudaSuccess) return bail("cudaMallocHost", e);
-    if ((e = cudaMallocHost(&ctx->h_probe, kMaxRanges * sizeof(ProbeOut))) != cudaSuccess) return bail("cudaMallocHost", e);
     memset(ctx->h_ctr, 0, sizeof(DevCounters));
     if ((e = cudaFuncSetAttribute(k_cigar_scan<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kScanSmemBytes)) != cudaSuccess ||
         (e = cudaFuncSetAttribute(k_cigar_scan<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kScanSmemBytes)) != cudaSuccess)
@@ -867,10 +729,6 @@ int inq_ctx_create(int device, inq_ctx **out)
     if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_cigar_scan<false>, kCtaThreads, kScanSmemBytes)) != cudaSuccess)
         return bail("occupancy(k_cigar_scan)", e);
     ctx->scan_ctas_per_sm = std::max(1, occ);
-#ifdef INQ_TIMING_EXPERIMENTS
-    if (const char *dbg = getenv("INQ_SCAN_DEBUG")) ctx->scan_debug = (uint32_t)atoi(dbg);
-    if (const char *dbg = getenv("INQ_PAIR_DEBUG")) ctx->pair_debug = (uint32_t)atoi(dbg);
-#endif
     *out = ctx;
     return INQ_OK;
 }
@@ -894,11 +752,8 @@ void inq_ctx_destroy(inq_ctx *ctx)
     release(ctx->events); release(ctx->t1); release(ctx->t2); release(ctx->valid);
     if (ctx->d_ctr) cudaFree(ctx->d_ctr);
     if (ctx->d_unsorted) cudaFree(ctx->d_unsorted);
-    if (ctx->d_probe) cudaFree(ctx->d_probe);
-    if (ctx->d_probe_tiles) cudaFree(ctx->d_probe_tiles);
     if (ctx->h_ctr) cudaFreeHost(ctx->h_ctr);
     if (ctx->h_total) cudaFreeHost(ctx->h_total);
-    if (ctx->h_probe) cudaFreeHost(ctx->h_probe);
     if (ctx->h_stage) cudaFreeHost(ctx->h_stage);
     if (ctx->h_route_stage) cudaFreeHost(ctx->h_route_stage);
     for (int i = 0; i < EV_COUNT; ++i)
@@ -915,36 +770,12 @@ int inq_set_option(inq_ctx *ctx, const char *name, int64_t value)
 {
     if (!ctx || !name) return INQ_ERR_ARG;
     const std::string n(name);
-    if (n == "ranges") {
-        if (value < 0 || value > kMaxRanges) return fail(ctx, INQ_ERR_ARG, "ranges must be in [0, %d]", kMaxRanges);
-        ctx->opt_ranges = (int)value;
-    } else if (n == "max_ranges") {
-        if (value < 1 || value > kMaxRanges) return fail(ctx, INQ_ERR_ARG, "max_ranges must be in [1, %d]", kMaxRanges);
-        ctx->opt_max_ranges = (int)value;
-    } else if (n == "min_range_tiles") {
-        if (value < 1) return fail(ctx, INQ_ERR_ARG, "min_range_tiles must be positive");
-        ctx->opt_min_range_tiles = value;
-    } else if (n == "graph") ctx->opt_graph = value != 0;
+    if (n == "graph") ctx->opt_graph = value != 0;
     else if (n == "timing") {
         if (value < 0 || value > 2) return fail(ctx, INQ_ERR_ARG, "timing must be 0 (off), 1 (pass and CIGAR scan) or 2 (every stage)");
         ctx->opt_timing = (int)value;
     }
-    else if (n == "push_kernel") ctx->opt_push_kernel = value != 0;
-    else if (n == "join_coop") ctx->opt_join_coop = value != 0;
-    else if (n == "evict_first") ctx->opt_evict_first = value != 0;
-    else if (n == "push_ctas") {
-        if (value < 1 || value > 1024) return fail(ctx, INQ_ERR_ARG, "push_ctas must be in [1, 1024]");
-        ctx->opt_push_ctas = (int)value;
-    }
-    else if (n == "median_pieces") {
-        if (value < 1 || value > kMaxMedianChunks / 2) return fail(ctx, INQ_ERR_ARG, "median_pieces must be in [1, %d]", kMaxMedianChunks / 2);
-        ctx->opt_median_pieces = (int)value;
-    } else if (n == "min_piece") {
-        if (value < 256) return fail(ctx, INQ_ERR_ARG, "min_piece must be at least 256 loci");
-        ctx->opt_min_piece = value;
-    }
     else return fail(ctx, INQ_ERR_ARG, "unknown option '%s'", name);
-    ctx->plan.valid = false;
     drop_graph(ctx);
     ctx->have_last_key = false;
     return INQ_OK;
@@ -1003,7 +834,7 @@ int inq_set_loci(inq_ctx *ctx, int32_t n_contigs, const int64_t *contig_locus_of
         CU_TRY(ctx, cudaGetLastError());
         CU_TRY(ctx, cudaMemcpyAsync(ctx->h_ctr, ctx->d_ctr, sizeof(DevCounters), cudaMemcpyDeviceToHost, s));
     }
-    // host copy of the running max of `end` per contig (the plan's "which loci are complete" test); overlaps the copies above
+    // host copy of the running max of `end` per contig (inq_push_reads_routed); overlaps the copies above
     ctx->h_contig_off.assign(contig_locus_offsets, contig_locus_offsets + n_contigs + 1);
     ctx->h_pmax.resize((size_t)L);
     ctx->h_lstart.assign(start, start + (L ? L : 0));
@@ -1250,24 +1081,13 @@ int inq_genotype(inq_ctx *ctx, uint32_t minlen, uint32_t support, int unphased, 
     TRY(ensure(ctx, ctx->wt, n_wt + 2));
     TRY(ensure(ctx, ctx->wtot, n_wt + 2));
     TRY(ensure(ctx, ctx->wt_sbase, n_wt + 1));
-    TRY(ensure(ctx, ctx->desc_wt, 2 * ((n_wt + kXsTile - 1) / kXsTile + 2 * kMaxRanges + 1)));       // even: k_zero clears it in 16-byte units
+    TRY(ensure(ctx, ctx->desc_wt, 2 * ((n_wt + kXsTile - 1) / kXsTile + 1)));       // even: k_zero clears it in 16-byte units
     if (ntiles) TRY(make_tensor_map(ctx, (uint64_t)ntiles * kTileWords));
     const uint64_t raw_slack = (uint64_t)ctx->sm_count * ctx->scan_ctas_per_sm * kScanWarps * kEvChunk;
     // event storage is sized speculatively (1/16 of the words; checked and regrown after the run); it hands out
     // kEvChunk-slot chunks and a warp strands the remainder of its chunk whenever a tile does not fit any more
     if (ctx->evraw.cap == 0) TRY(ensure(ctx, ctx->evraw, C / 16 + 4096 + raw_slack));
-    TRY(build_plan(ctx, n_wt));
-    if (getenv("INQ_JOIN_TRACE") && R) {
-        const uint64_t ctas = (R + 255) / 256;
-        if (ctas != ctx->join_trace_ctas) {
-            if (ctx->join_trace) cudaFree(ctx->join_trace);
-            ctx->join_trace = nullptr;
-            CU_TRY(ctx, cudaMalloc(&ctx->join_trace, (ctas * 3 + 8) * sizeof(unsigned long long)));
-            ctx->join_trace_ctas = ctas;
-            drop_graph(ctx);
-            ctx->have_last_key = false;
-        }
-    }
+    TRY(build_plan(ctx));
 
     // results go straight to the caller's arrays when those are pinned, otherwise through a pinned staging buffer
     const bool direct_out = L == 0 || (is_pinned(twice_h1) && is_pinned(twice_h2) && is_pinned(valid_mask));
@@ -1286,7 +1106,7 @@ int inq_genotype(inq_ctx *ctx, uint32_t minlen, uint32_t support, int unphased, 
         rp.ov = reinterpret_cast<uint8_t *>(rp.o2 + L);
     }
 
-    if (ctx->opt_push_kernel && L) {
+    if (L) {
         void *a = nullptr, *b = nullptr, *c = nullptr;
         if (cudaHostGetDevicePointer(&a, rp.o1, 0) == cudaSuccess && cudaHostGetDevicePointer(&b, rp.o2, 0) == cudaSuccess &&
             cudaHostGetDevicePointer(&c, rp.ov, 0) == cudaSuccess) {
@@ -1301,19 +1121,10 @@ int inq_genotype(inq_ctx *ctx, uint32_t minlen, uint32_t support, int unphased, 
     // the call buffer holds one slot per candidate; on the first call of a context its size is read back from a
     // join-only pre-pass, afterwards it is sized from the previous run and checked after the pass
     if (work && ctx->vals.cap == 0) {
-        const uint32_t loc_scan_tiles = (uint32_t)(((uint64_t)L + 1 + kXsTile - 1) / kXsTile);
-        ReadView rv{ctx->contig.p, ctx->rs.p, ctx->re.p, ctx->mapq.p, ctx->hp.p, ctx->flags.p, ctx->cig_off.p, R};
-        LocusView lv{ctx->contig_off.p, ctx->lstart.p, ctx->lend.p, ctx->lpmax.p, ctx->n_contigs};
         CU_TRY(ctx, cudaMemsetAsync(ctx->d_ctr, 0, sizeof(DevCounters), s));
         CU_TRY(ctx, cudaMemsetAsync(ctx->delta.p, 0, ((uint64_t)L + 2) * sizeof(uint32_t), s));
-        CU_TRY(ctx, cudaMemsetAsync(ctx->desc_scan.p, 0, 2 * ((uint64_t)loc_scan_tiles + 1) * sizeof(uint64_t), s));
-        k_join_ranges<<<(unsigned)((R + 255) / 256), 256, 0, s>>>(rv, lv, unphased, ctx->opt_join_coop, ctx->cand_lo.p, ctx->cand_n.p, ctx->delta.p, ctx->d_ctr, ctx->join_trace);
-        const unsigned g = std::min<unsigned>(loc_scan_tiles, (unsigned)ctx->sm_count * 4);
-        k_exclusive_scan<<<g, kXsThreads, 0, s>>>(ctx->delta.p, ctx->lcnt.p, (uint64_t)L + 1, loc_scan_tiles, ctx->desc_scan.p,
-                                                  &ctx->d_ctr->scan_counter[2], nullptr);
-        k_exclusive_scan<<<g, kXsThreads, 0, s>>>(ctx->lcnt.p + 1, ctx->seg_off.p, (uint64_t)L, loc_scan_tiles,
-                                                  ctx->desc_scan.p + loc_scan_tiles + 1, &ctx->d_ctr->scan_counter[3], &ctx->d_ctr->flags);
-        CU_TRY(ctx, cudaGetLastError());
+        CU_TRY(ctx, cudaMemsetAsync(ctx->desc_scan.p, 0, 2 * ((uint64_t)loc_scan_tiles(L) + 1) * sizeof(uint64_t), s));
+        TRY(launch_join(ctx, unphased, s));
         CU_TRY(ctx, cudaMemcpyAsync(ctx->h_total, ctx->seg_off.p + L, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
         CU_TRY(ctx, cudaStreamSynchronize(s));
         TRY(ensure(ctx, ctx->vals, (uint64_t)*ctx->h_total + 1));
@@ -1398,14 +1209,6 @@ int inq_genotype(inq_ctx *ctx, uint32_t minlen, uint32_t support, int unphased, 
     }
     if (!done) return fail(ctx, INQ_ERR_STATE, "internal: speculative buffers still too small after 4 attempts");
     ctx->last_n_events = (ntiles && L) ? ctx->h_total[3] : 0;      // .y of wt[n_wt]
-    if (ctx->join_trace) {
-        // experiments: dump the trace of the last pass (binary u64 triples: start ns, end ns, SM), plus the pass start
-        if (const char *path = getenv("INQ_JOIN_TRACE")) {
-            std::vector<unsigned long long> h(ctx->join_trace_ctas * 3);
-            CU_TRY(ctx, cudaMemcpy(h.data(), ctx->join_trace, h.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost));
-            if (FILE *f = fopen(path, "wb")) { fwrite(h.data(), sizeof(unsigned long long), h.size(), f); fclose(f); }
-        }
-    }
     if (!direct_out && L) {
         memcpy(twice_h1, rp.o1, (size_t)L * sizeof(int64_t));
         memcpy(twice_h2, rp.o2, (size_t)L * sizeof(int64_t));
@@ -1426,7 +1229,7 @@ int inq_genotype(inq_ctx *ctx, uint32_t minlen, uint32_t support, int unphased, 
         stats->op_visits = total(ST_OP_VISITS);
         stats->n_kernel_launches = launches;
         stats->n_tiles = ntiles;
-        stats->n_ranges = (uint32_t)ctx->plan.K;
+        stats->n_ranges = 1;
         stats->used_graph = used_graph ? 1u : 0u;
         stats->reads_sorted = ctx->plan.reads_sorted ? 1u : 0u;
         stats->n_median_chunks = (uint32_t)ctx->plan.n_chunks;
@@ -1436,23 +1239,18 @@ int inq_genotype(inq_ctx *ctx, uint32_t minlen, uint32_t support, int unphased, 
             if (rp.timing >= 2) {
                 stats->ms_join = el(EV_START, EV_JOIN);          // memsets + join + segment offsets, under the CIGAR scan
                 stats->ms_index = el(EV_START, EV_INDEX);        // ... of which the zeroing kernel
-                if (getenv("INQ_DEBUG_TIMING"))
-                    fprintf(stderr, "[inq timing] zero done %.3f  join done %.3f  offsets done %.3f  scan done %.3f ms after the start\n",
-                            el(EV_START, EV_INDEX), work ? el(EV_START, EV_JOIN0) : 0.f, el(EV_START, EV_JOIN), el(EV_START, EV_SCAN0 + 2 * (ctx->plan.K - 1) + 1));
-                for (int k = 0; k < ctx->plan.K; ++k) {
-                    stats->ms_cigar += el(EV_SCAN0 + 2 * k, EV_SCAN0 + 2 * k + 1);
-                    stats->ms_pairs += el(EV_PAIR0 + 2 * k, EV_PAIR0 + 2 * k + 1);
-                }
-                // prefix scan over the last range's warp-tile totals (incl. waiting for the join stream)
-                stats->ms_fixup = el(EV_SCAN0 + 2 * (ctx->plan.K - 1) + 1, EV_PAIR0 + 2 * (ctx->plan.K - 1));
+                stats->ms_cigar = el(EV_SCAN0, EV_SCAN1);
+                stats->ms_pairs = el(EV_PAIR0, EV_PAIR1);
+                // prefix scan over the warp-tile totals (incl. waiting for the join stream)
+                stats->ms_fixup = el(EV_SCAN1, EV_PAIR0);
                 stats->ms_median = el(EV_MED0, EV_MED1);
                 stats->ms_d2h = el(EV_MED1, EV_D2H);
             } else {
-                // S0 runs the K scans back to back right after the pass starts: start of the pass -> end of the last scan
-                // (a few us of fork on top of the kernels: the conservative side for a bandwidth figure)
-                stats->ms_cigar = el(EV_START, EV_SCAN0 + 2 * (ctx->plan.K - 1) + 1);
+                // S0 runs the scan right after the pass starts: start of the pass -> end of the scan
+                // (a few us of fork on top of the kernel: the conservative side for a bandwidth figure)
+                stats->ms_cigar = el(EV_START, EV_SCAN1);
             }
-            stats->ms_scan = el(EV_SCAN0 + 2 * (ctx->plan.K - 1) + 1, EV_END);      // what is left exposed after the last range is scanned
+            stats->ms_scan = el(EV_SCAN1, EV_END);           // what is left exposed after the CIGAR stream is scanned
         }
         stats->ms_h2d = ctx->ms_h2d;
     }

@@ -266,11 +266,8 @@ __host__ __device__ inline size_t zw_warp_bytes(uint32_t n_cols) { return (size_
 __global__ void __launch_bounds__(kZwMaxWarps * 32, 1)
 k_outlier_zscore_warp(const float *__restrict__ m, uint64_t n_rows, uint32_t n_cols, float minsize, float cutoff,
                       uint8_t *__restrict__ row_kept, unsigned long long *__restrict__ hits, uint64_t cap,
-                      CohortCounters *__restrict__ ctr, uint32_t dbg)
+                      CohortCounters *__restrict__ ctr)
 {
-#ifndef INQ_TIMING_EXPERIMENTS
-    dbg = 0;                                                  // timing experiments only exist in -DINQ_TIMING_EXPERIMENTS builds
-#endif
     extern __shared__ __align__(128) unsigned char zw_smem[];
     const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
     const uint32_t stride = zw_stride(n_cols);
@@ -310,7 +307,7 @@ k_outlier_zscore_warp(const float *__restrict__ m, uint64_t n_rows, uint32_t n_c
         // ---- one lane per row: sequential f32 sum + max, then the population variance (outlier.rs:18-31,81-90)
         float mean = 0.0f, sd = 0.0f, rinv = 0.0f;
         bool kept = false;
-        if (lane < nr && !(dbg & 2u)) {
+        if (lane < nr) {
             const float4 *row4 = reinterpret_cast<const float4 *>(rows + lane * stride);
             float sum = 0.0f, mx = -INFINITY;
 #pragma unroll 4
@@ -345,7 +342,7 @@ k_outlier_zscore_warp(const float *__restrict__ m, uint64_t n_rows, uint32_t n_c
         uint32_t *bits = reinterpret_cast<uint32_t *>(rows + 32 * stride) + lane * kZwMaskWords;
         const uint32_t n4 = n_cols / 4, nwords = (n4 + 7) / 8;
         uint32_t cnt = 0;
-        if (lane < nr && kept && !(dbg & 1u)) {
+        if (lane < nr && kept) {
             const float4 *row4 = reinterpret_cast<const float4 *>(rows + lane * stride);
             // The reference's test fl(fl(v - mean) / sd) >= cutoff (outlier.rs:109) is a step function of v: both roundings
             // are monotone for sd > 0. Its exact threshold -- the smallest f32 that passes -- is found once per row by
@@ -364,8 +361,7 @@ k_outlier_zscore_warp(const float *__restrict__ m, uint64_t n_rows, uint32_t n_c
                     return __uint_as_float(u);
                 };
                 float t = __fmaf_rn(cutoff, sd, mean);
-                if (dbg & 4u) { have_thr = true; thr = t; }              // (timing experiment: approximate threshold, wrong results)
-                else if (fabsf(t) <= 3.0e38f) {
+                if (fabsf(t) <= 3.0e38f) {
                     int guard = 0;
                     if (pred(t)) {
                         for (; guard < 16; ++guard) { const float d = step(t, false); if (!(fabsf(d) <= 3.0e38f) || !pred(d)) break; t = d; }
@@ -407,7 +403,7 @@ k_outlier_zscore_warp(const float *__restrict__ m, uint64_t n_rows, uint32_t n_c
 #pragma unroll
         for (int d = 1; d < 32; d <<= 1) { const uint32_t o = __shfl_up_sync(0xffffffffu, incl, d); if ((int)lane >= d) incl += o; }
         const uint32_t total = __shfl_sync(0xffffffffu, incl, 31);
-        if (total && !(dbg & 8u)) {
+        if (total) {
             unsigned long long base = 0;
             if (lane == 0) base = atomicAdd(&ctr->n_hits, (unsigned long long)total);
             unsigned long long slot = __shfl_sync(0xffffffffu, base, 0) + (incl - cnt);

@@ -7,7 +7,6 @@
 #include <algorithm>
 #include <cstdarg>
 #include <cstdio>
-#include <cstdlib>
 #include <cmath>
 #include <cstring>
 #include <string>
@@ -89,20 +88,14 @@ int inq_outlier(int device, int method, uint64_t n_rows, uint32_t n_cols, const 
         CC_TRY(cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, device));
         const size_t per_warp = zw_warp_bytes(n_cols);
         const int zw_warps = (int)std::min<size_t>(kZwMaxWarps, ((size_t)smem_max - 256) / per_warp);
-        uint32_t zw_dbg = 0;
-        bool force_rows = false;
-#ifdef INQ_TIMING_EXPERIMENTS
-        if (const char *e = getenv("INQ_ZW_DEBUG")) zw_dbg = (uint32_t)atoi(e);
-        if (const char *e = getenv("INQ_ZSCORE_ROWS")) force_rows = atoi(e) != 0;
-#endif
-        if (n_cols % 4 == 0 && n_cols <= 32u * kZwMaskWords && zw_warps >= 2 && !force_rows) {
+        if (n_cols % 4 == 0 && n_cols <= 32u * kZwMaskWords && zw_warps >= 2) {
             // every warp its own pipeline over groups of 32 rows (bulk async copies, one lane per row)
             const size_t smem = (size_t)zw_warps * per_warp + (size_t)zw_warps * 12 + 128;
             CC_TRY(cudaFuncSetAttribute(k_outlier_zscore_warp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
             const uint64_t groups = (n_rows + 31) / 32;
             const unsigned grid = (unsigned)std::min<uint64_t>((groups + zw_warps - 1) / zw_warps, (uint64_t)sms);
             k_outlier_zscore_warp<<<grid, zw_warps * 32, smem, g.s>>>((const float *)g.d_m, n_rows, n_cols, (float)minsize, zscore_cutoff,
-                                                                     (uint8_t *)g.d_kept, (unsigned long long *)g.d_hits, cap, (CohortCounters *)g.d_ctr, zw_dbg);
+                                                                     (uint8_t *)g.d_kept, (unsigned long long *)g.d_hits, cap, (CohortCounters *)g.d_ctr);
         } else if (res_smem <= 200u * 1024u) {
             // 32 rows fit in shared memory: the matrix is read once
             CC_TRY(cudaFuncSetAttribute(k_outlier_zscore_rows, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)res_smem));

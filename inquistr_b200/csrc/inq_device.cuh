@@ -45,17 +45,15 @@ constexpr uint64_t kKeyInf = ~0ull;
 constexpr int kStatSlots = 64;
 enum { ST_CANDIDATES = 0, ST_PAIRS, ST_READS_JOINED, ST_WORDS_JOINED, ST_OP_VISITS, ST_COUNT = 8 };
 
-constexpr int kMaxRanges = 16;              // the CIGAR stream is scanned in up to this many ranges of warp tiles (see inq_genotype)
 constexpr int kMaxMedianChunks = 48;        // the medians run in catalog chunks so that the result copy of one overlaps the next
 struct DevCounters {
     unsigned long long stat[kStatSlots][ST_COUNT];
     unsigned long long n_events;
     unsigned long long ev_alloc;      // event slots handed out to warps (chunks)
-    unsigned long long wt_carry[kMaxRanges + 1][2];   // warp-tile prefix {consumption, events} at the start of every scanned range
     unsigned int flags;
     unsigned int tile_counter;
     unsigned int scan_counter[4];
-    unsigned int wt_scan_counter[kMaxRanges];  // dynamic tile ids of k_exclusive_scan2, one per range
+    unsigned int wt_scan_counter;     // dynamic tile ids of k_exclusive_scan2
     unsigned int big_count[kMaxMedianChunks];  // per chunk of the catalog (see inq_genotype): loci for the CTA path
     unsigned int big_cursor[kMaxMedianChunks];
     unsigned int bad_hp_value;        // diagnostics: HP value and read index of one offending read
@@ -352,17 +350,9 @@ __device__ __forceinline__ void candidate_range_warp(bool unphased, const LocusV
 // the kernel adds +1/-1 to a difference array; its prefix sum is the number of candidate reads of
 // every locus, which sizes that locus' segment of the call buffer (an upper bound on its pairs).
 __global__ void __launch_bounds__(256)
-k_join_ranges(ReadView rv, LocusView lv, int unphased, int coop, uint32_t *__restrict__ cand_lo, uint32_t *__restrict__ cand_n,
-              uint32_t *__restrict__ delta /* L+1, zeroed */, DevCounters *__restrict__ ctr, unsigned long long *__restrict__ trace)
+k_join_ranges(ReadView rv, LocusView lv, int unphased, uint32_t *__restrict__ cand_lo, uint32_t *__restrict__ cand_n,
+              uint32_t *__restrict__ delta /* L+1, zeroed */, DevCounters *__restrict__ ctr)
 {
-    // (trace, experiments only: globaltimer at the start and the end of every CTA, and the SM it ran on)
-    if (trace && threadIdx.x == 0) {
-        unsigned long long t; unsigned int sm;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-        asm volatile("mov.u32 %0, %%smid;" : "=r"(sm));
-        trace[3ull * blockIdx.x] = t;
-        trace[3ull * blockIdx.x + 2] = sm;
-    }
     const uint64_t r = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
     int lo = 0, n = 0;
     int c = -1;
@@ -378,7 +368,7 @@ k_join_ranges(ReadView rv, LocusView lv, int unphased, int coop, uint32_t *__res
     // one contig for the whole warp? (all warps but the few that straddle a contig boundary)
     const int cmin = __reduce_min_sync(0xffffffffu, act ? c : 0x7fffffff), cmax = __reduce_max_sync(0xffffffffu, act ? c : -1);
     int hi = 0;
-    if (coop && cmin == cmax) {
+    if (cmin == cmax) {
         candidate_range_warp(unphased != 0, lv, cmin, act, rs, re, lo, hi);
     } else if (act) {
         candidate_range(unphased != 0, lv, c, rs, re, lo, hi);
@@ -404,14 +394,6 @@ k_join_ranges(ReadView rv, LocusView lv, int unphased, int coop, uint32_t *__res
     const uint32_t cand_w = __reduce_add_sync(0xffffffffu, (uint32_t)n);
     if (lane_id() == 0 && cand_w)
         atomicAdd(&ctr->stat[(blockIdx.x * 8u + (threadIdx.x >> 5)) % kStatSlots][ST_CANDIDATES], (unsigned long long)cand_w);
-    if (trace) {
-        __syncthreads();
-        if (threadIdx.x == 0) {
-            unsigned long long t;
-            asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
-            trace[3ull * blockIdx.x + 1] = t;
-        }
-    }
 }
 
 // ----------------------------------------------------------------------------------------------
@@ -461,18 +443,10 @@ struct ScanParams {
     uint2 *evraw;
     DevCounters *ctr;
     uint64_t raw_cap;             // capacity of evraw (slots)
-    uint64_t wt_begin;            // this launch scans warp tiles [wt_begin, n_wt)
     uint64_t n_wt;
     uint32_t thr;                 // (min(minlen, 2^28 - 1) << 4) | 15: an op is longer than minlen iff its word > thr
     uint32_t neg1;                // 0xFFFFFFFF as a run-time value (keeps thr - w a multiply-add on the FMA pipe)
-    uint32_t evict_first;         // 1: the CIGAR words are loaded with the L2 evict-first policy
-    uint32_t debug;               // timing experiments only, compiled in with -DINQ_TIMING_EXPERIMENTS: results are wrong when != 0
 };
-#ifdef INQ_TIMING_EXPERIMENTS
-#define INQ_DBG(x) (x)
-#else
-#define INQ_DBG(x) 0u             // the shipped library cannot be switched into a wrong-answer mode
-#endif
 
 #ifndef INQ_LANE_WORDS
 #define INQ_LANE_WORDS 32
@@ -514,20 +488,14 @@ constexpr size_t kScanSmemBytes = sizeof(ScanSmem) + 1024;   // slack to align t
 // (16-byte chunk index bits [2:4] ^= 128-byte row index bits [5:7])
 __device__ __forceinline__ uint32_t swz(uint32_t idx) { return idx ^ (((idx >> 5) & 7u) << 2); }
 
-// `policy`: L2 cache policy of the load, 0 = none. The stream is read exactly once, so its lines are marked evict-first:
+// `policy`: L2 cache policy of the load. The stream is read exactly once, so its lines are marked evict-first:
 // otherwise 10 GB of them flush the catalog and the per-read arrays out of the 126 MB L2, and every probe of the join
 // chain that runs next to the scan (and of the pair kernel after it) goes to the saturated HBM instead.
 __device__ __forceinline__ void tma_load_tile(void *dst_smem, const CUtensorMap *tmap, uint32_t row, uint64_t *bar, uint64_t policy)
 {
-    if (policy) {
-        asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%2, %3}], [%4], %5;"
-                     ::"r"(smem_u32(dst_smem)), "l"(tmap), "r"(0), "r"(row), "r"(smem_u32(bar)), "l"(policy)
-                     : "memory");
-    } else {
-        asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-                     ::"r"(smem_u32(dst_smem)), "l"(tmap), "r"(0), "r"(row), "r"(smem_u32(bar))
-                     : "memory");
-    }
+    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1, {%2, %3}], [%4], %5;"
+                 ::"r"(smem_u32(dst_smem)), "l"(tmap), "r"(0), "r"(row), "r"(smem_u32(bar)), "l"(policy)
+                 : "memory");
 }
 __device__ __forceinline__ uint64_t l2_evict_first_policy()
 {
@@ -548,9 +516,9 @@ k_cigar_scan(const __grid_constant__ CUtensorMap tmap, ScanParams p)
     const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     constexpr uint32_t kBoxBytes = kWarpTileWords * 4;
     constexpr uint32_t kRowsPerBox = kWarpTileWords / 32;       // 128-byte rows
-    const uint64_t gwid = p.wt_begin + (uint64_t)blockIdx.x * kScanWarps + warp, stride = (uint64_t)gridDim.x * kScanWarps;
+    const uint64_t gwid = (uint64_t)blockIdx.x * kScanWarps + warp, stride = (uint64_t)gridDim.x * kScanWarps;
     uint64_t *full = sm.full[warp];
-    const uint64_t l2_policy = p.evict_first ? l2_evict_first_policy() : 0ull;
+    const uint64_t l2_policy = l2_evict_first_policy();
 
     if (lane == 0) {
         for (int s = 0; s < kWarpStages; ++s) mbar_init(&full[s], 1);
@@ -599,7 +567,6 @@ k_cigar_scan(const __grid_constant__ CUtensorMap tmap, ScanParams p)
         //      snap[j]: bases consumed inside the lane's words before quad j (parked in shared memory below)
         uint32_t c = 0, evrev = 0;
         uint32_t snap[kQuads];
-        if (!(INQ_DBG(p.debug) & 8u))
 #pragma unroll
         for (int j = 0; j < (int)kQuads; ++j) {
             const uint32_t q = q0 + (uint32_t)j, row = q >> 3;
@@ -620,10 +587,6 @@ k_cigar_scan(const __grid_constant__ CUtensorMap tmap, ScanParams p)
                 // c += consumes ? len : 0 as one multiply-add (FMA pipe) instead of select + add (ALU pipe)
                 asm("mad.lo.u32 %0, %1, %2, %0;" : "+r"(c) : "r"(w >> 4), "r"(lut & 1u));
             }
-        }
-        else {
-#pragma unroll
-            for (int j = 0; j < (int)kQuads; ++j) snap[j] = 0;
         }
         const uint32_t ne = __popc(evrev);
         const uint32_t incl_c = warp_incl_scan(c), incl_e = warp_incl_scan(ne);
@@ -649,7 +612,7 @@ k_cigar_scan(const __grid_constant__ CUtensorMap tmap, ScanParams p)
             }
             chunk_cur += tot_e;
         }
-        if (lane == 31 && !(INQ_DBG(p.debug) & 16u)) {
+        if (lane == 31) {
             p.wt[gw] = make_uint2(incl_c, incl_e);
             p.wt_sbase[gw] = (uint32_t)sbase;
         }
@@ -665,7 +628,6 @@ k_cigar_scan(const __grid_constant__ CUtensorMap tmap, ScanParams p)
         const uint32_t n_q = tot_e + n_starts;                  // queries [0, tot_e) are the events in word order
         const uint32_t off_cur = (uint32_t)(g_cur - gw * kWarpTileWords);    // lane i: first word of read tf_lo + i
         uint32_t ev_left = evrev, ev_idx = excl_e;
-        if (!(INQ_DBG(p.debug) & 1u))
         for (uint32_t base = 0; base < n_q; base += 32) {
             // owners list their events with index in [base, base + 32): word order = descending bits of evrev
             while (ev_left && ev_idx < base + 32u) {
@@ -848,20 +810,16 @@ k_exclusive_scan(const uint32_t *in, uint32_t *out, uint64_t n, uint32_t ntiles,
 }
 
 // same for pairs of u32 (both components wrap mod 2^32; `y` is checked against 2^32): totals `in[0, n)` ->
-// exclusive prefixes `out[0, n]`. The CIGAR stream is scanned in ranges of warp tiles (inq_genotype); every
-// range continues from the prefix the previous one left in carry_in and leaves its own end in carry_out
-// (out[n], the end sentinel of this range, is the value the next range writes to the same slot again).
+// exclusive prefixes `out[0, n]`
 __global__ void __launch_bounds__(kXsThreads)
 k_exclusive_scan2(const uint2 *__restrict__ in, uint2 *__restrict__ out, uint64_t n, uint32_t ntiles,
                   uint64_t *__restrict__ desc_x, uint64_t *__restrict__ desc_y, unsigned int *__restrict__ tile_counter,
-                  const unsigned long long *__restrict__ carry_in, unsigned long long *__restrict__ carry_out,
                   unsigned int *__restrict__ overflow_flags)
 {
     __shared__ uint32_t wsx[kXsThreads / 32], wsy[kXsThreads / 32];
     __shared__ uint32_t tile_s;
     __shared__ uint64_t bx_s, by_s;
     const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const uint64_t cx = carry_in[0], cy = carry_in[1];
     while (true) {
         if (tid == 0) tile_s = atomicAdd(tile_counter, 1u);
         __syncthreads();
@@ -901,13 +859,11 @@ k_exclusive_scan2(const uint2 *__restrict__ in, uint2 *__restrict__ out, uint64_
                 }
             }
             if (lane == 0) {
-                bx_s = bx + cx;
-                by_s = by + cy;
+                bx_s = bx;
+                by_s = by;
                 if (t == ntiles - 1) {
-                    out[n] = make_uint2((uint32_t)(cx + bx + tx), (uint32_t)(cy + by + ty));
-                    carry_out[0] = (cx + bx + tx) & 0xFFFFFFFFull;
-                    carry_out[1] = cy + by + ty;
-                    if (overflow_flags && cy + by + ty > 0xFFFFFFFFull) atomicOr(overflow_flags, kFlagCountOverflow);
+                    out[n] = make_uint2((uint32_t)(bx + tx), (uint32_t)(by + ty));
+                    if (overflow_flags && by + ty > 0xFFFFFFFFull) atomicOr(overflow_flags, kFlagCountOverflow);
                 }
             }
         }
@@ -989,13 +945,12 @@ struct PairSmem {                           // per CTA of kPairWarps warps (dyna
     uint32_t joined[kPairWarps];
 };
 
-// reads [r_begin, r_end): the CIGAR stream is scanned in ranges of warp tiles and every range's reads are
-// evaluated as soon as their last word has been scanned (inq_genotype)
+// reads [r_begin, r_end) (the pass launches it once over [0, R); bounding r by rv.R instead doubles ptxas' spills)
 __global__ void __launch_bounds__(kPairWarps * 32, INQ_PAIR_MIN_CTAS)
 k_pair_eval(ReadView rv, uint64_t r_begin, uint64_t r_end, LocusView lv, int unphased, const uint32_t *__restrict__ cand_lo,
             const uint32_t *__restrict__ cand_n, EventSource es, const uint32_t *__restrict__ seg_off,
             unsigned long long *__restrict__ cursor, uint64_t *__restrict__ vals, uint64_t vals_cap,
-            DevCounters *__restrict__ ctr, uint32_t debug)
+            DevCounters *__restrict__ ctr)
 {
     // A warp owns 32 consecutive reads; their candidates are flattened and dealt to the lanes
     // 32 at a time (reads have 0..hundreds of candidates, a per-read loop leaves most lanes idle).
@@ -1117,8 +1072,7 @@ k_pair_eval(ReadView rv, uint64_t r_begin, uint64_t r_end, LocusView lv, int unp
         if (!pend) return;
         const uint32_t slot_k = pend_back ? (uint32_t)(pend_old >> 32) : (uint32_t)pend_old;
         const uint64_t slot = pend_back ? (uint64_t)pend_seg + (pend_cap - 1u - slot_k) : (uint64_t)pend_seg + slot_k;
-        if (INQ_DBG(debug) & 2u) {
-        } else if (slot_k < pend_cap && slot < vals_cap) vals[slot] = pend_key;
+        if (slot_k < pend_cap && slot < vals_cap) vals[slot] = pend_key;
         else atomicOr(&ctr->flags, kFlagValsOverflow);
         pend = false;
     };
@@ -1182,13 +1136,12 @@ k_pair_eval(ReadView rv, uint64_t r_begin, uint64_t r_end, LocusView lv, int unp
             ++npass;
             atomicOr(&s_joined[wid], 1u << j);
             // slot first: the atomic's round trip overlaps the rest of this iteration and the next one
-            old = (INQ_DBG(debug) & 1u) ? 0ull : atomicAdd(cursor + l, back ? (1ull << 32) : 1ull);
+            old = atomicAdd(cursor + l, back ? (1ull << 32) : 1ull);
             const uint32_t start_ext = (uint32_t)ls - 10u, end_ext = (uint32_t)le + 10u;
             const bool is2d = ((hf_j >> 8) & 1u) != 0u;
             int64_t call = 0;
             uint32_t clip = 0;
-            if (INQ_DBG(debug) & 4u) {
-            } else if (!(hf_j & (1u << 9))) {
+            if (!(hf_j & (1u << 9))) {
                 // the read's events sit in shared memory, sorted by anchor: binary search, then a short scan
                 const uint32_t ne = e1_j - e0_j;
                 const uint2 *sev = &s_ev[wid][eb_j];

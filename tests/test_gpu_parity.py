@@ -241,26 +241,22 @@ def test_size_independent_properties(ctx):
     assert np.all((d.valid & ~a.valid) == 0)
 
 
-# ------------------------------------------------------------------ range pipeline + CUDA graph
+# ------------------------------------------------------------------ CUDA graph
 def _pinned_out(n):
     import inquistr_b200 as q
     return (q.pinned_empty(n, np.int64), q.pinned_empty(n, np.int64), q.pinned_empty(n, np.uint8))
 
 
 @pytest.mark.parametrize("sort_reads", [True, False])
-@pytest.mark.parametrize("ranges", [2, 3, 7, 16])
-def test_range_pipeline_and_graph_replay(sort_reads, ranges):
-    """the pass cut into `ranges` ranges of warp tiles (pair / median work of range k under the scan of
-    range k+1), launched directly, captured, and replayed from the CUDA graph: same bits every time"""
+def test_graph_replay(sort_reads):
+    """the pass launched directly, captured, and replayed from the CUDA graph: same bits every time"""
     import inquistr_b200 as q
-    case = make_case(70 + ranges, n_contigs=3, contig_len=200_000, n_loci=700, n_reads=5000, sort_reads=sort_reads)
+    case = make_case(72, n_contigs=3, contig_len=200_000, n_loci=700, n_reads=5000, sort_reads=sort_reads)
     rd = case["reads"]
-    assert len(rd.cigar) // 1024 >= 3 * ranges
     rc, p1, p2, visits = O.genotype_loci(rd, case["n_contigs"], case["locus_contig"], case["locus_start"],
                                          case["locus_end"], 5, 3, False, threads=4)
     assert rc == 0
     with q.Context(0) as c:
-        c.set_option("ranges", ranges)
         c.set_loci(case["contig_off"], case["locus_start"], case["locus_end"])
         c.push(rd)
         out = _pinned_out(len(case["locus_start"]))
@@ -270,7 +266,7 @@ def test_range_pipeline_and_graph_replay(sort_reads, ranges):
             res = c.genotype(5, 3, False, out=out)
             assert same(res.phase1, p1) and same(res.phase2, p2), (it, res.stats)
             assert res.stats["op_visits"] == visits
-            assert res.stats["n_ranges"] == ranges
+            assert res.stats["n_ranges"] == 1
             assert res.stats["reads_sorted"] == int(sort_reads)
             graphs += res.stats["used_graph"]
         assert graphs == 3                                  # first call direct, then capture + replay
@@ -280,6 +276,8 @@ def test_range_pipeline_and_graph_replay(sort_reads, ranges):
         for it in range(3):
             res = c.genotype(0, 2, True, out=out)          # minlen 0: the event buffer regrows on the first of these
             assert same(res.phase1, u1) and same(res.phase2, u2)
+            if it == 0:
+                assert res.stats["used_graph"] == 0
         assert res.stats["used_graph"] == 1
         # pageable outputs: staged through the library's pinned buffer, no graph requirement on the caller
         res = c.genotype(5, 3, False)
@@ -293,20 +291,31 @@ def test_range_pipeline_and_graph_replay(sort_reads, ranges):
             q.free_pinned(a)
 
 
-def test_sorted_reads_finish_loci_early():
-    """coordinate-sorted reads: catalog chunks are reduced as soon as no later read can reach them"""
+def test_sorted_reads_are_flagged():
+    """coordinate-sorted reads of a real-shaped workload are recognised as sorted and genotyped like the oracle"""
     import inquistr_b200 as q
     from synth.synth import make_workload
     w = make_workload(3, scale=0.02, threads=4, pack_filter=True)
     with q.Context(0) as c:
-        c.set_option("ranges", 4)
         c.set_loci(w.contig_locus_off, w.locus_start, w.locus_end)
         c.push(w.reads)
         res = c.genotype(w.minlen, w.support, w.unphased)
-        assert res.stats["reads_sorted"] == 1 and res.stats["n_median_chunks"] >= 4
+        assert res.stats["reads_sorted"] == 1
         rc, p1, p2, visits = O.genotype_loci(w.reads, w.n_contigs, w.locus_contig, w.locus_start.astype(np.uint32),
                                              w.locus_end.astype(np.uint32), w.minlen, w.support, w.unphased, threads=8)
         assert rc == 0 and same(res.phase1, p1) and same(res.phase2, p2) and res.stats["op_visits"] == visits
+
+
+def test_set_option_accepts_only_graph_and_timing(ctx):
+    """the range pipeline and the experiment switches are gone: their names are unknown options"""
+    import inquistr_b200 as q
+    ctx.set_option("graph", 1)
+    ctx.set_option("timing", 1)
+    for name in ("ranges", "max_ranges", "min_range_tiles", "push_kernel", "join_coop", "evict_first", "push_ctas",
+                 "median_pieces", "min_piece"):
+        with pytest.raises(q.InqError) as ei:
+            ctx.set_option(name, 1)
+        assert ei.value.code == -2 and "unknown option" in str(ei.value), name
 
 
 def test_reserve_after_push_keeps_padding_and_tile_table(ctx):
