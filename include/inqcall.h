@@ -65,7 +65,7 @@ typedef struct inq_ctx inq_ctx;
 typedef struct inq_stats {
     uint64_t n_loci;
     uint64_t n_reads;
-    uint64_t n_cigar_words;      /* C  : packed CIGAR words resident on the device */
+    uint64_t n_cigar_words;      /* C  : BAM CIGAR words pushed (the device keeps them as about as many 16-bit units) */
     uint64_t n_cigar_words_joined; /* C_j: words of reads joined to >= 1 locus candidate */
     uint64_t n_reads_joined;
     uint64_t n_pairs;            /* P  : (read, locus) pairs that passed the filter into a bucket */
@@ -73,7 +73,8 @@ typedef struct inq_stats {
     uint64_t n_events;           /* I/D/S ops longer than minlen found by the CIGAR scan */
     uint64_t op_visits;          /* sum over pairs of n_cigar(read): what call.rs:382 executes */
     uint32_t n_kernel_launches;  /* kernels launched by the call (direct or replayed from the CUDA graph) */
-    uint32_t n_tiles;            /* CIGAR tiles scanned */
+    uint32_t n_tiles;            /* 32 KB tiles of the device CIGAR stream scanned: 16384 units each (before units were
+                                    16 bits, a tile held 8192 words, so the count is half what it was) */
     float ms_total;              /* start of the pass -> everything done, results in host memory */
     float ms_index;              /* memsets */
     float ms_join;               /* K1 read x locus overlap join + segment offsets (second stream, under K2) */
@@ -162,7 +163,8 @@ int inq_push_reads_routed(inq_ctx *ctx, uint64_t n_reads, const int32_t *contig,
                           const uint32_t *cigar_words, uint32_t filter, int host_threads,
                           uint64_t *n_taken);
 
-/* Optional: size the device buffers once before a series of pushes. */
+/* Optional: size the device buffers once before a series of pushes. The CIGAR stream gets room for n_cigar_words
+ * 16-bit units (one per word of ordinary reads); ops of 4095 or more bases take a few units more and grow it in place. */
 int inq_reserve_reads(inq_ctx *ctx, uint64_t n_reads, uint64_t n_cigar_words);
 
 /* Forget all pushed reads (device buffers are kept for reuse). */

@@ -88,7 +88,7 @@ const DriverApi &driver()
     return d;
 }
 
-// The packed CIGAR stream (the one multi-GB buffer) lives in a reserved virtual address range that is
+// The CIGAR unit stream (the one multi-GB buffer) lives in a reserved virtual address range that is
 // backed by physical chunks as reads arrive: growing it neither copies the stream nor moves its base
 // address (the TMA tensor map and a captured graph stay valid).
 struct VmStream {
@@ -165,13 +165,18 @@ struct inq_ctx {
     std::vector<int32_t> h_pmax, h_lstart;
     void *h_route_stage = nullptr;        // pinned staging of inq_push_reads_routed when the kept reads are scattered
 
-    // reads
-    uint64_t R = 0, C = 0;
+    // reads: C BAM words (the statistics count them), stored as U 16-bit units (inq_device.cuh, "CIGAR units")
+    uint64_t R = 0, C = 0, U = 0;
     DevBuf<int32_t> contig, rs, re;
     DevBuf<uint8_t> mapq, hp, flags;
-    DevBuf<uint64_t> cig_off;
-    DevBuf<uint32_t> cigar;               // cudaMalloc'ed fallback when the driver has no VMM API
+    DevBuf<uint64_t> cig_off, unit_off;
+    DevBuf<uint16_t> cigar;               // cudaMalloc'ed fallback when the driver has no VMM API
     VmStream vm;
+    // encoding at push: a double-buffered staging ring of BAM words and the per-chunk unit counts / offsets
+    DevBuf<uint32_t> push_stage, push_cnt, push_off;
+    DevBuf<uint64_t> push_desc;
+    DevBuf<unsigned int> push_ctr;        // tile counter and overflow flag of the offset scan
+    cudaEvent_t push_landed[2] = {}, push_free[2] = {};
     uint32_t *d_unsorted = nullptr;       // != 0: the pushed reads are not sorted by (contig, ref_start)
 
     // work buffers
@@ -181,7 +186,7 @@ struct inq_ctx {
     DevBuf<uint2> rd_pre, wt, wtot;
     DevBuf<uint64_t> desc_scan, desc_wt, vals;
     DevBuf<uint2> evraw;
-    CUtensorMap tmap;                 // 2-D view of the packed CIGAR stream: rows of 32 words, 128B swizzle
+    CUtensorMap tmap;                 // 2-D view of the unit stream: rows of 32 words (64 units), 128B swizzle
     const void *tmap_base = nullptr;
     uint64_t tmap_rows = 0;
     DevBuf<uint2> events;
@@ -322,18 +327,18 @@ int vm_ensure(inq_ctx *ctx, size_t bytes)
     return INQ_OK;
 }
 
-uint32_t *cigar_ptr(inq_ctx *ctx) { return driver().vmm ? reinterpret_cast<uint32_t *>(ctx->vm.base) : ctx->cigar.p; }
-uint64_t cigar_cap_words(inq_ctx *ctx) { return driver().vmm ? ctx->vm.mapped / 4 : ctx->cigar.cap; }
+uint16_t *cigar_ptr(inq_ctx *ctx) { return driver().vmm ? reinterpret_cast<uint16_t *>(ctx->vm.base) : ctx->cigar.p; }
+uint64_t cigar_cap_units(inq_ctx *ctx) { return driver().vmm ? ctx->vm.mapped / 2 : ctx->cigar.cap; }
 
-// (re)build the TMA descriptor of the CIGAR stream: uint32 [rows][32], box = one 4 KB warp tile, 128B swizzle
-int make_tensor_map(inq_ctx *ctx, uint64_t n_words_padded)
+// (re)build the TMA descriptor of the unit stream: uint32 [rows][32] (unit pairs), box = one 4 KB warp tile, 128B swizzle
+int make_tensor_map(inq_ctx *ctx, uint64_t n_units_padded)
 {
-    const uint64_t rows = n_words_padded / 32;
+    const uint64_t rows = n_units_padded / 64;
     if (ctx->tmap_base == cigar_ptr(ctx) && ctx->tmap_rows == rows) return INQ_OK;
     if (!driver().tmap_encode) return fail(ctx, INQ_ERR_CUDA, "cuTensorMapEncodeTiled is not available from the driver");
     const cuuint64_t gdim[2] = {32, rows};
     const cuuint64_t gstride[1] = {128};
-    const cuuint32_t box[2] = {32, (cuuint32_t)(kWarpTileWords / 32)};    // one warp tile
+    const cuuint32_t box[2] = {32, (cuuint32_t)(kWarpTileUnits / 64)};    // one warp tile
     const cuuint32_t estride[2] = {1, 1};
     CUresult r = driver().tmap_encode(&ctx->tmap, CU_TENSOR_MAP_DATA_TYPE_UINT32, 2, cigar_ptr(ctx), gdim, gstride, box, estride,
                                       CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
@@ -345,9 +350,22 @@ int make_tensor_map(inq_ctx *ctx, uint64_t n_words_padded)
     return INQ_OK;
 }
 
-int reserve_reads(inq_ctx *ctx, uint64_t nR, uint64_t nC, double growth)
+// Room for nU units of the stream. What must survive a regrow is everything inq_push_reads left behind: the `keep`
+// units written so far, the zero padding up to a tile boundary (+1 tile of slack) and the tile_first entries of
+// every warp tile up to the padded end plus the sentinel slot.
+int reserve_units(inq_ctx *ctx, uint64_t nU, uint64_t keep, double growth)
 {
-    const uint64_t R = ctx->R, C = ctx->C;
+    const uint64_t Upad = round_up(keep, kTileUnits);
+    const uint64_t need_units = round_up(nU, kTileUnits) + kTileUnits;
+    if (driver().vmm) TRY(vm_ensure(ctx, need_units * sizeof(uint16_t)));
+    else TRY(ensure(ctx, ctx->cigar, need_units, Upad, growth));
+    TRY(ensure(ctx, ctx->tile_first, std::max(cigar_cap_units(ctx), need_units) / kWarpTileUnits + 2, keep ? Upad / kWarpTileUnits + 1 : 0, 1.0));
+    return INQ_OK;
+}
+
+int reserve_reads(inq_ctx *ctx, uint64_t nR, uint64_t nU, double growth)
+{
+    const uint64_t R = ctx->R;
     TRY(ensure(ctx, ctx->contig, nR, R, growth));
     TRY(ensure(ctx, ctx->rs, nR, R, growth));
     TRY(ensure(ctx, ctx->re, nR, R, growth));
@@ -355,15 +373,8 @@ int reserve_reads(inq_ctx *ctx, uint64_t nR, uint64_t nC, double growth)
     TRY(ensure(ctx, ctx->hp, nR, R, growth));
     TRY(ensure(ctx, ctx->flags, nR, R, growth));
     TRY(ensure(ctx, ctx->cig_off, nR + 1, R + 1, growth));
-    // CIGAR stream is padded with zero words up to a tile boundary (+1 tile of slack). What must survive a
-    // regrow is everything inq_push_reads left behind: the words, their zero padding, and the tile_first
-    // entries of every warp tile up to the padded end plus the sentinel slot.
-    const uint64_t Cpad = R ? round_up(C, kTileWords) : 0;
-    const uint64_t need_words = round_up(nC, kTileWords) + kTileWords;
-    if (driver().vmm) TRY(vm_ensure(ctx, need_words * sizeof(uint32_t)));
-    else TRY(ensure(ctx, ctx->cigar, need_words, Cpad, growth));
-    TRY(ensure(ctx, ctx->tile_first, std::max(cigar_cap_words(ctx), need_words) / kWarpTileWords + 2, R ? Cpad / kWarpTileWords + 1 : 0, 1.0));
-    return INQ_OK;
+    TRY(ensure(ctx, ctx->unit_off, nR + 1, R + 1, growth));
+    return reserve_units(ctx, nU, R ? ctx->U : 0, growth);
 }
 
 // ---- small kernels of the orchestration layer ---------------------------------------------------
@@ -500,10 +511,10 @@ int enqueue_pass(inq_ctx *ctx, const RunParams &rp, bool capturing, uint32_t *n_
 {
     const Plan &pl = ctx->plan;
     const int64_t L = ctx->L;
-    const uint64_t R = ctx->R, C = ctx->C;
+    const uint64_t R = ctx->R, U = ctx->U;
     cudaStream_t s0 = ctx->stream, s1 = ctx->stream_join, s2 = ctx->stream_med, s3 = ctx->stream_copy;
-    const uint32_t ntiles = (uint32_t)((C + kTileWords - 1) / kTileWords);
-    const uint64_t n_wt = (uint64_t)ntiles * (kTileWords / kWarpTileWords);
+    const uint32_t ntiles = (uint32_t)((U + kTileUnits - 1) / kTileUnits);
+    const uint64_t n_wt = (uint64_t)ntiles * (kTileUnits / kWarpTileUnits);
     const bool work = R && L;
     const bool scan = n_wt && L;
     uint32_t launches = 0;
@@ -535,7 +546,7 @@ int enqueue_pass(inq_ctx *ctx, const RunParams &rp, bool capturing, uint32_t *n_
             add(ctx->desc_scan.p, 2 * ((uint64_t)loc_scan_tiles(L) + 1) * sizeof(uint64_t), ctx->desc_scan.cap * sizeof(uint64_t));
             biggest = ((uint64_t)L + 1) * sizeof(unsigned long long);
         }
-        if (!ntiles) add(ctx->wt.p, 2 * sizeof(uint2), ctx->wt.cap * sizeof(uint2));      // no CIGAR words at all
+        if (!ntiles) add(ctx->wt.p, 2 * sizeof(uint2), ctx->wt.cap * sizeof(uint2));      // no CIGAR units at all
         if (n_wt) add(ctx->desc_wt.p, ctx->desc_wt.cap * sizeof(uint64_t), ctx->desc_wt.cap * sizeof(uint64_t));
         if (z.n) {
             const unsigned g = (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((std::max<uint64_t>(biggest, 4096) / 16 + 255) / 256, (uint64_t)ctx->sm_count * 4));
@@ -561,13 +572,17 @@ int enqueue_pass(inq_ctx *ctx, const RunParams &rp, bool capturing, uint32_t *n_
     CU_TRY(ctx, stamp(EV_SCAN0, s0));
     if (scan) {
         ScanParams sp;
-        sp.tile_first = ctx->tile_first.p; sp.cig_off = ctx->cig_off.p; sp.rd_pre = ctx->rd_pre.p; sp.wt = ctx->wtot.p;
-        sp.wt_sbase = ctx->wt_sbase.p; sp.evraw = ctx->evraw.p; sp.ctr = ctx->d_ctr; sp.raw_cap = ctx->evraw.cap;
-        sp.n_wt = n_wt; sp.neg1 = 0xFFFFFFFFu;
-        sp.thr = (std::min<uint32_t>(rp.minlen, (1u << 28) - 1u) << 4) | 15u;      // BAM op lengths have 28 bits
+        sp.tile_first = ctx->tile_first.p; sp.unit_off = ctx->unit_off.p; sp.units = cigar_ptr(ctx); sp.rd_pre = ctx->rd_pre.p;
+        sp.wt = ctx->wtot.p; sp.wt_sbase = ctx->wt_sbase.p; sp.evraw = ctx->evraw.p; sp.ctr = ctx->d_ctr; sp.raw_cap = ctx->evraw.cap;
+        sp.n_wt = n_wt; sp.neg1 = 0xFFFFFFFFu; sp.minlen = rp.minlen;
+        // the unit field holds lengths up to 4094 exactly and 4095 for every longer I/D/S: from minlen 4095 on only
+        // those long heads can be events, and k_cigar_scan<true, true> checks their full length
+        const uint32_t thr16 = (std::min<uint32_t>(rp.minlen, kUnitLong - 1) << 4) | 15u;
+        sp.thr = (thr16 << 16) | 0xFFFFu;
         const unsigned grid = (unsigned)std::min<uint64_t>((n_wt + kScanWarps - 1) / kScanWarps, (uint64_t)ctx->sm_count * ctx->scan_ctas_per_sm);
-        if (sp.thr >> 31) k_cigar_scan<true><<<grid, kCtaThreads, kScanSmemBytes, s0>>>(ctx->tmap, sp);
-        else k_cigar_scan<false><<<grid, kCtaThreads, kScanSmemBytes, s0>>>(ctx->tmap, sp);
+        if (rp.minlen >= kUnitLong) k_cigar_scan<true, true><<<grid, kCtaThreads, kScanSmemBytes, s0>>>(ctx->tmap, sp);
+        else if (sp.thr >> 31) k_cigar_scan<true, false><<<grid, kCtaThreads, kScanSmemBytes, s0>>>(ctx->tmap, sp);
+        else k_cigar_scan<false, false><<<grid, kCtaThreads, kScanSmemBytes, s0>>>(ctx->tmap, sp);
         ++launches;
         CU_TRY(ctx, cudaGetLastError());
     }
@@ -596,7 +611,7 @@ int enqueue_pass(inq_ctx *ctx, const RunParams &rp, bool capturing, uint32_t *n_
         LocusView lv{ctx->contig_off.p, ctx->lstart.p, ctx->lend.p, ctx->lpmax.p, ctx->n_contigs};
         k_pair_eval<<<(unsigned)((R + threads - 1) / threads), threads, sizeof(PairSmem), s1>>>(
             rv, 0, R, lv, rp.unphased, ctx->cand_lo.p, ctx->cand_n.p,
-            EventSource{ctx->wt.p, ctx->rd_pre.p, ctx->wt_sbase.p, ctx->evraw.p, ctx->evraw.cap}, ctx->seg_off.p, ctx->cursor.p,
+            EventSource{ctx->unit_off.p, ctx->wt.p, ctx->rd_pre.p, ctx->wt_sbase.p, ctx->evraw.p, ctx->evraw.cap}, ctx->seg_off.p, ctx->cursor.p,
             ctx->vals.p, ctx->vals.cap, ctx->d_ctr);
         ++launches;
         CU_TRY(ctx, cudaGetLastError());
@@ -714,19 +729,23 @@ int inq_ctx_create(int device, inq_ctx **out)
         if ((e = cudaEventCreate(&ctx->ev[i])) != cudaSuccess) return bail("cudaEventCreate", e);
     for (int i = 0; i < DEP_COUNT; ++i)
         if ((e = cudaEventCreateWithFlags(&ctx->dep[i], cudaEventDisableTiming)) != cudaSuccess) return bail("cudaEventCreate", e);
+    for (int i = 0; i < 2; ++i)
+        if ((e = cudaEventCreateWithFlags(&ctx->push_landed[i], cudaEventDisableTiming)) != cudaSuccess ||
+            (e = cudaEventCreateWithFlags(&ctx->push_free[i], cudaEventDisableTiming)) != cudaSuccess) return bail("cudaEventCreate", e);
     if ((e = cudaMalloc(&ctx->d_ctr, sizeof(DevCounters))) != cudaSuccess) return bail("cudaMalloc", e);
     if ((e = cudaMalloc(&ctx->d_unsorted, sizeof(uint32_t))) != cudaSuccess) return bail("cudaMalloc", e);
     if ((e = cudaMemset(ctx->d_unsorted, 0, sizeof(uint32_t))) != cudaSuccess) return bail("cudaMemset", e);
     if ((e = cudaMallocHost(&ctx->h_ctr, sizeof(DevCounters))) != cudaSuccess) return bail("cudaMallocHost", e);
     if ((e = cudaMallocHost(&ctx->h_total, 64)) != cudaSuccess) return bail("cudaMallocHost", e);
     memset(ctx->h_ctr, 0, sizeof(DevCounters));
-    if ((e = cudaFuncSetAttribute(k_cigar_scan<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kScanSmemBytes)) != cudaSuccess ||
-        (e = cudaFuncSetAttribute(k_cigar_scan<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kScanSmemBytes)) != cudaSuccess)
+    if ((e = cudaFuncSetAttribute(k_cigar_scan<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kScanSmemBytes)) != cudaSuccess ||
+        (e = cudaFuncSetAttribute(k_cigar_scan<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kScanSmemBytes)) != cudaSuccess ||
+        (e = cudaFuncSetAttribute(k_cigar_scan<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kScanSmemBytes)) != cudaSuccess)
         return bail("cudaFuncSetAttribute(k_cigar_scan)", e);
     if ((e = cudaFuncSetAttribute(k_pair_eval, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(PairSmem))) != cudaSuccess)
         return bail("cudaFuncSetAttribute(k_pair_eval)", e);
     int occ = 0;
-    if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_cigar_scan<false>, kCtaThreads, kScanSmemBytes)) != cudaSuccess)
+    if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_cigar_scan<false, false>, kCtaThreads, kScanSmemBytes)) != cudaSuccess)
         return bail("occupancy(k_cigar_scan)", e);
     ctx->scan_ctas_per_sm = std::max(1, occ);
     *out = ctx;
@@ -742,7 +761,8 @@ void inq_ctx_destroy(inq_ctx *ctx)
     release(ctx->contig_off); release(ctx->lstart); release(ctx->lend); release(ctx->lpmax);
     release(ctx->contig); release(ctx->rs); release(ctx->re);
     release(ctx->mapq); release(ctx->hp); release(ctx->flags);
-    release(ctx->cig_off); release(ctx->cigar);
+    release(ctx->cig_off); release(ctx->unit_off); release(ctx->cigar);
+    release(ctx->push_stage); release(ctx->push_cnt); release(ctx->push_off); release(ctx->push_desc); release(ctx->push_ctr);
     if (ctx->vm.base) vm_release(ctx->vm);
     release(ctx->cand_lo); release(ctx->cand_n); release(ctx->ev_off);
     release(ctx->rd_pre); release(ctx->wt); release(ctx->wtot); release(ctx->wt_sbase); release(ctx->tile_first);
@@ -760,6 +780,10 @@ void inq_ctx_destroy(inq_ctx *ctx)
         if (ctx->ev[i]) cudaEventDestroy(ctx->ev[i]);
     for (int i = 0; i < DEP_COUNT; ++i)
         if (ctx->dep[i]) cudaEventDestroy(ctx->dep[i]);
+    for (int i = 0; i < 2; ++i) {
+        if (ctx->push_landed[i]) cudaEventDestroy(ctx->push_landed[i]);
+        if (ctx->push_free[i]) cudaEventDestroy(ctx->push_free[i]);
+    }
     cudaStream_t streams[4] = {ctx->stream_copy, ctx->stream_med, ctx->stream_join, ctx->stream};
     for (auto s : streams)
         if (s) cudaStreamDestroy(s);
@@ -858,7 +882,8 @@ int inq_reserve_reads(inq_ctx *ctx, uint64_t n_reads, uint64_t n_cigar_words)
 {
     if (!ctx) return INQ_ERR_ARG;
     CU_TRY(ctx, cudaSetDevice(ctx->device));
-    return reserve_reads(ctx, std::max(n_reads, ctx->R), std::max(n_cigar_words, ctx->C), 1.0);
+    // room for as many units as words: longer ops grow the stream in place when they are pushed
+    return reserve_reads(ctx, std::max(n_reads, ctx->R), std::max(n_cigar_words, ctx->U), 1.0);
 }
 
 int inq_clear_reads(inq_ctx *ctx)
@@ -867,23 +892,41 @@ int inq_clear_reads(inq_ctx *ctx)
     CU_TRY(ctx, cudaSetDevice(ctx->device));
     ctx->R = 0;
     ctx->C = 0;
+    ctx->U = 0;
     ++ctx->data_gen;
     CU_TRY(ctx, cudaMemsetAsync(ctx->d_unsorted, 0, sizeof(uint32_t), ctx->stream));
     return INQ_OK;
 }
 
+constexpr uint64_t kPushChunkWords = 1ull << 24;      // BAM words per encoding chunk (64 MB; a ring of up to two staging buffers)
+
+unsigned grid_for(uint64_t n) { return (unsigned)std::max<uint64_t>(1, std::min<uint64_t>((n + 255) / 256, 4096)); }
+
 // Appends n reads whose CIGAR words are words[cigar_off[0] .. cigar_off[n]) (cigar_off need not start at 0).
-// The copies are asynchronous; the caller synchronises ctx->stream before the host arrays may change.
+// The words go to the device in chunks through a two-buffer staging ring on S3, so that the copy of chunk k+1
+// overlaps the encoding of chunk k into units on S0: count the units of every word, scan the counts, read the
+// chunk's total back (the stream may have to grow), write the units and the unit offsets of the reads that start
+// in the chunk. The copies are asynchronous; the caller synchronises ctx->stream before the host arrays may change.
 static int push_impl(inq_ctx *ctx, uint64_t n, const int32_t *contig, const int32_t *ref_start, const int32_t *ref_end,
                      const uint8_t *mapq, const uint8_t *hp, const uint8_t *flags, const uint64_t *cigar_off, const uint32_t *words)
 {
     const uint64_t w0 = cigar_off[0], nw = cigar_off[n] - w0;
     if (ctx->R + n >= 0xFFFFFFFFull) return fail(ctx, INQ_ERR_TOO_LARGE, "inq_push_reads: more than 2^32-2 reads");
-    TRY(reserve_reads(ctx, ctx->R + n, ctx->C + nw, 1.5));
+    TRY(reserve_reads(ctx, ctx->R + n, ctx->U + nw, 1.5));
+    const uint64_t stage_words = std::min(nw, kPushChunkWords);
+    const uint64_t n_chunks = nw ? (nw + stage_words - 1) / stage_words : 0;
+    const uint32_t max_xt = (uint32_t)((stage_words + kXsTile - 1) / kXsTile);
+    if (nw) {
+        // the second buffer of the ring only when there is a second chunk: a push of up to 64 MB of words holds one
+        TRY(ensure(ctx, ctx->push_stage, std::min<uint64_t>(n_chunks, 2) * stage_words));
+        TRY(ensure(ctx, ctx->push_cnt, stage_words));
+        TRY(ensure(ctx, ctx->push_off, stage_words + 1));
+        TRY(ensure(ctx, ctx->push_desc, (uint64_t)max_xt + 1));
+        TRY(ensure(ctx, ctx->push_ctr, 2));
+    }
     ++ctx->data_gen;
-    cudaStream_t s = ctx->stream;
-    const uint64_t R0 = ctx->R, C0 = ctx->C;
-    uint32_t *cig = cigar_ptr(ctx);
+    cudaStream_t s = ctx->stream, sc = ctx->stream_copy;
+    const uint64_t R0 = ctx->R, C0 = ctx->C, U0 = ctx->U;
     CU_TRY(ctx, cudaMemcpyAsync(ctx->contig.p + R0, contig, n * sizeof(int32_t), cudaMemcpyHostToDevice, s));
     CU_TRY(ctx, cudaMemcpyAsync(ctx->rs.p + R0, ref_start, n * sizeof(int32_t), cudaMemcpyHostToDevice, s));
     CU_TRY(ctx, cudaMemcpyAsync(ctx->re.p + R0, ref_end, n * sizeof(int32_t), cudaMemcpyHostToDevice, s));
@@ -891,24 +934,67 @@ static int push_impl(inq_ctx *ctx, uint64_t n, const int32_t *contig, const int3
     CU_TRY(ctx, cudaMemcpyAsync(ctx->hp.p + R0, hp, n, cudaMemcpyHostToDevice, s));
     CU_TRY(ctx, cudaMemcpyAsync(ctx->flags.p + R0, flags, n, cudaMemcpyHostToDevice, s));
     CU_TRY(ctx, cudaMemcpyAsync(ctx->cig_off.p + R0, cigar_off, (n + 1) * sizeof(uint64_t), cudaMemcpyHostToDevice, s));
-    if (nw) CU_TRY(ctx, cudaMemcpyAsync(cig + C0, words + w0, nw * sizeof(uint32_t), cudaMemcpyHostToDevice, s));
     if (C0 != w0) {                                              // batch-local offsets -> offsets into the device stream (mod 2^64)
         k_rebase_offsets<<<(unsigned)std::min<uint64_t>((n + 1 + 255) / 256, 8192), 256, 0, s>>>(ctx->cig_off.p + R0, n + 1, C0 - w0);
         CU_TRY(ctx, cudaGetLastError());
     }
     k_check_sorted<<<(unsigned)std::min<uint64_t>((n + 255) / 256, 4096), 256, 0, s>>>(ctx->contig.p, ctx->rs.p, R0, n, ctx->d_unsorted);
     CU_TRY(ctx, cudaGetLastError());
-    const uint64_t C1 = C0 + nw, Cpad = round_up(C1, kTileWords);
-    if (Cpad > C1) CU_TRY(ctx, cudaMemsetAsync(cig + C1, 0, (Cpad - C1) * sizeof(uint32_t), s));
+
+    auto copy_chunk = [&](uint64_t k) -> int {
+        const uint64_t a = k * stage_words, m = std::min(stage_words, nw - a);
+        CU_TRY(ctx, cudaStreamWaitEvent(sc, ctx->push_free[k & 1], 0));      // the encoding of chunk k-2 is done with the buffer
+        CU_TRY(ctx, cudaMemcpyAsync(ctx->push_stage.p + (k & 1) * stage_words, words + w0 + a, m * sizeof(uint32_t), cudaMemcpyHostToDevice, sc));
+        CU_TRY(ctx, cudaEventRecord(ctx->push_landed[k & 1], sc));
+        return INQ_OK;
+    };
+    uint64_t U1 = U0;
+    if (n_chunks) TRY(copy_chunk(0));
+    for (uint64_t k = 0; k < n_chunks; ++k) {
+        if (k + 1 < n_chunks) TRY(copy_chunk(k + 1));
+        const uint64_t a = k * stage_words, m = std::min(stage_words, nw - a);
+        const uint32_t *src = ctx->push_stage.p + (k & 1) * stage_words;
+        const uint32_t xt = (uint32_t)((m + kXsTile - 1) / kXsTile);
+        CU_TRY(ctx, cudaStreamWaitEvent(s, ctx->push_landed[k & 1], 0));
+        k_unit_count<<<grid_for(m), 256, 0, s>>>(src, m, ctx->push_cnt.p);
+        CU_TRY(ctx, cudaMemsetAsync(ctx->push_desc.p, 0, ((uint64_t)xt + 1) * sizeof(uint64_t), s));
+        CU_TRY(ctx, cudaMemsetAsync(ctx->push_ctr.p, 0, 2 * sizeof(unsigned int), s));
+        k_exclusive_scan<<<std::min<unsigned>(xt, (unsigned)ctx->sm_count * 4), kXsThreads, 0, s>>>(
+            ctx->push_cnt.p, ctx->push_off.p, m, xt, ctx->push_desc.p, ctx->push_ctr.p, ctx->push_ctr.p + 1);
+        CU_TRY(ctx, cudaGetLastError());
+        CU_TRY(ctx, cudaMemcpyAsync(ctx->h_total + 12, ctx->push_off.p + m, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+        CU_TRY(ctx, cudaMemcpyAsync(ctx->h_total + 13, ctx->push_ctr.p + 1, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
+        CU_TRY(ctx, cudaStreamSynchronize(s));
+        if (ctx->h_total[13]) return fail(ctx, INQ_ERR_TOO_LARGE, "inq_push_reads: %llu CIGAR words expand to 2^32 units or more", (unsigned long long)m);
+        const uint64_t mu = ctx->h_total[12];
+        TRY(reserve_units(ctx, U1 + mu, U1, 1.5));
+        k_unit_write<<<grid_for(m), 256, 0, s>>>(src, m, ctx->push_off.p, cigar_ptr(ctx) + U1);
+        CU_TRY(ctx, cudaEventRecord(ctx->push_free[k & 1], s));
+        // unit offsets of the reads that start in the chunk (the last chunk also takes those that start at its end)
+        const uint64_t b = k + 1 == n_chunks ? nw + 1 : a + m;
+        const uint64_t ra = (uint64_t)(std::lower_bound(cigar_off, cigar_off + n + 1, w0 + a) - cigar_off);
+        const uint64_t rb = (uint64_t)(std::lower_bound(cigar_off, cigar_off + n + 1, w0 + b) - cigar_off);
+        if (rb > ra) k_read_units<<<grid_for(rb - ra), 256, 0, s>>>(ctx->cig_off.p, R0 + ra, rb - ra, C0 + a, ctx->push_off.p, U1, ctx->unit_off.p);
+        CU_TRY(ctx, cudaGetLastError());
+        U1 += mu;
+    }
+    if (!nw) {
+        k_read_units<<<grid_for(n + 1), 256, 0, s>>>(ctx->cig_off.p, R0, n + 1, 0, nullptr, U0, ctx->unit_off.p);
+        CU_TRY(ctx, cudaGetLastError());
+    }
+    uint16_t *units = cigar_ptr(ctx);
+    const uint64_t Upad = round_up(U1, kTileUnits);
+    if (Upad > U1) CU_TRY(ctx, cudaMemsetAsync(units + U1, 0, (Upad - U1) * sizeof(uint16_t), s));
     {
-        // reads starting per warp tile, for the tiles that gained words (k_cigar_scan leaves the tile-local
-        // prefix of every read start in rd_pre); cig_off[R0 + n] is the sentinel and counts as a start
-        const uint64_t t0 = C0 / kWarpTileWords, t1 = Cpad / kWarpTileWords;
-        k_tile_first<<<(unsigned)((t1 - t0 + 1 + 255) / 256), 256, 0, s>>>(ctx->cig_off.p, R0 + n + 1, t0, t1, ctx->tile_first.p);
+        // reads starting per warp tile, for the tiles that gained units (k_cigar_scan leaves the tile-local
+        // prefix of every read start in rd_pre); unit_off[R0 + n] is the sentinel and counts as a start
+        const uint64_t t0 = U0 / kWarpTileUnits, t1 = Upad / kWarpTileUnits;
+        k_tile_first<<<(unsigned)((t1 - t0 + 1 + 255) / 256), 256, 0, s>>>(ctx->unit_off.p, R0 + n + 1, t0, t1, ctx->tile_first.p);
         CU_TRY(ctx, cudaGetLastError());
     }
     ctx->R = R0 + n;
-    ctx->C = C1;
+    ctx->C = C0 + nw;
+    ctx->U = U1;
     return INQ_OK;
 }
 
@@ -1071,9 +1157,10 @@ int inq_genotype(inq_ctx *ctx, uint32_t minlen, uint32_t support, int unphased, 
     unphased = unphased != 0;
     CU_TRY(ctx, cudaSetDevice(ctx->device));
     cudaStream_t s = ctx->stream;
-    const uint32_t ntiles = (uint32_t)((C + kTileWords - 1) / kTileWords);
-    if ((C + kTileWords - 1) / kTileWords > 0x7FFFFFFFull) return fail(ctx, INQ_ERR_TOO_LARGE, "too many CIGAR words");
-    const uint64_t n_wt = (uint64_t)ntiles * (kTileWords / kWarpTileWords);
+    const uint64_t U = ctx->U;
+    const uint32_t ntiles = (uint32_t)((U + kTileUnits - 1) / kTileUnits);
+    if ((U + kTileUnits - 1) / kTileUnits > 0x7FFFFFFFull) return fail(ctx, INQ_ERR_TOO_LARGE, "too many CIGAR units");
+    const uint64_t n_wt = (uint64_t)ntiles * (kTileUnits / kWarpTileUnits);
     const bool work = R && L;
     TRY(ensure(ctx, ctx->cand_lo, R));
     TRY(ensure(ctx, ctx->cand_n, R));
@@ -1082,7 +1169,7 @@ int inq_genotype(inq_ctx *ctx, uint32_t minlen, uint32_t support, int unphased, 
     TRY(ensure(ctx, ctx->wtot, n_wt + 2));
     TRY(ensure(ctx, ctx->wt_sbase, n_wt + 1));
     TRY(ensure(ctx, ctx->desc_wt, 2 * ((n_wt + kXsTile - 1) / kXsTile + 1)));       // even: k_zero clears it in 16-byte units
-    if (ntiles) TRY(make_tensor_map(ctx, (uint64_t)ntiles * kTileWords));
+    if (ntiles) TRY(make_tensor_map(ctx, (uint64_t)ntiles * kTileUnits));
     const uint64_t raw_slack = (uint64_t)ctx->sm_count * ctx->scan_ctas_per_sm * kScanWarps * kEvChunk;
     // event storage is sized speculatively (1/16 of the words; checked and regrown after the run); it hands out
     // kEvChunk-slot chunks and a warp strands the remainder of its chunk whenever a tile does not fit any more
@@ -1270,7 +1357,7 @@ int inq_debug_events(inq_ctx *ctx, uint64_t *n_events, uint32_t *event_pos, int3
     if (ctx->events.cap < E + 1) { release(ctx->events); TRY(ensure(ctx, ctx->events, E + 1)); }
     if (E) {
         const uint64_t fix_warps = (R + 1 + 30) / 31;
-        k_read_fixup<<<(unsigned)((fix_warps * 32 + 255) / 256), 256, 0, ctx->stream>>>(ctx->cig_off.p, ctx->rs.p, R, ctx->wt.p, ctx->rd_pre.p,
+        k_read_fixup<<<(unsigned)((fix_warps * 32 + 255) / 256), 256, 0, ctx->stream>>>(ctx->unit_off.p, ctx->rs.p, R, ctx->wt.p, ctx->rd_pre.p,
                                                                                        ctx->wt_sbase.p, ctx->evraw.p, ctx->evraw.cap,
                                                                                        ctx->events.p, ctx->events.cap, ctx->ev_off.p, ctx->d_ctr);
         CU_TRY(ctx, cudaGetLastError());

@@ -7,7 +7,8 @@
 //   K3  k_locus_median*   sort / split / support / median      call.rs:308-321,365-369,497-522
 //
 // Layout in HBM (all structure-of-arrays, see DESIGN.md):
-//   reads : contig/ref_start/ref_end int32[R], mapq/hp/flags u8[R], cig_off u64[R+1], cigar u32[C]
+//   reads : contig/ref_start/ref_end int32[R], mapq/hp/flags u8[R], cig_off u64[R+1] (BAM words),
+//           unit_off u64[R+1], units u16[U] (the CIGAR stream as 16-bit units, see "CIGAR units" below)
 //   loci  : start/end/pmax_end int32[L] sorted by (contig,start), contig_off int64[n_contigs+1]
 //   events: uint2{pos1 (1-based anchor, u32), val = (signed len << 1) | is_softclip}[E], ev_off u32[R+1]
 //   calls : one segment per locus sized by its candidate count (seg_off u32[L+1]); H1 from the front,
@@ -22,7 +23,7 @@ namespace inq {
 
 // ----------------------------------------------------------------------------------------------
 // constants
-constexpr int kTileWords = 8192;            // padding granularity of the device CIGAR stream (32 KB)
+constexpr int kTileUnits = 16384;           // padding granularity of the device CIGAR stream (32 KB)
 
 constexpr uint32_t kFlagBadHp = 1u << 0;
 constexpr uint32_t kFlagMedianEmpty = 1u << 1;
@@ -118,16 +119,56 @@ __device__ __forceinline__ void fence_mbar_init()
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
 }
 
-// CIGAR word decode. BAM ops MIDNSHP=X -> 0..8; M,D,N,=,X consume the reference
-// (call.rs:384-392,404): bit mask 0b1_1000_1101.
-__device__ __forceinline__ uint32_t cig_consume(uint32_t w)
+// ----------------------------------------------------------------------------------------------
+// CIGAR units. BAM words are (len << 4) | op with ops MIDNSHP=X -> 0..8; M,D,N,=,X consume the reference
+// (call.rs:384-392,404), I,D,S longer than minlen are events (call.rs:388,394,400). The device keeps the
+// stream as 16-bit units (len << 4) | op, len < 4096, written when reads are pushed:
+//   - H, P, the invalid codes 9..15 and every op of length 0 are dropped: they consume nothing and are never events;
+//   - M, N, = and X longer than 4095 are split into pieces of at most 4095 with the same op (consumption adds up);
+//   - I, D and S of length >= 4095 are a head (4095 << 4) | op followed by two payload units that hold the full
+//     length (14 bits each, op codes 12..15: no consumption, no event). A long D's head consumes 4095 and is
+//     followed by N pieces for the rest, so that consumption still adds up unit by unit.
+// So for I/D/S the 12-bit field is the exact length below 4095 and 4095 exactly for a long head: the event test on
+// the field is exact for minlen < 4095; a larger minlen looks the heads' full length up (k_cigar_scan<_, true>).
+constexpr uint32_t kUnitLong = 4095;        // field of a long I/D/S head; longest piece of a split op
+
+__device__ __forceinline__ bool op_dropped(uint32_t op) { return op > 8u || op == 5u || op == 6u; }
+__device__ __forceinline__ bool op_event_class(uint32_t op) { return ((0x16u >> op) & 1u) != 0u; }
+__device__ __forceinline__ uint32_t split_pieces(uint32_t len) { return (len + kUnitLong - 1u) / kUnitLong; }
+__device__ __forceinline__ uint16_t payload_unit(uint32_t p14) { return (uint16_t)(((p14 >> 2) << 4) | 12u | (p14 & 3u)); }
+__device__ __forceinline__ uint32_t payload_value(uint32_t u) { return ((u >> 4) << 2) | (u & 3u); }
+// full length of the long head at unit index h of the stream
+__device__ __forceinline__ uint32_t long_head_len(const uint16_t *__restrict__ units, uint64_t h)
 {
-    return ((0x18Du >> (w & 15u)) & 1u) ? (w >> 4) : 0u;
+    return payload_value(__ldg(units + h + 1)) | (payload_value(__ldg(units + h + 2)) << 14);
 }
-// op is I, D or S and longer than minlen (call.rs:388,394,400 -- strict `>`)
-__device__ __forceinline__ bool cig_is_event(uint32_t w, uint32_t minlen)
+
+// units that BAM word w becomes
+__device__ __forceinline__ uint32_t unit_count(uint32_t w)
 {
-    return (((0x16u >> (w & 15u)) & 1u) != 0u) && ((w >> 4) > minlen);
+    const uint32_t op = w & 15u, len = w >> 4;
+    if (op_dropped(op) || len == 0u) return 0u;
+    if (!op_event_class(op)) return split_pieces(len);
+    if (len < kUnitLong) return 1u;
+    return op == 2u ? 3u + split_pieces(len - kUnitLong) : 3u;
+}
+__device__ __forceinline__ void unit_write(uint32_t w, uint16_t *__restrict__ out)
+{
+    const uint32_t op = w & 15u;
+    uint32_t len = w >> 4;
+    if (op_dropped(op) || len == 0u) return;
+    uint32_t split_op = op;
+    if (op_event_class(op)) {
+        if (len < kUnitLong) { out[0] = (uint16_t)w; return; }
+        out[0] = (uint16_t)((kUnitLong << 4) | op);
+        out[1] = payload_unit(len & 0x3FFFu);
+        out[2] = payload_unit(len >> 14);
+        if (op != 2u) return;
+        out += 3;
+        len -= kUnitLong;
+        split_op = 3u;                      // the rest of a long D: N pieces
+    }
+    for (; len; len -= min(len, kUnitLong)) *out++ = (uint16_t)((min(len, kUnitLong) << 4) | split_op);
 }
 
 template <typename T>
@@ -421,38 +462,41 @@ __device__ __forceinline__ uint64_t lookback(const uint64_t *__restrict__ desc, 
 }
 
 // ----------------------------------------------------------------------------------------------
-// K2: CIGAR scan. Persistent warps stream 4 KB "warp tiles" (1024 words) of the flat packed-CIGAR array
+// K2: CIGAR scan. Persistent warps stream 4 KB "warp tiles" (2048 units) of the flat CIGAR unit stream
 // through per-warp 2-stage shared-memory rings filled by TMA (2-D tensor map, 128B swizzle); each lane
-// owns 32 consecutive words. One pass over the words gives the lane's reference consumption
-// (call.rs:384-392,404) and its event mask (I/D/S ops longer than minlen, call.rs:388,394,400); two warp
-// scans turn that into warp-local prefixes. Nothing in this kernel depends on another CTA or warp:
+// owns 64 consecutive units (32 words of two units). One pass over the units gives the lane's reference
+// consumption (call.rs:384-392,404) and its event masks (I/D/S ops longer than minlen, call.rs:388,394,400);
+// two warp scans turn that into warp-local prefixes. Nothing in this kernel depends on another CTA or warp:
 // it writes
-//   rd_pre : warp-tile-local exclusive prefixes {consumption, events} at the first word of every read
+//   rd_pre : warp-tile-local exclusive prefixes {consumption, events} at the first unit of every read
 //            that starts inside the tile (tile_first, built when reads are pushed, names those reads)
 //   wt     : totals per warp tile (prefix-summed afterwards by k_exclusive_scan2)
 //   evraw  : {bases consumed inside the warp tile before the op, (signed len << 1) | is_S}
 //            for every event, stored per warp tile in chunks handed out by one atomic
 // and k_read_fixup turns these into per-read event lists with absolute anchors.
-// Each CIGAR word is read from HBM exactly once.
+// Each unit is read from HBM exactly once (the payload of a long I/D/S head once more, from L2).
 struct ScanParams {
-    const uint32_t *tile_first;   // [n_wt + 1] first read (index into cig_off, sentinel R included) starting in warp tile t or later
-    const uint64_t *cig_off;      // [R + 1] first CIGAR word of every read (+ sentinel)
-    uint2 *rd_pre;                // [R + 1] {consumption, events} inside the read's warp tile before its first word
+    const uint32_t *tile_first;   // [n_wt + 1] first read (index into unit_off, sentinel R included) starting in warp tile t or later
+    const uint64_t *unit_off;     // [R + 1] first unit of every read (+ sentinel)
+    const uint16_t *units;        // the unit stream (payloads of long heads)
+    uint2 *rd_pre;                // [R + 1] {consumption, events} inside the read's warp tile before its first unit
     uint2 *wt;                    // [n_wt] {consumption, events} totals per warp tile (prefix-summed by k_exclusive_scan2 into a second array)
     uint32_t *wt_sbase;           // [n_wt] storage slot of the warp tile's first event
     uint2 *evraw;
     DevCounters *ctr;
     uint64_t raw_cap;             // capacity of evraw (slots)
     uint64_t n_wt;
-    uint32_t thr;                 // (min(minlen, 2^28 - 1) << 4) | 15: an op is longer than minlen iff its word > thr
+    uint32_t thr;                 // (thr16 << 16) | 0xFFFF with thr16 = (min(minlen, 4094) << 4) | 15: a unit in the
+                                  // top half of a word is longer than minlen (up to 4094) iff the word > thr
     uint32_t neg1;                // 0xFFFFFFFF as a run-time value (keeps thr - w a multiply-add on the FMA pipe)
+    uint32_t minlen;              // full minlen (the long-head variant)
 };
 
 #ifndef INQ_LANE_WORDS
 #define INQ_LANE_WORDS 32
 #endif
-constexpr int kLaneWords = INQ_LANE_WORDS;               // consecutive CIGAR words per lane (16 or 32)
-constexpr int kWarpTileWords = 32 * kLaneWords;         // 1024 words = 4 KB = one TMA box
+constexpr int kLaneWords = INQ_LANE_WORDS;               // consecutive 32-bit words (unit pairs) per lane (16 or 32)
+constexpr int kWarpTileUnits = 64 * kLaneWords;         // 2048 units = 4 KB = one TMA box
 #ifndef INQ_SCAN_WARPS
 #define INQ_SCAN_WARPS 24
 #endif
@@ -465,31 +509,29 @@ constexpr int kWarpTileWords = 32 * kLaneWords;         // 1024 words = 4 KB = o
 constexpr int kScanWarps = INQ_SCAN_WARPS;              // warps per CTA, each fully autonomous
 constexpr int kCtaThreads = kScanWarps * 32;
 constexpr int kWarpStages = INQ_WARP_STAGES;             // per-warp ring of TMA boxes
-// 64-bit LUT read through one wrap-mode funnel shift by 2*op: result bit 0 = op consumes the reference
-// (M,D,N,=,X: lo bit 2*op), result bit 31 = op is I, D or S (hi bit 2*op-1)
-constexpr uint32_t kOpLutLo = (1u << 0) | (1u << 4) | (1u << 6) | (1u << 14) | (1u << 16);
-constexpr uint32_t kOpLutHi = (1u << 1) | (1u << 3) | (1u << 7);
+// 64-bit LUT read through one wrap-mode funnel shift by 2*op or 2*op+1: result bit 0 = op consumes the reference
+// (M,D,N,=,X: lo bits 2*op and 2*op+1), result bit 31 = op is I, D or S (hi bits 2*op-1 and 2*op). Both bits of each
+// op are set so that the shift of the top unit of a word can be word >> 15, whatever bit 15 holds.
+constexpr uint32_t kOpLutLo = (3u << 0) | (3u << 4) | (3u << 6) | (3u << 14) | (3u << 16);
+constexpr uint32_t kOpLutHi = (3u << 1) | (3u << 3) | (3u << 7);
 constexpr uint32_t kEvChunk = 1024;                     // event slots a warp takes per atomic
-// cig_consume through the LUT: branch-free, the multiply issues on the FMA pipe
-__device__ __forceinline__ uint32_t cig_consume_lut(uint32_t w)
+// consumption of unit u (bits above 15 zero) through the LUT: branch-free, the multiply issues on the FMA pipe
+__device__ __forceinline__ uint32_t unit_consume(uint32_t u)
 {
-    return (w >> 4) * (__funnelshift_r(kOpLutLo, kOpLutHi, w + w) & 1u);
+    return (u >> 4) * (__funnelshift_r(kOpLutLo, kOpLutHi, u + u) & 1u);
 }
+__device__ __forceinline__ uint32_t word_consume(uint32_t x) { return unit_consume(x & 0xFFFFu) + unit_consume(x >> 16); }
 
 struct ScanSmem {
-    alignas(1024) uint32_t stage[kScanWarps][kWarpStages][kWarpTileWords];   // 128B-swizzled by the TMA tensor map
-    uint32_t snap[kScanWarps][kLaneWords / 4][32];                            // per-quad cursor snapshots of every lane
-    uint16_t qlist[kScanWarps][32];                                           // word positions of one round of events
-    alignas(8) uint64_t full[kScanWarps][kWarpStages];                        // TMA landed (tx bytes)
+    alignas(1024) uint32_t stage[kScanWarps][kWarpStages][kWarpTileUnits / 2];   // 128B-swizzled by the TMA tensor map
+    uint32_t snap[kScanWarps][kLaneWords / 4][32];                                // per-quad cursor snapshots of every lane
+    uint16_t qlist[kScanWarps][32];                                               // unit positions of one round of events
+    alignas(8) uint64_t full[kScanWarps][kWarpStages];                            // TMA landed (tx bytes)
 };
 constexpr size_t kScanSmemBytes = sizeof(ScanSmem) + 1024;   // slack to align the swizzled stages to 1 KB
 
-// word index inside a warp tile -> word index in the 128B-swizzled stage buffer
-// (16-byte chunk index bits [2:4] ^= 128-byte row index bits [5:7])
-__device__ __forceinline__ uint32_t swz(uint32_t idx) { return idx ^ (((idx >> 5) & 7u) << 2); }
-
 // `policy`: L2 cache policy of the load. The stream is read exactly once, so its lines are marked evict-first:
-// otherwise 10 GB of them flush the catalog and the per-read arrays out of the 126 MB L2, and every probe of the join
+// otherwise 5 GB of them flush the catalog and the per-read arrays out of the 126 MB L2, and every probe of the join
 // chain that runs next to the scan (and of the pair kernel after it) goes to the saturated HBM instead.
 __device__ __forceinline__ void tma_load_tile(void *dst_smem, const CUtensorMap *tmap, uint32_t row, uint64_t *bar, uint64_t policy)
 {
@@ -503,10 +545,15 @@ __device__ __forceinline__ uint64_t l2_evict_first_policy()
     asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));
     return p;
 }
+// events among the first n words of a lane's mask (word i <-> bit kLaneWords-1-i)
+__device__ __forceinline__ uint32_t events_before(uint32_t m, uint32_t n) { return n ? __popc(m >> (kLaneWords - n)) : 0u; }
+
 // Every warp is an independent pipeline: it owns warp tiles gwid, gwid + W, gwid + 2W, ... (W = warps
 // in the grid), a kWarpStages-deep ring of 4 KB shared-memory boxes (one warp tile each) that it fills itself with TMA, and the
 // mbarriers of that ring. There is no block-level synchronisation and no producer warp.
-template <bool kThrHigh>
+// kThrHigh: thr >= 2^31 (minlen >= 2048). kLongOnly: minlen >= 4095, only long heads can be events and their full
+// length decides.
+template <bool kThrHigh, bool kLongOnly>
 __global__ void __launch_bounds__(kCtaThreads, INQ_SCAN_MIN_CTAS)
 k_cigar_scan(const __grid_constant__ CUtensorMap tmap, ScanParams p)
 {
@@ -514,8 +561,9 @@ k_cigar_scan(const __grid_constant__ CUtensorMap tmap, ScanParams p)
     // keep the pointer in the shared address space (LDS/STS, not generic loads)
     ScanSmem &sm = *reinterpret_cast<ScanSmem *>(smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u));
     const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    constexpr uint32_t kBoxBytes = kWarpTileWords * 4;
-    constexpr uint32_t kRowsPerBox = kWarpTileWords / 32;       // 128-byte rows
+    constexpr uint32_t kBoxBytes = kWarpTileUnits * 2;
+    constexpr uint32_t kRowsPerBox = kWarpTileUnits / 64;       // 128-byte rows
+    constexpr uint32_t kLaneUnits = 2 * kLaneWords;
     const uint64_t gwid = (uint64_t)blockIdx.x * kScanWarps + warp, stride = (uint64_t)gridDim.x * kScanWarps;
     uint64_t *full = sm.full[warp];
     const uint64_t l2_policy = l2_evict_first_policy();
@@ -533,21 +581,21 @@ k_cigar_scan(const __grid_constant__ CUtensorMap tmap, ScanParams p)
     }
     __syncwarp();
 
-    const uint32_t thr = p.thr;                                 // (w >> 4) > minlen  <=>  w > thr
+    const uint32_t thr = p.thr;
     const uint32_t neg1 = p.neg1;
     // this lane's kLaneWords consecutive words: quads q0..q0+kLaneWords/4-1 of the box; quad q lives in
     // 128-byte row q/8 at chunk (q%8) ^ (row%8) (128B swizzle) -> conflict-free LDS.128 across the warp
     constexpr uint32_t kQuads = kLaneWords / 4;
     const uint32_t q0 = lane * kQuads;
     uint64_t chunk_cur = 0, chunk_end = 0;                      // this warp's private range of event slots
-    // reads that start inside the current warp tile: [tf_lo, tf_hi), lane i holds the first word of read
+    // reads that start inside the current warp tile: [tf_lo, tf_hi), lane i holds the first unit of read
     // tf_lo + i. Both are fetched one iteration ahead so that their latency never shows.
     uint32_t tf_lo = 0, tf_hi = 0;
     uint64_t g_cur = 0;
     if (gwid < p.n_wt) {
         tf_lo = __ldg(p.tile_first + gwid);
         tf_hi = __ldg(p.tile_first + gwid + 1);
-        if (tf_lo + lane < tf_hi) g_cur = __ldg(p.cig_off + tf_lo + lane);
+        if (tf_lo + lane < tf_hi) g_cur = __ldg(p.unit_off + tf_lo + lane);
     }
 
     for (uint32_t it = 0;; ++it) {
@@ -563,9 +611,9 @@ k_cigar_scan(const __grid_constant__ CUtensorMap tmap, ScanParams p)
         const uint32_t *stage = sm.stage[warp][s];
         const uint4 *st4 = reinterpret_cast<const uint4 *>(stage);
 
-        // ---- one pass over the lane's words. evrev: bit (31 - i) <-> word i is an event;
-        //      snap[j]: bases consumed inside the lane's words before quad j (parked in shared memory below)
-        uint32_t c = 0, evrev = 0;
+        // ---- one pass over the lane's words. ev0 / ev1: bit (kLaneWords-1 - i) <-> the low / high unit of word i
+        //      is an event; snap[j]: bases consumed inside the lane's units before quad j (parked in shared memory below)
+        uint32_t c = 0, ev0 = 0, ev1 = 0;
         uint32_t snap[kQuads];
 #pragma unroll
         for (int j = 0; j < (int)kQuads; ++j) {
@@ -575,25 +623,44 @@ k_cigar_scan(const __grid_constant__ CUtensorMap tmap, ScanParams p)
             snap[j] = c;
 #pragma unroll
             for (int k = 0; k < 4; ++k) {
+                const uint32_t x = w4[k], y = x << 16;            // y: the low unit moved to the top half
                 // one funnel shift in wrap mode indexes the LUT by 2*op without masking the op first
-                const uint32_t w = w4[k], lut = __funnelshift_r(kOpLutLo, kOpLutHi, w + w);
-                // borrow of thr - w (<=> w > thr) lands in the sign bit of d | w (thr < 2^31) or d & w
-                // (thr >= 2^31); the subtraction is a multiply-add by a run-time -1 so that it issues on
-                // the FMA pipe. One LOP3 ands it with the op class, one funnel shift appends the sign bit.
-                uint32_t d;
-                asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(d) : "r"(w), "r"(neg1), "r"(thr));
-                const uint32_t t = kThrHigh ? (lut & (d & w)) : (lut & (d | w));
-                evrev = __funnelshift_l(t, evrev, 1);
+                // (x + x for the low unit, x >> 15 for the high one: the LUT has both bits of every op)
+                const uint32_t lut0 = __funnelshift_r(kOpLutLo, kOpLutHi, x + x);
+                const uint32_t lut1 = __funnelshift_r(kOpLutLo, kOpLutHi, x >> 15);
+                // borrow of thr - u (<=> u > thr for the unit u in the top half) lands in the sign bit of d | u
+                // (thr < 2^31) or d & u (thr >= 2^31); the subtraction is a multiply-add by a run-time -1 so that it
+                // issues on the FMA pipe. One LOP3 ands it with the op class, one funnel shift appends the sign bit.
+                uint32_t d0, d1;
+                asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(d0) : "r"(y), "r"(neg1), "r"(thr));
+                asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(d1) : "r"(x), "r"(neg1), "r"(thr));
+                const uint32_t t0 = kThrHigh ? (lut0 & (d0 & y)) : (lut0 & (d0 | y));
+                const uint32_t t1 = kThrHigh ? (lut1 & (d1 & x)) : (lut1 & (d1 | x));
+                ev0 = __funnelshift_l(t0, ev0, 1);
+                ev1 = __funnelshift_l(t1, ev1, 1);
                 // c += consumes ? len : 0 as one multiply-add (FMA pipe) instead of select + add (ALU pipe)
-                asm("mad.lo.u32 %0, %1, %2, %0;" : "+r"(c) : "r"(w >> 4), "r"(lut & 1u));
+                asm("mad.lo.u32 %0, %1, %2, %0;" : "+r"(c) : "r"(y >> 20), "r"(lut0 & 1u));
+                asm("mad.lo.u32 %0, %1, %2, %0;" : "+r"(c) : "r"(x >> 20), "r"(lut1 & 1u));
             }
         }
-        const uint32_t ne = __popc(evrev);
+        if (kLongOnly) {
+            // the candidates are the long heads (field 4095); an event only if the full length is > minlen
+            const uint64_t lane_u0 = gw * kWarpTileUnits + lane * kLaneUnits;
+            for (uint32_t m = ev0; m; m &= m - 1u) {
+                const uint32_t b = __ffs(m) - 1u;
+                if (long_head_len(p.units, lane_u0 + 2u * (kLaneWords - 1u - b)) <= p.minlen) ev0 ^= 1u << b;
+            }
+            for (uint32_t m = ev1; m; m &= m - 1u) {
+                const uint32_t b = __ffs(m) - 1u;
+                if (long_head_len(p.units, lane_u0 + 2u * (kLaneWords - 1u - b) + 1u) <= p.minlen) ev1 ^= 1u << b;
+            }
+        }
+        const uint32_t ne = __popc(ev0) + __popc(ev1);
         const uint32_t incl_c = warp_incl_scan(c), incl_e = warp_incl_scan(ne);
         const uint32_t excl_c = incl_c - c, excl_e = incl_e - ne;
         const uint32_t tot_e = __shfl_sync(0xffffffffu, incl_e, 31);
         uint64_t g_nxt = 0;
-        if (nf_lo + lane < nf_hi) g_nxt = __ldg(p.cig_off + nf_lo + lane);
+        if (nf_lo + lane < nf_hi) g_nxt = __ldg(p.unit_off + nf_lo + lane);
 
         // ---- event slots: contiguous per warp tile, taken from a warp-private chunk
         uint64_t sbase = chunk_cur;
@@ -617,23 +684,26 @@ k_cigar_scan(const __grid_constant__ CUtensorMap tmap, ScanParams p)
             p.wt_sbase[gw] = (uint32_t)sbase;
         }
 
-        // ---- position queries. Two things need the tile-local prefix at a word position: every event
-        //      (about 1 % of the words -> {bases consumed before the op, value}) and the first word of every
+        // ---- position queries. Two things need the tile-local prefix at a unit position: every event
+        //      (about 1 % of the units -> {bases consumed before the op, value}) and the first unit of every
         //      read that starts in the tile (-> rd_pre). They are dealt to the lanes 32 at a time (one round
-        //      for a typical tile): the lane that owns the word supplies its scan values by shuffle and its
-        //      per-quad snapshot through shared memory; at most 3 words are re-read from the stage.
+        //      for a typical tile): the lane that owns the unit supplies its scan values by shuffle and its
+        //      per-quad snapshot through shared memory; at most 4 words are re-read from the stage.
 #pragma unroll
         for (int j = 0; j < (int)kQuads; ++j) sm.snap[warp][j][lane] = snap[j];
         const uint32_t n_starts = tf_hi - tf_lo;
-        const uint32_t n_q = tot_e + n_starts;                  // queries [0, tot_e) are the events in word order
-        const uint32_t off_cur = (uint32_t)(g_cur - gw * kWarpTileWords);    // lane i: first word of read tf_lo + i
-        uint32_t ev_left = evrev, ev_idx = excl_e;
+        const uint32_t n_q = tot_e + n_starts;                  // queries [0, tot_e) are the events in unit order
+        const uint32_t off_cur = (uint32_t)(g_cur - gw * kWarpTileUnits);    // lane i: first unit of read tf_lo + i
+        uint32_t left0 = ev0, left1 = ev1, ev_idx = excl_e;
         for (uint32_t base = 0; base < n_q; base += 32) {
-            // owners list their events with index in [base, base + 32): word order = descending bits of evrev
-            while (ev_left && ev_idx < base + 32u) {
-                const uint32_t bit = 31u - (uint32_t)__clz(ev_left);
-                ev_left ^= 1u << bit;
-                sm.qlist[warp][ev_idx - base] = (uint16_t)(lane * kLaneWords + (kLaneWords - 1u - bit));
+            // owners list their events with index in [base, base + 32) in unit order: the next word of either mask,
+            // its low unit first
+            while ((left0 | left1) && ev_idx < base + 32u) {
+                const uint32_t i0 = __clz(left0) - (32u - kLaneWords), i1 = __clz(left1) - (32u - kLaneWords);
+                const bool lo = i0 <= i1;
+                const uint32_t i = lo ? i0 : i1;
+                if (lo) left0 ^= 1u << (kLaneWords - 1u - i); else left1 ^= 1u << (kLaneWords - 1u - i);
+                sm.qlist[warp][ev_idx - base] = (uint16_t)(lane * kLaneUnits + 2u * i + (lo ? 0u : 1u));
                 ++ev_idx;
             }
             __syncwarp();
@@ -643,25 +713,29 @@ k_cigar_scan(const __grid_constant__ CUtensorMap tmap, ScanParams p)
             const uint32_t spos = __shfl_sync(0xffffffffu, off_cur, si & 31u);
             uint32_t pos = 0;
             if (is_ev) pos = sm.qlist[warp][lane];
-            else if (act) pos = (si < 32u) ? spos : (uint32_t)(__ldg(p.cig_off + tf_lo + si) - gw * kWarpTileWords);
-            const uint32_t owner = pos / kLaneWords, k = pos % kLaneWords;
+            else if (act) pos = (si < 32u) ? spos : (uint32_t)(__ldg(p.unit_off + tf_lo + si) - gw * kWarpTileUnits);
+            const uint32_t owner = pos / kLaneUnits, k = pos % kLaneUnits;
             const uint32_t xc = __shfl_sync(0xffffffffu, excl_c, owner), xe = __shfl_sync(0xffffffffu, excl_e, owner);
-            const uint32_t er = __shfl_sync(0xffffffffu, evrev, owner);
+            const uint32_t er0 = __shfl_sync(0xffffffffu, ev0, owner), er1 = __shfl_sync(0xffffffffu, ev1, owner);
             if (act) {
-                const uint32_t j = k >> 2, kk = k & 3u, q = owner * kQuads + j, row = q >> 3;
+                const uint32_t i = k >> 1, h = k & 1u, j = i >> 2, kk = i & 3u, q = owner * kQuads + j, row = q >> 3;
                 const uint4 v = st4[row * 8 + ((q & 7u) ^ (row & 7u))];
-                // a zero word (M, length 0) consumes nothing: blank the words at and after the position
-                const uint32_t c_in = xc + sm.snap[warp][j][owner] + cig_consume_lut(kk > 0u ? v.x : 0u) +
-                                      cig_consume_lut(kk > 1u ? v.y : 0u) + cig_consume_lut(kk > 2u ? v.z : 0u);
+                const uint32_t x = kk == 0u ? v.x : kk == 1u ? v.y : kk == 2u ? v.z : v.w;
+                // a zero word (two zero units) consumes nothing: blank the words at and after the position
+                const uint32_t c_in = xc + sm.snap[warp][j][owner] + word_consume(kk > 0u ? v.x : 0u) +
+                                      word_consume(kk > 1u ? v.y : 0u) + word_consume(kk > 2u ? v.z : 0u) +
+                                      (h ? unit_consume(x & 0xFFFFu) : 0u);
                 if (is_ev) {
-                    const uint32_t w = kk == 0u ? v.x : kk == 1u ? v.y : kk == 2u ? v.z : v.w;
-                    const uint32_t len = w >> 4, op = w & 15u;
+                    const uint32_t u = h ? x >> 16 : x & 0xFFFFu, op = u & 15u;
+                    uint32_t len = u >> 4;
+                    if (len == kUnitLong) len = long_head_len(p.units, gw * kWarpTileUnits + pos);
                     const int32_t val = (int32_t)(((op == 2u) ? (0u - len) : len) << 1) | (int32_t)(op == 4u);
                     const uint64_t slot = sbase + qi;
                     if (slot < p.raw_cap) p.evraw[slot] = make_uint2(c_in, (uint32_t)val);
                     else atomicOr(&p.ctr->flags, kFlagEventOverflow);
                 } else if (pos) {
-                    const uint32_t e_in = k ? __popc(er >> (kLaneWords - k)) : 0u;     // word i <-> bit kLaneWords-1-i
+                    // units before k: the low units of words [0, (k+1)/2), the high units of words [0, k/2)
+                    const uint32_t e_in = events_before(er0, (k + 1u) >> 1) + events_before(er1, k >> 1);
                     p.rd_pre[tf_lo + si] = make_uint2(c_in, xe + e_in);
                 }
             }
@@ -682,31 +756,51 @@ k_cigar_scan(const __grid_constant__ CUtensorMap tmap, ScanParams p)
     }
 }
 
-// tile_first[t] = first entry of cig_off[0, n_entries) that is >= t * kWarpTileWords (n_entries if none), for
+// tile_first[t] = first entry of unit_off[0, n_entries) that is >= t * kWarpTileUnits (n_entries if none), for
 // warp tiles t0..t1: the reads that start inside warp tile t are [tile_first[t], tile_first[t+1]).
 // Runs when reads are pushed, not per genotyping pass.
 __global__ void __launch_bounds__(256)
-k_tile_first(const uint64_t *__restrict__ cig_off, uint64_t n_entries, uint64_t t0, uint64_t t1, uint32_t *__restrict__ tile_first)
+k_tile_first(const uint64_t *__restrict__ unit_off, uint64_t n_entries, uint64_t t0, uint64_t t1, uint32_t *__restrict__ tile_first)
 {
     const uint64_t t = t0 + blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
     if (t > t1) return;
-    const uint64_t target = t * kWarpTileWords;
+    const uint64_t target = t * kWarpTileUnits;
     uint64_t lo = 0, hi = n_entries;
     while (lo < hi) {
         const uint64_t mid = (lo + hi) >> 1;
-        if (__ldg(cig_off + mid) < target) lo = mid + 1; else hi = mid;
+        if (__ldg(unit_off + mid) < target) lo = mid + 1; else hi = mid;
     }
     tile_first[t] = (uint32_t)lo;
 }
 
+// ---- encoding at push: one chunk of BAM words -> units (count, exclusive scan of the counts, write)
+__global__ void k_unit_count(const uint32_t *__restrict__ words, uint64_t n, uint32_t *__restrict__ cnt)
+{
+    for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x)
+        cnt[i] = unit_count(words[i]);
+}
+__global__ void k_unit_write(const uint32_t *__restrict__ words, uint64_t n, const uint32_t *__restrict__ off, uint16_t *__restrict__ out)
+{
+    for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x)
+        unit_write(words[i], out + off[i]);
+}
+// unit_off[r] = ubase + off[cig_off[r] - wbase] for reads [r0, r0 + n) whose first word lies in the chunk that starts at
+// stream word wbase (off: the chunk's exclusive unit offsets, one past its end included; null: no words at all)
+__global__ void k_read_units(const uint64_t *__restrict__ cig_off, uint64_t r0, uint64_t n, uint64_t wbase,
+                             const uint32_t *__restrict__ off, uint64_t ubase, uint64_t *__restrict__ unit_off)
+{
+    for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x)
+        unit_off[r0 + i] = ubase + (off ? off[cig_off[r0 + i] - wbase] : 0u);
+}
+
 // Per read: (1) the index of its first event in CIGAR order and the stream-wide consumption prefix
-// at its first word = warp-tile prefix + the tile-local prefix k_cigar_scan left in rd_pre;
+// at its first unit = warp-tile prefix + the tile-local prefix k_cigar_scan left in rd_pre;
 // (2) its events moved from warp-tile storage into CIGAR order with absolute anchors:
 // pos1 = ref_start + 1 + bases consumed by the read before the op (the u32 cursor of call.rs:380).
 // A warp owns 31 reads; lane 31 only supplies the first-event index of the next read.
 // `wt` holds EXCLUSIVE prefixes here (k_exclusive_scan2 ran in between).
 __global__ void __launch_bounds__(256)
-k_read_fixup(const uint64_t *__restrict__ cig_off, const int32_t *__restrict__ rs, uint64_t R,
+k_read_fixup(const uint64_t *__restrict__ unit_off, const int32_t *__restrict__ rs, uint64_t R,
              const uint2 *__restrict__ wt, const uint2 *__restrict__ rd_pre,
              const uint32_t *__restrict__ wt_sbase, const uint2 *__restrict__ evraw, uint64_t raw_cap,
              uint2 *__restrict__ events, uint64_t ev_cap, uint32_t *__restrict__ ev_off, DevCounters *__restrict__ ctr)
@@ -717,11 +811,11 @@ k_read_fixup(const uint64_t *__restrict__ cig_off, const int32_t *__restrict__ r
     uint32_t e = 0, c = 0;
     uint64_t g = 0;
     if (r <= R) {
-        g = cig_off[r];
-        const uint2 w0 = wt[g / kWarpTileWords];
+        g = unit_off[r];
+        const uint2 w0 = wt[g / kWarpTileUnits];
         c = w0.x;
         e = w0.y;
-        if (g % kWarpTileWords) {
+        if (g % kWarpTileUnits) {
             const uint2 pre = rd_pre[r];
             c += pre.x;
             e += pre.y;
@@ -733,7 +827,7 @@ k_read_fixup(const uint64_t *__restrict__ cig_off, const int32_t *__restrict__ r
     if (r == R) { ctr->n_events = e; return; }
     if (e == e_next) return;
     const uint32_t base = (uint32_t)rs[r] + 1u - c;
-    uint64_t gw = g / kWarpTileWords;
+    uint64_t gw = g / kWarpTileUnits;
     uint2 pre = wt[gw];
     uint32_t hi = wt[gw + 1].y;
     for (uint32_t k = e; k < e_next; ++k) {
@@ -903,19 +997,20 @@ constexpr int kPairLociCache = 128;         // catalog entries per warp kept in 
 constexpr int kPairTileCache = 64;          // warp-tile prefixes per warp kept in shared memory
 
 struct EventSource {
+    const uint64_t *unit_off;     // [R + 1] first unit of every read (+ sentinel)
     const uint2 *wt;              // [n_wt + 1] exclusive prefixes {consumption, events} per warp tile
-    const uint2 *rd_pre;          // [R + 1] tile-local prefixes at each read's first word
+    const uint2 *rd_pre;          // [R + 1] tile-local prefixes at each read's first unit
     const uint32_t *wt_sbase;     // [n_wt] storage slot of the warp tile's first event
     const uint2 *evraw;           // {consumption inside the warp tile before the op, val}
     uint64_t raw_cap;
 };
 
-// stream-wide {consumption, events} prefix at CIGAR word g, which is the first word of read r
+// stream-wide {consumption, events} prefix at unit g, which is the first unit of read r
 __device__ __forceinline__ uint2 read_prefix(const EventSource &es, uint64_t g, uint64_t r)
 {
     const uint2 pre = es.rd_pre[r];                          // unconditional: not behind the load of g
-    uint2 v = es.wt[g / kWarpTileWords];
-    if (g % kWarpTileWords) {                               // (rd_pre is only written for reads starting inside a tile)
+    uint2 v = es.wt[g / kWarpTileUnits];
+    if (g % kWarpTileUnits) {                               // (rd_pre is only written for reads starting inside a tile)
         v.x += pre.x;
         v.y += pre.y;
     }
@@ -975,17 +1070,17 @@ k_pair_eval(ReadView rv, uint64_t r_begin, uint64_t r_end, LocusView lv, int unp
         rs = rv.rs[r];
         re = rv.re[r];
         hf = (uint32_t)rv.hp[r] | ((uint32_t)(rv.flags[r] & 1u) << 8) | ((uint32_t)(rv.flags[r] & 2u) << 9);   // bit 10: SA panic
-        const uint64_t g0 = rv.cig_off[r], g1 = rv.cig_off[r + 1];
+        const uint64_t g0 = es.unit_off[r], g1 = es.unit_off[r + 1];
         const uint2 p0 = read_prefix(es, g0, r), p1 = read_prefix(es, g1, r + 1);
         e0 = p0.y;
         e1 = p1.y;
         abase = (uint32_t)rs + 1u - p0.x;                       // anchor = abase + stream-wide consumption before the op
-        t_lo = (uint32_t)(g0 / kWarpTileWords);
-        t_hi = g1 > g0 ? (uint32_t)((g1 - 1) / kWarpTileWords) : t_lo;
-        words = (uint32_t)min(g1 - g0, (uint64_t)0xFFFFFFFFu);
+        t_lo = (uint32_t)(g0 / kWarpTileUnits);
+        t_hi = g1 > g0 ? (uint32_t)((g1 - 1) / kWarpTileUnits) : t_lo;
+        words = (uint32_t)min(rv.cig_off[r + 1] - rv.cig_off[r], (uint64_t)0xFFFFFFFFu);   // BAM words: the statistics
     }
     // the events of the warp's joined reads are one run [ev_lo, ev_hi) of the event stream, stored in the
-    // warp tiles [tile_lo, tile_hi]; the tile range only depends on cig_off, so its prefixes are fetched
+    // warp tiles [tile_lo, tile_hi]; the tile range only depends on unit_off, so its prefixes are fetched
     // while the per-read prefixes are still in flight
     const uint32_t tile_lo = __reduce_min_sync(0xffffffffu, n ? t_lo : 0xFFFFFFFFu);
     const uint32_t tile_hi = __reduce_max_sync(0xffffffffu, n ? t_hi : 0u);
