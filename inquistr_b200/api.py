@@ -8,7 +8,7 @@ from dataclasses import dataclass
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-_LIB_PATH = os.environ.get("INQ_LIB") or os.path.join(_HERE, "lib", "libinqcall.so")     # INQ_LIB: tools/ sweeps over library variants
+_LIB_PATH = os.path.join(_HERE, "lib", "libinqcall.so")
 _LIB = None
 
 INQ_OK = 0
@@ -47,16 +47,15 @@ class Stats(C.Structure):
         return {n: getattr(self, n) for n, _ in self._fields_}
 
 
-def load_library(path: str | None = None):
+def load_library():
     """Load libinqcall.so; raises OSError if it has not been built (python -m inquistr_b200.build)."""
     global _LIB
-    if _LIB is not None and path is None:
+    if _LIB is not None:
         return _LIB
-    p = path or _LIB_PATH
-    if not os.path.exists(p):
-        raise OSError(f"{p} not found: build it with `python -m inquistr_b200.build` "
+    if not os.path.exists(_LIB_PATH):
+        raise OSError(f"{_LIB_PATH} not found: build it with `python -m inquistr_b200.build` "
                       "(there is no CPU fallback)")
-    L = C.CDLL(p)
+    L = C.CDLL(_LIB_PATH)
     vp, u64, u32, i32 = C.c_void_p, C.c_uint64, C.c_uint32, C.c_int32
     L.inq_ctx_create.restype = C.c_int
     L.inq_ctx_create.argtypes = [C.c_int, C.POINTER(vp)]
@@ -85,8 +84,7 @@ def load_library(path: str | None = None):
     L.inq_set_option.argtypes = [vp, C.c_char_p, C.c_int64]
     L.inq_debug_events.restype = C.c_int
     L.inq_debug_events.argtypes = [vp, C.POINTER(u64), vp, vp, u64, vp]
-    if path is None:
-        _LIB = L
+    _LIB = L
     return L
 
 
@@ -138,8 +136,8 @@ class GenotypeResult:
 class Context:
     """One GPU context (inq_ctx). Mirrors the call order of the C ABI."""
 
-    def __init__(self, device: int = 0, lib=None):
-        self._lib = lib if lib is not None else load_library()   # `lib`: a load_library(path) handle (tools/ sweeps)
+    def __init__(self, device: int = 0):
+        self._lib = load_library()
         h = C.c_void_p()
         rc = self._lib.inq_ctx_create(int(device), C.byref(h))
         if rc != INQ_OK:

@@ -33,13 +33,10 @@ bool inflate_block(const uint8_t *in, size_t in_len, uint8_t *out, size_t out_le
 {
     if (out_len == 0) return true;
     // own one-shot decoder first (inflate_fast.hpp); zlib when it declines or the CRC disagrees
-    static const bool use_fast = [] { const char *e = getenv("INQ_FAST_INFLATE"); return !e || atoi(e) != 0; }();
-    if (use_fast) {
-        thread_local FastInflater fi;
-        if (fi.inflate(in, in_len, out, out_len) && crc32_buffer(out, out_len) == crc) {
-            g_fast_blocks.fetch_add(1, std::memory_order_relaxed);
-            return true;
-        }
+    thread_local FastInflater fi;
+    if (fi.inflate(in, in_len, out, out_len) && crc32_buffer(out, out_len) == crc) {
+        g_fast_blocks.fetch_add(1, std::memory_order_relaxed);
+        return true;
     }
     g_zlib_blocks.fetch_add(1, std::memory_order_relaxed);
     z_stream zs;

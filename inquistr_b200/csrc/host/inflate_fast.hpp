@@ -12,13 +12,6 @@
 
 namespace inqhost {
 
-#ifdef INQ_INFLATE_STATS
-inline uint64_t g_st[8];                // experiments: lookups / bytes by kind
-#define INQ_ST(i, n) (g_st[i] += (n))
-#else
-#define INQ_ST(i, n) ((void)0)
-#endif
-
 class FastInflater {
 public:
     // decodes exactly out_len bytes from in[0, in_len); in must be readable up to in + in_len + 8
@@ -245,7 +238,6 @@ inline bool FastInflater::read_dynamic_header()
     if (!build(lens, hlit, kLitBits, lit_, (int)(sizeof(lit_) / sizeof(lit_[0])), false)) return false;
     if (!build(lens + hlit, hdist, kDistBits, dist_, (int)(sizeof(dist_) / sizeof(dist_[0])), true)) return false;
     fixed_loaded_ = false;
-    INQ_ST(5, 1);
     return true;
 }
 
@@ -294,16 +286,7 @@ inline int FastInflater::prepare()
             if (!fixed_loaded_) { load_fixed(); fixed_loaded_ = true; }
             return kReady;
         }
-        if (btype == 2) {
-#ifdef INQ_INFLATE_STATS
-            const uint64_t t0_ = __builtin_ia32_rdtsc();
-#endif
-            const bool ok = read_dynamic_header();
-#ifdef INQ_INFLATE_STATS
-            g_st[2] += __builtin_ia32_rdtsc() - t0_;
-#endif
-            return ok ? kReady : kFail;
-        }
+        if (btype == 2) return read_dynamic_header() ? kReady : kFail;
         return kFail;
     }
 }
@@ -335,25 +318,21 @@ inline int FastInflater::prepare()
             P##bb >>= (e & 0xFFu);                                                                                    \
             P##bc -= (int)(e & 0xFFu);                                                                                \
             *P##out++ = (uint8_t)(e >> 16);                                                                           \
-            INQ_ST(0, 1); INQ_ST(1, 1);                                                                               \
             e = P##lit[(uint32_t)P##bb & kLitMask];                                                                   \
             if (e & kLitFlag) {                                                                                       \
                 P##bb >>= (e & 0xFFu);                                                                                \
                 P##bc -= (int)(e & 0xFFu);                                                                            \
                 *P##out++ = (uint8_t)(e >> 16);                                                                       \
-                INQ_ST(1, 1);                                                                                         \
                 e = P##lit[(uint32_t)P##bb & kLitMask];                                                               \
                 if (e & kLitFlag) {                                                                                   \
                     P##bb >>= (e & 0xFFu);                                                                            \
                     P##bc -= (int)(e & 0xFFu);                                                                        \
                     *P##out++ = (uint8_t)(e >> 16);                                                                   \
-                    INQ_ST(1, 1);                                                                                     \
                     e = P##lit[(uint32_t)P##bb & kLitMask];                                                           \
                     if (e & kLitFlag) {                                                                               \
                         P##bb >>= (e & 0xFFu);                                                                        \
                         P##bc -= (int)(e & 0xFFu);                                                                    \
                         *P##out++ = (uint8_t)(e >> 16);                                                               \
-                        INQ_ST(1, 1);                                                                                 \
                     }                                                                                                 \
                 }                                                                                                     \
             }                                                                                                         \
@@ -410,7 +389,6 @@ inline int FastInflater::prepare()
         const uint8_t *src = P##out - dist;                                                                           \
         uint8_t *dst = P##out;                                                                                        \
         P##out += len;                                                                                                \
-        INQ_ST(3, 1); INQ_ST(4, len); INQ_ST(6, dist < 8); INQ_ST(7, len > 8);                                        \
         if (dist >= 8) {                                                                                              \
             do {                                                                                                      \
                 uint64_t w;                                                                                           \

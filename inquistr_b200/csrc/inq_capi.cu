@@ -58,14 +58,15 @@ struct DriverApi {
     mem_release_fn release = nullptr;
     mem_free_fn addr_free = nullptr;
     mem_gran_fn granularity = nullptr;
-    bool vmm = false;
+    const char *missing = nullptr;    // the first of the entry points above that the driver does not provide
 };
 
-void *driver_symbol(const char *name)
+void *driver_symbol(const char *name, const char *&missing)
 {
     void *fn = nullptr;
     cudaDriverEntryPointQueryResult qres;
-    if (cudaGetDriverEntryPoint(name, &fn, cudaEnableDefault, &qres) != cudaSuccess || qres != cudaDriverEntryPointSuccess) return nullptr;
+    if (cudaGetDriverEntryPoint(name, &fn, cudaEnableDefault, &qres) != cudaSuccess || qres != cudaDriverEntryPointSuccess) fn = nullptr;
+    if (!fn && !missing) missing = name;
     return fn;
 }
 
@@ -73,16 +74,15 @@ const DriverApi &driver()
 {
     static DriverApi d = [] {
         DriverApi a;
-        a.tmap_encode = (tmap_encode_fn)driver_symbol("cuTensorMapEncodeTiled");
-        a.reserve = (mem_reserve_fn)driver_symbol("cuMemAddressReserve");
-        a.create = (mem_create_fn)driver_symbol("cuMemCreate");
-        a.map = (mem_map_fn)driver_symbol("cuMemMap");
-        a.set_access = (mem_access_fn)driver_symbol("cuMemSetAccess");
-        a.unmap = (mem_unmap_fn)driver_symbol("cuMemUnmap");
-        a.release = (mem_release_fn)driver_symbol("cuMemRelease");
-        a.addr_free = (mem_free_fn)driver_symbol("cuMemAddressFree");
-        a.granularity = (mem_gran_fn)driver_symbol("cuMemGetAllocationGranularity");
-        a.vmm = a.reserve && a.create && a.map && a.set_access && a.unmap && a.release && a.addr_free && a.granularity;
+        a.tmap_encode = (tmap_encode_fn)driver_symbol("cuTensorMapEncodeTiled", a.missing);
+        a.reserve = (mem_reserve_fn)driver_symbol("cuMemAddressReserve", a.missing);
+        a.create = (mem_create_fn)driver_symbol("cuMemCreate", a.missing);
+        a.map = (mem_map_fn)driver_symbol("cuMemMap", a.missing);
+        a.set_access = (mem_access_fn)driver_symbol("cuMemSetAccess", a.missing);
+        a.unmap = (mem_unmap_fn)driver_symbol("cuMemUnmap", a.missing);
+        a.release = (mem_release_fn)driver_symbol("cuMemRelease", a.missing);
+        a.addr_free = (mem_free_fn)driver_symbol("cuMemAddressFree", a.missing);
+        a.granularity = (mem_gran_fn)driver_symbol("cuMemGetAllocationGranularity", a.missing);
         return a;
     }();
     return d;
@@ -170,7 +170,6 @@ struct inq_ctx {
     DevBuf<int32_t> contig, rs, re;
     DevBuf<uint8_t> mapq, hp, flags;
     DevBuf<uint64_t> cig_off, unit_off;
-    DevBuf<uint16_t> cigar;               // cudaMalloc'ed fallback when the driver has no VMM API
     VmStream vm;
     // encoding at push: a double-buffered staging ring of BAM words and the per-chunk unit counts / offsets
     DevBuf<uint32_t> push_stage, push_cnt, push_off;
@@ -327,15 +326,13 @@ int vm_ensure(inq_ctx *ctx, size_t bytes)
     return INQ_OK;
 }
 
-uint16_t *cigar_ptr(inq_ctx *ctx) { return driver().vmm ? reinterpret_cast<uint16_t *>(ctx->vm.base) : ctx->cigar.p; }
-uint64_t cigar_cap_units(inq_ctx *ctx) { return driver().vmm ? ctx->vm.mapped / 2 : ctx->cigar.cap; }
+uint16_t *cigar_ptr(inq_ctx *ctx) { return reinterpret_cast<uint16_t *>(ctx->vm.base); }
 
 // (re)build the TMA descriptor of the unit stream: uint32 [rows][32] (unit pairs), box = one 4 KB warp tile, 128B swizzle
 int make_tensor_map(inq_ctx *ctx, uint64_t n_units_padded)
 {
     const uint64_t rows = n_units_padded / 64;
     if (ctx->tmap_base == cigar_ptr(ctx) && ctx->tmap_rows == rows) return INQ_OK;
-    if (!driver().tmap_encode) return fail(ctx, INQ_ERR_CUDA, "cuTensorMapEncodeTiled is not available from the driver");
     const cuuint64_t gdim[2] = {32, rows};
     const cuuint64_t gstride[1] = {128};
     const cuuint32_t box[2] = {32, (cuuint32_t)(kWarpTileUnits / 64)};    // one warp tile
@@ -350,16 +347,14 @@ int make_tensor_map(inq_ctx *ctx, uint64_t n_units_padded)
     return INQ_OK;
 }
 
-// Room for nU units of the stream. What must survive a regrow is everything inq_push_reads left behind: the `keep`
-// units written so far, the zero padding up to a tile boundary (+1 tile of slack) and the tile_first entries of
-// every warp tile up to the padded end plus the sentinel slot.
-int reserve_units(inq_ctx *ctx, uint64_t nU, uint64_t keep, double growth)
+// Room for nU units of the stream, padded to a tile boundary (+1 tile of slack). The stream grows in place; what
+// must survive a regrow of tile_first are the entries of the `keep` units written so far: every warp tile up to
+// their padded end plus the sentinel slot.
+int reserve_units(inq_ctx *ctx, uint64_t nU, uint64_t keep)
 {
-    const uint64_t Upad = round_up(keep, kTileUnits);
     const uint64_t need_units = round_up(nU, kTileUnits) + kTileUnits;
-    if (driver().vmm) TRY(vm_ensure(ctx, need_units * sizeof(uint16_t)));
-    else TRY(ensure(ctx, ctx->cigar, need_units, Upad, growth));
-    TRY(ensure(ctx, ctx->tile_first, std::max(cigar_cap_units(ctx), need_units) / kWarpTileUnits + 2, keep ? Upad / kWarpTileUnits + 1 : 0, 1.0));
+    TRY(vm_ensure(ctx, need_units * sizeof(uint16_t)));
+    TRY(ensure(ctx, ctx->tile_first, ctx->vm.mapped / 2 / kWarpTileUnits + 2, keep ? round_up(keep, kTileUnits) / kWarpTileUnits + 1 : 0, 1.0));
     return INQ_OK;
 }
 
@@ -374,7 +369,7 @@ int reserve_reads(inq_ctx *ctx, uint64_t nR, uint64_t nU, double growth)
     TRY(ensure(ctx, ctx->flags, nR, R, growth));
     TRY(ensure(ctx, ctx->cig_off, nR + 1, R + 1, growth));
     TRY(ensure(ctx, ctx->unit_off, nR + 1, R + 1, growth));
-    return reserve_units(ctx, nU, R ? ctx->U : 0, growth);
+    return reserve_units(ctx, nU, R ? ctx->U : 0);
 }
 
 // ---- small kernels of the orchestration layer ---------------------------------------------------
@@ -627,9 +622,9 @@ int enqueue_pass(inq_ctx *ctx, const RunParams &rp, bool capturing, uint32_t *n_
             CU_TRY(ctx, cudaStreamWaitEvent(s2, ctx->dep[DEP_PAIRED], 0));
             CU_TRY(ctx, stamp(EV_MED0, s2));
         }
-        k_locus_median<<<(unsigned)((((uint64_t)(l1 - l0) + kMedianLociPerWarp - 1) / kMedianLociPerWarp * 32 + 255) / 256), 256, 0, s2>>>(l0, l1, c, rp.unphased, rp.support, ctx->seg_off.p, ctx->cursor.p,
-                                                                                          ctx->vals.p, ctx->vals.cap, ctx->t1.p, ctx->t2.p, ctx->valid.p,
-                                                                                          ctx->big_list.p, ctx->d_ctr);
+        k_locus_median<<<(unsigned)(((uint64_t)(l1 - l0) * 32 + 255) / 256), 256, 0, s2>>>(l0, l1, c, rp.unphased, rp.support, ctx->seg_off.p, ctx->cursor.p,
+                                                                                     ctx->vals.p, ctx->vals.cap, ctx->t1.p, ctx->t2.p, ctx->valid.p,
+                                                                                     ctx->big_list.p, ctx->d_ctr);
         CU_TRY(ctx, cudaGetLastError());
         // the CTA path for the (rare) deep loci of the chunk, between two chunks on S2
         if (!pl.big_known || pl.need_big[c]) {
@@ -718,6 +713,12 @@ int inq_ctx_create(int device, inq_ctx **out)
         inq_ctx_destroy(ctx);
         return INQ_ERR_CUDA;
     }
+    // the CIGAR stream lives in a virtual address range (cuMem*) and is read through a TMA tensor map
+    if (const char *missing = driver().missing) {
+        fail(nullptr, INQ_ERR_CUDA, "the CUDA driver does not provide %s, which libinqcall needs", missing);
+        inq_ctx_destroy(ctx);
+        return INQ_ERR_CUDA;
+    }
     ctx->sm_count = prop.multiProcessorCount;
     // the HBM-bound scan gets the SMs first; pair / median CTAs fill what its one CTA per SM leaves free
     int prio_lo = 0, prio_hi = 0;
@@ -761,7 +762,7 @@ void inq_ctx_destroy(inq_ctx *ctx)
     release(ctx->contig_off); release(ctx->lstart); release(ctx->lend); release(ctx->lpmax);
     release(ctx->contig); release(ctx->rs); release(ctx->re);
     release(ctx->mapq); release(ctx->hp); release(ctx->flags);
-    release(ctx->cig_off); release(ctx->unit_off); release(ctx->cigar);
+    release(ctx->cig_off); release(ctx->unit_off);
     release(ctx->push_stage); release(ctx->push_cnt); release(ctx->push_off); release(ctx->push_desc); release(ctx->push_ctr);
     if (ctx->vm.base) vm_release(ctx->vm);
     release(ctx->cand_lo); release(ctx->cand_n); release(ctx->ev_off);
@@ -967,7 +968,7 @@ static int push_impl(inq_ctx *ctx, uint64_t n, const int32_t *contig, const int3
         CU_TRY(ctx, cudaStreamSynchronize(s));
         if (ctx->h_total[13]) return fail(ctx, INQ_ERR_TOO_LARGE, "inq_push_reads: %llu CIGAR words expand to 2^32 units or more", (unsigned long long)m);
         const uint64_t mu = ctx->h_total[12];
-        TRY(reserve_units(ctx, U1 + mu, U1, 1.5));
+        TRY(reserve_units(ctx, U1 + mu, U1));
         k_unit_write<<<grid_for(m), 256, 0, s>>>(src, m, ctx->push_off.p, cigar_ptr(ctx) + U1);
         CU_TRY(ctx, cudaEventRecord(ctx->push_free[k & 1], s));
         // unit offsets of the reads that start in the chunk (the last chunk also takes those that start at its end)

@@ -492,23 +492,12 @@ struct ScanParams {
     uint32_t minlen;              // full minlen (the long-head variant)
 };
 
-#ifndef INQ_LANE_WORDS
-#define INQ_LANE_WORDS 32
-#endif
-constexpr int kLaneWords = INQ_LANE_WORDS;               // consecutive 32-bit words (unit pairs) per lane (16 or 32)
+constexpr int kLaneWords = 32;                          // consecutive 32-bit words (unit pairs) per lane
 constexpr int kWarpTileUnits = 64 * kLaneWords;         // 2048 units = 4 KB = one TMA box
-#ifndef INQ_SCAN_WARPS
-#define INQ_SCAN_WARPS 24
-#endif
-#ifndef INQ_WARP_STAGES
-#define INQ_WARP_STAGES 2
-#endif
-#ifndef INQ_SCAN_MIN_CTAS
-#define INQ_SCAN_MIN_CTAS 1
-#endif
-constexpr int kScanWarps = INQ_SCAN_WARPS;              // warps per CTA, each fully autonomous
+constexpr int kScanWarps = 24;                          // warps per CTA, each fully autonomous
 constexpr int kCtaThreads = kScanWarps * 32;
-constexpr int kWarpStages = INQ_WARP_STAGES;             // per-warp ring of TMA boxes
+constexpr int kWarpStages = 2;                          // per-warp ring of TMA boxes
+constexpr int kScanMinCtas = 1;
 // 64-bit LUT read through one wrap-mode funnel shift by 2*op or 2*op+1: result bit 0 = op consumes the reference
 // (M,D,N,=,X: lo bits 2*op and 2*op+1), result bit 31 = op is I, D or S (hi bits 2*op-1 and 2*op). Both bits of each
 // op are set so that the shift of the top unit of a word can be word >> 15, whatever bit 15 holds.
@@ -554,7 +543,7 @@ __device__ __forceinline__ uint32_t events_before(uint32_t m, uint32_t n) { retu
 // kThrHigh: thr >= 2^31 (minlen >= 2048). kLongOnly: minlen >= 4095, only long heads can be events and their full
 // length decides.
 template <bool kThrHigh, bool kLongOnly>
-__global__ void __launch_bounds__(kCtaThreads, INQ_SCAN_MIN_CTAS)
+__global__ void __launch_bounds__(kCtaThreads, kScanMinCtas)
 k_cigar_scan(const __grid_constant__ CUtensorMap tmap, ScanParams p)
 {
     extern __shared__ __align__(1024) unsigned char smem_raw[];
@@ -982,17 +971,9 @@ k_exclusive_scan2(const uint2 *__restrict__ in, uint2 *__restrict__ out, uint64_
 // lives in warp tile t with wt[t].y <= k < wt[t+1].y at slot wt_sbase[t] + (k - wt[t].y), and its 1-based
 // anchor (the u32 cursor of call.rs:380) is ref_start + 1 + (wt[t].x + raw.x) - (consumption prefix at the
 // read's first word).
-#ifndef INQ_PAIR_POOL
-#define INQ_PAIR_POOL 256
-#endif
-#ifndef INQ_PAIR_WARPS
-#define INQ_PAIR_WARPS 4
-#endif
-#ifndef INQ_PAIR_MIN_CTAS
-#define INQ_PAIR_MIN_CTAS (40 / INQ_PAIR_WARPS)
-#endif
-constexpr int kPairWarps = INQ_PAIR_WARPS;  // warps per CTA of k_pair_eval (each warp works alone: no block-level sync)
-constexpr int kPairEvPool = INQ_PAIR_POOL;  // events per warp (32 consecutive reads) kept in shared memory
+constexpr int kPairWarps = 4;               // warps per CTA of k_pair_eval (each warp works alone: no block-level sync)
+constexpr int kPairMinCtas = 10;            // 40 warps per SM
+constexpr int kPairEvPool = 256;            // events per warp (32 consecutive reads) kept in shared memory
 constexpr int kPairLociCache = 128;         // catalog entries per warp kept in shared memory
 constexpr int kPairTileCache = 64;          // warp-tile prefixes per warp kept in shared memory
 
@@ -1041,7 +1022,7 @@ struct PairSmem {                           // per CTA of kPairWarps warps (dyna
 };
 
 // reads [r_begin, r_end) (the pass launches it once over [0, R); bounding r by rv.R instead doubles ptxas' spills)
-__global__ void __launch_bounds__(kPairWarps * 32, INQ_PAIR_MIN_CTAS)
+__global__ void __launch_bounds__(kPairWarps * 32, kPairMinCtas)
 k_pair_eval(ReadView rv, uint64_t r_begin, uint64_t r_end, LocusView lv, int unphased, const uint32_t *__restrict__ cand_lo,
             const uint32_t *__restrict__ cand_n, EventSource es, const uint32_t *__restrict__ seg_off,
             unsigned long long *__restrict__ cursor, uint64_t *__restrict__ vals, uint64_t vals_cap,
@@ -1512,14 +1493,7 @@ __device__ __forceinline__ void warp_locus(const uint64_t *__restrict__ vals, ui
 }
 
 constexpr int kMedianWarpMax = 128;         // loci with more calls go to the CTA kernel
-
-#ifndef INQ_MEDIAN_LOCI_PER_WARP
-#define INQ_MEDIAN_LOCI_PER_WARP 1     // measured: 1 -> 0.357 ms, 2 -> 0.369-0.389, 3 -> 0.473 (the kernel is issue-bound, not latency-bound)
-#endif
-#ifndef INQ_MEDIAN_MIN_CTAS
-#define INQ_MEDIAN_MIN_CTAS (INQ_MEDIAN_LOCI_PER_WARP == 1 ? 8 : 6)
-#endif
-constexpr int kMedianLociPerWarp = INQ_MEDIAN_LOCI_PER_WARP;
+constexpr int kMedianMinCtas = 8;
 
 // header of one locus' segment
 struct LocusSeg {
@@ -1593,44 +1567,26 @@ __device__ __forceinline__ void median_one(uint32_t l, uint32_t l0, int chunk, i
     }
 }
 
-// A warp owns kMedianLociPerWarp consecutive loci (default 1). Each locus costs two dependent round trips (segment header,
-// then its calls); with several loci per warp all headers and then all key loads are in flight together before any locus is
-// reduced -- measured, it does not pay: 68 % of the issue slots are busy already and the extra registers cost occupancy.
-__global__ void __launch_bounds__(256, INQ_MEDIAN_MIN_CTAS)
+// A warp owns one locus. Each locus costs two dependent round trips (segment header, then its calls). Warps that took
+// several loci, with all headers and then all key loads in flight together before any locus was reduced, were measured
+// and do not pay: 1 locus -> 0.357 ms, 2 -> 0.369-0.389, 3 -> 0.473. The kernel is issue-bound, not latency-bound: 68 %
+// of the issue slots are busy already and the extra registers cost occupancy.
+__global__ void __launch_bounds__(256, kMedianMinCtas)
 k_locus_median(uint32_t l0, uint32_t l1, int chunk, int unphased, uint32_t support, const uint32_t *__restrict__ seg_off,
                const unsigned long long *__restrict__ cursor, const uint64_t *__restrict__ vals, uint64_t vals_cap,
                int64_t *__restrict__ twice_h1, int64_t *__restrict__ twice_h2, uint8_t *__restrict__ valid,
                uint32_t *__restrict__ big_list, DevCounters *__restrict__ ctr)
 {
     // loci [l0, l1) of the catalog (chunk < kMaxMedianChunks); the chunk's CTA-path loci are listed in big_list[l0 ...]
-    const uint32_t lw = l0 + ((blockIdx.x * blockDim.x + threadIdx.x) >> 5) * (uint32_t)kMedianLociPerWarp;
-    if (lw >= l1) return;
-    LocusSeg h[kMedianLociPerWarp];
-    bool live[kMedianLociPerWarp], fast[kMedianLociPerWarp];
-    uint64_t pre[kMedianLociPerWarp];
-    // round trip 1: the headers of all the warp's loci
-    {
-        uint32_t so[kMedianLociPerWarp + 1];
-        unsigned long long cur[kMedianLociPerWarp];
-#pragma unroll
-        for (int i = 0; i <= kMedianLociPerWarp; ++i) so[i] = (lw + i <= l1) ? seg_off[lw + i] : 0u;
-#pragma unroll
-        for (int i = 0; i < kMedianLociPerWarp; ++i) {
-            live[i] = lw + i < l1;
-            cur[i] = live[i] ? cursor[lw + i] : 0ull;
-        }
-#pragma unroll
-        for (int i = 0; i < kMedianLociPerWarp; ++i) h[i] = locus_seg(so[i], live[i] ? so[i + 1] - so[i] : 0u, cur[i], vals_cap);
-    }
-    // round trip 2: the calls of the loci on the common path
-#pragma unroll
-    for (int i = 0; i < kMedianLociPerWarp; ++i) {
-        fast[i] = live[i] && h[i].ok && !unphased && h[i].nf <= 16u && h[i].nb <= 16u;
-        pre[i] = fast[i] ? fast16_load(vals, h[i]) : kKeyInf;
-    }
-#pragma unroll
-    for (int i = 0; i < kMedianLociPerWarp; ++i)
-        if (live[i]) median_one(lw + i, l0, chunk, unphased, support, h[i], fast[i], pre[i], vals, twice_h1, twice_h2, valid, big_list, ctr);
+    const uint32_t l = l0 + ((blockIdx.x * blockDim.x + threadIdx.x) >> 5);
+    if (l >= l1) return;
+    // round trip 1: the header
+    const uint32_t seg = seg_off[l], seg_end = seg_off[l + 1];
+    const LocusSeg h = locus_seg(seg, seg_end - seg, cursor[l], vals_cap);
+    // round trip 2: the calls, on the common path
+    const bool fast = h.ok && !unphased && h.nf <= 16u && h.nb <= 16u;
+    const uint64_t pre = fast ? fast16_load(vals, h) : kKeyInf;
+    median_one(l, l0, chunk, unphased, support, h, fast, pre, vals, twice_h1, twice_h2, valid, big_list, ctr);
 }
 
 // CTA-wide path for loci with more than kMedianWarpMax calls: bitonic sort in shared memory when
