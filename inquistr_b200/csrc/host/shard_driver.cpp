@@ -37,17 +37,9 @@ std::vector<size_t> balanced_cuts(size_t L, int n, const double *weight)
 
 ShardWorker::ShardWorker(int device, size_t lo, size_t hi, int n_contigs, const std::vector<int64_t> &contig_off,
                          const int32_t *lstart, const int32_t *lend, uint32_t minlen, uint32_t support, bool unphased, int n_batches)
-    : device_(device), lo_(lo), hi_(hi), n_contigs_(n_contigs), lstart_(lstart + lo), lend_(lend + lo), minlen_(minlen),
-      support_(support), unphased_(unphased)
+    : device_(device), lo_(lo), hi_(hi), lstart_(lstart + lo), lend_(lend + lo), minlen_(minlen), support_(support), unphased_(unphased)
 {
-    off_.resize(n_contigs + 1);
-    for (int c = 0; c <= n_contigs; ++c)
-        off_[c] = (int64_t)std::min<size_t>(std::max<size_t>((size_t)contig_off[c], lo), hi) - (int64_t)lo;
-    pmax_.resize(hi - lo);
-    for (int c = 0; c < n_contigs; ++c) {
-        int32_t m = INT32_MIN;
-        for (int64_t i = off_[c]; i < off_[c + 1]; ++i) { m = std::max(m, lend_[i]); pmax_[i] = m; }
-    }
+    reach_.build(n_contigs, contig_off.data(), lstart, lend, (int64_t)lo, (int64_t)hi);     // inq_set_loci reports its faults
     // staging batches: the reader fills one while others are on their way to the device (or wait for the context)
     batches_.resize((size_t)std::max(2, n_batches));
     for (ReadBatch &b : batches_) {
@@ -82,16 +74,6 @@ ShardWorker::~ShardWorker()
         th_.join();
     }
     for (ReadBatch &b : batches_) { free(b.cigar); free(b.meta_block); }
-}
-
-bool ShardWorker::reaches(int32_t tid, int32_t pos, int32_t end) const
-{
-    if (tid < 0 || tid >= n_contigs_) return false;
-    const int64_t l0 = off_[tid], l1 = off_[tid + 1];
-    if (l0 == l1) return false;
-    // loci with start - 10 < endpos, and among them one with end + 10 > pos (SURVEY 8a A4)
-    const int64_t hi = std::lower_bound(lstart_ + l0, lstart_ + l1, (int32_t)std::min<int64_t>((int64_t)end + 10, INT32_MAX)) - lstart_;
-    return hi != l0 && (int64_t)pmax_[hi - 1] + 10 > (int64_t)pos;
 }
 
 bool ShardWorker::failed()
@@ -180,7 +162,7 @@ void ShardWorker::run()
     int rc = inq_ctx_create(device_, &ctx);
     if (rc != INQ_OK) { fail(rc, inq_last_error(nullptr)); return; }
     // shard view of the catalog: offsets relative to the slice, loci coordinates as they are
-    rc = inq_set_loci(ctx, n_contigs_, off_.data(), lstart_, lend_);
+    rc = inq_set_loci(ctx, reach_.n_contigs(), reach_.offsets(), lstart_, lend_);
     if (rc != INQ_OK) { fail(rc, inq_last_error(ctx)); inq_ctx_destroy(ctx); return; }
     // the staging batches were handed to the reader as ordinary memory before the context existed (CUDA start-up takes
     // 1-2 s next to the inflate threads: the reader must not wait for it); page-lock them now for the pushes

@@ -24,6 +24,7 @@
 #include <vector>
 
 #include "../../../include/inqcall.h"
+#include "catalog_reach.hpp"
 
 namespace inqhost {
 
@@ -61,7 +62,7 @@ public:
     size_t lo() const { return lo_; }
     size_t hi() const { return hi_; }
     // would htslib's fetch return a record [pos, end) on tid for some locus of this shard?
-    bool reaches(int32_t tid, int32_t pos, int32_t end) const;
+    bool reaches(int32_t tid, int32_t pos, int32_t end) const { return reach_.reaches(tid, pos, end); }
     // append one record to the shard's current batch (reader thread); blocks while both batches are in flight
     void add(int32_t tid, int32_t pos, int32_t end, uint8_t mapq, uint8_t hp, uint8_t flags, const uint32_t *cigar, uint32_t n_cigar);
     bool failed();                       // the worker hit an error (the reader may stop early)
@@ -80,10 +81,9 @@ private:
 
     int device_;
     size_t lo_, hi_;
-    int n_contigs_;
-    std::vector<int64_t> off_;           // per-contig offsets relative to lo_
     const int32_t *lstart_, *lend_;      // slice base pointers
-    std::vector<int32_t> pmax_;          // running max of end within (contig, shard)
+    CatalogReach reach_;                 // the slice's contig offsets (relative to lo_) and its reach index: built by the
+                                         // constructor, so the reader routes with it before the context exists
     uint32_t minlen_, support_;
     bool unphased_;
 

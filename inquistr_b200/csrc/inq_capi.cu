@@ -13,6 +13,7 @@
 // of a shape and every retry (speculative buffer regrown, CTA-path guess wrong) launch the same DAG directly.
 #include "../../include/inqcall.h"
 #include "inq_device.cuh"
+#include "host/catalog_reach.hpp"
 
 #include <algorithm>
 #include <cstdarg>
@@ -161,8 +162,7 @@ struct inq_ctx {
     int64_t L = 0;
     DevBuf<int64_t> contig_off;
     DevBuf<int32_t> lstart, lend, lpmax;
-    std::vector<int64_t> h_contig_off;    // host copies for inq_push_reads_routed (which reads can reach a locus)
-    std::vector<int32_t> h_pmax, h_lstart;
+    inqhost::CatalogReach reach;          // host index of the catalog (valid while L > 0): which reads inq_push_reads_routed takes
     void *h_route_stage = nullptr;        // pinned staging of inq_push_reads_routed when the kept reads are scattered
 
     // reads: C BAM words (the statistics count them), stored as U 16-bit units (inq_device.cuh, "CIGAR units")
@@ -831,10 +831,13 @@ int inq_set_loci(inq_ctx *ctx, int32_t n_contigs, const int64_t *contig_locus_of
         if (contig_locus_offsets[c + 1] < contig_locus_offsets[c]) return fail(ctx, INQ_ERR_ARG, "inq_set_loci: offsets not monotonic");
     if (L > 0 && (!start || !end)) return fail(ctx, INQ_ERR_ARG, "inq_set_loci: start/end are NULL");
     if ((uint64_t)L * 2 + 2 > 0x7FFFFFFFull) return fail(ctx, INQ_ERR_TOO_LARGE, "inq_set_loci: too many loci (%lld)", (long long)L);
-    CU_TRY(ctx, cudaSetDevice(ctx->device));
     ctx->n_contigs = 0;
     ctx->L = 0;
     ++ctx->data_gen;
+    // one host pass checks the catalog and builds the running max of `end` that the join reads (lpmax)
+    const inqhost::CatalogFault bad = inqhost::catalog_fault(ctx->reach.build(n_contigs, contig_locus_offsets, start, end, 0, L));
+    if (bad.code != INQ_OK) return fail(ctx, bad.code, "%s", bad.message);
+    CU_TRY(ctx, cudaSetDevice(ctx->device));
     TRY(ensure(ctx, ctx->contig_off, (uint64_t)n_contigs + 1));
     TRY(ensure(ctx, ctx->lstart, (uint64_t)L));
     TRY(ensure(ctx, ctx->lend, (uint64_t)L));
@@ -853,27 +856,9 @@ int inq_set_loci(inq_ctx *ctx, int32_t n_contigs, const int64_t *contig_locus_of
     if (L) {
         CU_TRY(ctx, cudaMemcpyAsync(ctx->lstart.p, start, (size_t)L * sizeof(int32_t), cudaMemcpyHostToDevice, s));
         CU_TRY(ctx, cudaMemcpyAsync(ctx->lend.p, end, (size_t)L * sizeof(int32_t), cudaMemcpyHostToDevice, s));
-        CU_TRY(ctx, cudaMemsetAsync(ctx->d_ctr, 0, sizeof(DevCounters), s));
-        k_locus_check<<<std::min<int64_t>((L + 255) / 256, 4096), 256, 0, s>>>(n_contigs, ctx->contig_off.p, ctx->lstart.p, ctx->lend.p, &ctx->d_ctr->flags);
-        if (n_contigs > 0) k_locus_pmax<<<n_contigs, 1024, 0, s>>>(ctx->contig_off.p, ctx->lend.p, ctx->lpmax.p);
-        CU_TRY(ctx, cudaGetLastError());
-        CU_TRY(ctx, cudaMemcpyAsync(ctx->h_ctr, ctx->d_ctr, sizeof(DevCounters), cudaMemcpyDeviceToHost, s));
-    }
-    // host copy of the running max of `end` per contig (inq_push_reads_routed); overlaps the copies above
-    ctx->h_contig_off.assign(contig_locus_offsets, contig_locus_offsets + n_contigs + 1);
-    ctx->h_pmax.resize((size_t)L);
-    ctx->h_lstart.assign(start, start + (L ? L : 0));
-    for (int32_t c = 0; c < n_contigs; ++c) {
-        int32_t m = INT32_MIN;
-        for (int64_t i = contig_locus_offsets[c]; i < contig_locus_offsets[c + 1]; ++i) { m = std::max(m, end[i]); ctx->h_pmax[(size_t)i] = m; }
+        CU_TRY(ctx, cudaMemcpyAsync(ctx->lpmax.p, ctx->reach.pmax(), (size_t)L * sizeof(int32_t), cudaMemcpyHostToDevice, s));
     }
     CU_TRY(ctx, cudaStreamSynchronize(s));
-    if (L) {
-        const unsigned f = ctx->h_ctr->flags;
-        if (f & 4u) return fail(ctx, INQ_ERR_LOCUS_ORDER, "a locus has end < start (the reference panics, repeats.rs:102-104)");
-        if (f & 2u) return fail(ctx, INQ_ERR_LOCUS_ORDER, "loci must be sorted by start within each contig");
-        if (f & 1u) return fail(ctx, INQ_ERR_LOCUS_START, "a locus has start < 10: start-10 underflows u32 in the reference (call.rs:285)");
-    }
     ctx->n_contigs = n_contigs;
     ctx->L = L;
     return INQ_OK;
@@ -1040,25 +1025,16 @@ int inq_push_reads_routed(inq_ctx *ctx, uint64_t n, const int32_t *contig, const
     if (n == 0) return INQ_OK;
     TRY(check_push_args(ctx, n, contig, ref_start, ref_end, mapq, hp, flags, cigar_off, cigar_words));
     CU_TRY(ctx, cudaSetDevice(ctx->device));
+    if (!ctx->L) return INQ_OK;           // no catalog (or one without loci): no read reaches a locus
     const int nt = std::max(1, std::min(host_threads > 0 ? host_threads : (int)std::thread::hardware_concurrency(), 256));
     // 1. which reads would htslib's fetch return for some locus of this catalog (pos < end+10 && endpos > start-10,
     //    call.rs:285-288), minus the ones the per-read half of the filters rejects everywhere (call.rs:297-300,350-352)
     std::vector<uint8_t> keep(n);
-    const int64_t *coff = ctx->h_contig_off.data();
-    const int32_t *ls = ctx->h_lstart.data(), *pm = ctx->h_pmax.data();
-    const int32_t n_contigs = ctx->n_contigs;
+    const inqhost::CatalogReach &reach = ctx->reach;
     auto mark = [&](uint64_t a, uint64_t b) {
-        for (uint64_t i = a; i < b; ++i) {
-            uint8_t k = 0;
-            const int32_t c = contig[i];
-            if (c >= 0 && c < n_contigs && coff[c] != coff[c + 1] && !((filter & INQ_ROUTE_DROP_LOW_MAPQ) && mapq[i] <= 10) &&
-                !((filter & INQ_ROUTE_DROP_NO_HP) && hp[i] == INQ_HP_ABSENT)) {
-                const int32_t *b0 = ls + coff[c], *b1 = ls + coff[c + 1];
-                const int64_t hi = std::lower_bound(b0, b1, (int32_t)std::min<int64_t>((int64_t)ref_end[i] + 10, INT32_MAX)) - ls;
-                k = hi != coff[c] && (int64_t)pm[hi - 1] + 10 > (int64_t)ref_start[i];
-            }
-            keep[i] = k;
-        }
+        for (uint64_t i = a; i < b; ++i)
+            keep[i] = !((filter & INQ_ROUTE_DROP_LOW_MAPQ) && mapq[i] <= 10) && !((filter & INQ_ROUTE_DROP_NO_HP) && hp[i] == INQ_HP_ABSENT) &&
+                      reach.reaches(contig[i], ref_start[i], ref_end[i]);
     };
     auto parallel = [&](uint64_t total, auto fn) {
         const uint64_t per = (total + nt - 1) / nt;

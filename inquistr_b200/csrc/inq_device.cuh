@@ -200,55 +200,6 @@ __device__ __forceinline__ int lower_bound_i32(const int32_t *__restrict__ a, in
 }
 
 // ----------------------------------------------------------------------------------------------
-// locus prefix-max of end, one CTA per contig (used for the phased join's lower bound)
-__global__ void k_locus_pmax(const int64_t *__restrict__ contig_off, const int32_t *__restrict__ end,
-                             int32_t *__restrict__ pmax)
-{
-    __shared__ int32_t wmax[32];
-    __shared__ int32_t carry_s;
-    const int64_t a = contig_off[blockIdx.x], b = contig_off[blockIdx.x + 1];
-    if (threadIdx.x == 0) carry_s = INT32_MIN;
-    __syncthreads();
-    for (int64_t base = a; base < b; base += blockDim.x) {
-        int64_t i = base + threadIdx.x;
-        int32_t v = i < b ? end[i] : INT32_MIN;
-#pragma unroll
-        for (int d = 1; d < 32; d <<= 1) {
-            int32_t n = __shfl_up_sync(0xffffffffu, v, d);
-            if ((int)lane_id() >= d) v = max(v, n);
-        }
-        if (lane_id() == 31) wmax[threadIdx.x >> 5] = v;
-        __syncthreads();
-        int32_t pre = carry_s;
-        for (int w = 0; w < (int)(threadIdx.x >> 5); ++w) pre = max(pre, wmax[w]);
-        v = max(v, pre);
-        if (i < b) pmax[i] = v;
-        __syncthreads();
-        if (threadIdx.x == blockDim.x - 1) carry_s = v;
-        __syncthreads();
-    }
-}
-
-// validate the catalog: sorted by start within contig, start >= 10, end >= start
-__global__ void k_locus_check(int n_contigs, const int64_t *__restrict__ contig_off,
-                              const int32_t *__restrict__ start, const int32_t *__restrict__ end,
-                              unsigned int *__restrict__ bad /* bit0 start<10, bit1 order, bit2 end<start */)
-{
-    int64_t L = contig_off[n_contigs];
-    for (int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; i < L; i += (int64_t)gridDim.x * blockDim.x) {
-        unsigned int f = 0;
-        if (start[i] < 10) f |= 1u;
-        if (end[i] < start[i]) f |= 4u;
-        if (i > 0 && start[i - 1] > start[i]) {
-            // allowed only across a contig boundary
-            int lo = 0, hi = n_contigs;          // find contig of i: last c with off[c] <= i
-            while (lo < hi) { int m = (lo + hi) >> 1; if (contig_off[m + 1] <= i) lo = m + 1; else hi = m; }
-            if (contig_off[lo] != i) f |= 2u;
-        }
-        if (f) atomicOr(bad, f);
-    }
-}
-
 __global__ void k_rebase_offsets(uint64_t *__restrict__ off, uint64_t n, uint64_t base)
 {
     for (uint64_t i = blockIdx.x * (uint64_t)blockDim.x + threadIdx.x; i < n; i += (uint64_t)gridDim.x * blockDim.x)
