@@ -14,7 +14,8 @@
  *
  * inq_assoc: per-locus association of STR length with a trait (`inquistr-b200 assoc`, DESIGN.md 5e); the model is
  * this project's own (the reference has it only as an external R script): OLS with a Student t test, or logistic
- * IRLS as R's glm.fit without step-halving with a Wald z test; design [1, covariates..., x], x last.
+ * IRLS as R's glm.fit without step-halving with a Wald z test, or Firth-penalized logistic regression with a penalized
+ * likelihood-ratio test; design [1, covariates..., x], x last.
  */
 #ifndef INQCOHORT_H
 #define INQCOHORT_H
@@ -43,22 +44,27 @@ int inq_outlier(int device, int method, uint64_t n_rows, uint32_t n_cols, const 
 
 #define INQ_ASSOC_LINEAR 0         /* OLS, t test with n - rank degrees of freedom */
 #define INQ_ASSOC_LOGISTIC 1       /* binomial / logit IRLS, Wald z test, dispersion 1 */
+#define INQ_ASSOC_FIRTH 2          /* Firth-penalized logit (Jeffreys prior), penalized likelihood-ratio chi^2 test */
 #define INQ_ASSOC_SUM 0            /* predictor H1 + H2, missing if either is NaN */
 #define INQ_ASSOC_MAX 1            /* predictor max of the non-NaN alleles, missing if both are NaN */
 
 #define INQ_ASSOC_OK 0
 #define INQ_ASSOC_FEW_SAMPLES 1    /* n <= rank, or (logistic) only one class among the samples used */
 #define INQ_ASSOC_SINGULAR 2       /* x aliased by the intercept and covariates */
-#define INQ_ASSOC_NO_CONVERGENCE 3 /* logistic: 25 iterations without meeting the deviance criterion */
-#define INQ_ASSOC_SEPARATION 4     /* logistic: a fitted probability below 10 eps or above 1 - 10 eps */
+#define INQ_ASSOC_NO_CONVERGENCE 3 /* logistic: 25 iterations without meeting the deviance criterion;
+                                      firth: the full or the null fit took 100 steps without converging */
+#define INQ_ASSOC_SEPARATION 4     /* logistic: a fitted probability below 10 eps or above 1 - 10 eps (never for firth) */
 
 #define INQ_ASSOC_MAX_COV 30       /* design columns: intercept + covariates + x <= 32 */
 
 /* Tests every row of `haps` (host memory, row-major n_rows x 2 * n_samples f64: H1, H2 of each sample, NaN = no
- * call) for association with the trait `y[n_samples]` (logistic: every value 0 or 1), adjusted for the covariates
- * `cov` (row-major n_samples x n_cov, no missing values). Per row: beta, se, stat (t or z), two-sided p (NaN when
- * the status is FEW_SAMPLES or SINGULAR), n_used (samples with a predictor) and status (INQ_ASSOC_*);
+ * call) for association with the trait `y[n_samples]` (logistic and firth: every value 0 or 1), adjusted for the
+ * covariates `cov` (row-major n_samples x n_cov, no missing values). Per row: beta, se, stat (t or z), two-sided p
+ * (NaN when the status is FEW_SAMPLES or SINGULAR), n_used (samples with a predictor) and status (INQ_ASSOC_*);
  * n_iter (nullable) is the number of weighted solves of a logistic fit (0 for linear).
+ * INQ_ASSOC_FIRTH: beta and se = sqrt((I^-1)_xx) of the penalized full fit, stat the penalized likelihood-ratio
+ * chi^2 (full against x = 0, both fits penalized by the full model's log det I), p from chi^2 with 1 df, and n_iter
+ * the full fit's number of steps.
  * Returns 0 or a negative INQ_ERR_* code (inqcall.h); inq_cohort_last_error() describes the failure. */
 int inq_assoc(int device, int model, int predictor, uint64_t n_rows, uint32_t n_samples, const double *haps,
               const double *y, uint32_t n_cov, const double *cov, double *beta, double *se, double *stat, double *p,

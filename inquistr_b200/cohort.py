@@ -9,7 +9,7 @@ from .api import INQ_OK, InqError, load_library
 
 ZSCORE, DBSCAN = 0, 1
 INQ_ERR_NO_MODE, INQ_ERR_HITS_CAP = -15, -16
-LINEAR, LOGISTIC = 0, 1
+LINEAR, LOGISTIC, FIRTH = 0, 1, 2
 PRED_SUM, PRED_MAX = 0, 1
 ASSOC_OK, ASSOC_FEW_SAMPLES, ASSOC_SINGULAR, ASSOC_NO_CONVERGENCE, ASSOC_SEPARATION = 0, 1, 2, 3, 4
 ASSOC_STATUS_NAMES = ["ok", "few_samples", "singular", "no_convergence", "separation"]
@@ -62,6 +62,7 @@ def outlier(matrix, minsize: int = 10, cutoff: float = 3.0, method: str = "zscor
 def assoc(haps, y, cov=None, model: str = "linear", predictor: str = "sum", device: int = 0):
     """Per-row association of STR length with the trait y (include/inqcohort.h inq_assoc).
     haps: rows x 2*samples f64 (H1, H2 of each sample, NaN = no call); y: samples; cov: samples x n_cov or None.
+    model: "linear", "logistic" or "firth" (Firth-penalized logistic, stat = penalized likelihood-ratio chi^2).
     -> dict of per-row arrays beta, se, stat, p (f64), n (u32), status (u8, ASSOC_*), n_iter (u8), and ms_kernel."""
     h = np.ascontiguousarray(haps, dtype=np.float64)
     rows, cols = h.shape
@@ -78,7 +79,7 @@ def assoc(haps, y, cov=None, model: str = "linear", predictor: str = "sum", devi
     out["n_iter"] = np.zeros(rows, np.uint8)
     ms = C.c_float(0)
     L = _lib()
-    rc = L.inq_assoc(device, {"linear": LINEAR, "logistic": LOGISTIC}[model], {"sum": PRED_SUM, "max": PRED_MAX}[predictor],
+    rc = L.inq_assoc(device, {"linear": LINEAR, "logistic": LOGISTIC, "firth": FIRTH}[model], {"sum": PRED_SUM, "max": PRED_MAX}[predictor],
                      rows, ns, h.ctypes.data, yy.ctypes.data, c.shape[1], c.ctypes.data if c.size else None,
                      out["beta"].ctypes.data, out["se"].ctypes.data, out["stat"].ctypes.data, out["p"].ctypes.data,
                      out["n"].ctypes.data, out["status"].ctypes.data, out["n_iter"].ctypes.data, C.byref(ms))

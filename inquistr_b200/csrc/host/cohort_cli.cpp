@@ -317,9 +317,9 @@ void append_f64(std::string &out, double v)
 // `assoc`: one regression per row of a combined table (DESIGN.md 5e)
 int assoc_main(const std::vector<std::string> &v, int device)
 {
-    const char *usage = "assoc --phenotype <TSV> --trait <COL> --model <linear|logistic> [--covariates A,B,...] [--predictor sum|max] [--device N] <COMBINED>";
+    const char *usage = "assoc --phenotype <TSV> --trait <COL> --model <linear|logistic> [--firth] [--covariates A,B,...] [--predictor sum|max] [--device N] <COMBINED>";
     std::string combined, pheno, trait, model, predictor = "sum", covs, stats_json;
-    bool has_cov = false;
+    bool has_cov = false, firth = false;
     for (size_t i = 0; i < v.size(); ++i) {
         const std::string &a = v[i];
         auto value = [&](const char *name) -> std::string {
@@ -331,7 +331,8 @@ int assoc_main(const std::vector<std::string> &v, int device)
         else if (a == "--model") {
             model = value("--model <MODEL>");
             if (model != "linear" && model != "logistic") cusage("invalid value '" + model + "' for '--model <MODEL>'\n  [possible values: linear, logistic]", usage);
-        } else if (a == "--covariates") { covs = value("--covariates <A,B,...>"); has_cov = true; }
+        } else if (a == "--firth") firth = true;
+        else if (a == "--covariates") { covs = value("--covariates <A,B,...>"); has_cov = true; }
         else if (a == "--predictor") {
             predictor = value("--predictor <PREDICTOR>");
             if (predictor != "sum" && predictor != "max") cusage("invalid value '" + predictor + "' for '--predictor <PREDICTOR>'\n  [possible values: sum, max]", usage);
@@ -348,13 +349,16 @@ int assoc_main(const std::vector<std::string> &v, int device)
                    "      --phenotype <TSV>        tab-separated phenotype table with a header; first column: sample names\n"
                    "      --trait <COL>            response column\n"
                    "      --model <MODEL>          linear (OLS, t test) or logistic (0/1 trait, IRLS, Wald z test) [possible values: linear, logistic]\n"
+                   "      --firth                  with --model logistic: Firth-penalized fit (finite under separation) and\n"
+                   "                               penalized likelihood-ratio test\n"
                    "      --covariates <A,B,...>   0 to %d covariate columns; samples with a missing value (NA, NaN, empty) are left out\n"
                    "      --predictor <PREDICTOR>  per sample and locus: H1 + H2, or the larger allele [default: sum] [possible values: sum, max]\n"
                    "      --device <N>             CUDA device [default: 0]\n"
                    "      --stats-json <FILE>      write parse, device and output times to FILE\n"
                    "  -h, --help                   Print help\n\n"
                    "Output: chromosome begin end n beta se stat p status, one row per input row; status is one of ok,\n"
-                   "few_samples, singular, no_convergence, separation\n", usage, INQ_ASSOC_MAX_COV);
+                   "few_samples, singular, no_convergence, separation. With --firth, stat is the penalized likelihood-ratio\n"
+                   "chi-square (1 df) of x, p comes from it, and separation is never reported\n", usage, INQ_ASSOC_MAX_COV);
             return 0;
         } else if (!a.empty() && a[0] == '-' && a.size() > 1) cusage("unexpected argument '" + a + "' found", usage);
         else if (combined.empty()) combined = a;
@@ -366,6 +370,7 @@ int assoc_main(const std::vector<std::string> &v, int device)
     if (model.empty()) missing += "\n  --model <MODEL>";
     if (combined.empty()) missing += "\n  <COMBINED>";
     if (!missing.empty()) cusage("the following required arguments were not provided:" + missing, usage);
+    if (firth && model != "logistic") cusage("the argument '--firth' requires '--model logistic'", usage);
     std::vector<std::string> cov_names;
     if (has_cov && !covs.empty()) {
         size_t a = 0;
@@ -471,7 +476,7 @@ int assoc_main(const std::vector<std::string> &v, int device)
     const uint32_t ns = (uint32_t)use_idx.size();
     fputs("chromosome\tbegin\tend\tn\tbeta\tse\tstat\tp\tstatus\n", stdout);
     const char *status_names[] = {"ok", "few_samples", "singular", "no_convergence", "separation"};
-    const int mdl = logistic ? INQ_ASSOC_LOGISTIC : INQ_ASSOC_LINEAR, prd = predictor == "max" ? INQ_ASSOC_MAX : INQ_ASSOC_SUM;
+    const int mdl = firth ? INQ_ASSOC_FIRTH : logistic ? INQ_ASSOC_LOGISTIC : INQ_ASSOC_LINEAR, prd = predictor == "max" ? INQ_ASSOC_MAX : INQ_ASSOC_SUM;
 
     // rows in batches of at most 256 MB of values
     const size_t batch_rows = std::max<size_t>(1, (256u << 20) / ((size_t)ns * 2 * sizeof(double)));

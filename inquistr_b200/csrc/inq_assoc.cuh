@@ -304,4 +304,270 @@ k_assoc(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_samples, ui
     }
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// Firth-penalized logistic regression (DESIGN.md 5e, Firth). Per locus two fits, the full one (free set F = K) and
+// the null one (F = K \ {x}, beta_x = 0), each from beta = 0; K is the rank set decided at the first evaluation.
+// A step is two sweeps over the samples:
+//   A: at beta, eta, mu, w = mu (1 - mu), the deviance and I = X_K' W X_K; factor I = L D L' over K;
+//      D* = deviance - log det I. If D* rose, beta moves half way back to beta_prev and A runs again (<= 5 times).
+//   B: at the same beta, h_i = w_i x_i' I^-1 x_i, U* = X'(y - mu + h (1/2 - mu)), H = X' diag(w (1 + h)) X;
+//      delta_F = H_FF^-1 U*_F, lambda^2 = delta_F . U*_F; converged below 1e-10, else beta += delta.
+// For B, the factor of I is kept in per-warp shared memory as L^-1 (unit lower triangular) and 1/d, so lane l gets
+// h of its own sample as w sum_c (1/d_c) ((L^-1 u)_c)^2 from dot products of broadcast rows of L^-1 with its design
+// row u: no per-lane vector is held next to the accumulators. Centring x and the covariates is a unit-triangular
+// change of columns; it leaves every quantity of the iteration, and log det I, unchanged.
+constexpr int kFMaxSteps = 100;            // steps per fit
+constexpr int kFMaxHalvings = 5;           // halvings per step
+constexpr double kFLambda2 = 1e-10;        // convergence: delta_F . U*_F below this
+constexpr double kFRise = 1e-12;           // halve when D* > D*_prev + kFRise (|D*_prev| + 1)
+
+template <int P>
+__global__ void __launch_bounds__(kAWarps * 32)
+k_assoc_firth(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_samples, uint32_t p, int use_max,
+              const double *__restrict__ design, const double *__restrict__ shift, const double *__restrict__ y, AssocOut out)
+{
+    constexpr int S = P + 1;
+    __shared__ double s_des[kATile][S];
+    __shared__ double s_y[kATile];
+    __shared__ double s_beta[kAWarps][P];
+    __shared__ double s_li[kAWarps][P][P];     // L^-1 of the warp's last factor of I (identity outside K)
+    __shared__ double s_dinv[kAWarps][P];      // 1 / d_c for c in K, 0 elsewhere
+    __shared__ double s_full[kAWarps][3];      // the full fit's beta_x, se and D*
+    const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const uint64_t row = (uint64_t)blockIdx.x * kAWarps + warp;
+    const bool have = row < n_rows;
+    const double2 *h = reinterpret_cast<const double2 *>(haps + (have ? row : 0) * 2ull * n_samples);
+    const uint32_t xcol = p - 1;
+
+    // samples used, mean of x, cases
+    double sx = 0.0, sy = 0.0;
+    uint32_t cnt = 0;
+    if (have)
+        for (uint32_t s = lane; s < n_samples; s += 32) {
+            const double2 v = h[s];
+            const double x = use_max ? fmax(v.x, v.y) : v.x + v.y;
+            if (x == x) { sx += x; sy += y[s]; ++cnt; }
+        }
+    uint32_t n = cnt;
+#pragma unroll
+    for (int o = 16; o; o >>= 1) n += __shfl_xor_sync(0xffffffffu, n, o);
+    const double xbar = n ? warp_sum(sx) / n : 0.0;
+    const double cases = warp_sum(sy);
+
+    uint8_t status = INQ_ASSOC_OK;
+    bool done = !have;
+    if (have && (n == 0 || cases == 0.0 || cases == (double)n)) { status = INQ_ASSOC_FEW_SAMPLES; done = true; }
+    if (lane < P) s_beta[warp][lane] = 0.0;
+
+    const double my_shift = lane == xcol ? xbar : (lane < P ? shift[lane] : 0.0);
+    // b / b_prev: this lane's coefficient (lane < P); dpen: D* at b; dpen_prev: D* at b_prev; dx: pivot of x in I
+    double b = 0.0, b_prev = 0.0, dpen = 0.0, dpen_prev = 0.0, dx = 0.0;
+    uint32_t kmask = 0;
+    int fit = 0, t = 0, halvings = 0, t_full = 0;
+    bool first = true, sweep_b = false, conv_full = false;
+    for (;;) {
+        if (__syncthreads_and(done)) break;
+        // A: row `lane` of I, the deviance, the uncentred G_jj (first sweep only, for the rank rule)
+        // B: row `lane` of H and U*_lane
+        double G[P];
+#pragma unroll
+        for (int k = 0; k < P; ++k) G[k] = 0.0;
+        double gx = 0.0, rhs = 0.0, diag = 0.0, dsum = 0.0;
+        for (uint32_t s0 = 0; s0 < n_samples; s0 += kATile) {
+            __syncthreads();
+            for (uint32_t i = threadIdx.x; i < (uint32_t)kATile * P; i += blockDim.x) {
+                const uint32_t r = i / P, c = i % P, s = s0 + r;
+                s_des[r][c] = s < n_samples ? design[(uint64_t)s * P + c] : 0.0;
+            }
+            if (threadIdx.x < kATile) s_y[threadIdx.x] = s0 + threadIdx.x < n_samples ? y[s0 + threadIdx.x] : 0.0;
+            __syncthreads();
+            if (done) continue;
+            const uint32_t s = s0 + lane;
+            double xt = __longlong_as_double(0x7ff8000000000000ll);
+            if (s < n_samples) {
+                const double2 v = h[s];
+                xt = (use_max ? fmax(v.x, v.y) : v.x + v.y) - xbar;
+            }
+            const bool valid = xt == xt;
+            const double yl = s_y[lane];
+            double eta = 0.0;
+#pragma unroll
+            for (int k = 0; k < P; ++k) eta = fma(s_beta[warp][k], s_des[lane][k], eta);
+            eta = fma(s_beta[warp][xcol], xt, eta);     // the x slot of s_des is 0
+            double mu, omu;
+            logit_linkinv(eta, &mu, &omu);
+            const double w = mu * omu;
+            double W = w, r = 0.0;
+            if (!sweep_b) {
+                if (valid) dsum += yl != 0.0 ? -2.0 * log(mu) : -2.0 * log(omu);
+            } else {
+                // x' I^-1 x of this lane's sample: sum_c (1/d_c) z_c^2, z = L^-1 u, u = [design row, x]
+                double q = 0.0;
+#pragma unroll 1
+                for (int c = 0; c < (int)p; ++c) {
+                    double z = 0.0;
+#pragma unroll 4
+                    for (int k = 0; k <= c; ++k) z = fma(s_li[warp][k][c], s_des[lane][k], z);
+                    if (c == (int)xcol) z = fma(s_li[warp][c][c], xt, z);
+                    q = fma(s_dinv[warp][c] * z, z, q);
+                }
+                const double hh = w * q;
+                W = w * (1.0 + hh);
+                r = (yl != 0.0 ? omu : -mu) + hh * (0.5 - mu);
+            }
+            unsigned m = __ballot_sync(0xffffffffu, valid);
+            while (m) {
+                const int i = __ffs(m) - 1;
+                m &= m - 1;
+                const double xi = __shfl_sync(0xffffffffu, xt, i);
+                const double wi = __shfl_sync(0xffffffffu, W, i);
+                const double ri = __shfl_sync(0xffffffffu, r, i);
+                const double uj = lane == xcol ? xi : (lane < P ? s_des[i][lane < P ? lane : 0] : 0.0);
+                const double a = wi * uj;
+#pragma unroll
+                for (int k = 0; k < P; ++k) G[k] = fma(a, s_des[i][k], G[k]);
+                gx = fma(a, xi, gx);
+                rhs = fma(ri, uj, rhs);
+                if (first) {
+                    const double raw = uj + my_shift;
+                    diag = fma(wi * raw, raw, diag);
+                }
+            }
+        }
+        if (done) { continue; }
+#pragma unroll
+        for (int k = 0; k < P; ++k) if (k == (int)xcol) G[k] = gx;
+        if (!sweep_b) {
+            // LDL' of I over K (the first time: K by the rank rule); lane j > c keeps L_jc in G[c]
+            const double dev = warp_sum(dsum);
+            uint32_t kept = 0;
+            double logdet = 0.0, d_x = 0.0, my_dinv = 0.0;
+#pragma unroll
+            for (int c = 0; c < P; ++c) {
+                if (c >= (int)p) break;
+                const double d = __shfl_sync(0xffffffffu, G[c], c);
+                if (first) {
+                    const double sc = __shfl_sync(0xffffffffu, diag, c);
+                    if (!(d > kAAlias * sc)) continue;
+                } else if (!((kmask >> c) & 1u)) continue;
+                kept |= 1u << c;
+                logdet += log(d);
+                if (c == (int)xcol) d_x = d;
+                if ((int)lane == c) my_dinv = 1.0 / d;
+                const double l = G[c] / d;
+#pragma unroll
+                for (int k = c + 1; k < P; ++k) {
+                    if (k >= (int)p) break;
+                    const double gck = __shfl_sync(0xffffffffu, G[k], c);
+                    if ((int)lane > c) G[k] = fma(-l, gck, G[k]);
+                }
+                if ((int)lane > c) G[c] = l;
+            }
+            if (first) {
+                first = false;
+                kmask = kept;
+                if (n <= (uint32_t)__popc(kept)) { status = INQ_ASSOC_FEW_SAMPLES; done = true; }
+                else if (!((kept >> xcol) & 1u)) { status = INQ_ASSOC_SINGULAR; done = true; }
+                if (done) continue;
+            }
+            const double dnew = dev - logdet;
+            if (t > 0 && dnew > dpen_prev + kFRise * (fabs(dpen_prev) + 1.0) && halvings < kFMaxHalvings) {
+                b = 0.5 * (b + b_prev);
+                ++halvings;
+                __syncwarp();
+                if (lane < P) s_beta[warp][lane] = b;
+                __syncwarp();
+                continue;
+            }
+            dpen = dnew;
+            dx = d_x;
+            // L^-1 column by column from the rows of L in G (strictly lower, 0 outside K):
+            // (L^-1)_jk = -sum_{m = k..j-1} L_jm (L^-1)_mk, lane j gets row j once rows k..j-1 are final.
+            // Stored transposed, s_li[k][j] = (L^-1)_jk, so the lanes write consecutive words.
+            const bool my_kept = (kmask >> lane) & 1u;
+#pragma unroll
+            for (int m = 0; m < P; ++m)
+                if (!(m < (int)lane && my_kept && ((kmask >> m) & 1u))) G[m] = 0.0;
+            __syncwarp();
+#pragma unroll
+            for (int k = 0; k < P; ++k) {
+                double lk = (int)lane == k ? 1.0 : 0.0, acc = 0.0;
+#pragma unroll
+                for (int m = k; m < P - 1; ++m) {
+                    const double v = __shfl_sync(0xffffffffu, lk, m);
+                    acc = fma(G[m], v, acc);                    // G[m] = 0 unless m < lane
+                    if ((int)lane == m + 1) lk = -acc;
+                }
+                if (lane < P) s_li[warp][k][lane] = lk;
+            }
+            if (lane < P) s_dinv[warp][lane] = my_dinv;
+            __syncwarp();
+            sweep_b = true;
+            continue;
+        }
+        // B: delta_F = H_FF^-1 U*_F by LDL' over F, then back substitution
+        sweep_b = false;
+        const uint32_t fmask = fit == 0 ? kmask : kmask & ~(1u << xcol);
+        const double u = rhs;
+#pragma unroll
+        for (int c = 0; c < P; ++c) {
+            if (c >= (int)p || !((fmask >> c) & 1u)) continue;
+            const double d = __shfl_sync(0xffffffffu, G[c], c);
+            const double l = G[c] / d;
+            const double bc = __shfl_sync(0xffffffffu, rhs, c);
+#pragma unroll
+            for (int k = c + 1; k < P; ++k) {
+                if (k >= (int)p) break;
+                const double gck = __shfl_sync(0xffffffffu, G[k], c);
+                if ((int)lane > c) G[k] = fma(-l, gck, G[k]);
+            }
+            if ((int)lane > c) rhs = fma(-l, bc, rhs);
+        }
+        double acc = 0.0, delta = 0.0;
+#pragma unroll
+        for (int c = P - 1; c >= 0; --c) {
+            if (c >= (int)p || !((fmask >> c) & 1u)) continue;
+            const double dc = __shfl_sync(0xffffffffu, (rhs - acc) / G[c], c);
+            if ((int)lane == c) delta = dc;
+            if ((int)lane < c) acc = fma(G[c], dc, acc);
+        }
+        const double lam2 = warp_sum(lane < P && ((fmask >> lane) & 1u) ? delta * u : 0.0);
+        const bool conv = lam2 < kFLambda2;
+        if (!conv && t < kFMaxSteps) {
+            b_prev = b;
+            dpen_prev = dpen;
+            b += delta;
+            ++t;
+            halvings = 0;
+        } else if (fit == 0) {
+            // full fit done: keep its result, start the null fit from beta = 0
+            if (lane == xcol) { s_full[warp][0] = b; s_full[warp][1] = sqrt(1.0 / dx); s_full[warp][2] = dpen; }
+            t_full = t;
+            conv_full = conv;
+            fit = 1;
+            b = b_prev = 0.0;
+            t = halvings = 0;
+        } else {
+            if (lane == 0) {
+                const double stat = fmax(0.0, dpen - s_full[warp][2]);
+                out.beta[row] = s_full[warp][0]; out.se[row] = s_full[warp][1]; out.stat[row] = stat; out.p[row] = erfc(sqrt(0.5 * stat));
+            }
+            if (!conv_full || !conv) status = INQ_ASSOC_NO_CONVERGENCE;
+            done = true;
+        }
+        __syncwarp();
+        if (lane < P) s_beta[warp][lane] = b;
+        __syncwarp();
+    }
+    if (have && lane == 0) {
+        if (status == INQ_ASSOC_FEW_SAMPLES || status == INQ_ASSOC_SINGULAR) {
+            const double nan = __longlong_as_double(0x7ff8000000000000ll);
+            out.beta[row] = nan; out.se[row] = nan; out.stat[row] = nan; out.p[row] = nan;
+        }
+        out.n_used[row] = n;
+        out.status[row] = status;
+        if (out.n_iter) out.n_iter[row] = (uint8_t)t_full;
+    }
+}
+
 }  // namespace inqa

@@ -166,7 +166,7 @@ int inq_assoc(int device, int model, int predictor, uint64_t n_rows, uint32_t n_
 {
     using namespace inqa;
     if (ms_kernel) *ms_kernel = 0.f;
-    if (model != INQ_ASSOC_LINEAR && model != INQ_ASSOC_LOGISTIC) return cfail(INQ_ERR_ARG, "inq_assoc: unknown model %d", model);
+    if (model != INQ_ASSOC_LINEAR && model != INQ_ASSOC_LOGISTIC && model != INQ_ASSOC_FIRTH) return cfail(INQ_ERR_ARG, "inq_assoc: unknown model %d", model);
     if (predictor != INQ_ASSOC_SUM && predictor != INQ_ASSOC_MAX) return cfail(INQ_ERR_ARG, "inq_assoc: unknown predictor %d", predictor);
     if (n_cov > INQ_ASSOC_MAX_COV) return cfail(INQ_ERR_ARG, "inq_assoc: %u covariates (at most %d)", n_cov, INQ_ASSOC_MAX_COV);
     if (n_rows == 0) return INQ_OK;
@@ -175,7 +175,7 @@ int inq_assoc(int device, int model, int predictor, uint64_t n_rows, uint32_t n_
     if ((n_rows + kAWarps - 1) / kAWarps > 0x7FFFFFFFull) return cfail(INQ_ERR_TOO_LARGE, "inq_assoc: too many rows");
     for (uint32_t s = 0; s < n_samples; ++s) {
         if (!std::isfinite(y[s])) return cfail(INQ_ERR_ARG, "inq_assoc: trait of sample %u is not a finite number", s);
-        if (model == INQ_ASSOC_LOGISTIC && y[s] != 0.0 && y[s] != 1.0) return cfail(INQ_ERR_ARG, "inq_assoc: logistic trait of sample %u is not 0 or 1", s);
+        if (model != INQ_ASSOC_LINEAR && y[s] != 0.0 && y[s] != 1.0) return cfail(INQ_ERR_ARG, "inq_assoc: logistic trait of sample %u is not 0 or 1", s);
         for (uint32_t c = 0; c < n_cov; ++c)
             if (!std::isfinite(cov[(size_t)s * n_cov + c])) return cfail(INQ_ERR_ARG, "inq_assoc: covariate %u of sample %u is not a finite number", c, s);
     }
@@ -240,7 +240,14 @@ int inq_assoc(int device, int model, int predictor, uint64_t n_rows, uint32_t n_
     const int lg = model == INQ_ASSOC_LOGISTIC, mx = predictor == INQ_ASSOC_MAX;
     const double *dh = (const double *)d_haps, *dd = (const double *)d_des, *ds = (const double *)d_shift, *dy = (const double *)d_y;
     CC_TRY(cudaEventRecord(g.e0, g.s));
-    switch (P) {
+    if (model == INQ_ASSOC_FIRTH) {
+        switch (P) {
+        case 4: k_assoc_firth<4><<<grid, kAWarps * 32, 0, g.s>>>(dh, n_rows, n_samples, pdim, mx, dd, ds, dy, out); break;
+        case 8: k_assoc_firth<8><<<grid, kAWarps * 32, 0, g.s>>>(dh, n_rows, n_samples, pdim, mx, dd, ds, dy, out); break;
+        case 16: k_assoc_firth<16><<<grid, kAWarps * 32, 0, g.s>>>(dh, n_rows, n_samples, pdim, mx, dd, ds, dy, out); break;
+        default: k_assoc_firth<32><<<grid, kAWarps * 32, 0, g.s>>>(dh, n_rows, n_samples, pdim, mx, dd, ds, dy, out); break;
+        }
+    } else switch (P) {
     case 4: k_assoc<4><<<grid, kAWarps * 32, 0, g.s>>>(dh, n_rows, n_samples, pdim, lg, mx, dd, ds, dy, out); break;
     case 8: k_assoc<8><<<grid, kAWarps * 32, 0, g.s>>>(dh, n_rows, n_samples, pdim, lg, mx, dd, ds, dy, out); break;
     case 16: k_assoc<16><<<grid, kAWarps * 32, 0, g.s>>>(dh, n_rows, n_samples, pdim, lg, mx, dd, ds, dy, out); break;

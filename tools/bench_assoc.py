@@ -3,9 +3,11 @@
 samples, 12 covariates, 10 % missing calls, about 20 % constant loci, seeded. Prints one JSON line per model x
 predictor with the kernel time (CUDA events, H2D excluded; median of --reps runs after a warm-up), loci/s, the f64
 FMAs the fits need (from shapes and iteration counts) and GFLOP/s, and parity of --parity random loci against the
-numpy restatement (oracle/assoc.py, not R) with its host time. Then one line per model for the CLI on the same table
-written as TSV: wall time with text parse, device and output time separated (`--stats-json`). The card's name and
-power limit are read in the same run. Temporary files go to a temporary directory."""
+numpy restatement (oracle/assoc.py, not R) with its host time. `firth` lines (the case/control trait, `--firth`)
+report the steps of the full fit over every locus and of both fits on the parity loci (tests/firth_oracle.py, not
+logistf) instead of FMAs. Then one line per model for the CLI on the same table written as TSV: wall time with text
+parse, device and output time separated (`--stats-json`). The card's name and power limit are read in the same run.
+Temporary files go to a temporary directory."""
 import argparse
 import json
 import os
@@ -66,11 +68,12 @@ def main():
     args = ap.parse_args()
     from inquistr_b200 import cohort
     from oracle import assoc as A
+    from tests import firth_oracle as FO
     name = card()
     haps, cov, y_lin, y_bin = workload(args.rows, args.samples, args.cov)
     p = args.cov + 2
     sel = np.sort(np.random.default_rng(7).choice(args.rows, min(args.parity, args.rows), replace=False))
-    for model in ("linear", "logistic"):
+    for model in ("linear", "logistic", "firth"):
         y = y_lin if model == "linear" else y_bin
         for pred in ("sum", "max"):
             res = cohort.assoc(haps, y, cov, model, pred)                # warm-up
@@ -79,21 +82,31 @@ def main():
                 res = cohort.assoc(haps, y, cov, model, pred)
                 ms.append(res["ms_kernel"])
             med = float(np.median(ms))
-            f = fmas(res, p, model)
+            f = fmas(res, p, model) if model != "firth" else None
             t0 = time.perf_counter()
-            ref = A.assoc_matrix(haps[sel], y, cov, model, pred)
+            if model == "firth":
+                ref = FO.assoc_matrix(haps[sel], y, cov, pred)
+            else:
+                ref = A.assoc_matrix(haps[sel], y, cov, model, pred)
             oracle_s = time.perf_counter() - t0
             st = res["status"][sel]
             ok = (ref["status"] == A.OK) & (st == A.OK)
-            if model == "logistic":
+            if model != "linear":
                 ok &= res["n_iter"][sel] == ref["n_iter"]
             rb = np.abs(res["beta"][sel][ok] - ref["beta"][ok]) / (np.abs(ref["beta"][ok]) + ref["se"][ok])
             rs = np.abs(res["se"][sel][ok] / ref["se"][ok] - 1)
             lp = np.abs(np.log10(np.maximum(res["p"][sel][ok], 1e-300)) - np.log10(np.maximum(ref["p"][ok], 1e-300)))
+            steps = {}
+            if model == "firth":                                        # over the loci with a fit (not few_samples / singular)
+                fitted, rf = ~np.isin(res["status"], (1, 2)), ~np.isin(ref["status"], (1, 2))
+                steps = {"full_steps_mean": float(res["n_iter"][fitted].mean()), "full_steps_max": int(res["n_iter"][fitted].max()),
+                         "parity_full_steps_mean": float(ref["n_iter"][rf].mean()), "parity_full_steps_max": int(ref["n_iter"][rf].max()),
+                         "parity_null_steps_mean": float(ref["n_iter_null"][rf].mean()),
+                         "parity_null_steps_max": int(ref["n_iter_null"][rf].max())}
             print(json.dumps({
                 "bench": "assoc_kernel", "card": name, "model": model, "predictor": pred, "loci": args.rows,
                 "samples": args.samples, "covariates": args.cov, "kernel_ms_median": med, "kernel_ms_all": ms,
-                "loci_per_s": args.rows / (med * 1e-3), "f64_fma": f, "gflops": 2 * f / (med * 1e-3) / 1e9,
+                "loci_per_s": args.rows / (med * 1e-3), "f64_fma": f, "gflops": 2 * f / (med * 1e-3) / 1e9 if f else None, **steps,
                 "status_counts": {A.STATUS_NAMES[k]: int((res["status"] == k).sum()) for k in range(5)},
                 "mean_iterations": float(res["n_iter"][res["status"] != 1].mean()) if model == "logistic" else 0.0,
                 "parity": {"loci": int(len(sel)), "status_equal": bool(np.array_equal(st, ref["status"])),
@@ -121,10 +134,11 @@ def main():
             f.write("sample\tlin\tbin\t" + "\t".join(f"c{c}" for c in range(args.cov)) + "\n")
             for i, s in enumerate(samples):
                 f.write(f"{s}\t{float(y_lin[i])!r}\t{int(y_bin[i])}\t" + "\t".join(repr(float(v)) for v in cov[i]) + "\n")
-        for model, trait in (("linear", "lin"), ("logistic", "bin")):
+        for model, trait in (("linear", "lin"), ("logistic", "bin"), ("firth", "bin")):
             sj = os.path.join(d, "stats.json")
+            flags = ["--model", "logistic", "--firth"] if model == "firth" else ["--model", model]
             t0 = time.perf_counter()
-            r = subprocess.run([exe, "assoc", "--phenotype", ph, "--trait", trait, "--model", model, "--covariates",
+            r = subprocess.run([exe, "assoc", "--phenotype", ph, "--trait", trait, *flags, "--covariates",
                                 ",".join(f"c{c}" for c in range(args.cov)), "--stats-json", sj, table],
                                stdout=subprocess.PIPE, stderr=subprocess.PIPE)
             wall = time.perf_counter() - t0
