@@ -1,23 +1,28 @@
-// inq_assoc.cuh -- sm_100a kernel of `assoc`: per-locus linear / logistic regression of a trait on STR length.
+// inq_assoc.cuh -- sm_100a kernels of `assoc`: per-locus regression of a trait on STR length. k_assoc fits the
+// linear and the logistic model, k_assoc_firth the Firth-penalized logistic model (DESIGN.md 5e).
 //
-// One warp per locus, four loci per CTA. The design is [1, covariates..., x] with x last (p <= 32 columns); lane j
-// owns row j of the (weighted) Gram matrix G and entry j of X'Wz, in f64 registers (P = p rounded up to 4, 8, 16 or
-// 32 is a template parameter, so the rows stay in registers). The CTA stages tiles of 32 samples of the design rows
-// shared by all loci (intercept + covariates, centred by their mean over the samples used) and of the trait in
-// shared memory, so the sample count is not bounded by shared memory. Lane l of a warp reads sample s0 + l of its
-// locus (two haplotype values), forms the predictor, and computes that sample's eta, mu, weight and working response;
-// the warp then walks the valid samples of the tile and every lane adds its row's terms.
+// Both kernels have one layout. One warp per locus, four loci per CTA. The design is [1, covariates..., x] with x last
+// (p <= 32 columns); lane j owns row j of the matrix being accumulated and entry j of the right-hand side, in f64
+// registers (P = p rounded up to 4, 8, 16 or 32 is a template parameter, so the rows stay in registers). Each kernel
+// keeps its own iteration logic and builds every sweep over the samples from the same routines:
+//   locus_prepass    n (the samples with a call), the mean of x over them, and the sum of the trait over them.
+//   stage_tile       the CTA stages a tile of 32 samples of the design rows shared by all loci (intercept +
+//                    covariates, centred by their mean over the samples used) and of the trait in shared memory, so
+//                    the sample count is not bounded by shared memory.
+//   lane_x           lane l reads sample s0 + l of its locus (two haplotype values) and forms the centred predictor.
+//   lane_eta         eta of that sample under the warp's coefficients; the kernel then forms the sample's weight W and
+//                    the value v its right-hand side is built from.
+//   accumulate_tile  the warp walks the valid samples of the tile (ballot) and every lane adds its row's terms of
+//                    sum W u u' and of the right-hand side, and of the uncentred G_jj of the rank rule.
+//   ldl_solve        symmetric Gaussian elimination (LDL') without pivoting, one row per lane, over the columns the
+//                    caller keeps (a dropped column gets coefficient 0), then back substitution.
+//   write_tail       NaN for the loci without a fit; n, status and the iteration count of every locus.
+// The warps of a CTA run their sweeps in lock step (the tiles are shared); a warp whose locus is done idles.
 //
 // The predictor is centred per locus (mean over the samples used there), so the normal equations see centred
 // columns. The rank rule compares each elimination pivot d_j (the weighted residual sum of squares of column j
 // after the kept earlier columns, which centring does not change) with 1e-10 * G_jj of the UNcentred design.
-// Elimination is symmetric Gaussian elimination (LDL') without pivoting, one row per lane; an aliased column is
-// skipped (coefficient 0, rank - 1). With x last, (G^-1)_xx = 1 / d_x.
-//
-// Linear: pass 0 accumulates G (W = 1, z = y - mean y), solve, pass 1 sums the squared residuals.
-// Logistic (R's glm.fit without step-halving): pass t evaluates eta = X beta_t (t = 0: the start mu = (y + 1/2) / 2),
-// mu, the deviance of beta_t, and the weights / working response of the next solve, and accumulates that solve's G.
-// The warps of a CTA run their passes in lock step (the tiles are shared); a warp whose locus is done idles.
+// An aliased column is skipped (coefficient 0, rank - 1). With x last, (G^-1)_xx = 1 / d_x.
 #pragma once
 
 #include <cuda_runtime.h>
@@ -102,16 +107,166 @@ struct AssocOut {
     uint8_t *status, *n_iter;
 };
 
+__device__ __forceinline__ double predictor(double2 v, int use_max) { return use_max ? fmax(v.x, v.y) : v.x + v.y; }
+
+struct LocusSums {
+    uint32_t n;                            // samples with a call
+    double xbar, cases;                    // mean of x over them, sum of the trait over them
+};
+
+__device__ __forceinline__ LocusSums locus_prepass(const double2 *h, const double *__restrict__ y, uint32_t n_samples,
+                                                   int use_max, bool have, uint32_t lane)
+{
+    double sx = 0.0, sy = 0.0;
+    uint32_t cnt = 0;
+    if (have)
+        for (uint32_t s = lane; s < n_samples; s += 32) {
+            const double x = predictor(h[s], use_max);
+            if (x == x) { sx += x; sy += y[s]; ++cnt; }
+        }
+    uint32_t n = cnt;
+#pragma unroll
+    for (int o = 16; o; o >>= 1) n += __shfl_xor_sync(0xffffffffu, n, o);
+    return {n, n ? warp_sum(sx) / n : 0.0, warp_sum(sy)};
+}
+
 // design: n_samples x P (row stride P): [1, centred covariates..., 0 (the slot of x), 0 padding]
-// shift : P column shifts (covariate means; 0 for the intercept and x), to rebuild the uncentred G_jj
-// y     : n_samples trait values (linear: centred by their mean)
+// s_des has the odd row stride P + 1 in doubles, so lane-per-row reads spread over the banks. tid is threadIdx.x of the
+// caller: the kernel's read carries the range [0, kAWarps * 32) of __launch_bounds__, and with it the compiler needs no
+// guard in front of the first trip of the loop below (a read here would get a guard branch per tile).
+template <int P>
+__device__ __forceinline__ void stage_tile(double (*s_des)[P + 1], double *s_y, const double *__restrict__ design,
+                                           const double *__restrict__ y, uint32_t s0, uint32_t n_samples, uint32_t tid)
+{
+    __syncthreads();
+    for (uint32_t t = tid; t < (uint32_t)kATile * P; t += blockDim.x) {
+        const uint32_t r = t / P, c = t % P, s = s0 + r;
+        s_des[r][c] = s < n_samples ? design[(uint64_t)s * P + c] : 0.0;
+    }
+    if (tid < kATile) s_y[tid] = s0 + tid < n_samples ? y[s0 + tid] : 0.0;
+    __syncthreads();
+}
+
+// x - xbar of sample s; NaN for a sample without a call and for the padding of the last tile
+__device__ __forceinline__ double lane_x(const double2 *h, uint32_t s, uint32_t n_samples, int use_max, double xbar)
+{
+    double xt = __longlong_as_double(0x7ff8000000000000ll);
+    if (s < n_samples) xt = predictor(h[s], use_max) - xbar;
+    return xt;
+}
+
+template <int P>
+__device__ __forceinline__ double lane_eta(const double *beta, const double *des, uint32_t xcol, double xt)
+{
+    double eta = 0.0;
+#pragma unroll
+    for (int k = 0; k < P; ++k) eta = fma(beta[k], des[k], eta);
+    return fma(beta[xcol], xt, eta);       // the x slot of s_des is 0
+}
+
+// The ballot walk over the valid samples of the tile: u = [design row, x] of sample i, lane j adds W_i u_i u_ij to
+// row j of G (its x entry to gx: a run-time index into G would put G in local memory; put_x moves it in),
+// rhs_term(W_i u_ij, u_ij, v_i, rhs) to rhs and, with with_diag, W_i (u_ij + shift_j)^2 to diag, the uncentred G_jj.
+// Each kernel keeps its own expression for the right-hand side: fma(W u, z, .) and fma(W z, u, .) round differently.
+template <int P, class RhsTerm>
+__device__ __forceinline__ void accumulate_tile(double (&G)[P], double &gx, double &rhs, double &diag,
+                                                const double (*s_des)[P + 1], uint32_t lane, uint32_t xcol, bool valid,
+                                                double xt, double W, double v, double my_shift, bool with_diag,
+                                                RhsTerm rhs_term)
+{
+    unsigned m = __ballot_sync(0xffffffffu, valid);
+    while (m) {
+        const int i = __ffs(m) - 1;
+        m &= m - 1;
+        const double xi = __shfl_sync(0xffffffffu, xt, i);
+        const double wi = __shfl_sync(0xffffffffu, W, i);
+        const double vi = __shfl_sync(0xffffffffu, v, i);
+        const double uj = lane == xcol ? xi : (lane < P ? s_des[i][lane < P ? lane : 0] : 0.0);
+        const double a = wi * uj;
+#pragma unroll
+        for (int k = 0; k < P; ++k) G[k] = fma(a, s_des[i][k], G[k]);
+        gx = fma(a, xi, gx);
+        rhs = rhs_term(a, uj, vi, rhs);
+        if (with_diag) {
+            const double raw = uj + my_shift;
+            diag = fma(wi * raw, raw, diag);
+        }
+    }
+}
+
+template <int P>
+__device__ __forceinline__ void put_x(double (&G)[P], double gx, uint32_t xcol)
+{
+#pragma unroll
+    for (int k = 0; k < P; ++k) if (k == (int)xcol) G[k] = gx;
+}
+
+// Solves G b = rhs over the columns c < p that keep(c, d_c) accepts, d_c the pivot of column c after the kept earlier
+// columns; G is overwritten. -> this lane's coefficient (0 for a dropped column and for lanes >= p).
+template <int P, class Keep>
+__device__ __forceinline__ double ldl_solve(double (&G)[P], double rhs, uint32_t p, uint32_t lane, Keep keep)
+{
+    uint32_t kept = 0;
+#pragma unroll
+    for (int c = 0; c < P; ++c) {
+        if (c >= (int)p) break;
+        const double d = __shfl_sync(0xffffffffu, G[c], c);
+        if (!keep(c, d)) continue;
+        kept |= 1u << c;
+        const double l = G[c] / d;
+        const double bc = __shfl_sync(0xffffffffu, rhs, c);
+#pragma unroll
+        for (int k = c + 1; k < P; ++k) {
+            if (k >= (int)p) break;
+            const double gck = __shfl_sync(0xffffffffu, G[k], c);
+            if ((int)lane > c) G[k] = fma(-l, gck, G[k]);
+        }
+        if ((int)lane > c) rhs = fma(-l, bc, rhs);
+    }
+    double acc = 0.0, b = 0.0;
+#pragma unroll
+    for (int c = P - 1; c >= 0; --c) {
+        if (c >= (int)p || !((kept >> c) & 1u)) continue;
+        const double bc = __shfl_sync(0xffffffffu, (rhs - acc) / G[c], c);
+        if ((int)lane == c) b = bc;
+        if ((int)lane < c) acc = fma(G[c], bc, acc);
+    }
+    return b;
+}
+
+template <int P>
+__device__ __forceinline__ void publish_beta(double *s_beta, uint32_t lane, double b)
+{
+    __syncwarp();
+    if (lane < P) s_beta[lane] = b;
+    __syncwarp();
+}
+
+__device__ __forceinline__ void write_tail(const AssocOut &out, uint64_t row, bool have, uint32_t lane, uint32_t n,
+                                           uint8_t status, int n_iter)
+{
+    if (have && lane == 0) {
+        if (status == INQ_ASSOC_FEW_SAMPLES || status == INQ_ASSOC_SINGULAR) {
+            const double nan = __longlong_as_double(0x7ff8000000000000ll);
+            out.beta[row] = nan; out.se[row] = nan; out.stat[row] = nan; out.p[row] = nan;
+        }
+        out.n_used[row] = n;
+        out.status[row] = status;
+        if (out.n_iter) out.n_iter[row] = (uint8_t)n_iter;
+    }
+}
+
+// Linear: pass 0 accumulates G (W = 1, z = y - mean y), solve, pass 1 sums the squared residuals.
+// Logistic (R's glm.fit without step-halving): pass t evaluates eta = X beta_t (t = 0: the start mu = (y + 1/2) / 2),
+// mu, the deviance of beta_t, and the weights / working response of the next solve, and accumulates that solve's G.
+// shift: P column shifts (covariate means; 0 for the intercept and x), to rebuild the uncentred G_jj
+// y    : n_samples trait values (linear: centred by their mean)
 template <int P>
 __global__ void __launch_bounds__(kAWarps * 32)
 k_assoc(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_samples, uint32_t p, int logistic, int use_max,
         const double *__restrict__ design, const double *__restrict__ shift, const double *__restrict__ y, AssocOut out)
 {
-    constexpr int S = P + 1;                              // odd row stride in doubles: lane-per-row reads spread over banks
-    __shared__ double s_des[kATile][S];
+    __shared__ double s_des[kATile][P + 1];
     __shared__ double s_y[kATile];
     __shared__ double s_beta[kAWarps][P];
     const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -119,21 +274,7 @@ k_assoc(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_samples, ui
     const bool have = row < n_rows;
     const double2 *h = reinterpret_cast<const double2 *>(haps + (have ? row : 0) * 2ull * n_samples);
     const uint32_t xcol = p - 1;
-
-    // pass A: samples used, mean of x, cases
-    double sx = 0.0, sy = 0.0;
-    uint32_t cnt = 0;
-    if (have)
-        for (uint32_t s = lane; s < n_samples; s += 32) {
-            const double2 v = h[s];
-            const double x = use_max ? fmax(v.x, v.y) : v.x + v.y;
-            if (x == x) { sx += x; sy += y[s]; ++cnt; }
-        }
-    uint32_t n = cnt;
-#pragma unroll
-    for (int o = 16; o; o >>= 1) n += __shfl_xor_sync(0xffffffffu, n, o);
-    const double xbar = n ? warp_sum(sx) / n : 0.0;
-    const double cases = warp_sum(sy);
+    const auto [n, xbar, cases] = locus_prepass(h, y, n_samples, use_max, have, lane);
 
     uint8_t status = INQ_ASSOC_OK;
     bool done = !have;
@@ -149,31 +290,17 @@ k_assoc(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_samples, ui
         double G[P];
 #pragma unroll
         for (int k = 0; k < P; ++k) G[k] = 0.0;
-        double gx = 0.0, rhs = 0.0, diag = 0.0, dsum = 0.0;
+        double gx = 0.0, rhs = 0.0, diag = 0.0;
+        double dsum = 0.0;
         bool sep_l = false;
         const bool need_gram = !done && (logistic || pass == 0);
         for (uint32_t s0 = 0; s0 < n_samples; s0 += kATile) {
-            __syncthreads();
-            for (uint32_t t = threadIdx.x; t < (uint32_t)kATile * P; t += blockDim.x) {
-                const uint32_t r = t / P, c = t % P, s = s0 + r;
-                s_des[r][c] = s < n_samples ? design[(uint64_t)s * P + c] : 0.0;
-            }
-            if (threadIdx.x < kATile) s_y[threadIdx.x] = s0 + threadIdx.x < n_samples ? y[s0 + threadIdx.x] : 0.0;
-            __syncthreads();
+            stage_tile<P>(s_des, s_y, design, y, s0, n_samples, threadIdx.x);
             if (done) continue;
-            const uint32_t s = s0 + lane;
-            double xt = __longlong_as_double(0x7ff8000000000000ll);
-            if (s < n_samples) {
-                const double2 v = h[s];
-                xt = (use_max ? fmax(v.x, v.y) : v.x + v.y) - xbar;
-            }
+            const double xt = lane_x(h, s0 + lane, n_samples, use_max, xbar);
             const bool valid = xt == xt;
             const double yl = s_y[lane];
-            // eta of this lane's sample under the current coefficients
-            double eta = 0.0;
-#pragma unroll
-            for (int k = 0; k < P; ++k) eta = fma(s_beta[warp][k], s_des[lane][k], eta);
-            eta = fma(s_beta[warp][xcol], xt, eta);     // the x slot of s_des is 0
+            double eta = lane_eta<P>(s_beta[warp], s_des[lane], xcol, xt);
             double W = 1.0, z = yl;
             if (logistic) {
                 if (pass == 0) {
@@ -194,22 +321,8 @@ k_assoc(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_samples, ui
                 dsum = fma(r, r, dsum);
             }
             if (!need_gram) continue;
-            unsigned m = __ballot_sync(0xffffffffu, valid);
-            while (m) {
-                const int i = __ffs(m) - 1;
-                m &= m - 1;
-                const double xi = __shfl_sync(0xffffffffu, xt, i);
-                const double wi = __shfl_sync(0xffffffffu, W, i);
-                const double zi = __shfl_sync(0xffffffffu, z, i);
-                const double uj = lane == xcol ? xi : (lane < P ? s_des[i][lane < P ? lane : 0] : 0.0);
-                const double a = wi * uj;
-#pragma unroll
-                for (int k = 0; k < P; ++k) G[k] = fma(a, s_des[i][k], G[k]);
-                gx = fma(a, xi, gx);
-                rhs = fma(a, zi, rhs);
-                const double raw = uj + my_shift;
-                diag = fma(wi * raw, raw, diag);
-            }
+            accumulate_tile<P>(G, gx, rhs, diag, s_des, lane, xcol, valid, xt, W, z, my_shift, true,
+                               [](double a, double, double zi, double rhs) { return fma(a, zi, rhs); });
         }
         if (!done) {
             const double dev = warp_sum(dsum);             // deviance of the current coefficients (linear: RSS)
@@ -244,39 +357,16 @@ k_assoc(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_samples, ui
             }
             dev_old = dev;
             if (solve) {
-                // G[k] for the x column: gx; symmetric elimination, one row per lane
-#pragma unroll
-                for (int k = 0; k < P; ++k) if (k == (int)xcol) G[k] = gx;
+                put_x(G, gx, xcol);
                 uint32_t kept = 0;
-                int rk = 0;
                 double d_x = 0.0;
-#pragma unroll
-                for (int c = 0; c < P; ++c) {
-                    if (c >= (int)p) break;
-                    const double d = __shfl_sync(0xffffffffu, G[c], c);
-                    const double sc = __shfl_sync(0xffffffffu, diag, c);
-                    if (!(d > kAAlias * sc)) continue;          // aliased (or empty) column: dropped
+                const double b = ldl_solve<P>(G, rhs, p, lane, [&](int c, double d) {
+                    if (!(d > kAAlias * __shfl_sync(0xffffffffu, diag, c))) return false;   // aliased (or empty) column
                     kept |= 1u << c;
-                    ++rk;
                     if (c == (int)xcol) d_x = d;
-                    const double l = G[c] / d;
-                    const double bc = __shfl_sync(0xffffffffu, rhs, c);
-#pragma unroll
-                    for (int k = c + 1; k < P; ++k) {
-                        if (k >= (int)p) break;
-                        const double gck = __shfl_sync(0xffffffffu, G[k], c);
-                        if ((int)lane > c) G[k] = fma(-l, gck, G[k]);
-                    }
-                    if ((int)lane > c) rhs = fma(-l, bc, rhs);
-                }
-                double acc = 0.0, b = 0.0;
-#pragma unroll
-                for (int c = P - 1; c >= 0; --c) {
-                    if (c >= (int)p || !((kept >> c) & 1u)) continue;
-                    const double bc = __shfl_sync(0xffffffffu, (rhs - acc) / G[c], c);
-                    if ((int)lane == c) b = bc;
-                    if ((int)lane < c) acc = fma(G[c], bc, acc);
-                }
+                    return true;
+                });
+                const int rk = __popc(kept);
                 if (pass == 0) rank = rk;
                 if (pass == 0 && n <= (uint32_t)rk) { status = INQ_ASSOC_FEW_SAMPLES; done = true; }
                 else if (!((kept >> xcol) & 1u)) { status = INQ_ASSOC_SINGULAR; done = true; }
@@ -284,24 +374,14 @@ k_assoc(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_samples, ui
                     rank = rk;
                     dx = d_x;
                     beta_lane = b;
-                    __syncwarp();
-                    if (lane < P) s_beta[warp][lane] = b;
-                    __syncwarp();
+                    publish_beta<P>(s_beta[warp], lane, b);
                     if (logistic) ++iter;
                 }
             }
         }
         ++pass;
     }
-    if (have && lane == 0) {
-        if (status == INQ_ASSOC_FEW_SAMPLES || status == INQ_ASSOC_SINGULAR) {
-            const double nan = __longlong_as_double(0x7ff8000000000000ll);
-            out.beta[row] = nan; out.se[row] = nan; out.stat[row] = nan; out.p[row] = nan;
-        }
-        out.n_used[row] = n;
-        out.status[row] = status;
-        if (out.n_iter) out.n_iter[row] = (uint8_t)iter;
-    }
+    write_tail(out, row, have, lane, n, status, iter);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -326,8 +406,7 @@ __global__ void __launch_bounds__(kAWarps * 32)
 k_assoc_firth(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_samples, uint32_t p, int use_max,
               const double *__restrict__ design, const double *__restrict__ shift, const double *__restrict__ y, AssocOut out)
 {
-    constexpr int S = P + 1;
-    __shared__ double s_des[kATile][S];
+    __shared__ double s_des[kATile][P + 1];
     __shared__ double s_y[kATile];
     __shared__ double s_beta[kAWarps][P];
     __shared__ double s_li[kAWarps][P][P];     // L^-1 of the warp's last factor of I (identity outside K)
@@ -338,21 +417,7 @@ k_assoc_firth(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_sampl
     const bool have = row < n_rows;
     const double2 *h = reinterpret_cast<const double2 *>(haps + (have ? row : 0) * 2ull * n_samples);
     const uint32_t xcol = p - 1;
-
-    // samples used, mean of x, cases
-    double sx = 0.0, sy = 0.0;
-    uint32_t cnt = 0;
-    if (have)
-        for (uint32_t s = lane; s < n_samples; s += 32) {
-            const double2 v = h[s];
-            const double x = use_max ? fmax(v.x, v.y) : v.x + v.y;
-            if (x == x) { sx += x; sy += y[s]; ++cnt; }
-        }
-    uint32_t n = cnt;
-#pragma unroll
-    for (int o = 16; o; o >>= 1) n += __shfl_xor_sync(0xffffffffu, n, o);
-    const double xbar = n ? warp_sum(sx) / n : 0.0;
-    const double cases = warp_sum(sy);
+    const auto [n, xbar, cases] = locus_prepass(h, y, n_samples, use_max, have, lane);
 
     uint8_t status = INQ_ASSOC_OK;
     bool done = !have;
@@ -372,28 +437,15 @@ k_assoc_firth(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_sampl
         double G[P];
 #pragma unroll
         for (int k = 0; k < P; ++k) G[k] = 0.0;
-        double gx = 0.0, rhs = 0.0, diag = 0.0, dsum = 0.0;
+        double gx = 0.0, rhs = 0.0, diag = 0.0;
+        double dsum = 0.0;
         for (uint32_t s0 = 0; s0 < n_samples; s0 += kATile) {
-            __syncthreads();
-            for (uint32_t i = threadIdx.x; i < (uint32_t)kATile * P; i += blockDim.x) {
-                const uint32_t r = i / P, c = i % P, s = s0 + r;
-                s_des[r][c] = s < n_samples ? design[(uint64_t)s * P + c] : 0.0;
-            }
-            if (threadIdx.x < kATile) s_y[threadIdx.x] = s0 + threadIdx.x < n_samples ? y[s0 + threadIdx.x] : 0.0;
-            __syncthreads();
+            stage_tile<P>(s_des, s_y, design, y, s0, n_samples, threadIdx.x);
             if (done) continue;
-            const uint32_t s = s0 + lane;
-            double xt = __longlong_as_double(0x7ff8000000000000ll);
-            if (s < n_samples) {
-                const double2 v = h[s];
-                xt = (use_max ? fmax(v.x, v.y) : v.x + v.y) - xbar;
-            }
+            const double xt = lane_x(h, s0 + lane, n_samples, use_max, xbar);
             const bool valid = xt == xt;
             const double yl = s_y[lane];
-            double eta = 0.0;
-#pragma unroll
-            for (int k = 0; k < P; ++k) eta = fma(s_beta[warp][k], s_des[lane][k], eta);
-            eta = fma(s_beta[warp][xcol], xt, eta);     // the x slot of s_des is 0
+            const double eta = lane_eta<P>(s_beta[warp], s_des[lane], xcol, xt);
             double mu, omu;
             logit_linkinv(eta, &mu, &omu);
             const double w = mu * omu;
@@ -415,28 +467,11 @@ k_assoc_firth(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_sampl
                 W = w * (1.0 + hh);
                 r = (yl != 0.0 ? omu : -mu) + hh * (0.5 - mu);
             }
-            unsigned m = __ballot_sync(0xffffffffu, valid);
-            while (m) {
-                const int i = __ffs(m) - 1;
-                m &= m - 1;
-                const double xi = __shfl_sync(0xffffffffu, xt, i);
-                const double wi = __shfl_sync(0xffffffffu, W, i);
-                const double ri = __shfl_sync(0xffffffffu, r, i);
-                const double uj = lane == xcol ? xi : (lane < P ? s_des[i][lane < P ? lane : 0] : 0.0);
-                const double a = wi * uj;
-#pragma unroll
-                for (int k = 0; k < P; ++k) G[k] = fma(a, s_des[i][k], G[k]);
-                gx = fma(a, xi, gx);
-                rhs = fma(ri, uj, rhs);
-                if (first) {
-                    const double raw = uj + my_shift;
-                    diag = fma(wi * raw, raw, diag);
-                }
-            }
+            accumulate_tile<P>(G, gx, rhs, diag, s_des, lane, xcol, valid, xt, W, r, my_shift, first,
+                               [](double, double uj, double ri, double rhs) { return fma(ri, uj, rhs); });
         }
         if (done) { continue; }
-#pragma unroll
-        for (int k = 0; k < P; ++k) if (k == (int)xcol) G[k] = gx;
+        put_x(G, gx, xcol);
         if (!sweep_b) {
             // LDL' of I over K (the first time: K by the rank rule); lane j > c keeps L_jc in G[c]
             const double dev = warp_sum(dsum);
@@ -474,9 +509,7 @@ k_assoc_firth(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_sampl
             if (t > 0 && dnew > dpen_prev + kFRise * (fabs(dpen_prev) + 1.0) && halvings < kFMaxHalvings) {
                 b = 0.5 * (b + b_prev);
                 ++halvings;
-                __syncwarp();
-                if (lane < P) s_beta[warp][lane] = b;
-                __syncwarp();
+                publish_beta<P>(s_beta[warp], lane, b);
                 continue;
             }
             dpen = dnew;
@@ -495,7 +528,7 @@ k_assoc_firth(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_sampl
 #pragma unroll
                 for (int m = k; m < P - 1; ++m) {
                     const double v = __shfl_sync(0xffffffffu, lk, m);
-                    acc = fma(G[m], v, acc);                    // G[m] = 0 unless m < lane
+                    acc = fma(G[m], v, acc);                  // G[m] = 0 unless m < lane
                     if ((int)lane == m + 1) lk = -acc;
                 }
                 if (lane < P) s_li[warp][k][lane] = lk;
@@ -505,33 +538,11 @@ k_assoc_firth(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_sampl
             sweep_b = true;
             continue;
         }
-        // B: delta_F = H_FF^-1 U*_F by LDL' over F, then back substitution
+        // B: delta_F = H_FF^-1 U*_F over F; rhs keeps U*
         sweep_b = false;
         const uint32_t fmask = fit == 0 ? kmask : kmask & ~(1u << xcol);
-        const double u = rhs;
-#pragma unroll
-        for (int c = 0; c < P; ++c) {
-            if (c >= (int)p || !((fmask >> c) & 1u)) continue;
-            const double d = __shfl_sync(0xffffffffu, G[c], c);
-            const double l = G[c] / d;
-            const double bc = __shfl_sync(0xffffffffu, rhs, c);
-#pragma unroll
-            for (int k = c + 1; k < P; ++k) {
-                if (k >= (int)p) break;
-                const double gck = __shfl_sync(0xffffffffu, G[k], c);
-                if ((int)lane > c) G[k] = fma(-l, gck, G[k]);
-            }
-            if ((int)lane > c) rhs = fma(-l, bc, rhs);
-        }
-        double acc = 0.0, delta = 0.0;
-#pragma unroll
-        for (int c = P - 1; c >= 0; --c) {
-            if (c >= (int)p || !((fmask >> c) & 1u)) continue;
-            const double dc = __shfl_sync(0xffffffffu, (rhs - acc) / G[c], c);
-            if ((int)lane == c) delta = dc;
-            if ((int)lane < c) acc = fma(G[c], dc, acc);
-        }
-        const double lam2 = warp_sum(lane < P && ((fmask >> lane) & 1u) ? delta * u : 0.0);
+        const double delta = ldl_solve<P>(G, rhs, p, lane, [&](int c, double) { return ((fmask >> c) & 1u) != 0; });
+        const double lam2 = warp_sum(lane < P && ((fmask >> lane) & 1u) ? delta * rhs : 0.0);
         const bool conv = lam2 < kFLambda2;
         if (!conv && t < kFMaxSteps) {
             b_prev = b;
@@ -555,19 +566,9 @@ k_assoc_firth(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_sampl
             if (!conv_full || !conv) status = INQ_ASSOC_NO_CONVERGENCE;
             done = true;
         }
-        __syncwarp();
-        if (lane < P) s_beta[warp][lane] = b;
-        __syncwarp();
+        publish_beta<P>(s_beta[warp], lane, b);
     }
-    if (have && lane == 0) {
-        if (status == INQ_ASSOC_FEW_SAMPLES || status == INQ_ASSOC_SINGULAR) {
-            const double nan = __longlong_as_double(0x7ff8000000000000ll);
-            out.beta[row] = nan; out.se[row] = nan; out.stat[row] = nan; out.p[row] = nan;
-        }
-        out.n_used[row] = n;
-        out.status[row] = status;
-        if (out.n_iter) out.n_iter[row] = (uint8_t)t_full;
-    }
+    write_tail(out, row, have, lane, n, status, t_full);
 }
 
 }  // namespace inqa

@@ -10,6 +10,7 @@
 #include <cmath>
 #include <cstring>
 #include <string>
+#include <type_traits>
 #include <vector>
 
 namespace {
@@ -28,20 +29,35 @@ int cfail(int code, const char *fmt, ...)
 }
 
 struct Guard {                         // frees everything on every exit path
-    void *d_m = nullptr, *d_kept = nullptr, *d_hits = nullptr, *d_ctr = nullptr;
+    std::vector<void *> mem;
     cudaStream_t s = nullptr;
     cudaEvent_t e0 = nullptr, e1 = nullptr;
+    cudaError_t alloc(void **q, size_t bytes)
+    {
+        const cudaError_t e = cudaMalloc(q, bytes);
+        if (e == cudaSuccess) mem.push_back(*q);
+        return e;
+    }
     ~Guard()
     {
-        if (d_m) cudaFree(d_m);
-        if (d_kept) cudaFree(d_kept);
-        if (d_hits) cudaFree(d_hits);
-        if (d_ctr) cudaFree(d_ctr);
+        for (void *q : mem) cudaFree(q);
         if (e0) cudaEventDestroy(e0);
         if (e1) cudaEventDestroy(e1);
         if (s) cudaStreamDestroy(s);
     }
 };
+
+// Calls launch(std::integral_constant<int, P>()) for the padded design width P of inq_assoc's kernels: 4, 8, 16 or 32.
+template <class Launch>
+void with_width(int P, Launch launch)
+{
+    switch (P) {
+    case 4: launch(std::integral_constant<int, 4>()); break;
+    case 8: launch(std::integral_constant<int, 8>()); break;
+    case 16: launch(std::integral_constant<int, 16>()); break;
+    default: launch(std::integral_constant<int, 32>()); break;
+    }
+}
 
 #define CC_TRY(call)                                                                            \
     do {                                                                                        \
@@ -73,12 +89,13 @@ int inq_outlier(int device, int method, uint64_t n_rows, uint32_t n_cols, const 
     CC_TRY(cudaEventCreate(&g.e0));
     CC_TRY(cudaEventCreate(&g.e1));
     const size_t bytes = (size_t)n_rows * n_cols * sizeof(float);
-    CC_TRY(cudaMalloc(&g.d_m, bytes));
-    CC_TRY(cudaMalloc(&g.d_kept, n_rows));
-    CC_TRY(cudaMalloc(&g.d_hits, std::max<uint64_t>(cap, 1) * sizeof(unsigned long long)));
-    CC_TRY(cudaMalloc(&g.d_ctr, sizeof(CohortCounters)));
-    CC_TRY(cudaMemcpyAsync(g.d_m, values, bytes, cudaMemcpyHostToDevice, g.s));
-    CC_TRY(cudaMemsetAsync(g.d_ctr, 0, sizeof(CohortCounters), g.s));
+    void *d_m, *d_kept, *d_hits, *d_ctr;
+    CC_TRY(g.alloc(&d_m, bytes));
+    CC_TRY(g.alloc(&d_kept, n_rows));
+    CC_TRY(g.alloc(&d_hits, std::max<uint64_t>(cap, 1) * sizeof(unsigned long long)));
+    CC_TRY(g.alloc(&d_ctr, sizeof(CohortCounters)));
+    CC_TRY(cudaMemcpyAsync(d_m, values, bytes, cudaMemcpyHostToDevice, g.s));
+    CC_TRY(cudaMemsetAsync(d_ctr, 0, sizeof(CohortCounters), g.s));
     CC_TRY(cudaEventRecord(g.e0, g.s));
     if (method == INQ_OUTLIER_ZSCORE) {
         const uint32_t stride = n_cols | 1u;
@@ -94,18 +111,18 @@ int inq_outlier(int device, int method, uint64_t n_rows, uint32_t n_cols, const 
             CC_TRY(cudaFuncSetAttribute(k_outlier_zscore_warp, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
             const uint64_t groups = (n_rows + 31) / 32;
             const unsigned grid = (unsigned)std::min<uint64_t>((groups + zw_warps - 1) / zw_warps, (uint64_t)sms);
-            k_outlier_zscore_warp<<<grid, zw_warps * 32, smem, g.s>>>((const float *)g.d_m, n_rows, n_cols, (float)minsize, zscore_cutoff,
-                                                                     (uint8_t *)g.d_kept, (unsigned long long *)g.d_hits, cap, (CohortCounters *)g.d_ctr);
+            k_outlier_zscore_warp<<<grid, zw_warps * 32, smem, g.s>>>((const float *)d_m, n_rows, n_cols, (float)minsize, zscore_cutoff,
+                                                                     (uint8_t *)d_kept, (unsigned long long *)d_hits, cap, (CohortCounters *)d_ctr);
         } else if (res_smem <= 200u * 1024u) {
             // 32 rows fit in shared memory: the matrix is read once
             CC_TRY(cudaFuncSetAttribute(k_outlier_zscore_rows, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)res_smem));
             const unsigned grid = (unsigned)((n_rows + kZResRows - 1) / kZResRows);
-            k_outlier_zscore_rows<<<grid, kZResThreads, res_smem, g.s>>>((const float *)g.d_m, n_rows, n_cols, stride, (float)minsize, zscore_cutoff,
-                                                                        (uint8_t *)g.d_kept, (unsigned long long *)g.d_hits, cap, (CohortCounters *)g.d_ctr);
+            k_outlier_zscore_rows<<<grid, kZResThreads, res_smem, g.s>>>((const float *)d_m, n_rows, n_cols, stride, (float)minsize, zscore_cutoff,
+                                                                        (uint8_t *)d_kept, (unsigned long long *)d_hits, cap, (CohortCounters *)d_ctr);
         } else {
         const unsigned grid = (unsigned)((n_rows + kZRows - 1) / kZRows);
-        k_outlier_zscore<<<grid, kZRows, 0, g.s>>>((const float *)g.d_m, n_rows, n_cols, (float)minsize, zscore_cutoff,
-                                                   (uint8_t *)g.d_kept, (unsigned long long *)g.d_hits, cap, (CohortCounters *)g.d_ctr);
+        k_outlier_zscore<<<grid, kZRows, 0, g.s>>>((const float *)d_m, n_rows, n_cols, (float)minsize, zscore_cutoff,
+                                                   (uint8_t *)d_kept, (unsigned long long *)d_hits, cap, (CohortCounters *)d_ctr);
         }
     } else {
         uint32_t n2 = 32;
@@ -125,8 +142,8 @@ int inq_outlier(int device, int method, uint64_t n_rows, uint32_t n_cols, const 
             CC_TRY(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
             CC_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, (int)threads, smem));
             const unsigned grid = (unsigned)std::min<uint64_t>(n_rows, (uint64_t)sms * std::max(per_sm, 1));
-            kernel<<<grid, threads, smem, g.s>>>((const float *)g.d_m, n_rows, n_cols, n2, (float)minsize, min_points,
-                                                 (uint8_t *)g.d_kept, (unsigned long long *)g.d_hits, cap, (CohortCounters *)g.d_ctr);
+            kernel<<<grid, threads, smem, g.s>>>((const float *)d_m, n_rows, n_cols, n2, (float)minsize, min_points,
+                                                 (uint8_t *)d_kept, (unsigned long long *)d_hits, cap, (CohortCounters *)d_ctr);
             return INQ_OK;
         };
         int lrc;
@@ -143,8 +160,8 @@ int inq_outlier(int device, int method, uint64_t n_rows, uint32_t n_cols, const 
     CC_TRY(cudaGetLastError());
     CC_TRY(cudaEventRecord(g.e1, g.s));
     CohortCounters h;
-    CC_TRY(cudaMemcpyAsync(&h, g.d_ctr, sizeof(h), cudaMemcpyDeviceToHost, g.s));
-    if (row_kept) CC_TRY(cudaMemcpyAsync(row_kept, g.d_kept, n_rows, cudaMemcpyDeviceToHost, g.s));
+    CC_TRY(cudaMemcpyAsync(&h, d_ctr, sizeof(h), cudaMemcpyDeviceToHost, g.s));
+    if (row_kept) CC_TRY(cudaMemcpyAsync(row_kept, d_kept, n_rows, cudaMemcpyDeviceToHost, g.s));
     CC_TRY(cudaStreamSynchronize(g.s));
     if (ms_kernel) cudaEventElapsedTime(ms_kernel, g.e0, g.e1);
     if (h.no_mode)
@@ -153,7 +170,7 @@ int inq_outlier(int device, int method, uint64_t n_rows, uint32_t n_cols, const 
     *n_hits = h.n_hits;
     const uint64_t n = std::min<uint64_t>(h.n_hits, cap);
     if (n) {
-        CC_TRY(cudaMemcpy(hits, g.d_hits, n * sizeof(uint64_t), cudaMemcpyDeviceToHost));
+        CC_TRY(cudaMemcpy(hits, d_hits, n * sizeof(uint64_t), cudaMemcpyDeviceToHost));
         std::sort(hits, hits + n);                            // (row, column) = the reference's print order
     }
     if (h.n_hits > cap) return cfail(INQ_ERR_HITS_CAP, "inq_outlier: %llu outliers, capacity %llu", (unsigned long long)h.n_hits, (unsigned long long)cap);
@@ -200,36 +217,20 @@ int inq_assoc(int device, int model, int predictor, uint64_t n_rows, uint32_t n_
     }
 
     CC_TRY(cudaSetDevice(device));
-    struct AGuard {
-        std::vector<void *> p;
-        cudaStream_t s = nullptr;
-        cudaEvent_t e0 = nullptr, e1 = nullptr;
-        ~AGuard()
-        {
-            for (void *q : p) cudaFree(q);
-            if (e0) cudaEventDestroy(e0);
-            if (e1) cudaEventDestroy(e1);
-            if (s) cudaStreamDestroy(s);
-        }
-    } g;
-    auto dalloc = [&](void **q, size_t bytes) -> cudaError_t {
-        const cudaError_t e = cudaMalloc(q, bytes);
-        if (e == cudaSuccess) g.p.push_back(*q);
-        return e;
-    };
+    Guard g;
     CC_TRY(cudaStreamCreateWithFlags(&g.s, cudaStreamNonBlocking));
     CC_TRY(cudaEventCreate(&g.e0));
     CC_TRY(cudaEventCreate(&g.e1));
     const size_t hap_bytes = (size_t)n_rows * 2 * n_samples * sizeof(double);
     void *d_haps, *d_des, *d_shift, *d_y, *d_res, *d_n, *d_st, *d_it;
-    CC_TRY(dalloc(&d_haps, hap_bytes));
-    CC_TRY(dalloc(&d_des, design.size() * sizeof(double)));
-    CC_TRY(dalloc(&d_shift, shift.size() * sizeof(double)));
-    CC_TRY(dalloc(&d_y, n_samples * sizeof(double)));
-    CC_TRY(dalloc(&d_res, (size_t)n_rows * 4 * sizeof(double)));
-    CC_TRY(dalloc(&d_n, (size_t)n_rows * sizeof(uint32_t)));
-    CC_TRY(dalloc(&d_st, (size_t)n_rows));
-    CC_TRY(dalloc(&d_it, (size_t)n_rows));
+    CC_TRY(g.alloc(&d_haps, hap_bytes));
+    CC_TRY(g.alloc(&d_des, design.size() * sizeof(double)));
+    CC_TRY(g.alloc(&d_shift, shift.size() * sizeof(double)));
+    CC_TRY(g.alloc(&d_y, n_samples * sizeof(double)));
+    CC_TRY(g.alloc(&d_res, (size_t)n_rows * 4 * sizeof(double)));
+    CC_TRY(g.alloc(&d_n, (size_t)n_rows * sizeof(uint32_t)));
+    CC_TRY(g.alloc(&d_st, (size_t)n_rows));
+    CC_TRY(g.alloc(&d_it, (size_t)n_rows));
     CC_TRY(cudaMemcpyAsync(d_haps, haps, hap_bytes, cudaMemcpyHostToDevice, g.s));
     CC_TRY(cudaMemcpyAsync(d_des, design.data(), design.size() * sizeof(double), cudaMemcpyHostToDevice, g.s));
     CC_TRY(cudaMemcpyAsync(d_shift, shift.data(), shift.size() * sizeof(double), cudaMemcpyHostToDevice, g.s));
@@ -240,19 +241,11 @@ int inq_assoc(int device, int model, int predictor, uint64_t n_rows, uint32_t n_
     const int lg = model == INQ_ASSOC_LOGISTIC, mx = predictor == INQ_ASSOC_MAX;
     const double *dh = (const double *)d_haps, *dd = (const double *)d_des, *ds = (const double *)d_shift, *dy = (const double *)d_y;
     CC_TRY(cudaEventRecord(g.e0, g.s));
-    if (model == INQ_ASSOC_FIRTH) {
-        switch (P) {
-        case 4: k_assoc_firth<4><<<grid, kAWarps * 32, 0, g.s>>>(dh, n_rows, n_samples, pdim, mx, dd, ds, dy, out); break;
-        case 8: k_assoc_firth<8><<<grid, kAWarps * 32, 0, g.s>>>(dh, n_rows, n_samples, pdim, mx, dd, ds, dy, out); break;
-        case 16: k_assoc_firth<16><<<grid, kAWarps * 32, 0, g.s>>>(dh, n_rows, n_samples, pdim, mx, dd, ds, dy, out); break;
-        default: k_assoc_firth<32><<<grid, kAWarps * 32, 0, g.s>>>(dh, n_rows, n_samples, pdim, mx, dd, ds, dy, out); break;
-        }
-    } else switch (P) {
-    case 4: k_assoc<4><<<grid, kAWarps * 32, 0, g.s>>>(dh, n_rows, n_samples, pdim, lg, mx, dd, ds, dy, out); break;
-    case 8: k_assoc<8><<<grid, kAWarps * 32, 0, g.s>>>(dh, n_rows, n_samples, pdim, lg, mx, dd, ds, dy, out); break;
-    case 16: k_assoc<16><<<grid, kAWarps * 32, 0, g.s>>>(dh, n_rows, n_samples, pdim, lg, mx, dd, ds, dy, out); break;
-    default: k_assoc<32><<<grid, kAWarps * 32, 0, g.s>>>(dh, n_rows, n_samples, pdim, lg, mx, dd, ds, dy, out); break;
-    }
+    with_width(P, [&](auto width) {
+        constexpr int W = decltype(width)::value;
+        if (model == INQ_ASSOC_FIRTH) k_assoc_firth<W><<<grid, kAWarps * 32, 0, g.s>>>(dh, n_rows, n_samples, pdim, mx, dd, ds, dy, out);
+        else k_assoc<W><<<grid, kAWarps * 32, 0, g.s>>>(dh, n_rows, n_samples, pdim, lg, mx, dd, ds, dy, out);
+    });
     CC_TRY(cudaGetLastError());
     CC_TRY(cudaEventRecord(g.e1, g.s));
     CC_TRY(cudaMemcpyAsync(beta, r, n_rows * sizeof(double), cudaMemcpyDeviceToHost, g.s));

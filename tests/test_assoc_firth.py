@@ -1,6 +1,6 @@
 """`assoc --firth`: Firth-penalized logistic regression with a penalized likelihood-ratio test (DESIGN.md 5e, Firth).
-CPU: the numpy restatement (tests/firth_oracle.py) pinned by the closed forms of 2x2 tables, its modified score and
-its invariance under a change of x's scale; the CLI's and the ABI's error paths.
+CPU: the numpy restatement (oracle/assoc.py, model "firth") pinned by the closed forms of 2x2 tables, its modified
+score and its invariance under a change of x's scale; the CLI's and the ABI's error paths.
 GPU: inq_assoc with INQ_ASSOC_FIRTH against the restatement over a grid of shapes with case-only expansions, the
 closed forms through the kernel, edge loci, and the CLI end to end."""
 import subprocess
@@ -9,7 +9,6 @@ import numpy as np
 import pytest
 
 from oracle import assoc as A
-from tests import firth_oracle as F
 from tests.test_assoc import make_cohort, parse_output, run, write_table
 
 TABLES = [(12, 5, 7, 14), (9, 0, 4, 11), (3, 0, 0, 8), (40, 0, 0, 300), (1, 0, 30, 237)]
@@ -71,8 +70,8 @@ def separated_edge_loci(ns=60):
 def test_two_by_two_closed_forms():
     for table in TABLES:
         x, y = two_by_two(*table)
-        check_closed_form(F.fit_locus(x, y), table)
-    r = F.fit_locus(*two_by_two(*TABLES[0]))
+        check_closed_form(A.fit_locus(x, y, model="firth"), table)
+    r = A.fit_locus(*two_by_two(*TABLES[0]), model="firth")
     assert r["stat"] == pytest.approx(5.061824, abs=1e-6) and r["p"] == pytest.approx(0.0244585, abs=1e-7)
 
 
@@ -85,7 +84,7 @@ def test_modified_score_is_zero_at_the_solution():
         y = (rng.random(n) < 1 / (1 + np.exp(-(-1.5 + 0.3 * cov[:, 2])))).astype(float)
         if i % 2:
             x[np.flatnonzero(y)[:3]] = 2000.0 + 1000 * i                    # case-only expansions: separated
-        r = F.fit_locus(x, y, cov)
+        r = A.fit_locus(x, y, cov, "firth")
         assert r["status"] == A.OK and r["stat"] >= 0 and np.isfinite(r["beta"])
         X = np.column_stack([np.ones(n), cov, x])
         mu = A.linkinv(X @ r["coef"])
@@ -105,8 +104,8 @@ def test_invariant_under_a_change_of_scale_of_x():
     x = rng.gamma(2, 0.5, n)
     y = (rng.random(n) < 0.3).astype(float)
     x[np.flatnonzero(y)[:2]] = 9.0
-    a = F.fit_locus(x, y, cov)
-    b = F.fit_locus(1000 * x + 7, y, cov)
+    a = A.fit_locus(x, y, cov, "firth")
+    b = A.fit_locus(1000 * x + 7, y, cov, "firth")
     assert a["status"] == b["status"] == A.OK and a["n_iter"] == b["n_iter"]
     assert b["stat"] == pytest.approx(a["stat"], rel=1e-7) and b["p"] == pytest.approx(a["p"], rel=1e-6)
     assert b["beta"] * 1000 == pytest.approx(a["beta"], rel=1e-7) and b["se"] * 1000 == pytest.approx(a["se"], rel=1e-7)
@@ -118,10 +117,10 @@ def test_separated_locus_gets_a_finite_answer():
         x = A.predictor(haps[2, 0::2], haps[2, 1::2], pred)
         ml = A.fit_locus(x, y, cov, "logistic")
         assert ml["status"] in (A.SEPARATION, A.NO_CONVERGENCE)
-        r = F.fit_locus(x, y, cov)
+        r = A.fit_locus(x, y, cov, "firth")
         assert r["status"] == A.OK and np.isfinite(r["beta"]) and r["beta"] > 0 and np.isfinite(r["se"])
         assert 0 < r["p"] < 1e-6                                          # a separated locus is strong evidence
-    ref = F.assoc_matrix(haps, y, cov)
+    ref = A.assoc_matrix(haps, y, cov, "firth")
     assert list(ref["status"]) == [A.SINGULAR, A.OK, A.OK, A.FEW_SAMPLES, A.FEW_SAMPLES]
 
 
@@ -236,7 +235,7 @@ def test_gpu_firth_matches_oracle(rows, samples, n_cov, missing):
     c = cov if n_cov else None
     for pred in ("sum", "max"):
         got = cohort.assoc(haps, y, c, "firth", pred)
-        ref = F.assoc_matrix(haps, y, c, pred)                                 # every locus
+        ref = A.assoc_matrix(haps, y, c, "firth", pred)                        # every locus
         label = (rows, samples, n_cov, missing, pred)
         check_firth_parity(got, ref, label)
         if samples in (268, 2100):
@@ -265,7 +264,7 @@ def test_gpu_firth_edge_loci():
     haps = np.vstack([haps, one_class])
     for pred in ("sum", "max"):
         got = cohort.assoc(haps, y, cov, "firth", pred)
-        ref = F.assoc_matrix(haps, y, cov, pred)
+        ref = A.assoc_matrix(haps, y, cov, "firth", pred)
         check_firth_parity({k: v for k, v in got.items() if k != "ms_kernel"}, ref, pred)
         assert list(got["status"]) == [A.SINGULAR, A.OK, A.OK, A.FEW_SAMPLES, A.FEW_SAMPLES, A.FEW_SAMPLES], got["status"]
         assert list(got["n"][3:]) == [1, 0, 5]
@@ -312,7 +311,7 @@ def test_gpu_firth_cli_end_to_end(cli, tmp_path, gz):
         assert r.returncode == 0, r.stderr
         out = parse_output(r.stdout.decode())
         assert [tuple(o[:3]) for o in out] == [(c, str(b), str(e)) for c, b, e in loci]
-        ref = F.assoc_matrix(haps[:, cols], y, cov, pred)
+        ref = A.assoc_matrix(haps[:, cols], y, cov, "firth", pred)
         got = {k: np.array([float(o[j]) for o in out]) for j, k in ((4, "beta"), (5, "se"), (6, "stat"), (7, "p"))}
         got["n"] = np.array([int(o[3]) for o in out])
         got["status"] = np.array([A.STATUS_NAMES.index(o[8]) for o in out])

@@ -3,10 +3,10 @@
 samples, 12 covariates, 10 % missing calls, about 20 % constant loci, seeded. Prints one JSON line per model x
 predictor with the kernel time (CUDA events, H2D excluded; median of --reps runs after a warm-up), loci/s, the f64
 FMAs the fits need (from shapes and iteration counts) and GFLOP/s, and parity of --parity random loci against the
-numpy restatement (oracle/assoc.py, not R) with its host time. `firth` lines (the case/control trait, `--firth`)
-report the steps of the full fit over every locus and of both fits on the parity loci (tests/firth_oracle.py, not
-logistf) instead of FMAs. Then one line per model for the CLI on the same table written as TSV: wall time with text
-parse, device and output time separated (`--stats-json`). The card's name and power limit are read in the same run.
+numpy restatement (oracle/assoc.py, not R or logistf) with its host time. `firth` lines (the case/control trait,
+`--firth`) report the steps of the full fit over every locus and of both fits on the parity loci instead of FMAs.
+Then one line per model for the CLI on the same table written as TSV: wall time with text parse, device and output
+time separated (`--stats-json`). The card's name and power limit are read in the same run.
 Temporary files go to a temporary directory."""
 import argparse
 import json
@@ -38,7 +38,7 @@ def workload(rows, samples, n_cov, seed=2024):
     cov = np.empty((samples, n_cov))
     for c in range(n_cov):
         cov[:, c] = rng.normal(50, 15, samples) if c == 0 else (rng.integers(0, 2, samples) if c == 1 else rng.normal(0, 1, samples))
-    y_lin = 3 + 0.01 * cov[:, 0] + rng.normal(size=samples)
+    y_lin = 3 + (0.01 * cov[:, 0] if n_cov else 0.0) + rng.normal(size=samples)
     y_bin = (rng.random(samples) < 0.4).astype(float)
     return haps, cov, y_lin, y_bin
 
@@ -68,7 +68,6 @@ def main():
     args = ap.parse_args()
     from inquistr_b200 import cohort
     from oracle import assoc as A
-    from tests import firth_oracle as FO
     name = card()
     haps, cov, y_lin, y_bin = workload(args.rows, args.samples, args.cov)
     p = args.cov + 2
@@ -84,10 +83,7 @@ def main():
             med = float(np.median(ms))
             f = fmas(res, p, model) if model != "firth" else None
             t0 = time.perf_counter()
-            if model == "firth":
-                ref = FO.assoc_matrix(haps[sel], y, cov, pred)
-            else:
-                ref = A.assoc_matrix(haps[sel], y, cov, model, pred)
+            ref = A.assoc_matrix(haps[sel], y, cov, model, pred)
             oracle_s = time.perf_counter() - t0
             st = res["status"][sel]
             ok = (ref["status"] == A.OK) & (st == A.OK)
