@@ -569,15 +569,12 @@ int enqueue_pass(inq_ctx *ctx, const RunParams &rp, bool capturing, uint32_t *n_
         ScanParams sp;
         sp.tile_first = ctx->tile_first.p; sp.unit_off = ctx->unit_off.p; sp.units = cigar_ptr(ctx); sp.rd_pre = ctx->rd_pre.p;
         sp.wt = ctx->wtot.p; sp.wt_sbase = ctx->wt_sbase.p; sp.evraw = ctx->evraw.p; sp.ctr = ctx->d_ctr; sp.raw_cap = ctx->evraw.cap;
-        sp.n_wt = n_wt; sp.neg1 = 0xFFFFFFFFu; sp.minlen = rp.minlen;
+        sp.n_wt = n_wt; sp.ev_thr = scan_ev_thr(rp.minlen); sp.minlen = rp.minlen;
         // the unit field holds lengths up to 4094 exactly and 4095 for every longer I/D/S: from minlen 4095 on only
-        // those long heads can be events, and k_cigar_scan<true, true> checks their full length
-        const uint32_t thr16 = (std::min<uint32_t>(rp.minlen, kUnitLong - 1) << 4) | 15u;
-        sp.thr = (thr16 << 16) | 0xFFFFu;
+        // those long heads can be events, and k_cigar_scan<true> checks their full length
         const unsigned grid = (unsigned)std::min<uint64_t>((n_wt + kScanWarps - 1) / kScanWarps, (uint64_t)ctx->sm_count * ctx->scan_ctas_per_sm);
-        if (rp.minlen >= kUnitLong) k_cigar_scan<true, true><<<grid, kCtaThreads, kScanSmemBytes, s0>>>(ctx->tmap, sp);
-        else if (sp.thr >> 31) k_cigar_scan<true, false><<<grid, kCtaThreads, kScanSmemBytes, s0>>>(ctx->tmap, sp);
-        else k_cigar_scan<false, false><<<grid, kCtaThreads, kScanSmemBytes, s0>>>(ctx->tmap, sp);
+        if (rp.minlen >= kUnitLong) k_cigar_scan<true><<<grid, kCtaThreads, kScanSmemBytes, s0>>>(ctx->tmap, sp);
+        else k_cigar_scan<false><<<grid, kCtaThreads, kScanSmemBytes, s0>>>(ctx->tmap, sp);
         ++launches;
         CU_TRY(ctx, cudaGetLastError());
     }
@@ -739,14 +736,13 @@ int inq_ctx_create(int device, inq_ctx **out)
     if ((e = cudaMallocHost(&ctx->h_ctr, sizeof(DevCounters))) != cudaSuccess) return bail("cudaMallocHost", e);
     if ((e = cudaMallocHost(&ctx->h_total, 64)) != cudaSuccess) return bail("cudaMallocHost", e);
     memset(ctx->h_ctr, 0, sizeof(DevCounters));
-    if ((e = cudaFuncSetAttribute(k_cigar_scan<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kScanSmemBytes)) != cudaSuccess ||
-        (e = cudaFuncSetAttribute(k_cigar_scan<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kScanSmemBytes)) != cudaSuccess ||
-        (e = cudaFuncSetAttribute(k_cigar_scan<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kScanSmemBytes)) != cudaSuccess)
+    if ((e = cudaFuncSetAttribute(k_cigar_scan<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kScanSmemBytes)) != cudaSuccess ||
+        (e = cudaFuncSetAttribute(k_cigar_scan<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kScanSmemBytes)) != cudaSuccess)
         return bail("cudaFuncSetAttribute(k_cigar_scan)", e);
     if ((e = cudaFuncSetAttribute(k_pair_eval, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(PairSmem))) != cudaSuccess)
         return bail("cudaFuncSetAttribute(k_pair_eval)", e);
     int occ = 0;
-    if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_cigar_scan<false, false>, kCtaThreads, kScanSmemBytes)) != cudaSuccess)
+    if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_cigar_scan<false>, kCtaThreads, kScanSmemBytes)) != cudaSuccess)
         return bail("occupancy(k_cigar_scan)", e);
     ctx->scan_ctas_per_sm = std::max(1, occ);
     *out = ctx;

@@ -122,21 +122,37 @@ __device__ __forceinline__ void fence_mbar_init()
 // ----------------------------------------------------------------------------------------------
 // CIGAR units. BAM words are (len << 4) | op with ops MIDNSHP=X -> 0..8; M,D,N,=,X consume the reference
 // (call.rs:384-392,404), I,D,S longer than minlen are events (call.rs:388,394,400). The device keeps the
-// stream as 16-bit units (len << 4) | op, len < 4096, written when reads are pushed:
+// stream as 16-bit units written when reads are pushed. A unit carries what the scan asks of an op as bits, so that
+// both units of a 32-bit word are tested together with 32-bit arithmetic (k_cigar_scan):
+//   bit 15 C: consumes the reference; bits 14-13 sub; bit 12 E: I, D or S; bits 11-0: len
+//     M, N, =, X piece   C            len          I   E          len
+//     D or long-D head   C | E        len          S   E | sub 1  len
+//     payload (below)    sub = 2 payload bits, bits 11-0 = 12 payload bits (C = E = 0: no consumption, no event)
 //   - H, P, the invalid codes 9..15 and every op of length 0 are dropped: they consume nothing and are never events;
-//   - M, N, = and X longer than 4095 are split into pieces of at most 4095 with the same op (consumption adds up);
-//   - I, D and S of length >= 4095 are a head (4095 << 4) | op followed by two payload units that hold the full
-//     length (14 bits each, op codes 12..15: no consumption, no event). A long D's head consumes 4095 and is
-//     followed by N pieces for the rest, so that consumption still adds up unit by unit.
+//   - M, N, = and X longer than 4095 are split into pieces of at most 4095 (consumption adds up);
+//   - I, D and S of length >= 4095 are a head with len 4095 followed by two payload units that hold the full
+//     length (14 bits each). A long D's head consumes 4095 and is followed by N pieces for the rest, so that
+//     consumption still adds up unit by unit.
 // So for I/D/S the 12-bit field is the exact length below 4095 and 4095 exactly for a long head: the event test on
-// the field is exact for minlen < 4095; a larger minlen looks the heads' full length up (k_cigar_scan<_, true>).
+// the field is exact for minlen < 4095; a larger minlen looks the heads' full length up (k_cigar_scan<true>).
+// The all-zero unit (padding, and a payload of 0) consumes nothing and is never an event.
 constexpr uint32_t kUnitLong = 4095;        // field of a long I/D/S head; longest piece of a split op
+constexpr uint32_t kUnitLen = 0x0FFFu;
+constexpr uint32_t kUnitE = 1u << 12;
+constexpr uint32_t kUnitSub = 3u << 13;
+constexpr uint32_t kUnitS = 1u << 13;
+constexpr uint32_t kUnitC = 1u << 15;
 
 __device__ __forceinline__ bool op_dropped(uint32_t op) { return op > 8u || op == 5u || op == 6u; }
 __device__ __forceinline__ bool op_event_class(uint32_t op) { return ((0x16u >> op) & 1u) != 0u; }
+// flag bits of the units of a kept op
+__device__ __forceinline__ uint32_t op_unit_flags(uint32_t op)
+{
+    return op == 1u ? kUnitE : op == 2u ? kUnitC | kUnitE : op == 4u ? kUnitE | kUnitS : kUnitC;
+}
 __device__ __forceinline__ uint32_t split_pieces(uint32_t len) { return (len + kUnitLong - 1u) / kUnitLong; }
-__device__ __forceinline__ uint16_t payload_unit(uint32_t p14) { return (uint16_t)(((p14 >> 2) << 4) | 12u | (p14 & 3u)); }
-__device__ __forceinline__ uint32_t payload_value(uint32_t u) { return ((u >> 4) << 2) | (u & 3u); }
+__device__ __forceinline__ uint16_t payload_unit(uint32_t p14) { return (uint16_t)(((p14 & 3u) << 13) | (p14 >> 2)); }
+__device__ __forceinline__ uint32_t payload_value(uint32_t u) { return ((u & kUnitLen) << 2) | ((u >> 13) & 3u); }
 // full length of the long head at unit index h of the stream
 __device__ __forceinline__ uint32_t long_head_len(const uint16_t *__restrict__ units, uint64_t h)
 {
@@ -157,18 +173,18 @@ __device__ __forceinline__ void unit_write(uint32_t w, uint16_t *__restrict__ ou
     const uint32_t op = w & 15u;
     uint32_t len = w >> 4;
     if (op_dropped(op) || len == 0u) return;
-    uint32_t split_op = op;
+    uint32_t flags = op_unit_flags(op);
     if (op_event_class(op)) {
-        if (len < kUnitLong) { out[0] = (uint16_t)w; return; }
-        out[0] = (uint16_t)((kUnitLong << 4) | op);
+        if (len < kUnitLong) { out[0] = (uint16_t)(flags | len); return; }
+        out[0] = (uint16_t)(flags | kUnitLong);
         out[1] = payload_unit(len & 0x3FFFu);
         out[2] = payload_unit(len >> 14);
         if (op != 2u) return;
         out += 3;
         len -= kUnitLong;
-        split_op = 3u;                      // the rest of a long D: N pieces
+        flags = kUnitC;                     // the rest of a long D: N pieces
     }
-    for (; len; len -= min(len, kUnitLong)) *out++ = (uint16_t)((min(len, kUnitLong) << 4) | split_op);
+    for (; len; len -= min(len, kUnitLong)) *out++ = (uint16_t)(flags | min(len, kUnitLong));
 }
 
 template <typename T>
@@ -437,9 +453,7 @@ struct ScanParams {
     DevCounters *ctr;
     uint64_t raw_cap;             // capacity of evraw (slots)
     uint64_t n_wt;
-    uint32_t thr;                 // (thr16 << 16) | 0xFFFF with thr16 = (min(minlen, 4094) << 4) | 15: a unit in the
-                                  // top half of a word is longer than minlen (up to 4094) iff the word > thr
-    uint32_t neg1;                // 0xFFFFFFFF as a run-time value (keeps thr - w a multiply-add on the FMA pipe)
+    uint32_t ev_thr;              // scan_ev_thr(minlen), in both halves
     uint32_t minlen;              // full minlen (the long-head variant)
 };
 
@@ -449,18 +463,35 @@ constexpr int kScanWarps = 24;                          // warps per CTA, each f
 constexpr int kCtaThreads = kScanWarps * 32;
 constexpr int kWarpStages = 2;                          // per-warp ring of TMA boxes
 constexpr int kScanMinCtas = 1;
-// 64-bit LUT read through one wrap-mode funnel shift by 2*op or 2*op+1: result bit 0 = op consumes the reference
-// (M,D,N,=,X: lo bits 2*op and 2*op+1), result bit 31 = op is I, D or S (hi bits 2*op-1 and 2*op). Both bits of each
-// op are set so that the shift of the top unit of a word can be word >> 15, whatever bit 15 holds.
-constexpr uint32_t kOpLutLo = (3u << 0) | (3u << 4) | (3u << 6) | (3u << 14) | (3u << 16);
-constexpr uint32_t kOpLutHi = (3u << 1) | (3u << 3) | (3u << 7);
 constexpr uint32_t kEvChunk = 1024;                     // event slots a warp takes per atomic
-// consumption of unit u (bits above 15 zero) through the LUT: branch-free, the multiply issues on the FMA pipe
-__device__ __forceinline__ uint32_t unit_consume(uint32_t u)
+// 0xFFFF in each half of word x whose unit has C set, 0 otherwise: prmt's sign-replicate mode copies bit 15 into
+// bytes 0-1 and bit 31 into bytes 2-3 (__byte_perm drops the mode bit of the selector, hence the inline PTX)
+__device__ __forceinline__ uint32_t consume_mask(uint32_t x)
 {
-    return (u >> 4) * (__funnelshift_r(kOpLutLo, kOpLutHi, u + u) & 1u);
+    uint32_t m;
+    asm("prmt.b32 %0, %1, 0, 0xBB99;" : "=r"(m) : "r"(x));
+    return m;
 }
-__device__ __forceinline__ uint32_t word_consume(uint32_t x) { return unit_consume(x & 0xFFFFu) + unit_consume(x >> 16); }
+// consumption of both units of word x as two 16-bit sums (each at most 4095)
+__device__ __forceinline__ uint32_t word_consume2(uint32_t x) { return x & consume_mask(x) & 0x0FFF0FFFu; }
+__device__ __forceinline__ uint32_t word_consume(uint32_t x)
+{
+    const uint32_t a = word_consume2(x);
+    return (a & 0xFFFFu) + (a >> 16);
+}
+__device__ __forceinline__ uint32_t unit_consume(uint32_t u) { return (u & kUnitC) ? u & kUnitLen : 0u; }
+// Event test on both units of a word: bit 15 / bit 31 of ((x & 0x1FFF1FFF) | 0x80008000) - ev_thr is set exactly when
+// that unit has E set and len > minlen. Each half of ev_thr is 0x1000 + minlen + 1 (minlen < 4095), at most 0x1FFF:
+// the low half's minuend is >= 0x8000 > ev_thr, so it never borrows from the high half. From minlen 4094 on it is
+// 0x1FFF, which selects exactly the long heads (len 4095).
+inline uint32_t scan_ev_thr(uint32_t minlen)
+{
+    return (0x1000u + (minlen < kUnitLong - 1u ? minlen : kUnitLong - 1u) + 1u) * 0x00010001u;
+}
+__device__ __forceinline__ uint32_t word_events(uint32_t x, uint32_t ev_thr)
+{
+    return (((x & 0x1FFF1FFFu) | 0x80008000u) - ev_thr) & 0x80008000u;
+}
 
 struct ScanSmem {
     alignas(1024) uint32_t stage[kScanWarps][kWarpStages][kWarpTileUnits / 2];   // 128B-swizzled by the TMA tensor map
@@ -485,15 +516,33 @@ __device__ __forceinline__ uint64_t l2_evict_first_policy()
     asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(p));
     return p;
 }
-// events among the first n words of a lane's mask (word i <-> bit kLaneWords-1-i)
-__device__ __forceinline__ uint32_t events_before(uint32_t m, uint32_t n) { return n ? __popc(m >> (kLaneWords - n)) : 0u; }
+// A lane's event masks: evA for words 0-15, evB for words 16-31; bit i <-> the low unit of word i (of the 16),
+// bit 16 + i <-> its high unit. evs = evA | evB << 32.
+// events among the low units of the first nlo words and the high units of the first nhi words of one mask
+__device__ __forceinline__ uint32_t events_in_half(uint32_t m, uint32_t nlo, uint32_t nhi)
+{
+    return __popc(m & (((1u << nlo) - 1u) | (((1u << nhi) - 1u) << 16)));
+}
+// events among the first k units of a lane: the low units of words [0, (k+1)/2), the high units of words [0, k/2)
+__device__ __forceinline__ uint32_t events_before(uint64_t evs, uint32_t k)
+{
+    const uint32_t nlo = (k + 1u) >> 1, nhi = k >> 1, h = kLaneWords / 2;
+    return events_in_half((uint32_t)evs, min(nlo, h), min(nhi, h)) +
+           events_in_half((uint32_t)(evs >> 32), nlo - min(nlo, h), nhi - min(nhi, h));
+}
+// unit index inside the lane of the first event of evs (nonzero) in unit order, and that event's bit
+__device__ __forceinline__ uint32_t first_event(uint64_t evs, uint32_t &bit)
+{
+    const uint32_t b = __ffsll((evs | (evs >> 16)) & 0x0000FFFF0000FFFFull) - 1u;    // lowest word with an event
+    bit = (evs >> b) & 1u ? b : b + 16u;                                             // its low unit first
+    return 2u * ((b & 15u) | ((b >> 1) & 16u)) + ((bit >> 4) & 1u);
+}
 
 // Every warp is an independent pipeline: it owns warp tiles gwid, gwid + W, gwid + 2W, ... (W = warps
 // in the grid), a kWarpStages-deep ring of 4 KB shared-memory boxes (one warp tile each) that it fills itself with TMA, and the
 // mbarriers of that ring. There is no block-level synchronisation and no producer warp.
-// kThrHigh: thr >= 2^31 (minlen >= 2048). kLongOnly: minlen >= 4095, only long heads can be events and their full
-// length decides.
-template <bool kThrHigh, bool kLongOnly>
+// kLongOnly: minlen >= 4095, only long heads can be events and their full length decides.
+template <bool kLongOnly>
 __global__ void __launch_bounds__(kCtaThreads, kScanMinCtas)
 k_cigar_scan(const __grid_constant__ CUtensorMap tmap, ScanParams p)
 {
@@ -521,8 +570,7 @@ k_cigar_scan(const __grid_constant__ CUtensorMap tmap, ScanParams p)
     }
     __syncwarp();
 
-    const uint32_t thr = p.thr;
-    const uint32_t neg1 = p.neg1;
+    const uint32_t ev_thr = p.ev_thr;
     // this lane's kLaneWords consecutive words: quads q0..q0+kLaneWords/4-1 of the box; quad q lives in
     // 128-byte row q/8 at chunk (q%8) ^ (row%8) (128B swizzle) -> conflict-free LDS.128 across the warp
     constexpr uint32_t kQuads = kLaneWords / 4;
@@ -551,9 +599,9 @@ k_cigar_scan(const __grid_constant__ CUtensorMap tmap, ScanParams p)
         const uint32_t *stage = sm.stage[warp][s];
         const uint4 *st4 = reinterpret_cast<const uint4 *>(stage);
 
-        // ---- one pass over the lane's words. ev0 / ev1: bit (kLaneWords-1 - i) <-> the low / high unit of word i
-        //      is an event; snap[j]: bases consumed inside the lane's units before quad j (parked in shared memory below)
-        uint32_t c = 0, ev0 = 0, ev1 = 0;
+        // ---- one pass over the lane's words, both units of a word at once. evs: the lane's event masks (see
+        //      events_before); snap[j]: bases consumed inside the lane's units before quad j (parked in shared memory below)
+        uint32_t c = 0, evA = 0, evB = 0;
         uint32_t snap[kQuads];
 #pragma unroll
         for (int j = 0; j < (int)kQuads; ++j) {
@@ -561,41 +609,30 @@ k_cigar_scan(const __grid_constant__ CUtensorMap tmap, ScanParams p)
             const uint4 v = st4[row * 8 + ((q & 7u) ^ (row & 7u))];
             const uint32_t w4[4] = {v.x, v.y, v.z, v.w};
             snap[j] = c;
+            uint32_t a = 0;                                       // two 16-bit sums of at most 4 x 4095
 #pragma unroll
             for (int k = 0; k < 4; ++k) {
-                const uint32_t x = w4[k], y = x << 16;            // y: the low unit moved to the top half
-                // one funnel shift in wrap mode indexes the LUT by 2*op without masking the op first
-                // (x + x for the low unit, x >> 15 for the high one: the LUT has both bits of every op)
-                const uint32_t lut0 = __funnelshift_r(kOpLutLo, kOpLutHi, x + x);
-                const uint32_t lut1 = __funnelshift_r(kOpLutLo, kOpLutHi, x >> 15);
-                // borrow of thr - u (<=> u > thr for the unit u in the top half) lands in the sign bit of d | u
-                // (thr < 2^31) or d & u (thr >= 2^31); the subtraction is a multiply-add by a run-time -1 so that it
-                // issues on the FMA pipe. One LOP3 ands it with the op class, one funnel shift appends the sign bit.
-                uint32_t d0, d1;
-                asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(d0) : "r"(y), "r"(neg1), "r"(thr));
-                asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(d1) : "r"(x), "r"(neg1), "r"(thr));
-                const uint32_t t0 = kThrHigh ? (lut0 & (d0 & y)) : (lut0 & (d0 | y));
-                const uint32_t t1 = kThrHigh ? (lut1 & (d1 & x)) : (lut1 & (d1 | x));
-                ev0 = __funnelshift_l(t0, ev0, 1);
-                ev1 = __funnelshift_l(t1, ev1, 1);
-                // c += consumes ? len : 0 as one multiply-add (FMA pipe) instead of select + add (ALU pipe)
-                asm("mad.lo.u32 %0, %1, %2, %0;" : "+r"(c) : "r"(y >> 20), "r"(lut0 & 1u));
-                asm("mad.lo.u32 %0, %1, %2, %0;" : "+r"(c) : "r"(x >> 20), "r"(lut1 & 1u));
+                const uint32_t x = w4[k];
+                a += word_consume2(x);
+                // after 16 words the event bits of word i sit at bits i and 16 + i. The shifted mask has bits 15 and
+                // 31 clear, so an add does the or and fuses with the shift (one LEA.HI)
+                uint32_t &ev = j < (int)kQuads / 2 ? evA : evB;
+                ev = (ev >> 1) + word_events(x, ev_thr);
             }
+            c += (a & 0xFFFFu) + (a >> 16);
         }
+        uint64_t evs = evA | ((uint64_t)evB << 32);
         if (kLongOnly) {
             // the candidates are the long heads (field 4095); an event only if the full length is > minlen
             const uint64_t lane_u0 = gw * kWarpTileUnits + lane * kLaneUnits;
-            for (uint32_t m = ev0; m; m &= m - 1u) {
-                const uint32_t b = __ffs(m) - 1u;
-                if (long_head_len(p.units, lane_u0 + 2u * (kLaneWords - 1u - b)) <= p.minlen) ev0 ^= 1u << b;
-            }
-            for (uint32_t m = ev1; m; m &= m - 1u) {
-                const uint32_t b = __ffs(m) - 1u;
-                if (long_head_len(p.units, lane_u0 + 2u * (kLaneWords - 1u - b) + 1u) <= p.minlen) ev1 ^= 1u << b;
+            for (uint64_t m = evs; m;) {
+                uint32_t bit;
+                const uint32_t u = first_event(m, bit);
+                m ^= 1ull << bit;
+                if (long_head_len(p.units, lane_u0 + u) <= p.minlen) evs ^= 1ull << bit;
             }
         }
-        const uint32_t ne = __popc(ev0) + __popc(ev1);
+        const uint32_t ne = __popcll(evs);
         const uint32_t incl_c = warp_incl_scan(c), incl_e = warp_incl_scan(ne);
         const uint32_t excl_c = incl_c - c, excl_e = incl_e - ne;
         const uint32_t tot_e = __shfl_sync(0xffffffffu, incl_e, 31);
@@ -634,16 +671,15 @@ k_cigar_scan(const __grid_constant__ CUtensorMap tmap, ScanParams p)
         const uint32_t n_starts = tf_hi - tf_lo;
         const uint32_t n_q = tot_e + n_starts;                  // queries [0, tot_e) are the events in unit order
         const uint32_t off_cur = (uint32_t)(g_cur - gw * kWarpTileUnits);    // lane i: first unit of read tf_lo + i
-        uint32_t left0 = ev0, left1 = ev1, ev_idx = excl_e;
+        uint64_t left = evs;
+        uint32_t ev_idx = excl_e;
         for (uint32_t base = 0; base < n_q; base += 32) {
-            // owners list their events with index in [base, base + 32) in unit order: the next word of either mask,
-            // its low unit first
-            while ((left0 | left1) && ev_idx < base + 32u) {
-                const uint32_t i0 = __clz(left0) - (32u - kLaneWords), i1 = __clz(left1) - (32u - kLaneWords);
-                const bool lo = i0 <= i1;
-                const uint32_t i = lo ? i0 : i1;
-                if (lo) left0 ^= 1u << (kLaneWords - 1u - i); else left1 ^= 1u << (kLaneWords - 1u - i);
-                sm.qlist[warp][ev_idx - base] = (uint16_t)(lane * kLaneUnits + 2u * i + (lo ? 0u : 1u));
+            // owners list their events with index in [base, base + 32) in unit order
+            while (left && ev_idx < base + 32u) {
+                uint32_t bit;
+                const uint32_t u = first_event(left, bit);
+                left ^= 1ull << bit;
+                sm.qlist[warp][ev_idx - base] = (uint16_t)(lane * kLaneUnits + u);
                 ++ev_idx;
             }
             __syncwarp();
@@ -656,7 +692,7 @@ k_cigar_scan(const __grid_constant__ CUtensorMap tmap, ScanParams p)
             else if (act) pos = (si < 32u) ? spos : (uint32_t)(__ldg(p.unit_off + tf_lo + si) - gw * kWarpTileUnits);
             const uint32_t owner = pos / kLaneUnits, k = pos % kLaneUnits;
             const uint32_t xc = __shfl_sync(0xffffffffu, excl_c, owner), xe = __shfl_sync(0xffffffffu, excl_e, owner);
-            const uint32_t er0 = __shfl_sync(0xffffffffu, ev0, owner), er1 = __shfl_sync(0xffffffffu, ev1, owner);
+            const uint64_t er = __shfl_sync(0xffffffffu, evs, owner);
             if (act) {
                 const uint32_t i = k >> 1, h = k & 1u, j = i >> 2, kk = i & 3u, q = owner * kQuads + j, row = q >> 3;
                 const uint4 v = st4[row * 8 + ((q & 7u) ^ (row & 7u))];
@@ -666,17 +702,17 @@ k_cigar_scan(const __grid_constant__ CUtensorMap tmap, ScanParams p)
                                       word_consume(kk > 1u ? v.y : 0u) + word_consume(kk > 2u ? v.z : 0u) +
                                       (h ? unit_consume(x & 0xFFFFu) : 0u);
                 if (is_ev) {
-                    const uint32_t u = h ? x >> 16 : x & 0xFFFFu, op = u & 15u;
-                    uint32_t len = u >> 4;
+                    // E is set: D = C, S = sub 1, I otherwise
+                    const uint32_t u = h ? x >> 16 : x & 0xFFFFu;
+                    uint32_t len = u & kUnitLen;
                     if (len == kUnitLong) len = long_head_len(p.units, gw * kWarpTileUnits + pos);
-                    const int32_t val = (int32_t)(((op == 2u) ? (0u - len) : len) << 1) | (int32_t)(op == 4u);
+                    const int32_t val = (int32_t)(((u & kUnitC) ? (0u - len) : len) << 1) | (int32_t)((u & kUnitSub) != 0u);
                     const uint64_t slot = sbase + qi;
                     if (slot < p.raw_cap) p.evraw[slot] = make_uint2(c_in, (uint32_t)val);
                     else atomicOr(&p.ctr->flags, kFlagEventOverflow);
                 } else if (pos) {
                     // units before k: the low units of words [0, (k+1)/2), the high units of words [0, k/2)
-                    const uint32_t e_in = events_before(er0, (k + 1u) >> 1) + events_before(er1, k >> 1);
-                    p.rd_pre[tf_lo + si] = make_uint2(c_in, xe + e_in);
+                    p.rd_pre[tf_lo + si] = make_uint2(c_in, xe + events_before(er, k));
                 }
             }
             __syncwarp();                                       // qlist is rewritten in the next round
