@@ -70,6 +70,20 @@ int inq_assoc(int device, int model, int predictor, uint64_t n_rows, uint32_t n_
               const double *y, uint32_t n_cov, const double *cov, double *beta, double *se, double *stat, double *p,
               uint32_t *n_used, uint8_t *status, uint8_t *n_iter /* nullable */, float *ms_kernel /* nullable */);
 
+/* Several traits at once: every trait t (column t of y, row-major n_samples x n_traits, NaN = the sample is not used
+ * for t; logistic and firth: every other value 0 or 1; +-inf is rejected) gives, in column t of the row-major
+ * n_rows x n_traits outputs, exactly what inq_assoc gives for t alone over the samples where y is not NaN (bit for bit).
+ * All traits share the model, the predictor and the covariates (finite, as in inq_assoc). The haplotype matrix goes
+ * to the device once; traits with the same samples share one preparation, and the linear ones one Gram matrix per
+ * locus. ms_kernel is the summed kernel time of all sample sets.
+ * INQ_ERR_ARG for n_traits == 0 and for a trait without a value (the message names the trait index);
+ * INQ_ERR_TOO_LARGE when n_rows x n_traits does not fit in memory sizes, or one sample set's loci x traits exceed the
+ * launch shape (2^31 - 1 blocks of 4 loci for logistic and firth; of 4 loci and up to 4 to 16 linear traits (by the design width)). */
+int inq_assoc_traits(int device, int model, int predictor, uint64_t n_rows, uint32_t n_samples, const double *haps,
+                     uint32_t n_traits, const double *y, uint32_t n_cov, const double *cov, double *beta, double *se,
+                     double *stat, double *p, uint32_t *n_used, uint8_t *status, uint8_t *n_iter /* nullable */,
+                     float *ms_kernel /* nullable */);
+
 const char *inq_cohort_last_error(void);
 
 #ifdef __cplusplus

@@ -13,7 +13,7 @@ LINEAR, LOGISTIC, FIRTH = 0, 1, 2
 PRED_SUM, PRED_MAX = 0, 1
 ASSOC_OK, ASSOC_FEW_SAMPLES, ASSOC_SINGULAR, ASSOC_NO_CONVERGENCE, ASSOC_SEPARATION = 0, 1, 2, 3, 4
 ASSOC_STATUS_NAMES = ["ok", "few_samples", "singular", "no_convergence", "separation"]
-EXPORTS = ["inq_outlier", "inq_assoc", "inq_cohort_last_error"]
+EXPORTS = ["inq_outlier", "inq_assoc", "inq_assoc_traits", "inq_cohort_last_error"]
 
 _BOUND = False
 
@@ -29,6 +29,10 @@ def _lib():
         L.inq_assoc.argtypes = [C.c_int, C.c_int, C.c_int, C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p, C.c_uint32,
                                 C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                 C.c_void_p, C.POINTER(C.c_float)]
+        L.inq_assoc_traits.restype = C.c_int
+        L.inq_assoc_traits.argtypes = [C.c_int, C.c_int, C.c_int, C.c_uint64, C.c_uint32, C.c_void_p, C.c_uint32, C.c_void_p,
+                                       C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                       C.c_void_p, C.c_void_p, C.POINTER(C.c_float)]
         L.inq_cohort_last_error.restype = C.c_char_p
         L.inq_cohort_last_error.argtypes = []
         _BOUND = True
@@ -83,6 +87,37 @@ def assoc(haps, y, cov=None, model: str = "linear", predictor: str = "sum", devi
                      rows, ns, h.ctypes.data, yy.ctypes.data, c.shape[1], c.ctypes.data if c.size else None,
                      out["beta"].ctypes.data, out["se"].ctypes.data, out["stat"].ctypes.data, out["p"].ctypes.data,
                      out["n"].ctypes.data, out["status"].ctypes.data, out["n_iter"].ctypes.data, C.byref(ms))
+    if rc != INQ_OK:
+        raise InqError(rc, L.inq_cohort_last_error().decode())
+    out["ms_kernel"] = float(ms.value)
+    return out
+
+
+def assoc_traits(haps, Y, cov=None, model: str = "linear", predictor: str = "sum", device: int = 0):
+    """Per-row association of STR length with each column of Y (include/inqcohort.h inq_assoc_traits).
+    Y: samples x T, NaN = the sample is not used for that trait. Column t of every output equals what assoc gives for
+    trait t alone over the samples where it is not NaN.
+    -> dict of rows x T arrays beta, se, stat, p (f64), n (u32), status (u8), n_iter (u8), and ms_kernel."""
+    h = np.ascontiguousarray(haps, dtype=np.float64)
+    rows, cols = h.shape
+    if cols % 2:
+        raise ValueError("haps needs two columns per sample")
+    ns = cols // 2
+    yy = np.ascontiguousarray(Y, dtype=np.float64)
+    if yy.ndim != 2 or yy.shape[0] != ns:
+        raise ValueError("Y needs one row per sample")
+    nt = yy.shape[1]
+    c = np.zeros((ns, 0)) if cov is None else np.ascontiguousarray(np.asarray(cov, np.float64).reshape(ns, -1))
+    out = {k: np.zeros((rows, nt), np.float64) for k in ("beta", "se", "stat", "p")}
+    out["n"] = np.zeros((rows, nt), np.uint32)
+    out["status"] = np.zeros((rows, nt), np.uint8)
+    out["n_iter"] = np.zeros((rows, nt), np.uint8)
+    ms = C.c_float(0)
+    L = _lib()
+    rc = L.inq_assoc_traits(device, {"linear": LINEAR, "logistic": LOGISTIC, "firth": FIRTH}[model], {"sum": PRED_SUM, "max": PRED_MAX}[predictor],
+                            rows, ns, h.ctypes.data, nt, yy.ctypes.data, c.shape[1], c.ctypes.data if c.size else None,
+                            out["beta"].ctypes.data, out["se"].ctypes.data, out["stat"].ctypes.data, out["p"].ctypes.data,
+                            out["n"].ctypes.data, out["status"].ctypes.data, out["n_iter"].ctypes.data, C.byref(ms))
     if rc != INQ_OK:
         raise InqError(rc, L.inq_cohort_last_error().decode())
     out["ms_kernel"] = float(ms.value)

@@ -317,9 +317,9 @@ void append_f64(std::string &out, double v)
 // `assoc`: one regression per row of a combined table (DESIGN.md 5e)
 int assoc_main(const std::vector<std::string> &v, int device)
 {
-    const char *usage = "assoc --phenotype <TSV> --trait <COL> --model <linear|logistic> [--firth] [--covariates A,B,...] [--predictor sum|max] [--device N] <COMBINED>";
-    std::string combined, pheno, trait, model, predictor = "sum", covs, stats_json;
-    bool has_cov = false, firth = false;
+    const char *usage = "assoc --phenotype <TSV> --trait <COL> | --traits <A,B,...> --model <linear|logistic> [--firth] [--covariates A,B,...] [--predictor sum|max] [--device N] <COMBINED>";
+    std::string combined, pheno, trait, model, predictor = "sum", covs, trait_list, stats_json;
+    bool has_cov = false, firth = false, has_traits = false;
     for (size_t i = 0; i < v.size(); ++i) {
         const std::string &a = v[i];
         auto value = [&](const char *name) -> std::string {
@@ -328,6 +328,7 @@ int assoc_main(const std::vector<std::string> &v, int device)
         };
         if (a == "--phenotype") pheno = value("--phenotype <TSV>");
         else if (a == "--trait") trait = value("--trait <COL>");
+        else if (a == "--traits") { trait_list = value("--traits <A,B,...>"); has_traits = true; }
         else if (a == "--model") {
             model = value("--model <MODEL>");
             if (model != "linear" && model != "logistic") cusage("invalid value '" + model + "' for '--model <MODEL>'\n  [possible values: linear, logistic]", usage);
@@ -348,6 +349,8 @@ int assoc_main(const std::vector<std::string> &v, int device)
                    "Arguments:\n  <COMBINED>  combined table of calls (`call-cohort` or `combine` output, plain or gzip)\n\nOptions:\n"
                    "      --phenotype <TSV>        tab-separated phenotype table with a header; first column: sample names\n"
                    "      --trait <COL>            response column\n"
+                   "      --traits <A,B,...>       several response columns in one run (instead of --trait); a sample with a missing\n"
+                   "                               value (NA, NaN, empty) is left out for that trait only\n"
                    "      --model <MODEL>          linear (OLS, t test) or logistic (0/1 trait, IRLS, Wald z test) [possible values: linear, logistic]\n"
                    "      --firth                  with --model logistic: Firth-penalized fit (finite under separation) and\n"
                    "                               penalized likelihood-ratio test\n"
@@ -357,7 +360,8 @@ int assoc_main(const std::vector<std::string> &v, int device)
                    "      --stats-json <FILE>      write parse, device and output times to FILE\n"
                    "  -h, --help                   Print help\n\n"
                    "Output: chromosome begin end n beta se stat p status, one row per input row; status is one of ok,\n"
-                   "few_samples, singular, no_convergence, separation. With --firth, stat is the penalized likelihood-ratio\n"
+                   "few_samples, singular, no_convergence, separation. With --traits: chromosome begin end trait n beta se stat\n"
+                   "p status, one row per input row and trait in --traits order. With --firth, stat is the penalized likelihood-ratio\n"
                    "chi-square (1 df) of x, p comes from it, and separation is never reported\n", usage, INQ_ASSOC_MAX_COV);
             return 0;
         } else if (!a.empty() && a[0] == '-' && a.size() > 1) cusage("unexpected argument '" + a + "' found", usage);
@@ -366,19 +370,31 @@ int assoc_main(const std::vector<std::string> &v, int device)
     }
     std::string missing;
     if (pheno.empty()) missing += "\n  --phenotype <TSV>";
-    if (trait.empty()) missing += "\n  --trait <COL>";
+    if (has_traits && !trait.empty()) cusage("the argument '--traits <A,B,...>' cannot be used with '--trait <COL>'", usage);
+    if (trait.empty() && !has_traits) missing += "\n  --trait <COL>";
     if (model.empty()) missing += "\n  --model <MODEL>";
     if (combined.empty()) missing += "\n  <COMBINED>";
     if (!missing.empty()) cusage("the following required arguments were not provided:" + missing, usage);
     if (firth && model != "logistic") cusage("the argument '--firth' requires '--model logistic'", usage);
-    std::vector<std::string> cov_names;
-    if (has_cov && !covs.empty()) {
+    auto split_list = [](const std::string &s) {
+        std::vector<std::string> out;
         size_t a = 0;
         for (;;) {
-            const size_t b = covs.find(',', a);
-            cov_names.emplace_back(covs, a, b == std::string::npos ? std::string::npos : b - a);
+            const size_t b = s.find(',', a);
+            out.emplace_back(s, a, b == std::string::npos ? std::string::npos : b - a);
             if (b == std::string::npos) break;
             a = b + 1;
+        }
+        return out;
+    };
+    std::vector<std::string> cov_names, traits{trait};
+    if (has_cov && !covs.empty()) cov_names = split_list(covs);
+    if (has_traits) {
+        traits = split_list(trait_list);
+        for (size_t t = 0; t < traits.size(); ++t) {
+            if (traits[t].empty()) cusage("invalid value '" + trait_list + "' for '--traits <A,B,...>': an empty column name", usage);
+            for (size_t d = 0; d < t; ++d)
+                if (traits[d] == traits[t]) cusage("trait '" + traits[t] + "' is listed twice", usage);
         }
     }
     if (cov_names.size() > INQ_ASSOC_MAX_COV)
@@ -386,18 +402,21 @@ int assoc_main(const std::vector<std::string> &v, int device)
                std::to_string(INQ_ASSOC_MAX_COV), usage);
     for (size_t c = 0; c < cov_names.size(); ++c) {
         if (cov_names[c].empty()) cusage("invalid value '" + covs + "' for '--covariates <A,B,...>': an empty column name", usage);
-        if (cov_names[c] == trait) cusage("the trait '" + trait + "' is also listed as a covariate", usage);
+        for (const std::string &t : traits)
+            if (cov_names[c] == t) cusage("the trait '" + t + "' is also listed as a covariate", usage);
         for (size_t d = 0; d < c; ++d)
             if (cov_names[d] == cov_names[c]) cusage("covariate '" + cov_names[c] + "' is listed twice", usage);
     }
     const bool logistic = model == "logistic";
     const auto t_start = std::chrono::steady_clock::now();
 
-    // phenotype table: sample -> trait, covariates; rows with a missing value are left out
-    const size_t n_cov = cov_names.size();
-    std::unordered_map<std::string, std::vector<double>> ph;          // complete rows: [trait, covariates...]
+    // phenotype table: sample -> traits, covariates; rows with a missing covariate are left out, a missing trait value
+    // (NaN) leaves the sample out for that trait only
+    const size_t n_cov = cov_names.size(), n_tr = traits.size();
+    std::unordered_map<std::string, std::vector<double>> ph;          // rows with every covariate: [traits..., covariates...]
     std::unordered_set<std::string> ph_seen;
-    size_t ph_missing = 0;
+    size_t cov_missing = 0;
+    std::vector<size_t> ph_missing(n_tr, 0);                          // per trait: rows left out for it
     {
         LineReader pr;
         if (!exists(pheno) || !pr.open(pheno)) afail(pheno + ": cannot open the phenotype table");
@@ -406,7 +425,7 @@ int assoc_main(const std::vector<std::string> &v, int device)
         if (!pr.next(line)) afail(pheno + ":1: empty file (a header row is needed)");
         split_tabs(line, cols);
         const std::vector<std::string> head = cols;
-        std::vector<std::string> want_names{trait};                   // [trait, covariates...]
+        std::vector<std::string> want_names = traits;                 // [traits..., covariates...]
         want_names.insert(want_names.end(), cov_names.begin(), cov_names.end());
         std::vector<size_t> want;
         for (const std::string &name : want_names) {
@@ -422,17 +441,22 @@ int assoc_main(const std::vector<std::string> &v, int device)
             if (cols.size() != head.size())
                 afail(where + std::to_string(cols.size()) + " fields, the header has " + std::to_string(head.size()));
             if (!ph_seen.insert(cols[0]).second) afail(where + "column '" + head[0] + "': sample '" + cols[0] + "' appears twice");
-            std::vector<double> vals(want.size());
+            std::vector<double> vals(want.size(), NAN);
             bool complete = true;
             for (size_t w = 0; w < want.size(); ++w) {
                 const std::string &f = cols[want[w]];
-                if (f.empty() || f == "NA" || f == "NaN") { complete = false; continue; }
+                if (f.empty() || f == "NA" || f == "NaN") { if (w >= n_tr) complete = false; continue; }
                 if (!parse_f64(f, &vals[w])) afail(where + "column '" + head[want[w]] + "': '" + f + "' is not a number");
-                if (w == 0 && logistic && vals[w] != 0.0 && vals[w] != 1.0)
+                if (w < n_tr && logistic && vals[w] != 0.0 && vals[w] != 1.0)
                     afail(where + "column '" + head[want[w]] + "': '" + f + "' is not 0 or 1 (--model logistic)");
             }
-            if (complete) ph.emplace(cols[0], std::move(vals));
-            else ++ph_missing;
+            if (!complete) { ++cov_missing; continue; }
+            bool any = false;
+            for (size_t t = 0; t < n_tr; ++t) {
+                if (std::isnan(vals[t])) ++ph_missing[t];
+                else any = true;
+            }
+            if (any) ph.emplace(cols[0], std::move(vals));
         }
     }
 
@@ -449,8 +473,9 @@ int assoc_main(const std::vector<std::string> &v, int device)
     const size_t n_val = cols.size() - 3;
     if (n_val % 2) afail(combined + ":1: " + std::to_string(n_val) + " value columns: not in <S>_H1 <S>_H2 pairs");
     const size_t n_tab = n_val / 2;
-    std::vector<uint32_t> use_idx;                       // table sample index of every used sample, in table order
-    std::vector<double> y, cov;
+    std::vector<uint32_t> use_idx;                       // table sample index of every sample used for some trait, in table order
+    std::vector<double> y, cov;                          // y: use_idx.size() x n_tr, NaN = not used for that trait
+    size_t n_groups = 0;
     {
         std::unordered_set<std::string> names;
         for (size_t k = 0; k < n_tab; ++k) {
@@ -464,22 +489,38 @@ int assoc_main(const std::vector<std::string> &v, int device)
             const auto it = ph.find(s);
             if (it == ph.end()) continue;
             use_idx.push_back((uint32_t)k);
-            y.push_back(it->second[0]);
-            cov.insert(cov.end(), it->second.begin() + 1, it->second.end());
+            y.insert(y.end(), it->second.begin(), it->second.begin() + n_tr);
+            cov.insert(cov.end(), it->second.begin() + n_tr, it->second.end());
         }
         size_t ph_only = 0;
         for (const std::string &s : ph_seen) ph_only += !names.count(s);
-        fprintf(stderr, "assoc: %zu samples used, %zu in the table only, %zu in the phenotype table only (%zu phenotype rows with a missing value left out)\n",
-                use_idx.size(), n_tab - use_idx.size(), ph_only, ph_missing);
-        if (use_idx.empty()) afail("no sample is in both " + combined + " and " + pheno);
+        std::vector<size_t> used(n_tr, 0);
+        std::vector<std::vector<bool>> masks;            // the traits' sample sets, as inq_assoc_traits groups them
+        for (size_t t = 0; t < n_tr; ++t) {
+            std::vector<bool> m(use_idx.size());
+            for (size_t s = 0; s < use_idx.size(); ++s) used[t] += m[s] = !std::isnan(y[s * n_tr + t]);
+            if (std::find(masks.begin(), masks.end(), m) == masks.end()) masks.push_back(std::move(m));
+        }
+        n_groups = masks.size();
+        if (!has_traits) {
+            fprintf(stderr, "assoc: %zu samples used, %zu in the table only, %zu in the phenotype table only (%zu phenotype rows with a missing value left out)\n",
+                    use_idx.size(), n_tab - use_idx.size(), ph_only, cov_missing + ph_missing[0]);
+            if (use_idx.empty()) afail("no sample is in both " + combined + " and " + pheno);
+        } else {
+            for (size_t t = 0; t < n_tr; ++t)
+                fprintf(stderr, "assoc: trait '%s': %zu samples used, %zu in the table only, %zu in the phenotype table only (%zu phenotype rows with a missing value left out)\n",
+                        traits[t].c_str(), used[t], n_tab - used[t], ph_only, cov_missing + ph_missing[t]);
+            for (size_t t = 0; t < n_tr; ++t)
+                if (!used[t]) afail("trait '" + traits[t] + "': no sample is in both " + combined + " and " + pheno);
+        }
     }
     const uint32_t ns = (uint32_t)use_idx.size();
-    fputs("chromosome\tbegin\tend\tn\tbeta\tse\tstat\tp\tstatus\n", stdout);
+    fputs(has_traits ? "chromosome\tbegin\tend\ttrait\tn\tbeta\tse\tstat\tp\tstatus\n" : "chromosome\tbegin\tend\tn\tbeta\tse\tstat\tp\tstatus\n", stdout);
     const char *status_names[] = {"ok", "few_samples", "singular", "no_convergence", "separation"};
     const int mdl = firth ? INQ_ASSOC_FIRTH : logistic ? INQ_ASSOC_LOGISTIC : INQ_ASSOC_LINEAR, prd = predictor == "max" ? INQ_ASSOC_MAX : INQ_ASSOC_SUM;
 
-    // rows in batches of at most 256 MB of values
-    const size_t batch_rows = std::max<size_t>(1, (256u << 20) / ((size_t)ns * 2 * sizeof(double)));
+    // rows in batches of at most 256 MB of values and 64 MB of results (rows x traits x 38 bytes)
+    const size_t batch_rows = std::max<size_t>(1, std::min((256u << 20) / ((size_t)ns * 2 * sizeof(double)), (64u << 20) / (n_tr * 38)));
     std::vector<double> haps, beta, se, stat, pv, rowvals(n_val);
     std::vector<uint32_t> n_used;
     std::vector<uint8_t> status;
@@ -490,21 +531,26 @@ int assoc_main(const std::vector<std::string> &v, int device)
     auto flush = [&]() {
         const size_t rows = keys.size();
         if (!rows) return;
-        beta.resize(rows); se.resize(rows); stat.resize(rows); pv.resize(rows); n_used.resize(rows); status.resize(rows);
+        const size_t cells = rows * n_tr;
+        beta.resize(cells); se.resize(cells); stat.resize(cells); pv.resize(cells); n_used.resize(cells); status.resize(cells);
         const auto t0 = std::chrono::steady_clock::now();
-        const int rc = inq_assoc(device, mdl, prd, rows, ns, haps.data(), y.data(), (uint32_t)n_cov, n_cov ? cov.data() : nullptr,
-                                 beta.data(), se.data(), stat.data(), pv.data(), n_used.data(), status.data(), nullptr, nullptr);
+        const int rc = has_traits
+            ? inq_assoc_traits(device, mdl, prd, rows, ns, haps.data(), (uint32_t)n_tr, y.data(), (uint32_t)n_cov, n_cov ? cov.data() : nullptr,
+                               beta.data(), se.data(), stat.data(), pv.data(), n_used.data(), status.data(), nullptr, nullptr)
+            : inq_assoc(device, mdl, prd, rows, ns, haps.data(), y.data(), (uint32_t)n_cov, n_cov ? cov.data() : nullptr,
+                        beta.data(), se.data(), stat.data(), pv.data(), n_used.data(), status.data(), nullptr, nullptr);
         const auto t1 = std::chrono::steady_clock::now();
         s_device += std::chrono::duration<double>(t1 - t0).count();
         if (rc != INQ_OK) afail(inq_cohort_last_error());
         out.clear();
-        for (size_t r = 0; r < rows; ++r) {
-            out += keys[r];
+        for (size_t c = 0; c < cells; ++c) {
+            out += keys[c / n_tr];
             out.push_back('\t');
-            out += std::to_string(n_used[r]);
-            for (double x : {beta[r], se[r], stat[r], pv[r]}) { out.push_back('\t'); append_f64(out, x); }
+            if (has_traits) { out += traits[c % n_tr]; out.push_back('\t'); }
+            out += std::to_string(n_used[c]);
+            for (double x : {beta[c], se[c], stat[c], pv[c]}) { out.push_back('\t'); append_f64(out, x); }
             out.push_back('\t');
-            out += status[r] < 5 ? status_names[status[r]] : "?";
+            out += status[c] < 5 ? status_names[status[c]] : "?";
             out.push_back('\n');
             if (out.size() >= (4u << 20)) { fwrite(out.data(), 1, out.size(), stdout); out.clear(); }
         }
@@ -536,8 +582,8 @@ int assoc_main(const std::vector<std::string> &v, int device)
         const double total = std::chrono::duration<double>(std::chrono::steady_clock::now() - t_start).count();
         FILE *f = fopen(stats_json.c_str(), "w");
         if (!f) afail(stats_json + ": cannot write");
-        fprintf(f, "{\"rows\": %llu, \"samples_used\": %u, \"s_total\": %.6f, \"s_device\": %.6f, \"s_write\": %.6f, \"s_parse\": %.6f}\n",
-                (unsigned long long)n_rows, ns, total, s_device, s_write, total - s_device - s_write);
+        fprintf(f, "{\"rows\": %llu, \"samples_used\": %u, \"traits\": %zu, \"groups\": %zu, \"s_total\": %.6f, \"s_device\": %.6f, \"s_write\": %.6f, \"s_parse\": %.6f}\n",
+                (unsigned long long)n_rows, ns, n_tr, n_groups, total, s_device, s_write, total - s_device - s_write);
         fclose(f);
     }
     return 0;

@@ -1,7 +1,9 @@
 // inq_assoc.cuh -- sm_100a kernels of `assoc`: per-locus regression of a trait on STR length. k_assoc fits the
-// linear and the logistic model, k_assoc_firth the Firth-penalized logistic model (DESIGN.md 5e).
+// linear and the logistic model, k_assoc_firth the Firth-penalized logistic model (DESIGN.md 5e). For several traits
+// (inq_assoc_traits), k_assoc_traits runs the same per-locus fits once per trait, and k_assoc_linear_traits shares one
+// Gram matrix per locus between the linear traits of one sample set.
 //
-// Both kernels have one layout. One warp per locus, four loci per CTA. The design is [1, covariates..., x] with x last
+// All kernels have one layout. One warp per locus, four loci per CTA. The design is [1, covariates..., x] with x last
 // (p <= 32 columns); lane j owns row j of the matrix being accumulated and entry j of the right-hand side, in f64
 // registers (P = p rounded up to 4, 8, 16 or 32 is a template parameter, so the rows stay in registers). Each kernel
 // keeps its own iteration logic and builds every sweep over the samples from the same routines:
@@ -109,12 +111,22 @@ struct AssocOut {
 
 __device__ __forceinline__ double predictor(double2 v, int use_max) { return use_max ? fmax(v.x, v.y) : v.x + v.y; }
 
+// The samples of one trait group (k_assoc_traits, k_assoc_linear_traits): sample s of the group is column idx[s] of
+// the locus's haplotype row, or column s when idx is null (the group has every sample of the row).
+struct SampleSubset {
+    const double2 *h;
+    const uint32_t *__restrict__ idx;
+    __device__ __forceinline__ double2 operator[](uint32_t s) const { return idx ? h[idx[s]] : h[s]; }
+};
+
 struct LocusSums {
     uint32_t n;                            // samples with a call
     double xbar, cases;                    // mean of x over them, sum of the trait over them
 };
 
-__device__ __forceinline__ LocusSums locus_prepass(const double2 *h, const double *__restrict__ y, uint32_t n_samples,
+// H: the locus's haplotype pairs, h[s] for sample s: a double2 pointer, or SampleSubset
+template <class H>
+__device__ __forceinline__ LocusSums locus_prepass(const H &h, const double *__restrict__ y, uint32_t n_samples,
                                                    int use_max, bool have, uint32_t lane)
 {
     double sx = 0.0, sy = 0.0;
@@ -134,21 +146,28 @@ __device__ __forceinline__ LocusSums locus_prepass(const double2 *h, const doubl
 // s_des has the odd row stride P + 1 in doubles, so lane-per-row reads spread over the banks. tid is threadIdx.x of the
 // caller: the kernel's read carries the range [0, kAWarps * 32) of __launch_bounds__, and with it the compiler needs no
 // guard in front of the first trip of the loop below (a read here would get a guard branch per tile).
-template <int P>
+// K traits (k_assoc_linear_traits): s_y holds kATile rows of YS doubles, trait k of sample r at s_y[r * YS + k] (0 for
+// k >= kn), read from y[k * n_samples + s].
+template <int P, int K = 1, int YS = 1>
 __device__ __forceinline__ void stage_tile(double (*s_des)[P + 1], double *s_y, const double *__restrict__ design,
-                                           const double *__restrict__ y, uint32_t s0, uint32_t n_samples, uint32_t tid)
+                                           const double *__restrict__ y, uint32_t s0, uint32_t n_samples, uint32_t tid,
+                                           uint32_t kn = 1)
 {
     __syncthreads();
     for (uint32_t t = tid; t < (uint32_t)kATile * P; t += blockDim.x) {
         const uint32_t r = t / P, c = t % P, s = s0 + r;
         s_des[r][c] = s < n_samples ? design[(uint64_t)s * P + c] : 0.0;
     }
-    if (tid < kATile) s_y[tid] = s0 + tid < n_samples ? y[s0 + tid] : 0.0;
+    if (tid < kATile)
+#pragma unroll
+        for (int k = 0; k < K; ++k)
+            s_y[tid * YS + k] = s0 + tid < n_samples && (uint32_t)k < kn ? y[(uint64_t)k * n_samples + (s0 + tid)] : 0.0;
     __syncthreads();
 }
 
 // x - xbar of sample s; NaN for a sample without a call and for the padding of the last tile
-__device__ __forceinline__ double lane_x(const double2 *h, uint32_t s, uint32_t n_samples, int use_max, double xbar)
+template <class H>
+__device__ __forceinline__ double lane_x(const H &h, uint32_t s, uint32_t n_samples, int use_max, double xbar)
 {
     double xt = __longlong_as_double(0x7ff8000000000000ll);
     if (s < n_samples) xt = predictor(h[s], use_max) - xbar;
@@ -166,10 +185,11 @@ __device__ __forceinline__ double lane_eta(const double *beta, const double *des
 
 // The ballot walk over the valid samples of the tile: u = [design row, x] of sample i, lane j adds W_i u_i u_ij to
 // row j of G (its x entry to gx: a run-time index into G would put G in local memory; put_x moves it in),
-// rhs_term(W_i u_ij, u_ij, v_i, rhs) to rhs and, with with_diag, W_i (u_ij + shift_j)^2 to diag, the uncentred G_jj.
-// Each kernel keeps its own expression for the right-hand side: fma(W u, z, .) and fma(W z, u, .) round differently.
-template <int P, class RhsTerm>
-__device__ __forceinline__ void accumulate_tile(double (&G)[P], double &gx, double &rhs, double &diag,
+// rhs_term(rhs, W_i u_ij, u_ij, v_i, i) adds its terms to rhs and, with with_diag, W_i (u_ij + shift_j)^2 to diag,
+// the uncentred G_jj. Each kernel keeps its own expression for the right-hand side: fma(W u, z, .) and fma(W z, u, .)
+// round differently; k_assoc_linear_traits reads its K values of sample i from shared memory (v unused).
+template <int P, class Rhs, class RhsTerm>
+__device__ __forceinline__ void accumulate_tile(double (&G)[P], double &gx, Rhs &rhs, double &diag,
                                                 const double (*s_des)[P + 1], uint32_t lane, uint32_t xcol, bool valid,
                                                 double xt, double W, double v, double my_shift, bool with_diag,
                                                 RhsTerm rhs_term)
@@ -186,7 +206,7 @@ __device__ __forceinline__ void accumulate_tile(double (&G)[P], double &gx, doub
 #pragma unroll
         for (int k = 0; k < P; ++k) G[k] = fma(a, s_des[i][k], G[k]);
         gx = fma(a, xi, gx);
-        rhs = rhs_term(a, uj, vi, rhs);
+        rhs_term(rhs, a, uj, vi, i);
         if (with_diag) {
             const double raw = uj + my_shift;
             diag = fma(wi * raw, raw, diag);
@@ -201,10 +221,12 @@ __device__ __forceinline__ void put_x(double (&G)[P], double gx, uint32_t xcol)
     for (int k = 0; k < P; ++k) if (k == (int)xcol) G[k] = gx;
 }
 
-// Solves G b = rhs over the columns c < p that keep(c, d_c) accepts, d_c the pivot of column c after the kept earlier
-// columns; G is overwritten. -> this lane's coefficient (0 for a dropped column and for lanes >= p).
-template <int P, class Keep>
-__device__ __forceinline__ double ldl_solve(double (&G)[P], double rhs, uint32_t p, uint32_t lane, Keep keep)
+// Solves G b_r = rhs_r for R right-hand sides over the columns c < p that keep(c, d_c) accepts, d_c the pivot of column
+// c after the kept earlier columns; G is eliminated once and every right-hand side sees the operations of a solve of
+// its own. G and rhs are overwritten. -> b: this lane's coefficients (0 for a dropped column and for lanes >= p).
+template <int P, int R, class Keep>
+__device__ __forceinline__ void ldl_solve(double (&G)[P], double (&rhs)[R], double (&b)[R], uint32_t p, uint32_t lane,
+                                          Keep keep)
 {
     uint32_t kept = 0;
 #pragma unroll
@@ -214,24 +236,31 @@ __device__ __forceinline__ double ldl_solve(double (&G)[P], double rhs, uint32_t
         if (!keep(c, d)) continue;
         kept |= 1u << c;
         const double l = G[c] / d;
-        const double bc = __shfl_sync(0xffffffffu, rhs, c);
+        double bc[R];
+#pragma unroll
+        for (int r = 0; r < R; ++r) bc[r] = __shfl_sync(0xffffffffu, rhs[r], c);
 #pragma unroll
         for (int k = c + 1; k < P; ++k) {
             if (k >= (int)p) break;
             const double gck = __shfl_sync(0xffffffffu, G[k], c);
             if ((int)lane > c) G[k] = fma(-l, gck, G[k]);
         }
-        if ((int)lane > c) rhs = fma(-l, bc, rhs);
-    }
-    double acc = 0.0, b = 0.0;
 #pragma unroll
-    for (int c = P - 1; c >= 0; --c) {
-        if (c >= (int)p || !((kept >> c) & 1u)) continue;
-        const double bc = __shfl_sync(0xffffffffu, (rhs - acc) / G[c], c);
-        if ((int)lane == c) b = bc;
-        if ((int)lane < c) acc = fma(G[c], bc, acc);
+        for (int r = 0; r < R; ++r)
+            if ((int)lane > c) rhs[r] = fma(-l, bc[r], rhs[r]);
     }
-    return b;
+#pragma unroll
+    for (int r = 0; r < R; ++r) {
+        double acc = 0.0, br = 0.0;
+#pragma unroll
+        for (int c = P - 1; c >= 0; --c) {
+            if (c >= (int)p || !((kept >> c) & 1u)) continue;
+            const double bc = __shfl_sync(0xffffffffu, (rhs[r] - acc) / G[c], c);
+            if ((int)lane == c) br = bc;
+            if ((int)lane < c) acc = fma(G[c], bc, acc);
+        }
+        b[r] = br;
+    }
 }
 
 template <int P>
@@ -261,18 +290,16 @@ __device__ __forceinline__ void write_tail(const AssocOut &out, uint64_t row, bo
 // mu, the deviance of beta_t, and the weights / working response of the next solve, and accumulates that solve's G.
 // shift: P column shifts (covariate means; 0 for the intercept and x), to rebuild the uncentred G_jj
 // y    : n_samples trait values (linear: centred by their mean)
-template <int P>
-__global__ void __launch_bounds__(kAWarps * 32)
-k_assoc(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_samples, uint32_t p, int logistic, int use_max,
-        const double *__restrict__ design, const double *__restrict__ shift, const double *__restrict__ y, AssocOut out)
+// One locus of k_assoc / k_assoc_traits: h its haplotype pairs, have = the warp has a locus, row its output index.
+template <int P, class H>
+__device__ __forceinline__ void assoc_fit(uint32_t tid, const H &h, bool have, uint64_t row, uint32_t n_samples, uint32_t p, int logistic,
+                                          int use_max, const double *__restrict__ design, const double *__restrict__ shift,
+                                          const double *__restrict__ y, const AssocOut &out)
 {
     __shared__ double s_des[kATile][P + 1];
     __shared__ double s_y[kATile];
     __shared__ double s_beta[kAWarps][P];
-    const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const uint64_t row = (uint64_t)blockIdx.x * kAWarps + warp;
-    const bool have = row < n_rows;
-    const double2 *h = reinterpret_cast<const double2 *>(haps + (have ? row : 0) * 2ull * n_samples);
+    const uint32_t lane = tid & 31, warp = tid >> 5;
     const uint32_t xcol = p - 1;
     const auto [n, xbar, cases] = locus_prepass(h, y, n_samples, use_max, have, lane);
 
@@ -295,7 +322,7 @@ k_assoc(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_samples, ui
         bool sep_l = false;
         const bool need_gram = !done && (logistic || pass == 0);
         for (uint32_t s0 = 0; s0 < n_samples; s0 += kATile) {
-            stage_tile<P>(s_des, s_y, design, y, s0, n_samples, threadIdx.x);
+            stage_tile<P>(s_des, s_y, design, y, s0, n_samples, tid);
             if (done) continue;
             const double xt = lane_x(h, s0 + lane, n_samples, use_max, xbar);
             const bool valid = xt == xt;
@@ -322,7 +349,7 @@ k_assoc(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_samples, ui
             }
             if (!need_gram) continue;
             accumulate_tile<P>(G, gx, rhs, diag, s_des, lane, xcol, valid, xt, W, z, my_shift, true,
-                               [](double a, double, double zi, double rhs) { return fma(a, zi, rhs); });
+                               [](double &rhs, double a, double, double zi, int) { rhs = fma(a, zi, rhs); });
         }
         if (!done) {
             const double dev = warp_sum(dsum);             // deviance of the current coefficients (linear: RSS)
@@ -360,7 +387,8 @@ k_assoc(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_samples, ui
                 put_x(G, gx, xcol);
                 uint32_t kept = 0;
                 double d_x = 0.0;
-                const double b = ldl_solve<P>(G, rhs, p, lane, [&](int c, double d) {
+                double b[1], r1[1] = {rhs};
+                ldl_solve<P>(G, r1, b, p, lane, [&](int c, double d) {
                     if (!(d > kAAlias * __shfl_sync(0xffffffffu, diag, c))) return false;   // aliased (or empty) column
                     kept |= 1u << c;
                     if (c == (int)xcol) d_x = d;
@@ -373,8 +401,8 @@ k_assoc(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_samples, ui
                 else {
                     rank = rk;
                     dx = d_x;
-                    beta_lane = b;
-                    publish_beta<P>(s_beta[warp], lane, b);
+                    beta_lane = b[0];
+                    publish_beta<P>(s_beta[warp], lane, b[0]);
                     if (logistic) ++iter;
                 }
             }
@@ -382,6 +410,18 @@ k_assoc(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_samples, ui
         ++pass;
     }
     write_tail(out, row, have, lane, n, status, iter);
+}
+
+template <int P>
+__global__ void __launch_bounds__(kAWarps * 32)
+k_assoc(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_samples, uint32_t p, int logistic, int use_max,
+        const double *__restrict__ design, const double *__restrict__ shift, const double *__restrict__ y, AssocOut out)
+{
+    const uint32_t tid = threadIdx.x;
+    const uint64_t row = (uint64_t)blockIdx.x * kAWarps + (tid >> 5);
+    const bool have = row < n_rows;
+    assoc_fit<P>(tid, reinterpret_cast<const double2 *>(haps + (have ? row : 0) * 2ull * n_samples), have, row, n_samples, p,
+                 logistic, use_max, design, shift, y, out);
 }
 
 // ---------------------------------------------------------------------------------------------------------------
@@ -401,10 +441,10 @@ constexpr int kFMaxHalvings = 5;           // halvings per step
 constexpr double kFLambda2 = 1e-10;        // convergence: delta_F . U*_F below this
 constexpr double kFRise = 1e-12;           // halve when D* > D*_prev + kFRise (|D*_prev| + 1)
 
-template <int P>
-__global__ void __launch_bounds__(kAWarps * 32)
-k_assoc_firth(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_samples, uint32_t p, int use_max,
-              const double *__restrict__ design, const double *__restrict__ shift, const double *__restrict__ y, AssocOut out)
+template <int P, class H>
+__device__ __forceinline__ void firth_fit(uint32_t tid, const H &h, bool have, uint64_t row, uint32_t n_samples, uint32_t p, int use_max,
+                                          const double *__restrict__ design, const double *__restrict__ shift,
+                                          const double *__restrict__ y, const AssocOut &out)
 {
     __shared__ double s_des[kATile][P + 1];
     __shared__ double s_y[kATile];
@@ -412,10 +452,7 @@ k_assoc_firth(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_sampl
     __shared__ double s_li[kAWarps][P][P];     // L^-1 of the warp's last factor of I (identity outside K)
     __shared__ double s_dinv[kAWarps][P];      // 1 / d_c for c in K, 0 elsewhere
     __shared__ double s_full[kAWarps][3];      // the full fit's beta_x, se and D*
-    const uint32_t lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const uint64_t row = (uint64_t)blockIdx.x * kAWarps + warp;
-    const bool have = row < n_rows;
-    const double2 *h = reinterpret_cast<const double2 *>(haps + (have ? row : 0) * 2ull * n_samples);
+    const uint32_t lane = tid & 31, warp = tid >> 5;
     const uint32_t xcol = p - 1;
     const auto [n, xbar, cases] = locus_prepass(h, y, n_samples, use_max, have, lane);
 
@@ -440,7 +477,7 @@ k_assoc_firth(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_sampl
         double gx = 0.0, rhs = 0.0, diag = 0.0;
         double dsum = 0.0;
         for (uint32_t s0 = 0; s0 < n_samples; s0 += kATile) {
-            stage_tile<P>(s_des, s_y, design, y, s0, n_samples, threadIdx.x);
+            stage_tile<P>(s_des, s_y, design, y, s0, n_samples, tid);
             if (done) continue;
             const double xt = lane_x(h, s0 + lane, n_samples, use_max, xbar);
             const bool valid = xt == xt;
@@ -468,7 +505,7 @@ k_assoc_firth(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_sampl
                 r = (yl != 0.0 ? omu : -mu) + hh * (0.5 - mu);
             }
             accumulate_tile<P>(G, gx, rhs, diag, s_des, lane, xcol, valid, xt, W, r, my_shift, first,
-                               [](double, double uj, double ri, double rhs) { return fma(ri, uj, rhs); });
+                               [](double &rhs, double, double uj, double ri, int) { rhs = fma(ri, uj, rhs); });
         }
         if (done) { continue; }
         put_x(G, gx, xcol);
@@ -541,7 +578,9 @@ k_assoc_firth(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_sampl
         // B: delta_F = H_FF^-1 U*_F over F; rhs keeps U*
         sweep_b = false;
         const uint32_t fmask = fit == 0 ? kmask : kmask & ~(1u << xcol);
-        const double delta = ldl_solve<P>(G, rhs, p, lane, [&](int c, double) { return ((fmask >> c) & 1u) != 0; });
+        double dl[1], r1[1] = {rhs};
+        ldl_solve<P>(G, r1, dl, p, lane, [&](int c, double) { return ((fmask >> c) & 1u) != 0; });
+        const double delta = dl[0];
         const double lam2 = warp_sum(lane < P && ((fmask >> lane) & 1u) ? delta * rhs : 0.0);
         const bool conv = lam2 < kFLambda2;
         if (!conv && t < kFMaxSteps) {
@@ -569,6 +608,153 @@ k_assoc_firth(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_sampl
         publish_beta<P>(s_beta[warp], lane, b);
     }
     write_tail(out, row, have, lane, n, status, t_full);
+}
+
+template <int P>
+__global__ void __launch_bounds__(kAWarps * 32)
+k_assoc_firth(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_samples, uint32_t p, int use_max,
+              const double *__restrict__ design, const double *__restrict__ shift, const double *__restrict__ y, AssocOut out)
+{
+    const uint32_t tid = threadIdx.x;
+    const uint64_t row = (uint64_t)blockIdx.x * kAWarps + (tid >> 5);
+    const bool have = row < n_rows;
+    firth_fit<P>(tid, reinterpret_cast<const double2 *>(haps + (have ? row : 0) * 2ull * n_samples), have, row, n_samples, p,
+                 use_max, design, shift, y, out);
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// Several traits (inq_assoc_traits, DESIGN.md 5e, Several traits). A group is the traits of one sample set: its n_samples
+// samples are columns idx[s] of the haplotype rows (stride n_all samples; idx null: all of them), and its design, shifts
+// and traits (y: n_tr x n_samples, trait j of the group is output column tcol[j] of n_traits) are prepared over them
+// exactly as inq_assoc prepares a single trait, so every trait's fit is the single-trait fit bit for bit.
+
+// Logistic and Firth: W depends on the trait, so each CTA fits one trait of the group on kAWarps loci. The CTAs of one
+// block of loci for all traits of the group are adjacent: the haplotype rows come from HBM once, the other traits hit L2.
+template <int P, bool kFirth>
+__global__ void __launch_bounds__(kAWarps * 32)
+k_assoc_traits(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_all, const uint32_t *__restrict__ idx,
+               uint32_t n_samples, uint32_t p, int use_max, const double *__restrict__ design,
+               const double *__restrict__ shift, const double *__restrict__ y, uint32_t n_tr,
+               const uint32_t *__restrict__ tcol, uint32_t n_traits, AssocOut out)
+{
+    const uint32_t tid = threadIdx.x, j = blockIdx.x % n_tr;
+    const uint64_t row = (uint64_t)(blockIdx.x / n_tr) * kAWarps + (tid >> 5);
+    const bool have = row < n_rows;
+    const SampleSubset h{reinterpret_cast<const double2 *>(haps + (have ? row : 0) * 2ull * n_all), idx};
+    const uint64_t orow = row * n_traits + tcol[j];
+    const double *yj = y + (uint64_t)j * n_samples;
+    if constexpr (kFirth) firth_fit<P>(tid, h, have, orow, n_samples, p, use_max, design, shift, yj, out);
+    else assoc_fit<P>(tid, h, have, orow, n_samples, p, 1, use_max, design, shift, yj, out);
+}
+
+// Linear, shared Gram: G = X'X and the rank rule depend on the samples and covariates only. Each CTA takes kAWarps loci
+// and a chunk of up to K traits of the group (chunks of one block of loci adjacent, as above). Pass 0 accumulates G and
+// the uncentred G_jj once and X'y of the K traits with the operations of k_assoc's pass 0; one elimination of G solves
+// all K right-hand sides; pass 1 sums every trait's squared residuals. n, rank and the status are shared by the chunk.
+// K, the traits of one chunk, for the padded width P: the most for which ptxas reports no spill and no stack frame
+constexpr int lin_traits_chunk(int P) { return P <= 8 ? 16 : P == 16 ? 7 : 4; }
+
+template <int P, int K>
+__global__ void __launch_bounds__(kAWarps * 32)
+k_assoc_linear_traits(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_all, const uint32_t *__restrict__ idx,
+                      uint32_t n_samples, uint32_t p, int use_max, const double *__restrict__ design,
+                      const double *__restrict__ shift, const double *__restrict__ y, uint32_t n_tr,
+                      const uint32_t *__restrict__ tcol, uint32_t n_traits, AssocOut out)
+{
+    constexpr int YS = K | 1;                  // odd row stride: lane-per-row reads of s_y spread over the banks
+    __shared__ double s_des[kATile][P + 1];
+    __shared__ double s_y[kATile * YS];
+    __shared__ double s_beta[kAWarps][K][P];
+    const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const uint32_t n_chunks = (n_tr + K - 1) / K, chunk = blockIdx.x % n_chunks, k0 = chunk * K;
+    const uint32_t kn = min((uint32_t)K, n_tr - k0);
+    const uint64_t row = (uint64_t)(blockIdx.x / n_chunks) * kAWarps + warp;
+    const bool have = row < n_rows;
+    const SampleSubset h{reinterpret_cast<const double2 *>(haps + (have ? row : 0) * 2ull * n_all), idx};
+    const double *yk = y + (uint64_t)k0 * n_samples;
+    const uint32_t xcol = p - 1;
+    const auto [n, xbar, cases] = locus_prepass(h, yk, n_samples, use_max, have, lane);
+    (void)cases;
+
+    uint8_t status = INQ_ASSOC_OK;
+    bool done = !have;
+    if (have && n == 0) { status = INQ_ASSOC_FEW_SAMPLES; done = true; }
+    const double my_shift = lane == xcol ? xbar : (lane < P ? shift[lane] : 0.0);
+
+    // pass 0: row `lane` of G, X'y of each trait, uncentred G_jj
+    double G[P];
+#pragma unroll
+    for (int k = 0; k < P; ++k) G[k] = 0.0;
+    double gx = 0.0, rhs[K], diag = 0.0;
+#pragma unroll
+    for (int k = 0; k < K; ++k) rhs[k] = 0.0;
+    for (uint32_t s0 = 0; s0 < n_samples; s0 += kATile) {
+        stage_tile<P, K, YS>(s_des, s_y, design, yk, s0, n_samples, tid, kn);
+        if (done) continue;
+        const double xt = lane_x(h, s0 + lane, n_samples, use_max, xbar);
+        accumulate_tile<P>(G, gx, rhs, diag, s_des, lane, xcol, xt == xt, xt, 1.0, 0.0, my_shift, true,
+                           [&](double (&r)[K], double a, double, double, int i) {
+#pragma unroll
+                               for (int k = 0; k < K; ++k) r[k] = fma(a, s_y[i * YS + k], r[k]);
+                           });
+    }
+    int rank = 0;
+    double dx = 0.0, b[K];
+    if (!done) {
+        put_x(G, gx, xcol);
+        uint32_t kept = 0;
+        ldl_solve<P>(G, rhs, b, p, lane, [&](int c, double d) {
+            if (!(d > kAAlias * __shfl_sync(0xffffffffu, diag, c))) return false;   // aliased (or empty) column
+            kept |= 1u << c;
+            if (c == (int)xcol) dx = d;
+            return true;
+        });
+        rank = __popc(kept);
+        if (n <= (uint32_t)rank) { status = INQ_ASSOC_FEW_SAMPLES; done = true; }
+        else if (!((kept >> xcol) & 1u)) { status = INQ_ASSOC_SINGULAR; done = true; }
+        else {
+            __syncwarp();
+#pragma unroll
+            for (int k = 0; k < K; ++k)
+                if (lane < P) s_beta[warp][k][lane] = b[k];
+            __syncwarp();
+        }
+    }
+
+    // pass 1: residual sum of squares of each trait
+    double dsum[K];
+#pragma unroll
+    for (int k = 0; k < K; ++k) dsum[k] = 0.0;
+    if (!__syncthreads_and(done))
+        for (uint32_t s0 = 0; s0 < n_samples; s0 += kATile) {
+            stage_tile<P, K, YS>(s_des, s_y, design, yk, s0, n_samples, tid, kn);
+            if (done) continue;
+            const double xt = lane_x(h, s0 + lane, n_samples, use_max, xbar);
+            if (xt != xt) continue;
+#pragma unroll
+            for (int k = 0; k < K; ++k) {
+                if ((uint32_t)k >= kn) break;
+                const double r = s_y[lane * YS + k] - lane_eta<P>(s_beta[warp][k], s_des[lane], xcol, xt);
+                dsum[k] = fma(r, r, dsum[k]);
+            }
+        }
+    const double df = (double)n - rank;
+#pragma unroll
+    for (int k = 0; k < K; ++k) {
+        if ((uint32_t)k >= kn) break;
+        const uint64_t orow = row * n_traits + tcol[k0 + k];
+        if (!done) {
+            // as k_assoc's pass 1: the t statistic from the RSS
+            const double dev = warp_sum(dsum[k]);
+            const double se = sqrt(dev / df / dx);
+            const double beta = __shfl_sync(0xffffffffu, b[k], xcol);
+            if (lane == 0) {
+                const double t = beta / se;
+                out.beta[orow] = beta; out.se[orow] = se; out.stat[orow] = t; out.p[orow] = t_two_sided(t, df);
+            }
+        }
+        write_tail(out, orow, have, lane, n, status, 0);
+    }
 }
 
 }  // namespace inqa

@@ -8,6 +8,7 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cmath>
+#include <cstdint>
 #include <cstring>
 #include <string>
 #include <type_traits>
@@ -56,6 +57,74 @@ void with_width(int P, Launch launch)
     case 8: launch(std::integral_constant<int, 8>()); break;
     case 16: launch(std::integral_constant<int, 16>()); break;
     default: launch(std::integral_constant<int, 32>()); break;
+    }
+}
+
+// ---- assoc: the checks and the host preparation shared by inq_assoc and inq_assoc_traits
+
+int assoc_width(uint32_t pdim) { return pdim <= 4 ? 4 : pdim <= 8 ? 8 : pdim <= 16 ? 16 : 32; }
+
+int assoc_check_args(const char *fn, int model, int predictor, uint32_t n_cov)
+{
+    if (model != INQ_ASSOC_LINEAR && model != INQ_ASSOC_LOGISTIC && model != INQ_ASSOC_FIRTH) return cfail(INQ_ERR_ARG, "%s: unknown model %d", fn, model);
+    if (predictor != INQ_ASSOC_SUM && predictor != INQ_ASSOC_MAX) return cfail(INQ_ERR_ARG, "%s: unknown predictor %d", fn, predictor);
+    if (n_cov > INQ_ASSOC_MAX_COV) return cfail(INQ_ERR_ARG, "%s: %u covariates (at most %d)", fn, n_cov, INQ_ASSOC_MAX_COV);
+    return INQ_OK;
+}
+
+// y: n_samples x n_traits row-major, NaN allowed (not used for that trait) when nan_ok; cov: finite
+int assoc_check_values(const char *fn, int model, uint32_t n_samples, uint32_t n_traits, const double *y, bool nan_ok,
+                       uint32_t n_cov, const double *cov)
+{
+    for (uint32_t s = 0; s < n_samples; ++s) {
+        for (uint32_t t = 0; t < n_traits; ++t) {
+            const double v = y[(size_t)s * n_traits + t];
+            char what[32] = "trait";
+            if (n_traits > 1 || nan_ok) snprintf(what, sizeof(what), "trait %u", t);
+            if (nan_ok && std::isnan(v)) continue;
+            if (!std::isfinite(v)) return cfail(INQ_ERR_ARG, "%s: %s of sample %u is not a finite number%s", fn, what, s, nan_ok ? " or NaN" : "");
+            if (model != INQ_ASSOC_LINEAR && v != 0.0 && v != 1.0) return cfail(INQ_ERR_ARG, "%s: logistic %s of sample %u is not 0 or 1", fn, what, s);
+        }
+        for (uint32_t c = 0; c < n_cov; ++c)
+            if (!std::isfinite(cov[(size_t)s * n_cov + c])) return cfail(INQ_ERR_ARG, "%s: covariate %u of sample %u is not a finite number", fn, c, s);
+    }
+    return INQ_OK;
+}
+
+// One single-trait problem with several right-hand sides: the traits of one sample set.
+struct AssocGroup {
+    std::vector<uint32_t> idx;                 // its samples (columns of the haplotype rows) in order; empty: all of them
+    std::vector<uint32_t> traits;              // its traits (columns of y)
+    std::vector<double> design, shift, y;      // prepared over its samples; y: traits.size() x samples
+};
+
+// The kernels' inputs over the group's samples: design rows [1, covariates centred by their mean, 0 (x), 0 ...] (row
+// stride P), the P column shifts, and each trait (column t of y, row stride ld), centred by its mean for the linear model.
+void assoc_prepare(AssocGroup &gr, int model, int P, uint32_t n_all, uint32_t n_cov, const double *cov, const double *y, uint32_t ld)
+{
+    const uint32_t n = gr.idx.empty() ? n_all : (uint32_t)gr.idx.size();
+    auto sample = [&](uint32_t s) -> size_t { return gr.idx.empty() ? s : gr.idx[s]; };
+    gr.design.assign((size_t)n * P, 0.0);
+    gr.shift.assign(P, 0.0);
+    for (uint32_t c = 0; c < n_cov; ++c) {
+        double m = 0.0;
+        for (uint32_t s = 0; s < n; ++s) m += cov[sample(s) * n_cov + c];
+        gr.shift[1 + c] = m / n;
+    }
+    for (uint32_t s = 0; s < n; ++s) {
+        gr.design[(size_t)s * P] = 1.0;
+        for (uint32_t c = 0; c < n_cov; ++c) gr.design[(size_t)s * P + 1 + c] = cov[sample(s) * n_cov + c] - gr.shift[1 + c];
+    }
+    gr.y.resize(gr.traits.size() * (size_t)n);
+    for (size_t j = 0; j < gr.traits.size(); ++j) {
+        double *yj = gr.y.data() + j * n;
+        for (uint32_t s = 0; s < n; ++s) yj[s] = y[sample(s) * ld + gr.traits[j]];
+        if (model == INQ_ASSOC_LINEAR) {
+            double m = 0.0;
+            for (uint32_t s = 0; s < n; ++s) m += yj[s];
+            m /= n;
+            for (uint32_t s = 0; s < n; ++s) yj[s] -= m;
+        }
     }
 }
 
@@ -183,38 +252,17 @@ int inq_assoc(int device, int model, int predictor, uint64_t n_rows, uint32_t n_
 {
     using namespace inqa;
     if (ms_kernel) *ms_kernel = 0.f;
-    if (model != INQ_ASSOC_LINEAR && model != INQ_ASSOC_LOGISTIC && model != INQ_ASSOC_FIRTH) return cfail(INQ_ERR_ARG, "inq_assoc: unknown model %d", model);
-    if (predictor != INQ_ASSOC_SUM && predictor != INQ_ASSOC_MAX) return cfail(INQ_ERR_ARG, "inq_assoc: unknown predictor %d", predictor);
-    if (n_cov > INQ_ASSOC_MAX_COV) return cfail(INQ_ERR_ARG, "inq_assoc: %u covariates (at most %d)", n_cov, INQ_ASSOC_MAX_COV);
+    if (const int rc = assoc_check_args("inq_assoc", model, predictor, n_cov)) return rc;
     if (n_rows == 0) return INQ_OK;
     if (n_samples == 0) return cfail(INQ_ERR_ARG, "inq_assoc: no samples");
     if (!haps || !y || (n_cov && !cov) || !beta || !se || !stat || !p || !n_used || !status) return cfail(INQ_ERR_ARG, "inq_assoc: NULL array");
     if ((n_rows + kAWarps - 1) / kAWarps > 0x7FFFFFFFull) return cfail(INQ_ERR_TOO_LARGE, "inq_assoc: too many rows");
-    for (uint32_t s = 0; s < n_samples; ++s) {
-        if (!std::isfinite(y[s])) return cfail(INQ_ERR_ARG, "inq_assoc: trait of sample %u is not a finite number", s);
-        if (model != INQ_ASSOC_LINEAR && y[s] != 0.0 && y[s] != 1.0) return cfail(INQ_ERR_ARG, "inq_assoc: logistic trait of sample %u is not 0 or 1", s);
-        for (uint32_t c = 0; c < n_cov; ++c)
-            if (!std::isfinite(cov[(size_t)s * n_cov + c])) return cfail(INQ_ERR_ARG, "inq_assoc: covariate %u of sample %u is not a finite number", c, s);
-    }
+    if (const int rc = assoc_check_values("inq_assoc", model, n_samples, 1, y, false, n_cov, cov)) return rc;
     const uint32_t pdim = n_cov + 2;
-    const int P = pdim <= 4 ? 4 : pdim <= 8 ? 8 : pdim <= 16 ? 16 : 32;
-    // shared design rows [1, covariates centred by their mean, 0 (x), 0 ...]; the linear trait centred by its mean
-    std::vector<double> design((size_t)n_samples * P, 0.0), shift(P, 0.0), yc(y, y + n_samples);
-    for (uint32_t c = 0; c < n_cov; ++c) {
-        double m = 0.0;
-        for (uint32_t s = 0; s < n_samples; ++s) m += cov[(size_t)s * n_cov + c];
-        shift[1 + c] = m / n_samples;
-    }
-    for (uint32_t s = 0; s < n_samples; ++s) {
-        design[(size_t)s * P] = 1.0;
-        for (uint32_t c = 0; c < n_cov; ++c) design[(size_t)s * P + 1 + c] = cov[(size_t)s * n_cov + c] - shift[1 + c];
-    }
-    if (model == INQ_ASSOC_LINEAR) {
-        double m = 0.0;
-        for (uint32_t s = 0; s < n_samples; ++s) m += y[s];
-        m /= n_samples;
-        for (double &v : yc) v -= m;
-    }
+    const int P = assoc_width(pdim);
+    AssocGroup gr;
+    gr.traits = {0};
+    assoc_prepare(gr, model, P, n_samples, n_cov, cov, y, 1);
 
     CC_TRY(cudaSetDevice(device));
     Guard g;
@@ -224,17 +272,17 @@ int inq_assoc(int device, int model, int predictor, uint64_t n_rows, uint32_t n_
     const size_t hap_bytes = (size_t)n_rows * 2 * n_samples * sizeof(double);
     void *d_haps, *d_des, *d_shift, *d_y, *d_res, *d_n, *d_st, *d_it;
     CC_TRY(g.alloc(&d_haps, hap_bytes));
-    CC_TRY(g.alloc(&d_des, design.size() * sizeof(double)));
-    CC_TRY(g.alloc(&d_shift, shift.size() * sizeof(double)));
+    CC_TRY(g.alloc(&d_des, gr.design.size() * sizeof(double)));
+    CC_TRY(g.alloc(&d_shift, gr.shift.size() * sizeof(double)));
     CC_TRY(g.alloc(&d_y, n_samples * sizeof(double)));
     CC_TRY(g.alloc(&d_res, (size_t)n_rows * 4 * sizeof(double)));
     CC_TRY(g.alloc(&d_n, (size_t)n_rows * sizeof(uint32_t)));
     CC_TRY(g.alloc(&d_st, (size_t)n_rows));
     CC_TRY(g.alloc(&d_it, (size_t)n_rows));
     CC_TRY(cudaMemcpyAsync(d_haps, haps, hap_bytes, cudaMemcpyHostToDevice, g.s));
-    CC_TRY(cudaMemcpyAsync(d_des, design.data(), design.size() * sizeof(double), cudaMemcpyHostToDevice, g.s));
-    CC_TRY(cudaMemcpyAsync(d_shift, shift.data(), shift.size() * sizeof(double), cudaMemcpyHostToDevice, g.s));
-    CC_TRY(cudaMemcpyAsync(d_y, yc.data(), n_samples * sizeof(double), cudaMemcpyHostToDevice, g.s));
+    CC_TRY(cudaMemcpyAsync(d_des, gr.design.data(), gr.design.size() * sizeof(double), cudaMemcpyHostToDevice, g.s));
+    CC_TRY(cudaMemcpyAsync(d_shift, gr.shift.data(), gr.shift.size() * sizeof(double), cudaMemcpyHostToDevice, g.s));
+    CC_TRY(cudaMemcpyAsync(d_y, gr.y.data(), n_samples * sizeof(double), cudaMemcpyHostToDevice, g.s));
     double *r = (double *)d_res;
     const AssocOut out{r, r + n_rows, r + 2 * n_rows, r + 3 * n_rows, (uint32_t *)d_n, (uint8_t *)d_st, (uint8_t *)d_it};
     const unsigned grid = (unsigned)((n_rows + kAWarps - 1) / kAWarps);
@@ -255,6 +303,124 @@ int inq_assoc(int device, int model, int predictor, uint64_t n_rows, uint32_t n_
     CC_TRY(cudaMemcpyAsync(n_used, d_n, n_rows * sizeof(uint32_t), cudaMemcpyDeviceToHost, g.s));
     CC_TRY(cudaMemcpyAsync(status, d_st, n_rows, cudaMemcpyDeviceToHost, g.s));
     if (n_iter) CC_TRY(cudaMemcpyAsync(n_iter, d_it, n_rows, cudaMemcpyDeviceToHost, g.s));
+    CC_TRY(cudaStreamSynchronize(g.s));
+    if (ms_kernel) cudaEventElapsedTime(ms_kernel, g.e0, g.e1);
+    return INQ_OK;
+}
+
+int inq_assoc_traits(int device, int model, int predictor, uint64_t n_rows, uint32_t n_samples, const double *haps,
+                     uint32_t n_traits, const double *y, uint32_t n_cov, const double *cov, double *beta, double *se,
+                     double *stat, double *p, uint32_t *n_used, uint8_t *status, uint8_t *n_iter, float *ms_kernel)
+{
+    using namespace inqa;
+    if (ms_kernel) *ms_kernel = 0.f;
+    if (const int rc = assoc_check_args("inq_assoc_traits", model, predictor, n_cov)) return rc;
+    if (n_traits == 0) return cfail(INQ_ERR_ARG, "inq_assoc_traits: no traits");
+    if (n_rows == 0) return INQ_OK;
+    if (n_samples == 0) return cfail(INQ_ERR_ARG, "inq_assoc_traits: no samples");
+    if (!haps || !y || (n_cov && !cov) || !beta || !se || !stat || !p || !n_used || !status) return cfail(INQ_ERR_ARG, "inq_assoc_traits: NULL array");
+    if (n_rows > (uint64_t)SIZE_MAX / 64 / n_traits) return cfail(INQ_ERR_TOO_LARGE, "inq_assoc_traits: %llu rows x %u traits", (unsigned long long)n_rows, n_traits);
+    if (const int rc = assoc_check_values("inq_assoc_traits", model, n_samples, n_traits, y, true, n_cov, cov)) return rc;
+    // group the traits by their sample set (NaN pattern), groups in the order of their first trait
+    std::vector<AssocGroup> groups;
+    {
+        std::vector<std::vector<bool>> masks;
+        for (uint32_t t = 0; t < n_traits; ++t) {
+            std::vector<bool> m(n_samples);
+            uint32_t cnt = 0;
+            for (uint32_t s = 0; s < n_samples; ++s) cnt += m[s] = !std::isnan(y[(size_t)s * n_traits + t]);
+            if (!cnt) return cfail(INQ_ERR_ARG, "inq_assoc_traits: trait %u has no value (every sample NaN)", t);
+            size_t k = 0;
+            while (k < masks.size() && masks[k] != m) ++k;
+            if (k == masks.size()) {
+                masks.push_back(m);
+                groups.emplace_back();
+                if (cnt < n_samples)
+                    for (uint32_t s = 0; s < n_samples; ++s)
+                        if (m[s]) groups[k].idx.push_back(s);
+            }
+            groups[k].traits.push_back(t);
+        }
+    }
+    const uint32_t pdim = n_cov + 2;
+    const int P = assoc_width(pdim);
+    const int K = lin_traits_chunk(P);
+    const uint64_t blocks = (n_rows + kAWarps - 1) / kAWarps;
+    for (const AssocGroup &gr : groups) {
+        const uint64_t per = model == INQ_ASSOC_LINEAR ? (gr.traits.size() + K - 1) / K : gr.traits.size();
+        if (blocks > 0x7FFFFFFFull / per)
+            return cfail(INQ_ERR_TOO_LARGE, "inq_assoc_traits: %llu rows x %zu traits of one sample set exceed the launch shape",
+                         (unsigned long long)n_rows, gr.traits.size());
+    }
+    for (AssocGroup &gr : groups) assoc_prepare(gr, model, P, n_samples, n_cov, cov, y, n_traits);
+
+    CC_TRY(cudaSetDevice(device));
+    Guard g;
+    CC_TRY(cudaStreamCreateWithFlags(&g.s, cudaStreamNonBlocking));
+    CC_TRY(cudaEventCreate(&g.e0));
+    CC_TRY(cudaEventCreate(&g.e1));
+    // the haplotype matrix goes to the device once; each group reads its samples through its index
+    const size_t hap_bytes = (size_t)n_rows * 2 * n_samples * sizeof(double), cells = (size_t)n_rows * n_traits;
+    void *d_haps, *d_res, *d_n, *d_st, *d_it;
+    CC_TRY(g.alloc(&d_haps, hap_bytes));
+    CC_TRY(g.alloc(&d_res, cells * 4 * sizeof(double)));
+    CC_TRY(g.alloc(&d_n, cells * sizeof(uint32_t)));
+    CC_TRY(g.alloc(&d_st, cells));
+    CC_TRY(g.alloc(&d_it, cells));
+    CC_TRY(cudaMemcpyAsync(d_haps, haps, hap_bytes, cudaMemcpyHostToDevice, g.s));
+    struct DevGroup { const double *des, *shift, *y; const uint32_t *idx, *tcol; };
+    std::vector<DevGroup> dg(groups.size());
+    auto upload = [&](const void *src, size_t bytes, const void **dst) -> int {
+        void *q;
+        CC_TRY(g.alloc(&q, bytes));
+        CC_TRY(cudaMemcpyAsync(q, src, bytes, cudaMemcpyHostToDevice, g.s));
+        *dst = q;
+        return INQ_OK;
+    };
+    for (size_t k = 0; k < groups.size(); ++k) {
+        const AssocGroup &gr = groups[k];
+        DevGroup &d = dg[k];
+        int rc = upload(gr.design.data(), gr.design.size() * sizeof(double), (const void **)&d.des);
+        if (!rc) rc = upload(gr.shift.data(), gr.shift.size() * sizeof(double), (const void **)&d.shift);
+        if (!rc) rc = upload(gr.y.data(), gr.y.size() * sizeof(double), (const void **)&d.y);
+        if (!rc) rc = upload(gr.traits.data(), gr.traits.size() * sizeof(uint32_t), (const void **)&d.tcol);
+        d.idx = nullptr;
+        if (!rc && !gr.idx.empty()) rc = upload(gr.idx.data(), gr.idx.size() * sizeof(uint32_t), (const void **)&d.idx);
+        if (rc) return rc;
+    }
+    double *r = (double *)d_res;
+    const AssocOut out{r, r + cells, r + 2 * cells, r + 3 * cells, (uint32_t *)d_n, (uint8_t *)d_st, (uint8_t *)d_it};
+    const int mx = predictor == INQ_ASSOC_MAX;
+    const double *dh = (const double *)d_haps;
+    CC_TRY(cudaEventRecord(g.e0, g.s));
+    for (size_t k = 0; k < groups.size(); ++k) {
+        const DevGroup &d = dg[k];
+        const uint32_t ng = groups[k].idx.empty() ? n_samples : (uint32_t)groups[k].idx.size(), nt = (uint32_t)groups[k].traits.size();
+        with_width(P, [&](auto width) {
+            constexpr int W = decltype(width)::value;
+            if (model == INQ_ASSOC_LINEAR) {
+                constexpr int KW = lin_traits_chunk(W);
+                const unsigned grid = (unsigned)(blocks * ((nt + KW - 1) / KW));
+                k_assoc_linear_traits<W, KW><<<grid, kAWarps * 32, 0, g.s>>>(dh, n_rows, n_samples, d.idx, ng, pdim, mx, d.des, d.shift, d.y, nt,
+                                                                            d.tcol, n_traits, out);
+            } else {
+                const unsigned grid = (unsigned)(blocks * nt);
+                if (model == INQ_ASSOC_FIRTH)
+                    k_assoc_traits<W, true><<<grid, kAWarps * 32, 0, g.s>>>(dh, n_rows, n_samples, d.idx, ng, pdim, mx, d.des, d.shift, d.y, nt, d.tcol, n_traits, out);
+                else
+                    k_assoc_traits<W, false><<<grid, kAWarps * 32, 0, g.s>>>(dh, n_rows, n_samples, d.idx, ng, pdim, mx, d.des, d.shift, d.y, nt, d.tcol, n_traits, out);
+            }
+        });
+        CC_TRY(cudaGetLastError());
+    }
+    CC_TRY(cudaEventRecord(g.e1, g.s));
+    CC_TRY(cudaMemcpyAsync(beta, r, cells * sizeof(double), cudaMemcpyDeviceToHost, g.s));
+    CC_TRY(cudaMemcpyAsync(se, r + cells, cells * sizeof(double), cudaMemcpyDeviceToHost, g.s));
+    CC_TRY(cudaMemcpyAsync(stat, r + 2 * cells, cells * sizeof(double), cudaMemcpyDeviceToHost, g.s));
+    CC_TRY(cudaMemcpyAsync(p, r + 3 * cells, cells * sizeof(double), cudaMemcpyDeviceToHost, g.s));
+    CC_TRY(cudaMemcpyAsync(n_used, d_n, cells * sizeof(uint32_t), cudaMemcpyDeviceToHost, g.s));
+    CC_TRY(cudaMemcpyAsync(status, d_st, cells, cudaMemcpyDeviceToHost, g.s));
+    if (n_iter) CC_TRY(cudaMemcpyAsync(n_iter, d_it, cells, cudaMemcpyDeviceToHost, g.s));
     CC_TRY(cudaStreamSynchronize(g.s));
     if (ms_kernel) cudaEventElapsedTime(ms_kernel, g.e0, g.e1);
     return INQ_OK;

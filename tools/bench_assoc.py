@@ -6,7 +6,11 @@ FMAs the fits need (from shapes and iteration counts) and GFLOP/s, and parity of
 numpy restatement (oracle/assoc.py, not R or logistf) with its host time. `firth` lines (the case/control trait,
 `--firth`) report the steps of the full fit over every locus and of both fits on the parity loci instead of FMAs.
 Then one line per model for the CLI on the same table written as TSV: wall time with text parse, device and output
-time separated (`--stats-json`). The card's name and power limit are read in the same run.
+time separated (`--stats-json`). With --traits, `assoc_traits` lines: the kernel time of one inq_assoc_traits call
+for 1, 8 and 32 linear traits and for 8 logistic and 8 Firth traits (seeded extra traits; the last quarter of them
+share one distinct NaN pattern, so they form a second sample set) against that many times the single-trait kernel
+of the same run, and the CLI wall time of `--traits` with 8 traits against 8 `--trait` runs on the same TSV.
+The card's name and power limit are read in the same run.
 Temporary files go to a temporary directory."""
 import argparse
 import json
@@ -43,6 +47,19 @@ def workload(rows, samples, n_cov, seed=2024):
     return haps, cov, y_lin, y_bin
 
 
+def traits_matrix(y0, T, model, seed=99):
+    """T traits for --traits: y0 first, then seeded ones of the same kind; the last T // 4 share one NaN pattern."""
+    rng = np.random.default_rng(seed)
+    n = len(y0)
+    Y = np.empty((n, T))
+    Y[:, 0] = y0
+    for t in range(1, T):
+        Y[:, t] = rng.normal(3, 1, n) if model == "linear" else (rng.random(n) < 0.4).astype(float)
+    if T >= 4:
+        Y[rng.random(n) < 0.1, T - T // 4:] = np.nan
+    return Y
+
+
 def fmas(res, p, model):
     """f64 FMAs of the passes over the samples, n samples used and p design columns per locus:
     linear   one Gram pass, n * (p^2 + p) for G and X'y, and one residual pass, n * p for eta: n * (p^2 + 2p);
@@ -65,6 +82,7 @@ def main():
     ap.add_argument("--reps", type=int, default=5)
     ap.add_argument("--parity", type=int, default=2000)
     ap.add_argument("--no-cli", action="store_true")
+    ap.add_argument("--traits", action="store_true")
     args = ap.parse_args()
     from inquistr_b200 import cohort
     from oracle import assoc as A
@@ -72,6 +90,7 @@ def main():
     haps, cov, y_lin, y_bin = workload(args.rows, args.samples, args.cov)
     p = args.cov + 2
     sel = np.sort(np.random.default_rng(7).choice(args.rows, min(args.parity, args.rows), replace=False))
+    single_ms = {}
     for model in ("linear", "logistic", "firth"):
         y = y_lin if model == "linear" else y_bin
         for pred in ("sum", "max"):
@@ -81,6 +100,7 @@ def main():
                 res = cohort.assoc(haps, y, cov, model, pred)
                 ms.append(res["ms_kernel"])
             med = float(np.median(ms))
+            single_ms[model, pred] = med
             f = fmas(res, p, model) if model != "firth" else None
             t0 = time.perf_counter()
             ref = A.assoc_matrix(haps[sel], y, cov, model, pred)
@@ -110,6 +130,18 @@ def main():
                            "compared": int(ok.sum()), "max_beta_err_rel_to_abs_beta_plus_se": float(rb.max()) if ok.any() else None,
                            "max_se_rel_err": float(rs.max()) if ok.any() else None, "max_dlog10_p": float(lp.max()) if ok.any() else None},
                 "numpy_oracle_s": oracle_s, "numpy_oracle_loci_per_s": len(sel) / oracle_s}), flush=True)
+    if args.traits:
+        for model, T in (("linear", 1), ("linear", 8), ("linear", 32), ("logistic", 8), ("firth", 8)):
+            Y = traits_matrix(y_lin if model == "linear" else y_bin, T, model)
+            cohort.assoc_traits(haps, Y, cov, model, "sum")               # warm-up
+            ms = [cohort.assoc_traits(haps, Y, cov, model, "sum")["ms_kernel"] for _ in range(args.reps)]
+            med = float(np.median(ms))
+            groups = len({tuple(np.isnan(Y[:, t])) for t in range(T)})
+            print(json.dumps({"bench": "assoc_traits_kernel", "card": name, "model": model, "predictor": "sum", "traits": T,
+                              "groups": groups, "loci": args.rows, "samples": args.samples, "covariates": args.cov,
+                              "kernel_ms_median": med, "kernel_ms_all": ms, "single_trait_kernel_ms": single_ms[model, "sum"],
+                              "traits_x_single_ms": T * single_ms[model, "sum"],
+                              "speedup": T * single_ms[model, "sum"] / med}), flush=True)
     if args.no_cli:
         return
     from inquistr_b200 import build
@@ -143,6 +175,30 @@ def main():
             print(json.dumps({"bench": "assoc_cli", "card": name, "model": model, "predictor": "sum", "rc": r.returncode,
                               "table_bytes": os.path.getsize(table), "table_write_s": write_s, "wall_s": wall,
                               "rows_out": out_rows, **st, "stderr_tail": r.stderr.decode()[-300:]}), flush=True)
+        if not args.traits:
+            return
+        Y = traits_matrix(y_lin, 8, "linear")
+        ph8 = os.path.join(d, "pheno8.tsv")
+        with open(ph8, "w") as f:
+            f.write("sample\t" + "\t".join(f"t{t}" for t in range(8)) + "\t" + "\t".join(f"c{c}" for c in range(args.cov)) + "\n")
+            for i, s in enumerate(samples):
+                f.write(s + "\t" + "\t".join("NA" if np.isnan(v) else repr(float(v)) for v in Y[i]) + "\t" +
+                        "\t".join(repr(float(v)) for v in cov[i]) + "\n")
+        covs = ",".join(f"c{c}" for c in range(args.cov))
+
+        def cli_run(*trait_args):
+            sj = os.path.join(d, "stats.json")
+            t0 = time.perf_counter()
+            r = subprocess.run([exe, "assoc", "--phenotype", ph8, *trait_args, "--model", "linear", "--covariates", covs,
+                                "--stats-json", sj, table], stdout=subprocess.DEVNULL, stderr=subprocess.PIPE)
+            return time.perf_counter() - t0, r.returncode, json.load(open(sj)) if r.returncode == 0 else {}
+
+        wall, rc, st = cli_run("--traits", ",".join(f"t{t}" for t in range(8)))
+        singles = [cli_run("--trait", f"t{t}") for t in range(8)]
+        print(json.dumps({"bench": "assoc_traits_cli", "card": name, "model": "linear", "traits": 8, "rc": rc, "wall_s": wall, **st,
+                          "single_runs_wall_s": sum(w for w, _, _ in singles), "single_runs_rc": [c for _, c, _ in singles],
+                          "single_runs_s_parse": sum(x.get("s_parse", 0.0) for _, _, x in singles),
+                          "single_runs_s_device": sum(x.get("s_device", 0.0) for _, _, x in singles)}), flush=True)
 
 
 if __name__ == "__main__":
