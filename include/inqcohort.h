@@ -15,7 +15,8 @@
  * inq_assoc: per-locus association of STR length with a trait (`inquistr-b200 assoc`, DESIGN.md 5e); the model is
  * this project's own (the reference has it only as an external R script): OLS with a Student t test, or logistic
  * IRLS as R's glm.fit without step-halving with a Wald z test, or Firth-penalized logistic regression with a penalized
- * likelihood-ratio test; design [1, covariates..., x], x last.
+ * likelihood-ratio test; design [1, covariates..., x], x last. inq_assoc_cox fits Cox proportional hazards of a
+ * censored time (age at onset) instead.
  */
 #ifndef INQCOHORT_H
 #define INQCOHORT_H
@@ -83,6 +84,25 @@ int inq_assoc_traits(int device, int model, int predictor, uint64_t n_rows, uint
                      uint32_t n_traits, const double *y, uint32_t n_cov, const double *cov, double *beta, double *se,
                      double *stat, double *p, uint32_t *n_used, uint8_t *status, uint8_t *n_iter /* nullable */,
                      float *ms_kernel /* nullable */);
+
+#define INQ_COX_EFRON 0            /* Efron's approximation for tied event times (coxph's default) */
+#define INQ_COX_BRESLOW 1          /* Breslow's approximation */
+
+/* Cox proportional-hazards regression of a censored time on STR length (`assoc --model cox`, DESIGN.md 5e, Cox), as
+ * R's coxph(Surv(time, event) ~ covariates + x) with ties = "efron" or "breslow" and coxph.control's defaults:
+ * partial likelihood over u = [covariates..., x] (no intercept), Newton iteration with step-halving, at most 20
+ * iterations, converged when |loglik - loglik_old| <= 1e-9 |loglik|. time[n_samples]: any finite number;
+ * event[n_samples]: 1 = event at that time, 0 = censored at it (still at risk there). Per row: beta and
+ * se = sqrt((I^-1)_xx) of the fit, stat the Wald z, p = erfc(|z| / sqrt 2), n_used and status as inq_assoc, and
+ * n_iter (nullable) the Newton iterations. Statuses: FEW_SAMPLES (no event among the samples used, or n <= rank),
+ * SINGULAR, NO_CONVERGENCE (20 iterations), SEPARATION (a converged fit whose last Newton step for x, |(I^-1 U)_x|,
+ * exceeds 1e-9 and sqrt(1e-9) |beta|: the coefficient may be infinite, coxph's toler.inf rule).
+ * INQ_ERR_ARG names the sample for a non-finite time or covariate and an event that is not 0 or 1;
+ * INQ_ERR_TOO_LARGE when the rows exceed the launch shape (2^31 - 1 blocks of 4 loci). */
+int inq_assoc_cox(int device, int ties, int predictor, uint64_t n_rows, uint32_t n_samples, const double *haps,
+                  const double *time, const uint8_t *event, uint32_t n_cov, const double *cov, double *beta, double *se,
+                  double *stat, double *p, uint32_t *n_used, uint8_t *status, uint8_t *n_iter /* nullable */,
+                  float *ms_kernel /* nullable */);
 
 const char *inq_cohort_last_error(void);
 

@@ -26,7 +26,8 @@ def build_libinqcall(force: bool = False, verbose: bool = False) -> str:
     os.makedirs(LIBDIR, exist_ok=True)
     target = os.path.join(LIBDIR, "libinqcall.so")
     inc = os.path.join(os.path.dirname(HERE), "include")
-    units = [os.path.join(CSRC, "inq_capi.cu"), os.path.join(CSRC, "inq_cohort_capi.cu"), os.path.join(CSRC, "inq_inflate_capi.cu")]
+    units = [os.path.join(CSRC, "inq_capi.cu"), os.path.join(CSRC, "inq_cohort_capi.cu"), os.path.join(CSRC, "inq_cox_launch.cu"),
+             os.path.join(CSRC, "inq_inflate_capi.cu")]
     sources = units + [os.path.join(CSRC, "inq_device.cuh"), os.path.join(CSRC, "inq_cohort.cuh"), os.path.join(CSRC, "inq_assoc.cuh"), os.path.join(CSRC, "inq_inflate.cuh"),
                        os.path.join(CSRC, "host", "catalog_reach.hpp"),
                        os.path.join(inc, "inqcall.h"), os.path.join(inc, "inqcohort.h"), os.path.join(inc, "inqbgzf.h")]

@@ -13,7 +13,8 @@ LINEAR, LOGISTIC, FIRTH = 0, 1, 2
 PRED_SUM, PRED_MAX = 0, 1
 ASSOC_OK, ASSOC_FEW_SAMPLES, ASSOC_SINGULAR, ASSOC_NO_CONVERGENCE, ASSOC_SEPARATION = 0, 1, 2, 3, 4
 ASSOC_STATUS_NAMES = ["ok", "few_samples", "singular", "no_convergence", "separation"]
-EXPORTS = ["inq_outlier", "inq_assoc", "inq_assoc_traits", "inq_cohort_last_error"]
+COX_EFRON, COX_BRESLOW = 0, 1
+EXPORTS = ["inq_outlier", "inq_assoc", "inq_assoc_traits", "inq_assoc_cox", "inq_cohort_last_error"]
 
 _BOUND = False
 
@@ -33,6 +34,10 @@ def _lib():
         L.inq_assoc_traits.argtypes = [C.c_int, C.c_int, C.c_int, C.c_uint64, C.c_uint32, C.c_void_p, C.c_uint32, C.c_void_p,
                                        C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                        C.c_void_p, C.c_void_p, C.POINTER(C.c_float)]
+        L.inq_assoc_cox.restype = C.c_int
+        L.inq_assoc_cox.argtypes = [C.c_int, C.c_int, C.c_int, C.c_uint64, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                    C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                    C.c_void_p, C.c_void_p, C.POINTER(C.c_float)]
         L.inq_cohort_last_error.restype = C.c_char_p
         L.inq_cohort_last_error.argtypes = []
         _BOUND = True
@@ -118,6 +123,38 @@ def assoc_traits(haps, Y, cov=None, model: str = "linear", predictor: str = "sum
                             rows, ns, h.ctypes.data, nt, yy.ctypes.data, c.shape[1], c.ctypes.data if c.size else None,
                             out["beta"].ctypes.data, out["se"].ctypes.data, out["stat"].ctypes.data, out["p"].ctypes.data,
                             out["n"].ctypes.data, out["status"].ctypes.data, out["n_iter"].ctypes.data, C.byref(ms))
+    if rc != INQ_OK:
+        raise InqError(rc, L.inq_cohort_last_error().decode())
+    out["ms_kernel"] = float(ms.value)
+    return out
+
+
+def assoc_cox(haps, time, event, cov=None, ties: str = "efron", predictor: str = "sum", device: int = 0):
+    """Per-row Cox proportional-hazards regression of (time, event) on STR length (include/inqcohort.h inq_assoc_cox).
+    haps: rows x 2*samples f64 (NaN = no call); time: samples (finite); event: samples, 1 = event, 0 = censored;
+    cov: samples x n_cov or None. ties: "efron" or "breslow". stat is the Wald z.
+    -> dict of per-row arrays beta, se, stat, p (f64), n (u32), status (u8, ASSOC_*), n_iter (u8), and ms_kernel."""
+    h = np.ascontiguousarray(haps, dtype=np.float64)
+    rows, cols = h.shape
+    if cols % 2:
+        raise ValueError("haps needs two columns per sample")
+    ns = cols // 2
+    t = np.ascontiguousarray(time, dtype=np.float64)
+    e = np.asarray(event, dtype=np.float64)
+    if t.shape != (ns,) or e.shape != (ns,):
+        raise ValueError("time and event need one value per sample")
+    ev = np.ascontiguousarray(np.where(e == 0, 0, np.where(e == 1, 1, 2)), dtype=np.uint8)    # 2: rejected by the ABI
+    c = np.zeros((ns, 0)) if cov is None else np.ascontiguousarray(np.asarray(cov, np.float64).reshape(ns, -1))
+    out = {k: np.zeros(rows, np.float64) for k in ("beta", "se", "stat", "p")}
+    out["n"] = np.zeros(rows, np.uint32)
+    out["status"] = np.zeros(rows, np.uint8)
+    out["n_iter"] = np.zeros(rows, np.uint8)
+    ms = C.c_float(0)
+    L = _lib()
+    rc = L.inq_assoc_cox(device, {"efron": COX_EFRON, "breslow": COX_BRESLOW}[ties], {"sum": PRED_SUM, "max": PRED_MAX}[predictor],
+                         rows, ns, h.ctypes.data, t.ctypes.data, ev.ctypes.data, c.shape[1], c.ctypes.data if c.size else None,
+                         out["beta"].ctypes.data, out["se"].ctypes.data, out["stat"].ctypes.data, out["p"].ctypes.data,
+                         out["n"].ctypes.data, out["status"].ctypes.data, out["n_iter"].ctypes.data, C.byref(ms))
     if rc != INQ_OK:
         raise InqError(rc, L.inq_cohort_last_error().decode())
     out["ms_kernel"] = float(ms.value)

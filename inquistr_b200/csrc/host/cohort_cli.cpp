@@ -317,9 +317,9 @@ void append_f64(std::string &out, double v)
 // `assoc`: one regression per row of a combined table (DESIGN.md 5e)
 int assoc_main(const std::vector<std::string> &v, int device)
 {
-    const char *usage = "assoc --phenotype <TSV> --trait <COL> | --traits <A,B,...> --model <linear|logistic> [--firth] [--covariates A,B,...] [--predictor sum|max] [--device N] <COMBINED>";
-    std::string combined, pheno, trait, model, predictor = "sum", covs, trait_list, stats_json;
-    bool has_cov = false, firth = false, has_traits = false;
+    const char *usage = "assoc --phenotype <TSV> --trait <COL> | --traits <A,B,...> --model <linear|logistic|cox> [--firth] [--event <COL>] [--ties efron|breslow] [--covariates A,B,...] [--predictor sum|max] [--device N] <COMBINED>";
+    std::string combined, pheno, trait, model, predictor = "sum", covs, trait_list, stats_json, event_col, ties;
+    bool has_cov = false, firth = false, has_traits = false, has_event = false;
     for (size_t i = 0; i < v.size(); ++i) {
         const std::string &a = v[i];
         auto value = [&](const char *name) -> std::string {
@@ -331,8 +331,13 @@ int assoc_main(const std::vector<std::string> &v, int device)
         else if (a == "--traits") { trait_list = value("--traits <A,B,...>"); has_traits = true; }
         else if (a == "--model") {
             model = value("--model <MODEL>");
-            if (model != "linear" && model != "logistic") cusage("invalid value '" + model + "' for '--model <MODEL>'\n  [possible values: linear, logistic]", usage);
+            if (model != "linear" && model != "logistic" && model != "cox") cusage("invalid value '" + model + "' for '--model <MODEL>'\n  [possible values: linear, logistic, cox]", usage);
         } else if (a == "--firth") firth = true;
+        else if (a == "--event") { event_col = value("--event <COL>"); has_event = true; }
+        else if (a == "--ties") {
+            ties = value("--ties <TIES>");
+            if (ties != "efron" && ties != "breslow") cusage("invalid value '" + ties + "' for '--ties <TIES>'\n  [possible values: efron, breslow]", usage);
+        }
         else if (a == "--covariates") { covs = value("--covariates <A,B,...>"); has_cov = true; }
         else if (a == "--predictor") {
             predictor = value("--predictor <PREDICTOR>");
@@ -352,6 +357,10 @@ int assoc_main(const std::vector<std::string> &v, int device)
                    "      --traits <A,B,...>       several response columns in one run (instead of --trait); a sample with a missing\n"
                    "                               value (NA, NaN, empty) is left out for that trait only\n"
                    "      --model <MODEL>          linear (OLS, t test) or logistic (0/1 trait, IRLS, Wald z test) [possible values: linear, logistic]\n"
+                   "                               or cox (Cox proportional hazards, Wald z test): --trait is the time (age at onset or at\n"
+                   "                               last visit), --event the event column\n"
+                   "      --event <COL>            with --model cox: 1 = event (onset) at the time, 0 = censored (no onset yet)\n"
+                   "      --ties <TIES>            with --model cox: tied event times [default: efron] [possible values: efron, breslow]\n"
                    "      --firth                  with --model logistic: Firth-penalized fit (finite under separation) and\n"
                    "                               penalized likelihood-ratio test\n"
                    "      --covariates <A,B,...>   0 to %d covariate columns; samples with a missing value (NA, NaN, empty) are left out\n"
@@ -362,7 +371,8 @@ int assoc_main(const std::vector<std::string> &v, int device)
                    "Output: chromosome begin end n beta se stat p status, one row per input row; status is one of ok,\n"
                    "few_samples, singular, no_convergence, separation. With --traits: chromosome begin end trait n beta se stat\n"
                    "p status, one row per input row and trait in --traits order. With --firth, stat is the penalized likelihood-ratio\n"
-                   "chi-square (1 df) of x, p comes from it, and separation is never reported\n", usage, INQ_ASSOC_MAX_COV);
+                   "chi-square (1 df) of x, p comes from it, and separation is never reported. With --model cox, stat is the Wald z\n"
+                   "of x and a sample missing its time or event is left out\n", usage, INQ_ASSOC_MAX_COV);
             return 0;
         } else if (!a.empty() && a[0] == '-' && a.size() > 1) cusage("unexpected argument '" + a + "' found", usage);
         else if (combined.empty()) combined = a;
@@ -376,6 +386,12 @@ int assoc_main(const std::vector<std::string> &v, int device)
     if (combined.empty()) missing += "\n  <COMBINED>";
     if (!missing.empty()) cusage("the following required arguments were not provided:" + missing, usage);
     if (firth && model != "logistic") cusage("the argument '--firth' requires '--model logistic'", usage);
+    const bool cox = model == "cox";
+    if (has_event && !cox) cusage("the argument '--event <COL>' requires '--model cox'", usage);
+    if (!ties.empty() && !cox) cusage("the argument '--ties <TIES>' requires '--model cox'", usage);
+    if (cox && has_traits) cusage("the argument '--traits <A,B,...>' cannot be used with '--model cox'", usage);
+    if (cox && !has_event) cusage("the following required arguments were not provided:\n  --event <COL> (with --model cox)", usage);
+    if (cox && event_col == trait) cusage("the event column '" + event_col + "' is also the time column (--trait)", usage);
     auto split_list = [](const std::string &s) {
         std::vector<std::string> out;
         size_t a = 0;
@@ -404,16 +420,17 @@ int assoc_main(const std::vector<std::string> &v, int device)
         if (cov_names[c].empty()) cusage("invalid value '" + covs + "' for '--covariates <A,B,...>': an empty column name", usage);
         for (const std::string &t : traits)
             if (cov_names[c] == t) cusage("the trait '" + t + "' is also listed as a covariate", usage);
+        if (cox && cov_names[c] == event_col) cusage("the event column '" + event_col + "' is also listed as a covariate", usage);
         for (size_t d = 0; d < c; ++d)
             if (cov_names[d] == cov_names[c]) cusage("covariate '" + cov_names[c] + "' is listed twice", usage);
     }
     const bool logistic = model == "logistic";
     const auto t_start = std::chrono::steady_clock::now();
 
-    // phenotype table: sample -> traits, covariates; rows with a missing covariate are left out, a missing trait value
-    // (NaN) leaves the sample out for that trait only
-    const size_t n_cov = cov_names.size(), n_tr = traits.size();
-    std::unordered_map<std::string, std::vector<double>> ph;          // rows with every covariate: [traits..., covariates...]
+    // phenotype table: sample -> traits, covariates; rows with a missing covariate (or, for cox, event) are left out, a
+    // missing trait value (NaN) leaves the sample out for that trait only
+    const size_t n_cov = cov_names.size(), n_tr = traits.size(), n_ev = cox ? 1 : 0;
+    std::unordered_map<std::string, std::vector<double>> ph;          // rows with every covariate: [traits..., event, covariates...]
     std::unordered_set<std::string> ph_seen;
     size_t cov_missing = 0;
     std::vector<size_t> ph_missing(n_tr, 0);                          // per trait: rows left out for it
@@ -425,7 +442,8 @@ int assoc_main(const std::vector<std::string> &v, int device)
         if (!pr.next(line)) afail(pheno + ":1: empty file (a header row is needed)");
         split_tabs(line, cols);
         const std::vector<std::string> head = cols;
-        std::vector<std::string> want_names = traits;                 // [traits..., covariates...]
+        std::vector<std::string> want_names = traits;                 // [traits..., event (cox), covariates...]
+        if (cox) want_names.push_back(event_col);
         want_names.insert(want_names.end(), cov_names.begin(), cov_names.end());
         std::vector<size_t> want;
         for (const std::string &name : want_names) {
@@ -449,6 +467,8 @@ int assoc_main(const std::vector<std::string> &v, int device)
                 if (!parse_f64(f, &vals[w])) afail(where + "column '" + head[want[w]] + "': '" + f + "' is not a number");
                 if (w < n_tr && logistic && vals[w] != 0.0 && vals[w] != 1.0)
                     afail(where + "column '" + head[want[w]] + "': '" + f + "' is not 0 or 1 (--model logistic)");
+                if (cox && w == n_tr && vals[w] != 0.0 && vals[w] != 1.0)
+                    afail(where + "column '" + head[want[w]] + "': '" + f + "' is not 0 or 1 (--event)");
             }
             if (!complete) { ++cov_missing; continue; }
             bool any = false;
@@ -475,6 +495,7 @@ int assoc_main(const std::vector<std::string> &v, int device)
     const size_t n_tab = n_val / 2;
     std::vector<uint32_t> use_idx;                       // table sample index of every sample used for some trait, in table order
     std::vector<double> y, cov;                          // y: use_idx.size() x n_tr, NaN = not used for that trait
+    std::vector<uint8_t> event;                          // cox: the event of every sample used
     size_t n_groups = 0;
     {
         std::unordered_set<std::string> names;
@@ -490,7 +511,8 @@ int assoc_main(const std::vector<std::string> &v, int device)
             if (it == ph.end()) continue;
             use_idx.push_back((uint32_t)k);
             y.insert(y.end(), it->second.begin(), it->second.begin() + n_tr);
-            cov.insert(cov.end(), it->second.begin() + n_tr, it->second.end());
+            if (cox) event.push_back((uint8_t)it->second[n_tr]);
+            cov.insert(cov.end(), it->second.begin() + n_tr + n_ev, it->second.end());
         }
         size_t ph_only = 0;
         for (const std::string &s : ph_seen) ph_only += !names.count(s);
@@ -518,6 +540,7 @@ int assoc_main(const std::vector<std::string> &v, int device)
     fputs(has_traits ? "chromosome\tbegin\tend\ttrait\tn\tbeta\tse\tstat\tp\tstatus\n" : "chromosome\tbegin\tend\tn\tbeta\tse\tstat\tp\tstatus\n", stdout);
     const char *status_names[] = {"ok", "few_samples", "singular", "no_convergence", "separation"};
     const int mdl = firth ? INQ_ASSOC_FIRTH : logistic ? INQ_ASSOC_LOGISTIC : INQ_ASSOC_LINEAR, prd = predictor == "max" ? INQ_ASSOC_MAX : INQ_ASSOC_SUM;
+    const int tie = ties == "breslow" ? INQ_COX_BRESLOW : INQ_COX_EFRON;
 
     // rows in batches of at most 256 MB of values and 64 MB of results (rows x traits x 38 bytes)
     const size_t batch_rows = std::max<size_t>(1, std::min((256u << 20) / ((size_t)ns * 2 * sizeof(double)), (64u << 20) / (n_tr * 38)));
@@ -534,7 +557,10 @@ int assoc_main(const std::vector<std::string> &v, int device)
         const size_t cells = rows * n_tr;
         beta.resize(cells); se.resize(cells); stat.resize(cells); pv.resize(cells); n_used.resize(cells); status.resize(cells);
         const auto t0 = std::chrono::steady_clock::now();
-        const int rc = has_traits
+        const int rc = cox
+            ? inq_assoc_cox(device, tie, prd, rows, ns, haps.data(), y.data(), event.data(), (uint32_t)n_cov, n_cov ? cov.data() : nullptr,
+                            beta.data(), se.data(), stat.data(), pv.data(), n_used.data(), status.data(), nullptr, nullptr)
+            : has_traits
             ? inq_assoc_traits(device, mdl, prd, rows, ns, haps.data(), (uint32_t)n_tr, y.data(), (uint32_t)n_cov, n_cov ? cov.data() : nullptr,
                                beta.data(), se.data(), stat.data(), pv.data(), n_used.data(), status.data(), nullptr, nullptr)
             : inq_assoc(device, mdl, prd, rows, ns, haps.data(), y.data(), (uint32_t)n_cov, n_cov ? cov.data() : nullptr,

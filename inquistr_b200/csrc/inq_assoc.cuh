@@ -757,4 +757,226 @@ k_assoc_linear_traits(const double *__restrict__ haps, uint64_t n_rows, uint32_t
     }
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// Cox proportional hazards (inq_assoc_cox, DESIGN.md 5e, Cox): partial likelihood of (time, event) on u = [covariates...,
+// x] (no intercept: column 0 of the shared design never enters the kept set K), Efron or Breslow ties, Newton
+// iteration with coxph.fit's control flow. The samples come in ascending time order (idx), event[s] is 0 or 1 and
+// tgroup[s] the rank of sample s's distinct time. One evaluation at beta is two sweeps over the samples:
+//   A  descending time, tiles last to first, lanes 31 to 0: the risk-set sums B (samples of R(tau) outside D(tau)) and
+//      the pending tie group's deaths A, S0 = B0 + A0 and lane j's S1_j = B1_j + A1_j, scaled by exp(-M) with M the
+//      running maximum of eta over the samples added (online softmax: no risk-set sum is 0 or inf for any finite
+//      beta). Closing the group of an event time tau (m deaths) adds, with d0_k = B0 + (1 - f_k) A0 and
+//      d1_k = B1 + (1 - f_k) A1 (f_k = k / m for Efron, 0 for Breslow; no subtraction),
+//        loglik  sum_D (eta - M) - sum_k log d0_k,
+//        U_j     sum_D u_j - B1_j c - A1_j g,    c = sum_k 1 / d0_k, g = sum_k (1 - f_k) / d0_k,
+//        I       -(a B1 B1' + b (B1 A1' + A1 B1') + e A1 A1'),   a, b, e = sum_k (1, 1 - f_k, (1 - f_k)^2) / d0_k^2,
+//      and stores (tau's group, c, g, M) to the warp's scratch.
+//   B  ascending time: Lambda = sum over event times tau <= t_s of c_tau exp(-M_tau), kept relative to the last M,
+//      gives W_s = r_s (Lambda_s, or Lambda before t_s + g for a death at t_s) >= 0, and accumulate_tile adds
+//      sum_s W_s u_s u_s' = sum_tau sum_k d2_k / d0_k to I (first evaluation: the uncentred I+_jj of the rank rule).
+// Every quantity is invariant under adding one constant to every eta and under shifting a column, so the kernel uses
+// the centred design. A grid-stride loop over blocks of loci keeps the scratch (n_samples entries per warp slot) fixed.
+constexpr int kCMaxIter = 20;                          // coxph.control(iter.max = 20)
+constexpr double kCEps = 1e-9;                         // coxph.control(eps = 1e-9)
+constexpr double kCTolerInf = 3.1622776601683795e-05;  // coxph.control(toler.inf = sqrt(eps))
+
+template <int P, bool kEfron>
+__global__ void __launch_bounds__(kAWarps * 32, 1)
+k_assoc_cox(const double *__restrict__ haps, uint64_t n_rows, uint32_t n_all, const uint32_t *__restrict__ idx,
+            uint32_t n_samples, uint32_t p, int use_max, const double *__restrict__ design,
+            const double *__restrict__ shift, const double *__restrict__ event, const uint32_t *__restrict__ tgroup,
+            double4 *scratch, AssocOut out)
+{
+    __shared__ double s_des[kATile][P + 1];
+    __shared__ double s_y[kATile];             // event of the tile's samples
+    __shared__ double s_beta[kAWarps][P];
+    const uint32_t tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const uint32_t xcol = p - 1;
+    const int n_tiles = (int)((n_samples + kATile - 1) / kATile);
+    const uint64_t n_blocks = (n_rows + kAWarps - 1) / kAWarps;
+    double4 *scr = scratch + ((uint64_t)blockIdx.x * kAWarps + warp) * n_samples;
+    const double ninf = -__longlong_as_double(0x7ff0000000000000ll);
+    for (uint64_t blk = blockIdx.x; blk < n_blocks; blk += gridDim.x) {
+        const uint64_t row = blk * kAWarps + warp;
+        const bool have = row < n_rows;
+        const SampleSubset h{reinterpret_cast<const double2 *>(haps + (have ? row : 0) * 2ull * n_all), idx};
+        const auto [n, xbar, events] = locus_prepass(h, event, n_samples, use_max, have, lane);
+
+        uint8_t status = INQ_ASSOC_OK;
+        bool done = !have;
+        if (have && (n == 0 || events == 0.0)) { status = INQ_ASSOC_FEW_SAMPLES; done = true; }
+        if (lane < P) s_beta[warp][lane] = 0.0;
+        const double my_shift = lane == xcol ? xbar : (lane < P ? shift[lane] : 0.0);
+        // b / bnew: this lane's coefficient of beta and beta_new; ll: loglik at beta
+        double b = 0.0, bnew = 0.0, ll = 0.0;
+        uint32_t kmask = 0;
+        int iter = 0;
+        bool first = true, halving = false;
+        for (;;) {
+            if (__syncthreads_and(done)) break;
+            double G[P];
+#pragma unroll
+            for (int k = 0; k < P; ++k) G[k] = 0.0;
+            double gx = 0.0, U = 0.0, diag = 0.0, lle = 0.0;
+            // A: B0, A0 and lane j's B1_j, A1_j scaled by exp(-M); the pending group's sum_D (eta - M), sum_D u_j, m
+            double B0 = 0.0, A0 = 0.0, B1 = 0.0, A1 = 0.0, Deta = 0.0, DU = 0.0, M = ninf;
+            uint32_t m = 0, cur = 0xffffffffu, ne = 0;
+            auto close = [&]() {
+                if (m) {
+                    double lsum, c, g, a, bb, e;
+                    if constexpr (kEfron) {
+                        lsum = c = g = a = bb = e = 0.0;
+                        for (uint32_t k = 0; k < m; ++k) {
+                            const double of = 1.0 - (double)k / (double)m;
+                            const double id = 1.0 / fma(of, A0, B0);
+                            lsum += log(fma(of, A0, B0));
+                            c += id; g = fma(of, id, g);
+                            const double id2 = id * id;
+                            a += id2; bb = fma(of, id2, bb); e = fma(of * of, id2, e);
+                        }
+                    } else {
+                        const double d0 = B0 + A0, id = 1.0 / d0;
+                        lsum = (double)m * log(d0); c = g = (double)m * id; a = bb = e = c * id;
+                    }
+                    lle += Deta - lsum;
+                    U += DU - fma(B1, c, A1 * g);
+#pragma unroll
+                    for (int k = 0; k < P; ++k) {
+                        const double b1k = __shfl_sync(0xffffffffu, B1, k), a1k = __shfl_sync(0xffffffffu, A1, k);
+                        const double v = fma(a * B1, b1k, fma(bb, fma(B1, a1k, A1 * b1k), e * A1 * a1k));
+                        if (k == (int)xcol) gx -= v;
+                        else G[k] -= v;
+                    }
+                    if (lane == 0) scr[ne] = make_double4((double)cur, c, g, M);
+                    ++ne;
+                }
+                B0 += A0; B1 += A1;
+                A0 = A1 = Deta = DU = 0.0;
+                m = 0;
+            };
+            for (int t = n_tiles - 1; t >= 0; --t) {
+                const uint32_t s0 = (uint32_t)t * kATile;
+                stage_tile<P>(s_des, s_y, design, event, s0, n_samples, tid);
+                if (done) continue;
+                const double xt = lane_x(h, s0 + lane, n_samples, use_max, xbar);
+                const bool valid = xt == xt;
+                const double eta = lane_eta<P>(s_beta[warp], s_des[lane], xcol, xt);
+                const uint32_t tg = valid ? tgroup[s0 + lane] : 0u;
+                // M after this lane's sample is added: the maximum over it, the higher lanes and the later tiles
+                double mloc = valid ? eta : ninf;
+#pragma unroll
+                for (int o = 1; o < 32; o <<= 1) {
+                    const double q = __shfl_down_sync(0xffffffffu, mloc, o);
+                    if (lane + o < 32) mloc = fmax(mloc, q);
+                }
+                mloc = fmax(mloc, M);
+                const double r = exp(eta - mloc);
+                unsigned msk = __ballot_sync(0xffffffffu, valid);
+                while (msk) {
+                    const int i = 31 - __clz(msk);
+                    msk &= ~(1u << i);
+                    const uint32_t tgi = __shfl_sync(0xffffffffu, tg, i);
+                    if (tgi != cur) { close(); cur = tgi; }
+                    const double mi = __shfl_sync(0xffffffffu, mloc, i);
+                    if (mi > M) {
+                        const double sc = exp(M - mi);
+                        B0 *= sc; A0 *= sc; B1 *= sc; A1 *= sc;
+                        if (m) Deta -= (double)m * (mi - M);
+                        M = mi;
+                    }
+                    const double ri = __shfl_sync(0xffffffffu, r, i), xi = __shfl_sync(0xffffffffu, xt, i);
+                    const double ei = __shfl_sync(0xffffffffu, eta, i);
+                    const double uj = lane == xcol ? xi : (lane < P ? s_des[i][lane < P ? lane : 0] : 0.0);
+                    if (s_y[i] != 0.0) { A0 += ri; A1 = fma(ri, uj, A1); DU += uj; Deta += ei - M; ++m; }
+                    else { B0 += ri; B1 = fma(ri, uj, B1); }
+                }
+            }
+            if (!done) close();
+            // B: Lt = Lambda exp(M_c) at the last event time seen, Lp the same before it, gc its g
+            double Lt = 0.0, Lp = 0.0, gc = 0.0, Mc = 0.0;
+            bool here = false;
+            int e = (int)ne - 1;
+            cur = 0xffffffffu;
+            for (uint32_t s0 = 0; s0 < n_samples; s0 += kATile) {
+                stage_tile<P>(s_des, s_y, design, event, s0, n_samples, tid);
+                if (done) continue;
+                const double xt = lane_x(h, s0 + lane, n_samples, use_max, xbar);
+                const bool valid = xt == xt;
+                const double eta = lane_eta<P>(s_beta[warp], s_des[lane], xcol, xt);
+                const uint32_t tg = valid ? tgroup[s0 + lane] : 0u;
+                double lam = 0.0, mref = 0.0;
+                unsigned msk = __ballot_sync(0xffffffffu, valid);
+                while (msk) {
+                    const int i = __ffs(msk) - 1;
+                    msk &= msk - 1;
+                    const uint32_t tgi = __shfl_sync(0xffffffffu, tg, i);
+                    if (tgi != cur) {
+                        cur = tgi;
+                        here = false;
+                        if (e >= 0) {
+                            const double4 sc = scr[e];
+                            if (sc.x == (double)tgi) {
+                                Lp = Lt > 0.0 ? Lt * exp(sc.w - Mc) : 0.0;
+                                Lt = Lp + sc.y;
+                                gc = sc.z;
+                                Mc = sc.w;
+                                here = true;
+                                --e;
+                            }
+                        }
+                    }
+                    if ((int)lane == i) { lam = here && s_y[i] != 0.0 ? Lp + gc : Lt; mref = Mc; }
+                }
+                // eta <= mref wherever lam > 0: the sample is in the risk set that gave mref
+                const double W = lam > 0.0 ? lam * exp(eta - mref) : 0.0;
+                double none = 0.0;
+                accumulate_tile<P>(G, gx, none, diag, s_des, lane, xcol, valid, xt, W, 0.0, my_shift, first,
+                                   [](double &, double, double, double, int) {});
+            }
+            if (done) continue;
+            put_x(G, gx, xcol);
+            uint32_t kept = 0;
+            double d_x = 0.0, dl[1], r1[1] = {U};
+            ldl_solve<P>(G, r1, dl, p, lane, [&](int c, double d) {
+                const bool k = first ? c > 0 && d > kAAlias * __shfl_sync(0xffffffffu, diag, c) : ((kmask >> c) & 1u) != 0;
+                if (k) { kept |= 1u << c; if (c == (int)xcol) d_x = d; }
+                return k;
+            });
+            const double delta = dl[0];            // this lane's entry of I^-1 U
+            if (first) {
+                first = false;
+                kmask = kept;
+                if (n <= (uint32_t)__popc(kept)) { status = INQ_ASSOC_FEW_SAMPLES; done = true; }
+                else if (!((kept >> xcol) & 1u)) { status = INQ_ASSOC_SINGULAR; done = true; }
+                else { ll = lle; bnew = b + delta; publish_beta<P>(s_beta[warp], lane, bnew); }
+                continue;
+            }
+            ++iter;
+            const bool conv = fabs(lle - ll) <= kCEps * fabs(lle) && !halving;
+            if (conv || iter == kCMaxIter) {
+                const double bx = __shfl_sync(0xffffffffu, bnew, xcol), dx = fabs(__shfl_sync(0xffffffffu, delta, xcol));
+                if (!conv) status = INQ_ASSOC_NO_CONVERGENCE;
+                else if (dx > kCEps && dx > kCTolerInf * fabs(bx)) status = INQ_ASSOC_SEPARATION;
+                if (lane == 0) {
+                    const double se = sqrt(1.0 / d_x), zs = bx / se;
+                    out.beta[row] = bx; out.se[row] = se; out.stat[row] = zs; out.p[row] = erfc(fabs(zs) * M_SQRT1_2);
+                }
+                done = true;
+                continue;
+            }
+            if (lle < ll) { halving = true; bnew = 0.5 * (b + bnew); }
+            else { halving = false; ll = lle; b = bnew; bnew = b + delta; }
+            publish_beta<P>(s_beta[warp], lane, bnew);
+        }
+        write_tail(out, row, have, lane, n, status, iter);
+    }
+}
+
+// The Cox launches live in a translation unit of their own (inq_cox_launch.cu): instantiated next to the other assoc
+// kernels, k_assoc_cox changed the compiled code of k_assoc_linear_traits.
+cudaError_t cox_occupancy(int P, bool efron, int *per_sm);
+void cox_launch(int P, bool efron, unsigned grid, cudaStream_t s, const double *haps, uint64_t n_rows, uint32_t n_all,
+                const uint32_t *idx, uint32_t n_samples, uint32_t p, int use_max, const double *design, const double *shift,
+                const double *event, const uint32_t *tgroup, double4 *scratch, AssocOut out);
+
 }  // namespace inqa

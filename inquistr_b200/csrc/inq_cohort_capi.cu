@@ -426,4 +426,87 @@ int inq_assoc_traits(int device, int model, int predictor, uint64_t n_rows, uint
     return INQ_OK;
 }
 
+int inq_assoc_cox(int device, int ties, int predictor, uint64_t n_rows, uint32_t n_samples, const double *haps,
+                  const double *time, const uint8_t *event, uint32_t n_cov, const double *cov, double *beta, double *se,
+                  double *stat, double *p, uint32_t *n_used, uint8_t *status, uint8_t *n_iter, float *ms_kernel)
+{
+    using namespace inqa;
+    if (ms_kernel) *ms_kernel = 0.f;
+    if (ties != INQ_COX_EFRON && ties != INQ_COX_BRESLOW) return cfail(INQ_ERR_ARG, "inq_assoc_cox: unknown ties method %d", ties);
+    if (const int rc = assoc_check_args("inq_assoc_cox", INQ_ASSOC_LINEAR, predictor, n_cov)) return rc;
+    if (n_rows == 0) return INQ_OK;
+    if (n_samples == 0) return cfail(INQ_ERR_ARG, "inq_assoc_cox: no samples");
+    if (!haps || !time || !event || (n_cov && !cov) || !beta || !se || !stat || !p || !n_used || !status) return cfail(INQ_ERR_ARG, "inq_assoc_cox: NULL array");
+    if ((n_rows + kAWarps - 1) / kAWarps > 0x7FFFFFFFull) return cfail(INQ_ERR_TOO_LARGE, "inq_assoc_cox: too many rows");
+    for (uint32_t s = 0; s < n_samples; ++s) {
+        if (!std::isfinite(time[s])) return cfail(INQ_ERR_ARG, "inq_assoc_cox: time of sample %u is not a finite number", s);
+        if (event[s] > 1) return cfail(INQ_ERR_ARG, "inq_assoc_cox: event of sample %u is not 0 or 1", s);
+    }
+    std::vector<double> ev(event, event + n_samples);
+    if (const int rc = assoc_check_values("inq_assoc_cox", INQ_ASSOC_LINEAR, n_samples, 1, ev.data(), false, n_cov, cov)) return rc;
+    // the samples in ascending time order (stable: ties keep the sample order), and the rank of each one's distinct time
+    AssocGroup gr;
+    gr.traits = {0};
+    gr.idx.resize(n_samples);
+    for (uint32_t s = 0; s < n_samples; ++s) gr.idx[s] = s;
+    std::stable_sort(gr.idx.begin(), gr.idx.end(), [&](uint32_t a, uint32_t b) { return time[a] < time[b]; });
+    std::vector<uint32_t> tg(n_samples);
+    for (uint32_t s = 1; s < n_samples; ++s) tg[s] = tg[s - 1] + (time[gr.idx[s]] != time[gr.idx[s - 1]]);
+    const uint32_t pdim = n_cov + 2;
+    const int P = assoc_width(pdim);
+    assoc_prepare(gr, INQ_ASSOC_LOGISTIC, P, n_samples, n_cov, cov, ev.data(), 1);      // y: the event, not centred
+
+    CC_TRY(cudaSetDevice(device));
+    Guard g;
+    CC_TRY(cudaStreamCreateWithFlags(&g.s, cudaStreamNonBlocking));
+    CC_TRY(cudaEventCreate(&g.e0));
+    CC_TRY(cudaEventCreate(&g.e1));
+    // grid-stride over blocks of loci: a grid of resident CTAs, its scratch (one entry per sample and warp) <= 1 GiB
+    int sms = 0, per_sm = 0;
+    CC_TRY(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, device));
+    CC_TRY(cox_occupancy(P, ties == INQ_COX_EFRON, &per_sm));
+    const uint64_t blocks = (n_rows + kAWarps - 1) / kAWarps;
+    const uint64_t slot_bytes = (uint64_t)kAWarps * n_samples * sizeof(double4);
+    const unsigned grid = (unsigned)std::max<uint64_t>(1, std::min({blocks, (uint64_t)sms * std::max(per_sm, 1), (uint64_t)((1ull << 30) / slot_bytes)}));
+    const size_t hap_bytes = (size_t)n_rows * 2 * n_samples * sizeof(double);
+    void *d_haps, *d_des, *d_shift, *d_y, *d_idx, *d_tg, *d_scr, *d_res, *d_n, *d_st, *d_it;
+    CC_TRY(g.alloc(&d_haps, hap_bytes));
+    CC_TRY(g.alloc(&d_des, gr.design.size() * sizeof(double)));
+    CC_TRY(g.alloc(&d_shift, gr.shift.size() * sizeof(double)));
+    CC_TRY(g.alloc(&d_y, n_samples * sizeof(double)));
+    CC_TRY(g.alloc(&d_idx, n_samples * sizeof(uint32_t)));
+    CC_TRY(g.alloc(&d_tg, n_samples * sizeof(uint32_t)));
+    CC_TRY(g.alloc(&d_scr, grid * slot_bytes));
+    CC_TRY(g.alloc(&d_res, (size_t)n_rows * 4 * sizeof(double)));
+    CC_TRY(g.alloc(&d_n, (size_t)n_rows * sizeof(uint32_t)));
+    CC_TRY(g.alloc(&d_st, (size_t)n_rows));
+    CC_TRY(g.alloc(&d_it, (size_t)n_rows));
+    CC_TRY(cudaMemcpyAsync(d_haps, haps, hap_bytes, cudaMemcpyHostToDevice, g.s));
+    CC_TRY(cudaMemcpyAsync(d_des, gr.design.data(), gr.design.size() * sizeof(double), cudaMemcpyHostToDevice, g.s));
+    CC_TRY(cudaMemcpyAsync(d_shift, gr.shift.data(), gr.shift.size() * sizeof(double), cudaMemcpyHostToDevice, g.s));
+    CC_TRY(cudaMemcpyAsync(d_y, gr.y.data(), n_samples * sizeof(double), cudaMemcpyHostToDevice, g.s));
+    CC_TRY(cudaMemcpyAsync(d_idx, gr.idx.data(), n_samples * sizeof(uint32_t), cudaMemcpyHostToDevice, g.s));
+    CC_TRY(cudaMemcpyAsync(d_tg, tg.data(), n_samples * sizeof(uint32_t), cudaMemcpyHostToDevice, g.s));
+    double *r = (double *)d_res;
+    const AssocOut out{r, r + n_rows, r + 2 * n_rows, r + 3 * n_rows, (uint32_t *)d_n, (uint8_t *)d_st, (uint8_t *)d_it};
+    const int mx = predictor == INQ_ASSOC_MAX;
+    const double *dh = (const double *)d_haps, *dd = (const double *)d_des, *ds = (const double *)d_shift, *dy = (const double *)d_y;
+    const uint32_t *di = (const uint32_t *)d_idx, *dt = (const uint32_t *)d_tg;
+    double4 *dscr = (double4 *)d_scr;
+    CC_TRY(cudaEventRecord(g.e0, g.s));
+    cox_launch(P, ties == INQ_COX_EFRON, grid, g.s, dh, n_rows, n_samples, di, n_samples, pdim, mx, dd, ds, dy, dt, dscr, out);
+    CC_TRY(cudaGetLastError());
+    CC_TRY(cudaEventRecord(g.e1, g.s));
+    CC_TRY(cudaMemcpyAsync(beta, r, n_rows * sizeof(double), cudaMemcpyDeviceToHost, g.s));
+    CC_TRY(cudaMemcpyAsync(se, r + n_rows, n_rows * sizeof(double), cudaMemcpyDeviceToHost, g.s));
+    CC_TRY(cudaMemcpyAsync(stat, r + 2 * n_rows, n_rows * sizeof(double), cudaMemcpyDeviceToHost, g.s));
+    CC_TRY(cudaMemcpyAsync(p, r + 3 * n_rows, n_rows * sizeof(double), cudaMemcpyDeviceToHost, g.s));
+    CC_TRY(cudaMemcpyAsync(n_used, d_n, n_rows * sizeof(uint32_t), cudaMemcpyDeviceToHost, g.s));
+    CC_TRY(cudaMemcpyAsync(status, d_st, n_rows, cudaMemcpyDeviceToHost, g.s));
+    if (n_iter) CC_TRY(cudaMemcpyAsync(n_iter, d_it, n_rows, cudaMemcpyDeviceToHost, g.s));
+    CC_TRY(cudaStreamSynchronize(g.s));
+    if (ms_kernel) cudaEventElapsedTime(ms_kernel, g.e0, g.e1);
+    return INQ_OK;
+}
+
 }  // extern "C"

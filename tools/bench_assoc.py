@@ -10,9 +10,15 @@ time separated (`--stats-json`). With --traits, `assoc_traits` lines: the kernel
 for 1, 8 and 32 linear traits and for 8 logistic and 8 Firth traits (seeded extra traits; the last quarter of them
 share one distinct NaN pattern, so they form a second sample set) against that many times the single-trait kernel
 of the same run, and the CLI wall time of `--traits` with 8 traits against 8 `--trait` runs on the same TSV.
+With --cox, only the Cox lines (and the logistic `sum` kernel on the same loci, for comparison): seeded Weibull onset
+ages rounded to whole years (so times are tied) with about half of them censored; per ties method (Efron, Breslow)
+with `sum`, the kernel time (median of --reps after a warm-up), loci/s, mean and max Newton iterations and status
+counts, parity of --parity random loci against tests/cox_reference.py's assoc_cox_matrix (run on every host core; its wall
+time and the worker count are reported), and the CLI (`--model cox --stats-json`) on the same table as TSV.
 The card's name and power limit are read in the same run.
 Temporary files go to a temporary directory."""
 import argparse
+import concurrent.futures
 import json
 import os
 import subprocess
@@ -45,6 +51,97 @@ def workload(rows, samples, n_cov, seed=2024):
     y_lin = 3 + (0.01 * cov[:, 0] if n_cov else 0.0) + rng.normal(size=samples)
     y_bin = (rng.random(samples) < 0.4).astype(float)
     return haps, cov, y_lin, y_bin
+
+
+def onsets(samples, seed=2025):
+    """Onset ages: Weibull(shape 3, scale 55) rounded to whole years; about half the samples censored."""
+    rng = np.random.default_rng(seed)
+    t = np.round(55 * rng.weibull(3.0, samples))
+    ev = (rng.random(samples) < 0.5).astype(float)
+    return t, ev
+
+
+def _cox_oracle(job):
+    from tests import cox_reference
+    haps, t, ev, cov, ties = job
+    return cox_reference.assoc_cox_matrix(haps, t, ev, cov, ties, "sum")
+
+
+def cox_bench(args, name, haps, cov, y_bin):
+    from inquistr_b200 import cohort
+    from oracle import assoc as A
+    t, ev = onsets(args.samples)
+    res = cohort.assoc(haps, y_bin, cov, "logistic", "sum")
+    lms = float(np.median([cohort.assoc(haps, y_bin, cov, "logistic", "sum")["ms_kernel"] for _ in range(args.reps)]))
+    print(json.dumps({"bench": "assoc_kernel", "card": name, "model": "logistic", "predictor": "sum", "loci": args.rows,
+                      "samples": args.samples, "covariates": args.cov, "kernel_ms_median": lms}), flush=True)
+    sel = np.sort(np.random.default_rng(7).choice(args.rows, min(args.parity, args.rows), replace=False))
+    workers = os.cpu_count() or 1
+    for ties in ("efron", "breslow"):
+        cohort.assoc_cox(haps, t, ev, cov, ties, "sum")                   # warm-up
+        ms = []
+        for _ in range(args.reps):
+            res = cohort.assoc_cox(haps, t, ev, cov, ties, "sum")
+            ms.append(res["ms_kernel"])
+        med = float(np.median(ms))
+        t0 = time.perf_counter()
+        chunks = np.array_split(sel, workers * 4)
+        with concurrent.futures.ProcessPoolExecutor(workers) as ex:
+            parts = list(ex.map(_cox_oracle, [(haps[c], t, ev, cov, ties) for c in chunks if len(c)]))
+        ref = {k: np.concatenate([q[k] for q in parts]) for k in parts[0]}
+        oracle_s = time.perf_counter() - t0
+        st = res["status"][sel]
+        ok = (ref["status"] == A.OK) & (st == A.OK) & (res["n_iter"][sel] == ref["n_iter"])
+        rb = np.abs(res["beta"][sel][ok] - ref["beta"][ok]) / (np.abs(ref["beta"][ok]) + ref["se"][ok])
+        rs = np.abs(res["se"][sel][ok] / ref["se"][ok] - 1)
+        lp = np.abs(np.log10(np.maximum(res["p"][sel][ok], 1e-300)) - np.log10(np.maximum(ref["p"][ok], 1e-300)))
+        fitted = ~np.isin(res["status"], (1, 2))
+        print(json.dumps({
+            "bench": "assoc_cox_kernel", "card": name, "ties": ties, "predictor": "sum", "loci": args.rows,
+            "samples": args.samples, "covariates": args.cov, "events": int(ev.sum()), "distinct_times": int(len(np.unique(t))),
+            "kernel_ms_median": med, "kernel_ms_all": ms, "loci_per_s": args.rows / (med * 1e-3),
+            "logistic_sum_kernel_ms": lms, "ratio_to_logistic": med / lms,
+            "mean_iterations": float(res["n_iter"][fitted].mean()), "max_iterations": int(res["n_iter"][fitted].max()),
+            "status_counts": {A.STATUS_NAMES[k]: int((res["status"] == k).sum()) for k in range(5)},
+            "parity": {"loci": int(len(sel)), "status_equal": bool(np.array_equal(st, ref["status"])),
+                       "iter_equal": bool(np.array_equal(res["n_iter"][sel], ref["n_iter"])), "compared": int(ok.sum()),
+                       "max_beta_err_rel_to_abs_beta_plus_se": float(rb.max()) if ok.any() else None,
+                       "max_se_rel_err": float(rs.max()) if ok.any() else None, "max_dlog10_p": float(lp.max()) if ok.any() else None},
+            "numpy_oracle_wall_s": oracle_s, "numpy_oracle_workers": workers}), flush=True)
+    if args.no_cli:
+        return
+    from inquistr_b200 import build
+    exe = os.path.join(os.path.dirname(build.__file__), "bin", "inquistr-b200")
+    with tempfile.TemporaryDirectory() as d:
+        samples = [f"S{i}" for i in range(args.samples)]
+        table = write_table(d, haps, samples)
+        ph = os.path.join(d, "pheno.tsv")
+        with open(ph, "w") as f:
+            f.write("sample\tonset\taffected\t" + "\t".join(f"c{c}" for c in range(args.cov)) + "\n")
+            for i, s in enumerate(samples):
+                f.write(f"{s}\t{t[i]:g}\t{int(ev[i])}\t" + "\t".join(repr(float(v)) for v in cov[i]) + "\n")
+        for ties in ("efron", "breslow"):
+            sj = os.path.join(d, "stats.json")
+            t0 = time.perf_counter()
+            r = subprocess.run([exe, "assoc", "--phenotype", ph, "--trait", "onset", "--model", "cox", "--event", "affected",
+                                "--ties", ties, "--covariates", ",".join(f"c{c}" for c in range(args.cov)), "--stats-json", sj, table],
+                               stdout=subprocess.PIPE, stderr=subprocess.PIPE)
+            wall = time.perf_counter() - t0
+            st = json.load(open(sj)) if r.returncode == 0 else {}
+            print(json.dumps({"bench": "assoc_cox_cli", "card": name, "ties": ties, "predictor": "sum", "rc": r.returncode,
+                              "table_bytes": os.path.getsize(table), "wall_s": wall, "rows_out": r.stdout.count(b"\n") - 1,
+                              **st, "stderr_tail": r.stderr.decode()[-300:]}), flush=True)
+
+
+def write_table(d, haps, samples):
+    lut = np.array([f"{v / 2:g}" for v in range(0, 6001)] + ["NaN"], dtype=object)
+    idx = np.where(np.isnan(haps), 6001, np.nan_to_num(haps * 2).astype(np.int64))
+    table = os.path.join(d, "cohort.tsv")
+    with open(table, "w") as f:
+        f.write("chromosome\tbegin\tend\t" + "\t".join(f"{s}_H1\t{s}_H2" for s in samples) + "\n")
+        for i in range(len(haps)):
+            f.write(f"chr{1 + i // 30000}\t{1000 + 100 * i}\t{1040 + 100 * i}\t" + "\t".join(lut[idx[i]]) + "\n")
+    return table
 
 
 def traits_matrix(y0, T, model, seed=99):
@@ -83,11 +180,15 @@ def main():
     ap.add_argument("--parity", type=int, default=2000)
     ap.add_argument("--no-cli", action="store_true")
     ap.add_argument("--traits", action="store_true")
+    ap.add_argument("--cox", action="store_true")
     args = ap.parse_args()
     from inquistr_b200 import cohort
     from oracle import assoc as A
     name = card()
     haps, cov, y_lin, y_bin = workload(args.rows, args.samples, args.cov)
+    if args.cox:
+        cox_bench(args, name, haps, cov, y_bin)
+        return
     p = args.cov + 2
     sel = np.sort(np.random.default_rng(7).choice(args.rows, min(args.parity, args.rows), replace=False))
     single_ms = {}
@@ -148,14 +249,8 @@ def main():
     exe = os.path.join(os.path.dirname(build.__file__), "bin", "inquistr-b200")
     with tempfile.TemporaryDirectory() as d:
         samples = [f"S{i}" for i in range(args.samples)]
-        lut = np.array([f"{v / 2:g}" for v in range(0, 6001)] + ["NaN"], dtype=object)
-        idx = np.where(np.isnan(haps), 6001, np.nan_to_num(haps * 2).astype(np.int64))
         t0 = time.perf_counter()
-        table = os.path.join(d, "cohort.tsv")
-        with open(table, "w") as f:
-            f.write("chromosome\tbegin\tend\t" + "\t".join(f"{s}_H1\t{s}_H2" for s in samples) + "\n")
-            for i in range(args.rows):
-                f.write(f"chr{1 + i // 30000}\t{1000 + 100 * i}\t{1040 + 100 * i}\t" + "\t".join(lut[idx[i]]) + "\n")
+        table = write_table(d, haps, samples)
         write_s = time.perf_counter() - t0
         ph = os.path.join(d, "pheno.tsv")
         with open(ph, "w") as f:
