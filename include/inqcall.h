@@ -89,6 +89,10 @@ typedef struct inq_stats {
     uint32_t used_graph;         /* 1: the pass was replayed from a captured CUDA graph */
     uint32_t reads_sorted;       /* 1: reads were pushed in (contig, ref_start) order */
     uint32_t n_median_chunks;
+    uint32_t n_passes;           /* passes run for this call: more than 1 when a speculatively sized buffer was too small,
+                                    the CTA-path guess was wrong or a call needed 64-bit keys */
+    uint32_t key_bytes;          /* width of the call keys of the last pass: 4, or 8 once these reads had a call outside
+                                    [-2^29, 2^29) */
 } inq_stats;
 
 /* Create / destroy a context bound to CUDA device `device`. */

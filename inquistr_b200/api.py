@@ -40,7 +40,7 @@ class Stats(C.Structure):
         ("ms_cigar", C.c_float), ("ms_fixup", C.c_float), ("ms_scan", C.c_float), ("ms_pairs", C.c_float),
         ("ms_median", C.c_float), ("ms_h2d", C.c_float), ("ms_d2h", C.c_float),
         ("n_ranges", C.c_uint32), ("used_graph", C.c_uint32), ("reads_sorted", C.c_uint32),
-        ("n_median_chunks", C.c_uint32),
+        ("n_median_chunks", C.c_uint32), ("n_passes", C.c_uint32), ("key_bytes", C.c_uint32),
     ]
 
     def as_dict(self):

@@ -134,10 +134,12 @@ struct GraphKey {
     uint32_t minlen = 0, support = 0;
     int unphased = 0, timing = 0;
     const void *o1 = nullptr, *o2 = nullptr, *ov = nullptr;
+    bool wide_keys = false;
     bool operator==(const GraphKey &o) const
     {
         return data_gen == o.data_gen && buf_gen == o.buf_gen && minlen == o.minlen && support == o.support &&
-               unphased == o.unphased && timing == o.timing && o1 == o.o1 && o2 == o.o2 && ov == o.ov;
+               unphased == o.unphased && timing == o.timing && o1 == o.o1 && o2 == o.o2 && ov == o.ov &&
+               wide_keys == o.wide_keys;
     }
 };
 
@@ -183,7 +185,8 @@ struct inq_ctx {
     DevBuf<unsigned long long> cursor;
     DevBuf<uint32_t> wt_sbase, tile_first;
     DevBuf<uint2> rd_pre, wt, wtot;
-    DevBuf<uint64_t> desc_scan, desc_wt, vals;
+    DevBuf<uint64_t> desc_scan, desc_wt;
+    DevBuf<uint32_t> vals;                // call keys, one per candidate: 32-bit words, two per key with 64-bit keys
     DevBuf<uint2> evraw;
     CUtensorMap tmap;                 // 2-D view of the unit stream: rows of 32 words (64 units), 128B swizzle
     const void *tmap_base = nullptr;
@@ -203,6 +206,7 @@ struct inq_ctx {
     uint64_t last_n_events = 0;
 
     uint64_t data_gen = 1, buf_gen = 1;
+    uint64_t wide_gen = 0;                // == data_gen: these reads have a call outside 30 bits, the pass uses 64-bit keys
     Plan plan;
     cudaGraphExec_t graph = nullptr;
     GraphKey graph_key, last_key;
@@ -256,6 +260,12 @@ int ensure(inq_ctx *ctx, DevBuf<T> &b, uint64_t need, uint64_t keep = 0, double 
     ++ctx->buf_gen;                   // a captured graph holds the old pointer
     return INQ_OK;
 }
+
+// The call keys are 32 bits wide until a pass over the current reads meets a call outside [-2^29, 2^29) (the pair kernel
+// raises kFlagWideCall); from then on, until the reads change, they are 64 bits wide.
+bool wide_keys(const inq_ctx *ctx) { return ctx->wide_gen == ctx->data_gen; }
+uint64_t vals_keys(const inq_ctx *ctx) { return wide_keys(ctx) ? ctx->vals.cap / 2 : ctx->vals.cap; }
+int ensure_vals(inq_ctx *ctx, uint64_t keys) { return ensure(ctx, ctx->vals, wide_keys(ctx) ? 2 * keys : keys); }
 
 template <typename T>
 void release(DevBuf<T> &b)
@@ -597,14 +607,21 @@ int enqueue_pass(inq_ctx *ctx, const RunParams &rp, bool capturing, uint32_t *n_
     // ---- S1: K2b once the stream is scanned ; S2: K3 per catalog chunk ; S3: result copies
     CU_TRY(ctx, cudaStreamWaitEvent(s1, ctx->dep[DEP_SCANNED], 0));
     CU_TRY(ctx, stamp(EV_PAIR0, s1));
+    const bool wide = wide_keys(ctx);
+    uint64_t *vals64 = reinterpret_cast<uint64_t *>(ctx->vals.p);
+    const uint64_t vcap = vals_keys(ctx);
     if (work) {
         const unsigned threads = kPairWarps * 32;
         ReadView rv{ctx->contig.p, ctx->rs.p, ctx->re.p, ctx->mapq.p, ctx->hp.p, ctx->flags.p, ctx->cig_off.p, R};
         LocusView lv{ctx->contig_off.p, ctx->lstart.p, ctx->lend.p, ctx->lpmax.p, ctx->n_contigs};
-        k_pair_eval<<<(unsigned)((R + threads - 1) / threads), threads, sizeof(PairSmem), s1>>>(
-            rv, 0, R, lv, rp.unphased, ctx->cand_lo.p, ctx->cand_n.p,
-            EventSource{ctx->unit_off.p, ctx->wt.p, ctx->rd_pre.p, ctx->wt_sbase.p, ctx->evraw.p, ctx->evraw.cap}, ctx->seg_off.p, ctx->cursor.p,
-            ctx->vals.p, ctx->vals.cap, ctx->d_ctr);
+        const EventSource es{ctx->unit_off.p, ctx->wt.p, ctx->rd_pre.p, ctx->wt_sbase.p, ctx->evraw.p, ctx->evraw.cap};
+        const unsigned grid = (unsigned)((R + threads - 1) / threads);
+        if (wide)
+            k_pair_eval<uint64_t><<<grid, threads, sizeof(PairSmem), s1>>>(rv, 0, R, lv, rp.unphased, ctx->cand_lo.p, ctx->cand_n.p, es,
+                                                                           ctx->seg_off.p, ctx->cursor.p, vals64, vcap, ctx->d_ctr);
+        else
+            k_pair_eval<uint32_t><<<grid, threads, sizeof(PairSmem), s1>>>(rv, 0, R, lv, rp.unphased, ctx->cand_lo.p, ctx->cand_n.p, es,
+                                                                           ctx->seg_off.p, ctx->cursor.p, ctx->vals.p, vcap, ctx->d_ctr);
         ++launches;
         CU_TRY(ctx, cudaGetLastError());
     }
@@ -619,14 +636,23 @@ int enqueue_pass(inq_ctx *ctx, const RunParams &rp, bool capturing, uint32_t *n_
             CU_TRY(ctx, cudaStreamWaitEvent(s2, ctx->dep[DEP_PAIRED], 0));
             CU_TRY(ctx, stamp(EV_MED0, s2));
         }
-        k_locus_median<<<(unsigned)(((uint64_t)(l1 - l0) * 32 + 255) / 256), 256, 0, s2>>>(l0, l1, c, rp.unphased, rp.support, ctx->seg_off.p, ctx->cursor.p,
-                                                                                     ctx->vals.p, ctx->vals.cap, ctx->t1.p, ctx->t2.p, ctx->valid.p,
-                                                                                     ctx->big_list.p, ctx->d_ctr);
+        const unsigned grid = (unsigned)(((uint64_t)(l1 - l0) * 32 + 255) / 256);
+        if (wide)
+            k_locus_median<uint64_t><<<grid, 256, 0, s2>>>(l0, l1, c, rp.unphased, rp.support, ctx->seg_off.p, ctx->cursor.p, vals64, vcap,
+                                                           ctx->t1.p, ctx->t2.p, ctx->valid.p, ctx->big_list.p, ctx->d_ctr);
+        else
+            k_locus_median<uint32_t><<<grid, 256, 0, s2>>>(l0, l1, c, rp.unphased, rp.support, ctx->seg_off.p, ctx->cursor.p, ctx->vals.p, vcap,
+                                                           ctx->t1.p, ctx->t2.p, ctx->valid.p, ctx->big_list.p, ctx->d_ctr);
         CU_TRY(ctx, cudaGetLastError());
         // the CTA path for the (rare) deep loci of the chunk, between two chunks on S2
         if (!pl.big_known || pl.need_big[c]) {
-            k_locus_median_big<<<(unsigned)ctx->sm_count * 2, kBigThreads, 0, s2>>>(l0, c, rp.unphased, rp.support, ctx->seg_off.p, ctx->cursor.p, ctx->vals.p,
-                                                                                  ctx->vals.cap, ctx->t1.p, ctx->t2.p, ctx->valid.p, ctx->big_list.p, ctx->d_ctr);
+            const unsigned big_grid = (unsigned)ctx->sm_count * 2;
+            if (wide)
+                k_locus_median_big<uint64_t><<<big_grid, kBigThreads, 0, s2>>>(l0, c, rp.unphased, rp.support, ctx->seg_off.p, ctx->cursor.p, vals64, vcap,
+                                                                               ctx->t1.p, ctx->t2.p, ctx->valid.p, ctx->big_list.p, ctx->d_ctr);
+            else
+                k_locus_median_big<uint32_t><<<big_grid, kBigThreads, 0, s2>>>(l0, c, rp.unphased, rp.support, ctx->seg_off.p, ctx->cursor.p, ctx->vals.p,
+                                                                               vcap, ctx->t1.p, ctx->t2.p, ctx->valid.p, ctx->big_list.p, ctx->d_ctr);
             ++launches;
         }
         ++launches;
@@ -717,12 +743,15 @@ int inq_ctx_create(int device, inq_ctx **out)
         return INQ_ERR_CUDA;
     }
     ctx->sm_count = prop.multiProcessorCount;
-    // the HBM-bound scan gets the SMs first; pair / median CTAs fill what its one CTA per SM leaves free
+    // the HBM-bound scan gets the SMs first; pair / median CTAs fill what its one CTA per SM leaves free. The result
+    // pushes on S3 get them first too: they are PCIe-bound, and a push that waits behind the next median chunk's CTAs
+    // leaves the link idle, so the last pushes would end the pass well after the last median
     int prio_lo = 0, prio_hi = 0;
     if ((e = cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi)) != cudaSuccess) return bail("cudaDeviceGetStreamPriorityRange", e);
     cudaStream_t *streams[4] = {&ctx->stream, &ctx->stream_join, &ctx->stream_med, &ctx->stream_copy};
     for (int i = 0; i < 4; ++i)
-        if ((e = cudaStreamCreateWithPriority(streams[i], cudaStreamNonBlocking, i == 0 ? prio_hi : prio_lo)) != cudaSuccess) return bail("cudaStreamCreate", e);
+        if ((e = cudaStreamCreateWithPriority(streams[i], cudaStreamNonBlocking, (i == 0 || i == 3) ? prio_hi : prio_lo)) != cudaSuccess)
+            return bail("cudaStreamCreate", e);
     for (int i = 0; i < EV_COUNT; ++i)
         if ((e = cudaEventCreate(&ctx->ev[i])) != cudaSuccess) return bail("cudaEventCreate", e);
     for (int i = 0; i < DEP_COUNT; ++i)
@@ -739,7 +768,8 @@ int inq_ctx_create(int device, inq_ctx **out)
     if ((e = cudaFuncSetAttribute(k_cigar_scan<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kScanSmemBytes)) != cudaSuccess ||
         (e = cudaFuncSetAttribute(k_cigar_scan<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kScanSmemBytes)) != cudaSuccess)
         return bail("cudaFuncSetAttribute(k_cigar_scan)", e);
-    if ((e = cudaFuncSetAttribute(k_pair_eval, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(PairSmem))) != cudaSuccess)
+    if ((e = cudaFuncSetAttribute(k_pair_eval<uint32_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(PairSmem))) != cudaSuccess ||
+        (e = cudaFuncSetAttribute(k_pair_eval<uint64_t>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(PairSmem))) != cudaSuccess)
         return bail("cudaFuncSetAttribute(k_pair_eval)", e);
     int occ = 0;
     if ((e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, k_cigar_scan<false>, kCtaThreads, kScanSmemBytes)) != cudaSuccess)
@@ -1187,13 +1217,14 @@ int inq_genotype(inq_ctx *ctx, uint32_t minlen, uint32_t support, int unphased, 
         TRY(launch_join(ctx, unphased, s));
         CU_TRY(ctx, cudaMemcpyAsync(ctx->h_total, ctx->seg_off.p + L, sizeof(uint32_t), cudaMemcpyDeviceToHost, s));
         CU_TRY(ctx, cudaStreamSynchronize(s));
-        TRY(ensure(ctx, ctx->vals, (uint64_t)*ctx->h_total + 1));
+        TRY(ensure_vals(ctx, (uint64_t)*ctx->h_total + 1));
     }
 
-    uint32_t launches = 0;
+    uint32_t launches = 0, passes = 0;
     bool used_graph = false, done = false;
     for (int attempt = 0; attempt < 4 && !done; ++attempt) {
-        const GraphKey key{ctx->data_gen, ctx->buf_gen, minlen, support, unphased, rp.timing, rp.o1, rp.o2, rp.ov};
+        const GraphKey key{ctx->data_gen, ctx->buf_gen, minlen, support, unphased, rp.timing, rp.o1, rp.o2, rp.ov, wide_keys(ctx)};
+        ++passes;
         used_graph = false;
         if (ctx->graph && !(ctx->graph_key == key)) drop_graph(ctx);
         if (ctx->opt_graph && !ctx->graph && ctx->have_last_key && ctx->last_key == key) {
@@ -1204,7 +1235,9 @@ int inq_genotype(inq_ctx *ctx, uint32_t minlen, uint32_t support, int unphased, 
             cudaError_t e = cudaStreamEndCapture(s, &g);
             if (rc != INQ_OK) { if (g) cudaGraphDestroy(g); return rc; }
             if (e != cudaSuccess) return fail(ctx, INQ_ERR_CUDA, "cudaStreamEndCapture: %s", cudaGetErrorString(e));
-            e = cudaGraphInstantiate(&ctx->graph, g, 0);
+            // the nodes keep the priorities of the streams they were captured from (without the flag, every node runs at
+            // the priority of S0, which the graph is launched into)
+            e = cudaGraphInstantiateWithFlags(&ctx->graph, g, cudaGraphInstantiateFlagUseNodePriority);
             cudaGraphDestroy(g);
             if (e != cudaSuccess) { ctx->graph = nullptr; return fail(ctx, INQ_ERR_CUDA, "cudaGraphInstantiate: %s", cudaGetErrorString(e)); }
             ctx->graph_key = key;
@@ -1237,9 +1270,14 @@ int inq_genotype(inq_ctx *ctx, uint32_t minlen, uint32_t support, int unphased, 
             TRY(ensure(ctx, ctx->evraw, need_raw));
             retry = true;
         }
-        if (work && (uint64_t)*ctx->h_total + 1 > ctx->vals.cap) {
+        if (f & kFlagWideCall) {
+            // a call outside 30 bits: the medians of this pass are incomplete; these reads take 64-bit keys from now on
+            ctx->wide_gen = ctx->data_gen;
+            retry = true;
+        }
+        if (work && (uint64_t)*ctx->h_total + 1 > vals_keys(ctx)) {
             release(ctx->vals);
-            TRY(ensure(ctx, ctx->vals, (uint64_t)*ctx->h_total + 1));
+            TRY(ensure_vals(ctx, (uint64_t)*ctx->h_total + 1));
             retry = true;
         }
         if (retry) { ctx->have_last_key = false; continue; }       // buffers moved: the next attempt launches directly
@@ -1293,6 +1331,8 @@ int inq_genotype(inq_ctx *ctx, uint32_t minlen, uint32_t support, int unphased, 
         stats->used_graph = used_graph ? 1u : 0u;
         stats->reads_sorted = ctx->plan.reads_sorted ? 1u : 0u;
         stats->n_median_chunks = (uint32_t)ctx->plan.n_chunks;
+        stats->n_passes = passes;
+        stats->key_bytes = wide_keys(ctx) ? 8u : 4u;
         if (rp.timing) {
             auto el = [&](int a, int b) { float ms = 0.f; if (cudaEventElapsedTime(&ms, ctx->ev[a], ctx->ev[b]) != cudaSuccess) { cudaGetLastError(); ms = 0.f; } return ms; };
             stats->ms_total = el(EV_START, EV_END);

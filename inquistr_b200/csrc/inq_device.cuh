@@ -31,6 +31,7 @@ constexpr uint32_t kFlagEventOverflow = 1u << 2;
 constexpr uint32_t kFlagValsOverflow = 1u << 3;
 constexpr uint32_t kFlagCountOverflow = 1u << 4;
 constexpr uint32_t kFlagBadSa = 1u << 5;
+constexpr uint32_t kFlagWideCall = 1u << 6;   // a pass with 32-bit call keys met a call outside [-2^29, 2^29)
 
 constexpr uint64_t kDescAggregate = 1ull << 62;
 constexpr uint64_t kDescPrefix = 2ull << 62;
@@ -83,6 +84,12 @@ __device__ __forceinline__ uint32_t lanemask_lt()
 {
     uint32_t m;
     asm("mov.u32 %0, %%lanemask_lt;" : "=r"(m));
+    return m;
+}
+__device__ __forceinline__ uint32_t lanemask_le()
+{
+    uint32_t m;
+    asm("mov.u32 %0, %%lanemask_le;" : "=r"(m));
     return m;
 }
 
@@ -999,20 +1006,42 @@ __device__ __forceinline__ uint2 event_at(const EventSource &es, uint32_t k, uin
     return make_uint2(w.x + raw.x, raw.y);
 }
 
+// Call keys: 64-bit keys are ((call + 2^61) << 1) | clip with the H2 marker in bit 63. While every call of the reads
+// fits 30 bits the pass runs on 32-bit keys of the same layout (bias 2^29, H2 marker in bit 31): half the bytes from
+// k_pair_eval to k_locus_median, and half the shuffles and compares of the sorting networks. A call outside that range
+// raises kFlagWideCall and the host repeats the pass with 64-bit keys.
+template <typename T> struct KeyTraits;
+template <> struct KeyTraits<uint64_t> {
+    static constexpr uint64_t hap = kKeyHapBit, inf = kKeyInf;
+    static __device__ __forceinline__ int64_t call(uint64_t k) { return (int64_t)((k & ~hap) >> 1) - kCallBias; }
+};
+template <> struct KeyTraits<uint32_t> {
+    static constexpr uint32_t hap = 1u << 31, inf = 0xFFFFFFFFu;
+    static constexpr int32_t bias = 1 << 29;
+    static __device__ __forceinline__ int64_t call(uint32_t k) { return (int64_t)((int32_t)((k & ~hap) >> 1) - bias); }
+};
+
+// one read with candidates, as the candidate loop of k_pair_eval reads it: two 16-byte shared-memory loads
+struct PairRead {
+    uint4 a;                                // rs, re, lo - (flat index of its first candidate), abase
+    uint4 b;                                // eb (first staged event), number of events, hf | lane << 16, BAM words
+};
+
 struct PairSmem {                           // per CTA of kPairWarps warps (dynamic shared memory)
     uint2 ev[kPairWarps][kPairEvPool];
-    uint32_t off[kPairWarps][32];
+    PairRead rd[kPairWarps][32];            // the warp's reads with candidates, compacted in lane order
     uint32_t ty[kPairWarps][kPairTileCache + 1], tx[kPairWarps][kPairTileCache], tsb[kPairWarps][kPairTileCache];
-    int32_t ls[kPairWarps][kPairLociCache], le[kPairWarps][kPairLociCache];
+    int2 lse[kPairWarps][kPairLociCache];   // start, end
     uint32_t seg[kPairWarps][kPairLociCache + 1];
-    uint32_t joined[kPairWarps];
 };
 
 // reads [r_begin, r_end) (the pass launches it once over [0, R); bounding r by rv.R instead doubles ptxas' spills)
+// KeyT: uint32_t (calls outside [-2^29, 2^29) raise kFlagWideCall and are not stored) or uint64_t
+template <typename KeyT>
 __global__ void __launch_bounds__(kPairWarps * 32, kPairMinCtas)
 k_pair_eval(ReadView rv, uint64_t r_begin, uint64_t r_end, LocusView lv, int unphased, const uint32_t *__restrict__ cand_lo,
             const uint32_t *__restrict__ cand_n, EventSource es, const uint32_t *__restrict__ seg_off,
-            unsigned long long *__restrict__ cursor, uint64_t *__restrict__ vals, uint64_t vals_cap,
+            unsigned long long *__restrict__ cursor, KeyT *__restrict__ vals, uint64_t vals_cap,
             DevCounters *__restrict__ ctr)
 {
     // A warp owns 32 consecutive reads; their candidates are flattened and dealt to the lanes
@@ -1025,8 +1054,8 @@ k_pair_eval(ReadView rv, uint64_t r_begin, uint64_t r_end, LocusView lv, int unp
     // round trip overlaps the next candidate.
     extern __shared__ __align__(16) unsigned char pair_smem_raw[];
     PairSmem &sm = *reinterpret_cast<PairSmem *>(pair_smem_raw);
-    auto &s_off = sm.off; auto &s_joined = sm.joined; auto &s_ev = sm.ev;
-    auto &s_ty = sm.ty; auto &s_tx = sm.tx; auto &s_tsb = sm.tsb; auto &s_ls = sm.ls; auto &s_le = sm.le; auto &s_seg = sm.seg;
+    auto &s_ev = sm.ev;
+    auto &s_ty = sm.ty; auto &s_tx = sm.tx; auto &s_tsb = sm.tsb; auto &s_lse = sm.lse; auto &s_seg = sm.seg;
     const uint32_t lane = lane_id(), wid = threadIdx.x >> 5;
     const uint64_t r = r_begin + blockIdx.x * (uint64_t)blockDim.x + threadIdx.x;
     uint32_t n = 0, lo = 0, e0 = 0xFFFFFFFFu, e1 = 0xFFFFFFFFu, hf = 0, words = 0, t_lo = 0, t_hi = 0, abase = 0;
@@ -1103,11 +1132,16 @@ k_pair_eval(ReadView rv, uint64_t r_begin, uint64_t r_end, LocusView lv, int unp
         }
     }
     if (n && e1 - ev_lo > (uint32_t)kPairEvPool) hf |= 1u << 9;      // not (entirely) staged: searched in global memory
-    const uint32_t eb = e0 - ev_lo;                                   // first staged event of the read
     const uint32_t incl = warp_incl_scan(n);
     const uint32_t total = __shfl_sync(0xffffffffu, incl, 31);
-    s_off[wid][lane] = incl - n;
-    if (lane == 0) s_joined[wid] = 0u;
+    const uint32_t off = incl - n;                                    // flat index of the read's first candidate
+    // the record of a read with candidates goes to its rank among them: the loop below finds the read of a candidate by
+    // counting the reads that start in front of it (reads without candidates start nowhere)
+    const uint32_t with_cands = __ballot_sync(0xffffffffu, n != 0);
+    if (n) {
+        sm.rd[wid][__popc(with_cands & lanemask_lt())] =
+            PairRead{make_uint4((uint32_t)rs, (uint32_t)re, lo - off, abase), make_uint4(e0 - ev_lo, e1 - e0, hf | (lane << 16), words)};
+    }
     // slice of the catalog this warp touches
     const uint32_t lo_min = __reduce_min_sync(0xffffffffu, n ? lo : 0xFFFFFFFFu);
     const uint32_t hi_max = __reduce_max_sync(0xffffffffu, n ? lo + n : 0u);
@@ -1115,20 +1149,20 @@ k_pair_eval(ReadView rv, uint64_t r_begin, uint64_t r_end, LocusView lv, int unp
     if (cached) {
         const uint32_t span = hi_max - lo_min;
         for (uint32_t i = lane; i < span; i += 32) {
-            s_ls[wid][i] = __ldg(lv.start + lo_min + i);
-            s_le[wid][i] = __ldg(lv.end + lo_min + i);
+            s_lse[wid][i] = make_int2(__ldg(lv.start + lo_min + i), __ldg(lv.end + lo_min + i));
         }
         for (uint32_t i = lane; i <= span; i += 32) s_seg[wid][i] = __ldg(seg_off + lo_min + i);
     }
     __syncwarp();
 
     uint32_t npass = 0;                 // pairs that land in a bucket
+    uint32_t joined_bits = 0;           // lanes of the warp whose reads had a pair land here
     uint64_t visits = 0;                // CIGAR words the reference walks: every passing pair, incl. HP 0
     bool bad_hp = false, bad_sa = false;
     // deferred store of the previous candidate
-    bool pend = false;
+    bool pend = false, wide = false;
     unsigned long long pend_old = 0;
-    uint64_t pend_key = 0;
+    KeyT pend_key = 0;
     uint32_t pend_seg = 0, pend_cap = 0;
     bool pend_back = false;
     auto flush_pending = [&]() {
@@ -1140,31 +1174,27 @@ k_pair_eval(ReadView rv, uint64_t r_begin, uint64_t r_end, LocusView lv, int unp
         pend = false;
     };
 
+    uint32_t owner = 0xFFFFFFFFu;       // rank of the read that owns flat index base - 1
     for (uint32_t base = 0; base < total; base += 32) {
         const uint32_t k = base + lane;
         const bool active = k < total;
-        // owning read: the last j with s_off[j] <= k
-        uint32_t j = 0;
-#pragma unroll
-        for (uint32_t step = 16; step >= 1; step >>= 1)
-            if (active && s_off[wid][j + step] <= k) j += step;
-        const uint32_t idx = k - s_off[wid][j];
-        const int32_t rs_j = __shfl_sync(0xffffffffu, rs, j), re_j = __shfl_sync(0xffffffffu, re, j);
-        const uint32_t hf_j = __shfl_sync(0xffffffffu, hf, j), lo_j = __shfl_sync(0xffffffffu, lo, j);
-        const uint32_t e0_j = __shfl_sync(0xffffffffu, e0, j), e1_j = __shfl_sync(0xffffffffu, e1, j);
-        const uint32_t eb_j = __shfl_sync(0xffffffffu, eb, j);
-        const uint32_t tlo_j = __shfl_sync(0xffffffffu, t_lo, j), thi_j = __shfl_sync(0xffffffffu, t_hi, j);
-        const uint32_t abase_j = __shfl_sync(0xffffffffu, abase, j);
-        const uint32_t words_j = __shfl_sync(0xffffffffu, words, j);
+        // owning read: the reads starting in [base, base + 32) as a bit mask over the positions, counted up to k
+        const uint32_t starts = __reduce_or_sync(0xffffffffu, (n && off - base < 32u) ? 1u << (off - base) : 0u);
+        const PairRead &pr = sm.rd[wid][owner + __popc(starts & lanemask_le())];
+        owner += __popc(starts);
+        const uint4 ra = pr.a, rb = pr.b;
+        const int32_t rs_j = (int32_t)ra.x, re_j = (int32_t)ra.y;
+        const uint32_t abase_j = ra.w, eb_j = rb.x, ne_j = rb.y, hf_j = rb.z & 0xFFFFu, j = rb.z >> 16;
         bool emit = false;
         uint32_t l = 0, h = 0, seg = 0, cap = 0;
         int32_t ls = 0, le = 0;
         if (active) {
-            l = lo_j + idx;
+            l = k + ra.z;
             h = hf_j & 0xFFu;
             if (cached) {
-                ls = s_ls[wid][l - lo_min];
-                le = s_le[wid][l - lo_min];
+                const int2 se = s_lse[wid][l - lo_min];
+                ls = se.x;
+                le = se.y;
                 seg = s_seg[wid][l - lo_min];
                 cap = s_seg[wid][l - lo_min + 1] - seg;
             } else {
@@ -1174,7 +1204,7 @@ k_pair_eval(ReadView rv, uint64_t r_begin, uint64_t r_end, LocusView lv, int unp
                 cap = __ldg(seg_off + l + 1) - seg;
             }
             if (pair_passes(unphased != 0, rs_j, re_j, ls, le)) {
-                visits += words_j;                          // call.rs:357 runs before the bucket lookup
+                visits += rb.w;                             // call.rs:357 runs before the bucket lookup
                 emit = true;
                 if (hf_j & (1u << 10)) {                    // call.rs:394 -> 431: the walk panics inside is_accidental_2d
                     bad_sa = true;
@@ -1193,11 +1223,11 @@ k_pair_eval(ReadView rv, uint64_t r_begin, uint64_t r_end, LocusView lv, int unp
             }
         }
         unsigned long long old = 0;
-        uint64_t key = 0;
+        KeyT key = 0;
         const bool back = !unphased && h == 2u;
         if (emit) {
             ++npass;
-            atomicOr(&s_joined[wid], 1u << j);
+            joined_bits |= 1u << j;
             // slot first: the atomic's round trip overlaps the rest of this iteration and the next one
             old = atomicAdd(cursor + l, back ? (1ull << 32) : 1ull);
             const uint32_t start_ext = (uint32_t)ls - 10u, end_ext = (uint32_t)le + 10u;
@@ -1206,7 +1236,7 @@ k_pair_eval(ReadView rv, uint64_t r_begin, uint64_t r_end, LocusView lv, int unp
             uint32_t clip = 0;
             if (!(hf_j & (1u << 9))) {
                 // the read's events sit in shared memory, sorted by anchor: binary search, then a short scan
-                const uint32_t ne = e1_j - e0_j;
+                const uint32_t ne = ne_j;
                 const uint2 *sev = &s_ev[wid][eb_j];
                 uint32_t a = 0, b = ne;
                 while (a < b) {
@@ -1224,14 +1254,16 @@ k_pair_eval(ReadView rv, uint64_t r_begin, uint64_t r_end, LocusView lv, int unp
                 }
             } else {
                 // long event list, read from the warp-tile storage: anchors increase along the read, so a
-                // binary search finds the first event with pos1 > start_ext; then a short scan
+                // binary search finds the first event with pos1 > start_ext; then a short scan. The tile search runs over
+                // the warp's tiles: they hold the read's, and the tile of an event is the same over any range that does
+                const uint32_t e0_j = ev_lo + eb_j, e1_j = e0_j + ne_j;
                 uint32_t a = e0_j, b = e1_j;
                 while (a < b) {
                     const uint32_t m = (a + b) >> 1;
-                    if (abase_j + event_at(es, m, tlo_j, thi_j).x > start_ext) b = m; else a = m + 1;
+                    if (abase_j + event_at(es, m, tile_lo, tile_hi).x > start_ext) b = m; else a = m + 1;
                 }
                 for (uint32_t e = a; e < e1_j; ++e) {
-                    const uint2 ev = event_at(es, e, tlo_j, thi_j);
+                    const uint2 ev = event_at(es, e, tile_lo, tile_hi);
                     if (!(abase_j + ev.x < end_ext)) break;
                     const int32_t v = (int32_t)ev.y;
                     const uint32_t is_s = (uint32_t)v & 1u;
@@ -1240,7 +1272,14 @@ k_pair_eval(ReadView rv, uint64_t r_begin, uint64_t r_end, LocusView lv, int unp
                     clip |= is_s;
                 }
             }
-            key = ((uint64_t)(call + kCallBias) << 1) | clip;
+            if constexpr (sizeof(KeyT) == 8) {
+                key = ((uint64_t)(call + kCallBias) << 1) | clip;
+            } else if (call >= -(int64_t)KeyTraits<uint32_t>::bias && call < (int64_t)KeyTraits<uint32_t>::bias) {
+                key = ((uint32_t)(call + KeyTraits<uint32_t>::bias) << 1) | clip;
+            } else {
+                wide = true;                                // the slot stays taken and unwritten: the pass is repeated
+                emit = false;
+            }
         }
         flush_pending();                                    // store of the previous candidate
         if (emit) {
@@ -1255,12 +1294,13 @@ k_pair_eval(ReadView rv, uint64_t r_begin, uint64_t r_end, LocusView lv, int unp
     flush_pending();
     __syncwarp();
     // statistics (one atomic per warp per counter)
-    const bool joined = ((s_joined[wid] >> lane) & 1u) != 0u;
+    const bool joined = ((__reduce_or_sync(0xffffffffu, joined_bits) >> lane) & 1u) != 0u;
     const uint32_t pass_w = __reduce_add_sync(0xffffffffu, npass);
     const uint32_t join_w = __popc(__ballot_sync(0xffffffffu, joined));
     const uint64_t words_w = warp_sum(joined ? (uint64_t)words : 0ull);
     const uint64_t visits_w = warp_sum(visits);
     const uint32_t bad_w = __any_sync(0xffffffffu, bad_hp), bad_sa_w = __any_sync(0xffffffffu, bad_sa);
+    const uint32_t wide_w = __any_sync(0xffffffffu, wide);
     if (lane == 0) {
         // one of kStatSlots copies per warp: no block barrier, and no single hot address in L2
         unsigned long long *slot = ctr->stat[(blockIdx.x * (uint32_t)kPairWarps + wid) % kStatSlots];
@@ -1270,6 +1310,7 @@ k_pair_eval(ReadView rv, uint64_t r_begin, uint64_t r_end, LocusView lv, int unp
         if (visits_w) atomicAdd(slot + ST_OP_VISITS, (unsigned long long)visits_w);
         if (bad_w) atomicOr(&ctr->flags, kFlagBadHp);
         if (bad_sa_w) atomicOr(&ctr->flags, kFlagBadSa);
+        if (wide_w) atomicOr(&ctr->flags, kFlagWideCall);
     }
 }
 
@@ -1278,20 +1319,6 @@ k_pair_eval(ReadView rv, uint64_t r_begin, uint64_t r_end, LocusView lv, int unp
 // Keys are 63-bit ((call + bias) << 1 | clip): ascending key order == (value, Span before Clip).
 // Phased loci set bit 63 on H2 keys so one sort orders [H1 | H2]; unphased loci split the sorted
 // run at n/2 (call.rs:314).
-
-// Key traits: 64-bit keys are ((call + 2^61) << 1) | clip with the H2 marker in bit 63; when every
-// call of a locus fits 30 bits the same layout is used in 32 bits (bias 2^29, H2 marker bit 31),
-// which halves the shuffles and compares of the sorting network.
-template <typename T> struct KeyTraits;
-template <> struct KeyTraits<uint64_t> {
-    static constexpr uint64_t hap = kKeyHapBit, inf = kKeyInf;
-    static __device__ __forceinline__ int64_t call(uint64_t k) { return (int64_t)((k & ~hap) >> 1) - kCallBias; }
-};
-template <> struct KeyTraits<uint32_t> {
-    static constexpr uint32_t hap = 1u << 31, inf = 0xFFFFFFFFu;
-    static constexpr int32_t bias = 1 << 29;
-    static __device__ __forceinline__ int64_t call(uint32_t k) { return (int64_t)((int32_t)((k & ~hap) >> 1) - bias); }
-};
 
 // all-ascending bitonic network over K striped registers per lane (element i = k*32 + lane)
 // N < K * 32 sorts every aligned run of N elements on its own
@@ -1423,14 +1450,40 @@ __device__ __forceinline__ void median_halves32(uint32_t key, uint32_t nf, uint3
 
 // kSplit > 0 (phased only): H1 lives at positions [0, nf) and H2 at [kSplit, kSplit + nb) and the two
 // runs of kSplit elements are sorted independently (a shorter network than one sort over both).
-template <int K, int kSplit = 0>
-__device__ __forceinline__ void warp_locus(const uint64_t *__restrict__ vals, uint32_t seg, uint32_t cap, uint32_t nf,
+// 32-bit keys are sorted as they are; 64-bit keys are narrowed to 32 bits where every call of the locus fits.
+template <int K, int kSplit, typename KeyT>
+__device__ __forceinline__ void warp_locus(const KeyT *__restrict__ vals, uint32_t seg, uint32_t cap, uint32_t nf,
                                            uint32_t nb, uint32_t n1, bool phased, uint32_t support, int64_t *t1,
                                            int64_t *t2, uint32_t *valid, bool *panicked)
 {
     const uint32_t ntot = nf + nb;
     constexpr int kSortN = kSplit ? kSplit : K * 32;
     const uint32_t a2 = kSplit ? (uint32_t)kSplit : n1;              // first position of the second part
+    if constexpr (sizeof(KeyT) == 4) {
+        uint32_t k32[K];
+#pragma unroll
+        for (int k = 0; k < K; ++k) {
+            const uint32_t i = k * 32 + lane_id();
+            uint32_t v = KeyTraits<uint32_t>::inf;
+            if constexpr (kSplit > 0) {
+                if (i < nf) v = vals[seg + i];
+                else if (i >= (uint32_t)kSplit && i - (uint32_t)kSplit < nb) v = vals[seg + cap - nb + (i - (uint32_t)kSplit)];
+            } else {
+                if (i < nf) v = vals[seg + i];
+                else if (i < ntot) v = vals[seg + cap - nb + (i - nf)] | (phased ? KeyTraits<uint32_t>::hap : 0u);
+            }
+            k32[k] = v;
+        }
+        warp_sort<K, uint32_t, kSortN>(k32);
+        if constexpr (K == 1 && kSplit == 16) {
+            median_halves32(k32[0], nf, nb, support, t1, t2, valid, panicked);
+        } else {
+            const bool v1 = warp_median_part<K, uint32_t>(k32, 0, n1, support, t1, panicked);
+            const bool v2 = warp_median_part<K, uint32_t>(k32, a2, ntot - n1, support, t2, panicked);
+            *valid = (v1 ? 1u : 0u) | (v2 ? 2u : 0u);
+        }
+        return;
+    }
     uint64_t key[K];
     bool have_k[K];
     bool small = true;                      // every call fits the 32-bit key layout
@@ -1441,12 +1494,12 @@ __device__ __forceinline__ void warp_locus(const uint64_t *__restrict__ vals, ui
         bool have;
         if constexpr (kSplit > 0) {
             have = (i < nf) || (i >= (uint32_t)kSplit && i - (uint32_t)kSplit < nb);
-            if (i < nf) v = vals[seg + i];
-            else if (have) v = vals[seg + cap - nb + (i - (uint32_t)kSplit)];
+            if (i < nf) v = (uint64_t)vals[seg + i];
+            else if (have) v = (uint64_t)vals[seg + cap - nb + (i - (uint32_t)kSplit)];
         } else {
             have = i < ntot;
-            if (i < nf) v = vals[seg + i];
-            else if (have) v = vals[seg + cap - nb + (i - nf)] | (phased ? kKeyHapBit : 0ull);
+            if (i < nf) v = (uint64_t)vals[seg + i];
+            else if (have) v = (uint64_t)vals[seg + cap - nb + (i - nf)] | (phased ? kKeyHapBit : 0ull);
         }
         if (have) {
             const int64_t c = key_call(v);
@@ -1498,17 +1551,19 @@ __device__ __forceinline__ LocusSeg locus_seg(uint32_t seg, uint32_t cap, unsign
     return h;
 }
 // the common phased case (both haplotypes <= 16 calls): lane i < 16 holds H1's call i, lane 16 + i H2's call i
-__device__ __forceinline__ uint64_t fast16_load(const uint64_t *__restrict__ vals, const LocusSeg &h)
+template <typename KeyT>
+__device__ __forceinline__ KeyT fast16_load(const KeyT *__restrict__ vals, const LocusSeg &h)
 {
     const uint32_t i = lane_id();
     if (i < h.nf) return vals[h.seg + i];
     if (i >= 16u && i - 16u < h.nb) return vals[h.seg + h.cap - h.nb + (i - 16u)];
-    return kKeyInf;
+    return KeyTraits<KeyT>::inf;
 }
 
-// one locus: everything after the header. `pre`: the keys of the fast path, already loaded (kKeyInf lanes are empty).
-__device__ __forceinline__ void median_one(uint32_t l, uint32_t l0, int chunk, int unphased, uint32_t support, const LocusSeg &h, bool fast, uint64_t pre,
-                                           const uint64_t *__restrict__ vals, int64_t *__restrict__ twice_h1, int64_t *__restrict__ twice_h2,
+// one locus: everything after the header. `pre`: the keys of the fast path, already loaded (inf lanes are empty).
+template <typename KeyT>
+__device__ __forceinline__ void median_one(uint32_t l, uint32_t l0, int chunk, int unphased, uint32_t support, const LocusSeg &h, bool fast, KeyT pre,
+                                           const KeyT *__restrict__ vals, int64_t *__restrict__ twice_h1, int64_t *__restrict__ twice_h2,
                                            uint8_t *__restrict__ valid, uint32_t *__restrict__ big_list, DevCounters *__restrict__ ctr)
 {
     if (!h.ok) {                                        // speculatively sized call buffer too small: the run is repeated
@@ -1522,7 +1577,14 @@ __device__ __forceinline__ void median_one(uint32_t l, uint32_t l0, int chunk, i
     uint32_t vm = 0;
     bool panicked = false;
     bool done = false;
-    if (fast) {
+    if constexpr (sizeof(KeyT) == 4) {
+        if (fast) {                                     // keys are here already
+            uint32_t k32[1] = {pre};
+            warp_sort<1, uint32_t, 16>(k32);
+            median_halves32(k32[0], nf, nb, support, &t1, &t2, &vm, &panicked);
+            done = true;
+        }
+    } else if (fast) {
         // keys are here already: 32-bit layout when every call fits 30 bits (practically always)
         const bool have = pre != kKeyInf;
         const int64_t c = key_call(pre);
@@ -1536,11 +1598,11 @@ __device__ __forceinline__ void median_one(uint32_t l, uint32_t l0, int chunk, i
         }
     }
     if (!done) {
-        if (!unphased && nf <= 16 && nb <= 16) warp_locus<1, 16>(vals, seg, cap, nf, nb, n1, true, support, &t1, &t2, &vm, &panicked);
-        else if (ntot <= 32) warp_locus<1>(vals, seg, cap, nf, nb, n1, !unphased, support, &t1, &t2, &vm, &panicked);
-        else if (!unphased && nf <= 32 && nb <= 32) warp_locus<2, 32>(vals, seg, cap, nf, nb, n1, true, support, &t1, &t2, &vm, &panicked);
-        else if (ntot <= 64) warp_locus<2>(vals, seg, cap, nf, nb, n1, !unphased, support, &t1, &t2, &vm, &panicked);
-        else if (ntot <= kMedianWarpMax) warp_locus<4>(vals, seg, cap, nf, nb, n1, !unphased, support, &t1, &t2, &vm, &panicked);
+        if (!unphased && nf <= 16 && nb <= 16) warp_locus<1, 16, KeyT>(vals, seg, cap, nf, nb, n1, true, support, &t1, &t2, &vm, &panicked);
+        else if (ntot <= 32) warp_locus<1, 0, KeyT>(vals, seg, cap, nf, nb, n1, !unphased, support, &t1, &t2, &vm, &panicked);
+        else if (!unphased && nf <= 32 && nb <= 32) warp_locus<2, 32, KeyT>(vals, seg, cap, nf, nb, n1, true, support, &t1, &t2, &vm, &panicked);
+        else if (ntot <= 64) warp_locus<2, 0, KeyT>(vals, seg, cap, nf, nb, n1, !unphased, support, &t1, &t2, &vm, &panicked);
+        else if (ntot <= kMedianWarpMax) warp_locus<4, 0, KeyT>(vals, seg, cap, nf, nb, n1, !unphased, support, &t1, &t2, &vm, &panicked);
         else {
             if (lane_id() == 0) big_list[l0 + atomicAdd(&ctr->big_count[chunk], 1u)] = l;
             return;
@@ -1558,9 +1620,10 @@ __device__ __forceinline__ void median_one(uint32_t l, uint32_t l0, int chunk, i
 // several loci, with all headers and then all key loads in flight together before any locus was reduced, were measured
 // and do not pay: 1 locus -> 0.357 ms, 2 -> 0.369-0.389, 3 -> 0.473. The kernel is issue-bound, not latency-bound: 68 %
 // of the issue slots are busy already and the extra registers cost occupancy.
+template <typename KeyT>
 __global__ void __launch_bounds__(256, kMedianMinCtas)
 k_locus_median(uint32_t l0, uint32_t l1, int chunk, int unphased, uint32_t support, const uint32_t *__restrict__ seg_off,
-               const unsigned long long *__restrict__ cursor, const uint64_t *__restrict__ vals, uint64_t vals_cap,
+               const unsigned long long *__restrict__ cursor, const KeyT *__restrict__ vals, uint64_t vals_cap,
                int64_t *__restrict__ twice_h1, int64_t *__restrict__ twice_h2, uint8_t *__restrict__ valid,
                uint32_t *__restrict__ big_list, DevCounters *__restrict__ ctr)
 {
@@ -1572,7 +1635,7 @@ k_locus_median(uint32_t l0, uint32_t l1, int chunk, int unphased, uint32_t suppo
     const LocusSeg h = locus_seg(seg, seg_end - seg, cursor[l], vals_cap);
     // round trip 2: the calls, on the common path
     const bool fast = h.ok && !unphased && h.nf <= 16u && h.nb <= 16u;
-    const uint64_t pre = fast ? fast16_load(vals, h) : kKeyInf;
+    const KeyT pre = fast ? fast16_load(vals, h) : KeyTraits<KeyT>::inf;
     median_one(l, l0, chunk, unphased, support, h, fast, pre, vals, twice_h1, twice_h2, valid, big_list, ctr);
 }
 
@@ -1581,7 +1644,8 @@ k_locus_median(uint32_t l0, uint32_t l1, int chunk, int unphased, uint32_t suppo
 constexpr int kBigThreads = 256;
 constexpr int kBigSmemKeys = 4096;
 
-__device__ __forceinline__ void block_part_median(volatile uint64_t *a, uint32_t lo, uint32_t n, uint32_t support,
+template <typename KeyT>
+__device__ __forceinline__ void block_part_median(volatile KeyT *a, uint32_t lo, uint32_t n, uint32_t support,
                                                   int64_t *twice, bool *ok, bool *panicked, uint32_t *sh_cnt,
                                                   unsigned long long *sh_acc)
 {
@@ -1594,7 +1658,7 @@ __device__ __forceinline__ void block_part_median(volatile uint64_t *a, uint32_t
     __syncthreads();
     uint32_t my_s = 0, my_c = 0;
     for (uint32_t i = tid; i < n; i += blockDim.x) {
-        if (a[lo + i] & 1ull) ++my_c; else ++my_s;
+        if (a[lo + i] & 1u) ++my_c; else ++my_s;
     }
     my_s = warp_sum(my_s);
     my_c = warp_sum(my_c);
@@ -1610,8 +1674,8 @@ __device__ __forceinline__ void block_part_median(volatile uint64_t *a, uint32_t
     for (uint32_t base = 0; base < n; base += blockDim.x) {
         const uint32_t i = base + tid;
         const bool in = i < n;
-        const uint64_t k = in ? a[lo + i] : 0ull;
-        const bool is_clip = in && (k & 1ull), is_span = in && !(k & 1ull);
+        const KeyT k = in ? a[lo + i] : (KeyT)0;
+        const bool is_clip = in && (k & 1u), is_span = in && !(k & 1u);
         const uint32_t cb = __ballot_sync(0xffffffffu, is_clip);
         if (lane_id() == 0) wtot[0][tid >> 5] = __popc(cb);
         __syncthreads();
@@ -1624,7 +1688,7 @@ __device__ __forceinline__ void block_part_median(volatile uint64_t *a, uint32_t
         uint32_t rank = sh_cnt[2] + __popc(sb & lanemask_lt());
         for (uint32_t w = 0; w < (tid >> 5); ++w) rank += wtot[1][w];
         if (sel) {
-            const int64_t v = key_call(k);
+            const int64_t v = KeyTraits<KeyT>::call(k);
             if (rank == t1) atomicAdd(sh_acc, (unsigned long long)v);
             if (rank == t2) atomicAdd(sh_acc, (unsigned long long)v);
         }
@@ -1641,13 +1705,15 @@ __device__ __forceinline__ void block_part_median(volatile uint64_t *a, uint32_t
     *ok = true;
 }
 
+template <typename KeyT>
 __global__ void __launch_bounds__(kBigThreads)
 k_locus_median_big(uint32_t l0, int chunk, int unphased, uint32_t support, const uint32_t *__restrict__ seg_off,
-                   const unsigned long long *__restrict__ cursor, uint64_t *__restrict__ vals, uint64_t vals_cap,
+                   const unsigned long long *__restrict__ cursor, KeyT *__restrict__ vals, uint64_t vals_cap,
                    int64_t *__restrict__ twice_h1, int64_t *__restrict__ twice_h2, uint8_t *__restrict__ valid,
                    const uint32_t *__restrict__ big_list, DevCounters *__restrict__ ctr)
 {
-    __shared__ uint64_t skeys[kBigSmemKeys];
+    constexpr KeyT hap = KeyTraits<KeyT>::hap, inf = KeyTraits<KeyT>::inf;
+    __shared__ KeyT skeys[kBigSmemKeys];
     __shared__ uint32_t item_s;
     __shared__ uint32_t sh_cnt[4];
     __shared__ unsigned long long sh_acc;
@@ -1665,20 +1731,20 @@ k_locus_median_big(uint32_t l0, int chunk, int unphased, uint32_t support, const
         uint32_t ntot = nf + nb;
         const uint32_t n1 = unphased ? (ntot >> 1) : nf;
         const uint32_t n2 = ntot - n1;
-        volatile uint64_t *a;
+        volatile KeyT *a;
         if (ntot <= (uint32_t)kBigSmemKeys) {
             for (uint32_t i = tid; i < ntot; i += blockDim.x) {
-                uint64_t v;
+                KeyT v;
                 if (i < nf) v = vals[seg + i];
-                else v = vals[seg + cap - nb + (i - nf)] | (unphased ? 0ull : kKeyHapBit);
+                else v = vals[seg + cap - nb + (i - nf)] | (unphased ? (KeyT)0 : hap);
                 skeys[i] = v;
             }
             a = skeys;
         } else {
             // sort the whole segment in place; the unused gap between front and back becomes +inf keys
             for (uint32_t i = nf + tid; i < cap; i += blockDim.x) {
-                if (i < cap - nb) vals[seg + i] = kKeyInf;
-                else if (!unphased) vals[seg + i] |= kKeyHapBit;
+                if (i < cap - nb) vals[seg + i] = inf;
+                else if (!unphased) vals[seg + i] |= hap;
             }
             a = vals + seg;
             ntot = cap;
@@ -1691,7 +1757,7 @@ k_locus_median_big(uint32_t l0, int chunk, int unphased, uint32_t support, const
             for (uint32_t i = tid; i < npow; i += blockDim.x) {
                 const uint32_t j = i ^ (blk - 1);
                 if (i < j && j < ntot) {
-                    const uint64_t x = a[i], y = a[j];
+                    const KeyT x = a[i], y = a[j];
                     if (x > y) { a[i] = y; a[j] = x; }
                 }
             }
@@ -1700,7 +1766,7 @@ k_locus_median_big(uint32_t l0, int chunk, int unphased, uint32_t support, const
                 for (uint32_t i = tid; i < npow; i += blockDim.x) {
                     const uint32_t j = i ^ d;
                     if (i < j && j < ntot) {
-                        const uint64_t x = a[i], y = a[j];
+                        const KeyT x = a[i], y = a[j];
                         if (x > y) { a[i] = y; a[j] = x; }
                     }
                 }
